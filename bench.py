@@ -2,10 +2,12 @@
 """Headline benchmark: CMS AE (24 -> 15) compress + decompress of a synthetic 100M-row x 24-col float32
 table per GPU (BASELINE.json configs[1]), plus one training epoch as a secondary line.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--rows R]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--rows R] [--dump-outputs DIR]
 
 One step = one pass of the hot path over the table: column min/max -> normalise+encode -> latent, then
 decode+un-normalise -> reconstruction.  `value` = rows / step time with the table resident in HBM.
+`--dump-outputs DIR` writes what the last timed step computed (features, and latent and reconstruction at a fixed
+sample of rows) as .npy files, so that two builds run with the same arguments can be compared output for output.
 `e2e` = the same pass through the C-ABI host entry points (bb_compress_host / bb_decompress_host) with
 pinned HOST buffers, H2D / D2H copies inside the timed region.  N > 1: one process per GPU (torchrun), the
 table is row-sharded (100M rows per GPU, weak scaling), the only exchange is the 2 x 24 column min / max.
@@ -30,6 +32,8 @@ sys.path.insert(0, ROOT)
 FLOP_PER_ROW = 61100          # SURVEY 8(d): 2 * (24*200 + 200*100 + 100*50 + 50*15) per direction
 BYTES_PER_ROW = 156           # 96 in + 60 out (fp32 latent) per direction
 METRIC = "compress+decompress rows/s (CMS AE 24->15, table resident in HBM)"
+DUMP_ROWS = 1 << 18           # rows --dump-outputs samples: 41 MB of float32 latent + reconstruction whatever --rows
+DUMP_SEED = 0
 
 
 def load_peaks():
@@ -44,6 +48,25 @@ def load_peaks():
 def golden_state_dict():
     g = np.load(os.path.join(ROOT, "tests", "golden", "ae_cms.npz"))
     return {k[3:]: g[k] for k in g.files if k.startswith("sd/")}
+
+
+def dump_rows(n):
+    """the sorted row indices --dump-outputs samples from an n-row table: every row when n <= DUMP_ROWS; drawn from a
+    fixed seed and n alone, so runs with the same --rows sample the same rows"""
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(n, size=min(n, DUMP_ROWS), replace=False))
+
+
+def dump_outputs(out_dir, z, y, mn, rg):
+    """what a caller of the timed path receives, as float32 / float64 .npy files: features.npy (2 x 24: column min and
+    range), latent.npy and reconstruction.npy at the rows of dump_rows (float32), rows.npy (those indices, float64)"""
+    import torch
+    rows = dump_rows(z.shape[0])
+    idx = torch.from_numpy(rows).to(z.device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in (("features", torch.stack([mn, rg])), ("latent", z.index_select(0, idx)),
+                    ("reconstruction", y.index_select(0, idx))):
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+    np.save(os.path.join(out_dir, "rows.npy"), rows.astype(np.float64))
 
 
 class ClockSampler:
@@ -300,10 +323,12 @@ def run_ours(args):
     sync_all()
     t_start.record()
     for _ in range(args.steps):
-        step(timed_kernels=True)
+        features = step(timed_kernels=True)
     t_end.record()
     sync_all()
     total_ms = t_start.elapsed_time(t_end)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, z, y, *features)  # before the sweep below reuses z and y
     if codec.auto_precision == "split16" and codec.range_flag():
         raise RuntimeError("fp16 range guard tripped on the synthetic table: timed steps are invalid")
     clocks = sampler.stop() if rank == 0 else None
@@ -768,7 +793,13 @@ def main():
     ap.add_argument("--no-modes", action="store_true")
     ap.add_argument("--no-sweep", action="store_true", help="skip the 1B-row strong-scaling sweep (BASELINE configs[4])")
     ap.add_argument("--cfd-blocks", type=int, default=600_000)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="--impl ours: write the last timed step's outputs as DIR/<name>.npy (rank 0's shard under torchrun)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

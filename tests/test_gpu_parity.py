@@ -9,7 +9,7 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import rel_l2, rel_max, sub_sd
+from conftest import ROOT, rel_l2, rel_max, sub_sd
 from oracle import baler_oracle as orc
 from baler_b200 import engine, synth
 from baler_b200.modules import models
@@ -452,3 +452,40 @@ def test_error_bounded_deltas_vs_reference(golden, tmp_path, monkeypatch):
         same[r, c] = False
     scale = np.abs(ref).max(axis=0)
     assert (np.abs(dec - ref)[same] <= 1e-3 * np.broadcast_to(scale, dec.shape)[same]).all()  # float16 deltas: 2^-11 relative
+
+
+def test_bench_dump_outputs(ae, tmp_path):
+    """bench.py --dump-outputs: the features of the last timed step and its latent and reconstruction at the sampled rows,
+    the same whatever --steps (which sets the number of timed steps), equal to the oracle's compress / decompress"""
+    import json
+    import subprocess
+    import sys
+
+    sd = ae[1]
+    n = 300_000  # more rows than the dump samples
+    runs = []
+    for steps in (1, 3):
+        out = tmp_path / ("steps%d" % steps)
+        cmd = [sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--steps", str(steps), "--warmup", "1",
+               "--rows", str(n), "--no-sweep", "--no-cpu", "--no-modes", "--no-e2e", "--no-train", "--no-cfd",
+               "--dump-outputs", str(out)]
+        r = subprocess.run(cmd, capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stderr[-2000:]
+        d = json.loads(r.stdout.strip().splitlines()[-1])
+        assert d["steps"] == steps and d["gpu_launches"] == 3 * steps
+        files = {p.name[:-4]: np.load(p) for p in out.iterdir()}
+        assert sorted(files) == ["features", "latent", "reconstruction", "rows"]
+        assert all(a.dtype in (np.float32, np.float64) for a in files.values())
+        assert sum(a.nbytes for a in files.values()) <= 64 << 20
+        runs.append(files)
+    for k in runs[0]:
+        assert np.array_equal(runs[0][k], runs[1][k]), k
+    got = runs[0]
+    rows = got["rows"].astype(np.int64)
+    assert len(rows) < n and np.all(np.diff(rows) > 0)
+    table = synth.cms_table_device(n, seed=synth.CMS_SEED).cpu().numpy()
+    feats = orc.find_minmax(table)
+    assert np.array_equal(got["features"], feats)
+    z_ref = orc.compress(sd, table)[rows]
+    close(got["latent"], z_ref)
+    close(got["reconstruction"], orc.decompress(sd, z_ref, feats))

@@ -1,6 +1,6 @@
 import os, sys, time
 import numpy as np, torch
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from baler_b200 import synth
 from baler_b200.modules import models
 nb = 600000

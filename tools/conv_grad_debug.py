@@ -1,9 +1,10 @@
 import os, sys
-sys.path.insert(0, "/root/repo"); sys.path.insert(0, "/root/repo/tests")
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
 import numpy as np, torch
 import test_gpu_cfd as T
 from baler_b200 import engine
-g = np.load("/root/repo/tests/golden/conv_train.npz")
+g = np.load(os.path.join(ROOT, "tests", "golden", "conv_train.npz"))
 m = T._conv_model()
 tr, sp = T._conv_trainer(m)
 x = torch.from_numpy(g["blocks"]).cuda()
