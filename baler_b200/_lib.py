@@ -11,9 +11,9 @@ LIB_PATH = os.path.join(HERE, "libbaler_b200.so")
 
 BB_F32, BB_F16, BB_F64 = 0, 1, 2
 BB_ACT_NONE, BB_ACT_LEAKY, BB_ACT_RELU = 0, 1, 2
-BB_PREC_AUTO, BB_PREC_FP32, BB_PREC_SPLIT16, BB_PREC_FAST16 = 0, 1, 2, 3
+BB_PREC_AUTO, BB_PREC_FP32, BB_PREC_SPLIT16, BB_PREC_FAST16, BB_PREC_FP64 = 0, 1, 2, 3, 4
 PRECISIONS = {"auto": BB_PREC_AUTO, "exact": BB_PREC_AUTO, "fp32": BB_PREC_FP32,
-              "split16": BB_PREC_SPLIT16, "fast": BB_PREC_FAST16, "fast16": BB_PREC_FAST16}
+              "split16": BB_PREC_SPLIT16, "fast": BB_PREC_FAST16, "fast16": BB_PREC_FAST16, "fp64": BB_PREC_FP64}
 
 
 class BalerB200Error(RuntimeError):
@@ -46,12 +46,17 @@ _SIGNATURES = {
     "bb_model_chain_precision": (C.c_int, [_P, C.c_int]),
     "bb_model_range_flag": (C.c_int, [_P, C.c_int, C.POINTER(C.c_int)]),
     "bb_colminmax_f32": (C.c_int, [_P, _P, C.c_int64, C.c_int, _P, _P, _P]),
+    "bb_colminmax_f64": (C.c_int, [_P, _P, C.c_int64, C.c_int, _P, _P, _P]),
     "bb_normalize_f32": (C.c_int, [_P, _P, C.c_int64, C.c_int, _P, _P, _P, _P]),
     "bb_renormalize_f32": (C.c_int, [_P, _P, C.c_int64, C.c_int, _P, _P, _P, _P]),
     "bb_encode_f32": (C.c_int, [_P, _P, C.c_int64, _P, _P, _P, C.c_int, C.c_int, _P]),
     "bb_decode_f32": (C.c_int, [_P, _P, C.c_int, C.c_int64, _P, _P, _P, C.c_int, _P]),
+    "bb_encode_f64": (C.c_int, [_P, _P, C.c_int64, _P, _P, _P, _P]),
+    "bb_decode_f64": (C.c_int, [_P, _P, C.c_int64, _P, _P, _P, _P]),
     "bb_compress_host": (C.c_int, [_P, _P, C.c_int64, _P, C.c_int, _P, C.c_int, C.c_int]),
     "bb_decompress_host": (C.c_int, [_P, _P, C.c_int, C.c_int64, _P, _P, C.c_int, C.c_int]),
+    "bb_compress_host_f64": (C.c_int, [_P, _P, C.c_int64, _P, C.c_int, _P]),
+    "bb_decompress_host_f64": (C.c_int, [_P, _P, C.c_int64, _P, _P]),
     "bb_trainer_create": (C.c_int, [_P, C.c_int, C.c_int, _P, _P, C.c_int, _PP]),
     "bb_trainer_create_dbn": (C.c_int, [_P, C.c_int, C.c_int, _P, _P, _P, _P, _P, _P, _P, C.c_int, _PP]),
     "bb_trainer_set_dropout": (C.c_int, [_P, C.c_uint64, _P]),

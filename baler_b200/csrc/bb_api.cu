@@ -101,6 +101,7 @@ void free_chain(Chain* c) {
   release(c->g5_blob_dev);
   release(c->g5_bias_dev);
   bb_tc_release(c);
+  bb_chain_f64_release(c);
 }
 
 // the chain has a tensor-core form: one of the fused tcgen05 kernels, or the layered mma.sync GEMMs for shapes too
@@ -112,13 +113,22 @@ int resolve_precision(const bb_model* m, const Chain* c, int precision) {
   return precision;
 }
 
+// features (pre_* / post_*) are float32, or float64 (feat_dtype BB_F64) on the float64 path only
 int run_chain(bb_model* m, const Chain* c, const void* in, int in_dtype, int64_t n_rows,
-              const float* pre_min, const float* pre_range, const float* post_min,
-              const float* post_range, void* out, int out_dtype, int precision, cudaStream_t stream) {
+              const void* pre_min_v, const void* pre_range_v, const void* post_min_v,
+              const void* post_range_v, int feat_dtype, void* out, int out_dtype, int precision, cudaStream_t stream) {
   if (!m || (!in && n_rows) || (!out && n_rows) || n_rows < 0) return BB_ERR_INVALID;
-  if ((pre_min == nullptr) != (pre_range == nullptr) || (post_min == nullptr) != (post_range == nullptr))
+  if ((pre_min_v == nullptr) != (pre_range_v == nullptr) || (post_min_v == nullptr) != (post_range_v == nullptr))
     return BB_ERR_INVALID;
-  if ((in_dtype != BB_F32 && in_dtype != BB_F16) || (out_dtype != BB_F32 && out_dtype != BB_F16)) return BB_ERR_INVALID;
+  if (precision == BB_PREC_FP64)
+    return bb_chain_f64_launch(m->ctx, c, in, in_dtype, n_rows, pre_min_v, pre_range_v, post_min_v, post_range_v, feat_dtype,
+                               out, out_dtype, stream);
+  if ((in_dtype != BB_F32 && in_dtype != BB_F16) || (out_dtype != BB_F32 && out_dtype != BB_F16) || feat_dtype != BB_F32)
+    return BB_ERR_INVALID;
+  const float* pre_min = (const float*)pre_min_v;
+  const float* pre_range = (const float*)pre_range_v;
+  const float* post_min = (const float*)post_min_v;
+  const float* post_range = (const float*)post_range_v;
   const int p = resolve_precision(m, c, precision);
   if (p == BB_PREC_FP32) {
     if (!c->f32_ok)  // weights do not fit shared memory: one GEMM launch per layer
@@ -326,7 +336,7 @@ int pipe_init(bb_model* m, size_t in_bytes, size_t out_bytes) {
   return BB_OK;
 }
 
-// pinned float32 bounce buffers (two slots) of the float64 host paths, grown on demand and kept
+// pinned bounce buffers (two slots, float32 or float64 chunks) of the float64 host paths, grown on demand and kept
 int pinned_init(bb_model* m, int io, size_t bytes) {
   if (m->pinned_bytes[io] >= bytes) return BB_OK;
   for (int s = 0; s < 2; ++s) {
@@ -476,6 +486,21 @@ void host_colminmax(const float* x, int64_t n_rows, int F, float* mn_out, float*
   }
 }
 
+// page-locked host memory (cudaMallocHost / cudaHostRegister): copies to and from it run asynchronously at the PCIe rate
+bool host_pinned(const void* p) {
+  cudaPointerAttributes a;
+  if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
+    cudaGetLastError();
+    return false;
+  }
+  return a.type == cudaMemoryTypeHost;
+}
+
+// memcpy of n bytes on the library's worker threads (float64 chunks between a pageable caller buffer and a pinned slot)
+void copy_parallel(void* dst, const void* src, size_t n) {
+  host_parallel_ranges(n, [=](size_t lo, size_t hi) { memcpy((char*)dst + lo, (const char*)src + lo, hi - lo); });
+}
+
 // device copy of the whole table between the two passes of bb_compress_host, when it fits in half of the free memory
 float* resident_get(bb_model* m, size_t bytes) {
   if (getenv("BALER_B200_NO_RESIDENT")) return nullptr;  // test hook: take the two-pass streaming path of tables that do not fit
@@ -503,13 +528,30 @@ void model_trim(bb_model* m) {
   for (Chain* c : {&m->enc, &m->dec}) {
     if (c->lay_scratch) cudaFree(c->lay_scratch);
     c->lay_scratch = nullptr; c->lay_scratch_bytes = 0;
+    bb_chain_f64_release(c);  // the float64 weight image: packed again by the next BB_PREC_FP64 call
   }
+  if (m->feat64_dev) cudaFree(m->feat64_dev);
+  m->feat64_dev = nullptr;
 }
 
-// range = max - min on device (float32 subtraction, like numpy on a float32 table)
-__global__ void range_kernel(const float* mn, const float* mx, float* rg, int c) {
+// range = max - min on device (one subtraction in the table's dtype, like numpy)
+template <typename T>
+__global__ void range_kernel(const T* mn, const T* mx, T* rg, int c) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < c) rg[i] = __fsub_rn(mx[i], mn[i]);
+  if (i < c) rg[i] = mx[i] - mn[i];
+}
+
+void launch_range(const void* mn, const void* mx, void* rg, int c, int dtype, cudaStream_t s) {
+  if (dtype == BB_F64) range_kernel<double><<<(c + 127) / 128, 128, 0, s>>>((const double*)mn, (const double*)mx, (double*)rg, c);
+  else range_kernel<float><<<(c + 127) / 128, 128, 0, s>>>((const float*)mn, (const float*)mx, (float*)rg, c);
+}
+
+// [min | range | max] of the table's dtype on the device: float32 features in feat_dev, float64 ones in feat64_dev
+int features_dev(bb_model* m, int dtype, char** out) {
+  if (dtype == BB_F64 && !m->feat64_dev)
+    BB_CUDA(cudaMalloc(&m->feat64_dev, 3 * sizeof(double) * std::max(m->enc.desc.in_dim, m->dec.desc.out_dim)));
+  *out = dtype == BB_F64 ? (char*)m->feat64_dev : (char*)m->feat_dev;
+  return BB_OK;
 }
 
 }  // namespace
@@ -614,21 +656,41 @@ int bb_model_auto_precision(const bb_model* m) {
 int bb_colminmax_f32(bb_ctx* ctx, const float* x_dev, int64_t n_rows, int n_cols, float* min_dev,
                      float* max_dev, bb_stream_t stream) {
   if (!ctx || (!x_dev && n_rows) || !min_dev || !max_dev) return BB_ERR_INVALID;
-  return bb_colminmax_launch(ctx, x_dev, n_rows, n_cols, min_dev, max_dev, 1, (cudaStream_t)stream);
+  return bb_colminmax_launch(ctx, x_dev, BB_F32, n_rows, n_cols, min_dev, max_dev, 1, (cudaStream_t)stream);
+}
+
+int bb_colminmax_f64(bb_ctx* ctx, const double* x_dev, int64_t n_rows, int n_cols, double* min_dev,
+                     double* max_dev, bb_stream_t stream) {
+  if (!ctx || (!x_dev && n_rows) || !min_dev || !max_dev) return BB_ERR_INVALID;
+  return bb_colminmax_launch(ctx, x_dev, BB_F64, n_rows, n_cols, min_dev, max_dev, 1, (cudaStream_t)stream);
 }
 
 int bb_encode_f32(bb_model* m, const float* x_dev, int64_t n_rows, const float* min_dev,
                   const float* range_dev, void* z_dev, int z_dtype, int precision, bb_stream_t stream) {
   if (!m) return BB_ERR_INVALID;
-  return run_chain(m, &m->enc, x_dev, BB_F32, n_rows, min_dev, range_dev, nullptr, nullptr, z_dev, z_dtype,
+  return run_chain(m, &m->enc, x_dev, BB_F32, n_rows, min_dev, range_dev, nullptr, nullptr, BB_F32, z_dev, z_dtype,
                    precision, (cudaStream_t)stream);
 }
 
 int bb_decode_f32(bb_model* m, const void* z_dev, int z_dtype, int64_t n_rows, const float* min_dev,
                   const float* range_dev, float* y_dev, int precision, bb_stream_t stream) {
   if (!m) return BB_ERR_INVALID;
-  return run_chain(m, &m->dec, z_dev, z_dtype, n_rows, nullptr, nullptr, min_dev, range_dev, y_dev, BB_F32,
+  return run_chain(m, &m->dec, z_dev, z_dtype, n_rows, nullptr, nullptr, min_dev, range_dev, BB_F32, y_dev, BB_F32,
                    precision, (cudaStream_t)stream);
+}
+
+int bb_encode_f64(bb_model* m, const double* x_dev, int64_t n_rows, const double* min_dev, const double* range_dev,
+                  double* z_dev, bb_stream_t stream) {
+  if (!m) return BB_ERR_INVALID;
+  return run_chain(m, &m->enc, x_dev, BB_F64, n_rows, min_dev, range_dev, nullptr, nullptr, BB_F64, z_dev, BB_F64,
+                   BB_PREC_FP64, (cudaStream_t)stream);
+}
+
+int bb_decode_f64(bb_model* m, const double* z_dev, int64_t n_rows, const double* min_dev, const double* range_dev,
+                  double* y_dev, bb_stream_t stream) {
+  if (!m) return BB_ERR_INVALID;
+  return run_chain(m, &m->dec, z_dev, BB_F64, n_rows, nullptr, nullptr, min_dev, range_dev, BB_F64, y_dev, BB_F64,
+                   BB_PREC_FP64, (cudaStream_t)stream);
 }
 
 int bb_host_convert(const void* src, int src_dtype, void* dst, int dst_dtype, int64_t n) {
@@ -645,44 +707,58 @@ int bb_host_colminmax_f32(const float* x_host, int64_t n_rows, int n_cols, float
   return BB_OK;
 }
 
-int bb_compress_host(bb_model* m, const float* x_host, int64_t n_rows, float* features_host,
-                     int recompute_minmax, void* z_host, int z_dtype, int precision) {
+}  // extern "C"
+
+namespace {
+
+// The host-buffer compress pipeline of bb_compress_host (x_dtype BB_F32: float32 table and features) and
+// bb_compress_host_f64 (x_dtype BB_F64: float64 table and features, precision BB_PREC_FP64).
+int compress_host(bb_model* m, const void* x_host, int x_dtype, int64_t n_rows, void* features_host,
+                  int recompute_minmax, void* z_host, int z_dtype, int precision) {
   if (!m || (!x_host && n_rows) || (!z_host && n_rows) || n_rows < 0) return BB_ERR_INVALID;
   if (z_dtype != BB_F32 && z_dtype != BB_F16 && z_dtype != BB_F64) return BB_ERR_INVALID;
   if (recompute_minmax && !features_host) return BB_ERR_INVALID;
+  if (x_dtype == BB_F64 && precision != BB_PREC_FP64) return BB_ERR_INVALID;
   BB_CUDA(cudaSetDevice(m->ctx->device));
   const int F = m->enc.desc.in_dim, Z = m->enc.desc.out_dim;
-  const int dev_dtype = (z_dtype == BB_F16) ? BB_F16 : BB_F32;
+  const size_t xs = dtype_size(x_dtype);  // bytes per element of the table and of its features
+  // device output dtype: the float32 / fp16 kernels write float32 for a float64 latent (widened on the host below); the
+  // float64 kernel writes whatever is asked
+  const int dev_dtype = (z_dtype == BB_F64 && precision != BB_PREC_FP64) ? BB_F32 : z_dtype;
   const int64_t chunk = pipe_chunk_rows(n_rows);
   const int64_t n_chunks = n_rows ? (n_rows + chunk - 1) / chunk : 0;
-  const size_t in_b = (size_t)chunk * F * sizeof(float), out_b = (size_t)chunk * Z * dtype_size(dev_dtype);
+  const size_t in_b = (size_t)chunk * F * xs, out_b = (size_t)chunk * Z * dtype_size(dev_dtype);
   int rc = pipe_init(m, in_b, out_b);
   if (rc != BB_OK) return rc;
-  float* fmin = m->feat_dev;
-  float* frange = m->feat_dev + F;
-  float* fmax = m->feat_dev + 2 * F;
+  char* feat = nullptr;
+  rc = features_dev(m, x_dtype, &feat);
+  if (rc != BB_OK) return rc;
+  char* fmin = feat;
+  char* frange = feat + F * xs;
+  char* fmax = feat + 2 * F * xs;
   const bool norm = features_host != nullptr;
+  const char* xh = (const char*)x_host;
 
   // Column statistics of THIS table (helper.py:500-502): either a first streaming pass that keeps
   // the table resident when it fits, or the features handed in.
-  float* resident = nullptr;
+  char* resident = nullptr;
   std::vector<cudaEvent_t> ev_up;  // resident path: upload of chunk k complete
   if (norm && recompute_minmax && n_rows) {
-    resident = resident_get(m, (size_t)n_rows * F * sizeof(float));
+    resident = (char*)resident_get(m, (size_t)n_rows * F * xs);
     // the host scan pays when 16 host threads are free for it (measured on a 32-CPU node: 2 ranks 483 M rows/s against 414
     // with the device pass, 4 ranks of 8 threads each 385 against 557: the scans then compete with four uploads for the host's
-    // memory bandwidth; the device pass below costs nothing on the host)
-    if (resident && host_scan_threads() >= 16 && !getenv("BALER_B200_DEVICE_MINMAX")) {
+    // memory bandwidth; the device pass below costs nothing on the host).  (float32 tables: the host scan has no float64 form)
+    if (resident && x_dtype == BB_F32 && host_scan_threads() >= 16 && !getenv("BALER_B200_DEVICE_MINMAX")) {
       // the table fits: queue the whole upload now, find the column min / max on host threads meanwhile, and let the
       // encode + latent download of the chunks that have landed run against the rest of the upload
       // (the scan starts first, on its own threads: queuing copies from pageable memory blocks the calling thread)
       std::vector<float> mm(2 * (size_t)F);
-      std::thread scan(host_colminmax, x_host, n_rows, F, mm.data(), mm.data() + F);
+      std::thread scan(host_colminmax, (const float*)x_host, n_rows, F, mm.data(), mm.data() + F);
       ev_up.resize((size_t)n_chunks, nullptr);
       cudaError_t up_rc = cudaSuccess;
       for (int64_t k = 0; k < n_chunks && up_rc == cudaSuccess; ++k) {
         const int64_t r0 = k * chunk, rows = std::min(chunk, n_rows - r0);
-        up_rc = cudaMemcpyAsync(resident + (size_t)r0 * F, x_host + (size_t)r0 * F, (size_t)rows * F * sizeof(float), cudaMemcpyHostToDevice, m->s_copy_in);
+        up_rc = cudaMemcpyAsync(resident + (size_t)r0 * F * xs, xh + (size_t)r0 * F * xs, (size_t)rows * F * xs, cudaMemcpyHostToDevice, m->s_copy_in);
         if (up_rc == cudaSuccess) up_rc = cudaEventCreateWithFlags(&ev_up[(size_t)k], cudaEventDisableTiming);
         if (up_rc == cudaSuccess) up_rc = cudaEventRecord(ev_up[(size_t)k], m->s_copy_in);
       }
@@ -693,8 +769,8 @@ int bb_compress_host(bb_model* m, const float* x_host, int64_t n_rows, float* fe
       }
       BB_CUDA(cudaMemcpyAsync(fmin, mm.data(), F * sizeof(float), cudaMemcpyHostToDevice, m->s_compute));
       BB_CUDA(cudaMemcpyAsync(fmax, mm.data() + F, F * sizeof(float), cudaMemcpyHostToDevice, m->s_compute));
-      range_kernel<<<(F + 127) / 128, 128, 0, m->s_compute>>>(fmin, fmax, frange, F);
-      BB_CUDA(cudaMemcpyAsync(features_host, fmin, 2 * F * sizeof(float), cudaMemcpyDeviceToHost, m->s_compute));
+      launch_range(fmin, fmax, frange, F, x_dtype, m->s_compute);
+      BB_CUDA(cudaMemcpyAsync(features_host, fmin, 2 * F * xs, cudaMemcpyDeviceToHost, m->s_compute));
       BB_CUDA(cudaStreamSynchronize(m->s_compute));  // (mm goes out of scope; features_host is final)
     } else {
       // a first streaming pass for the statistics on the device (column min / max kernel per chunk as it lands), which
@@ -702,68 +778,70 @@ int bb_compress_host(bb_model* m, const float* x_host, int64_t n_rows, float* fe
       for (int64_t k = 0; k < n_chunks; ++k) {
         const int64_t r0 = k * chunk, rows = std::min(chunk, n_rows - r0);
         const int s = (int)(k & 1);
-        float* dst = resident ? resident + (size_t)r0 * F : (float*)m->stage_dev[0][s];
+        char* dst = resident ? resident + (size_t)r0 * F * xs : (char*)m->stage_dev[0][s];
         if (!resident && k >= 2) BB_CUDA(cudaStreamWaitEvent(m->s_copy_in, m->ev_done[s], 0));
-        BB_CUDA(cudaMemcpyAsync(dst, x_host + (size_t)r0 * F, (size_t)rows * F * sizeof(float), cudaMemcpyHostToDevice, m->s_copy_in));
+        BB_CUDA(cudaMemcpyAsync(dst, xh + (size_t)r0 * F * xs, (size_t)rows * F * xs, cudaMemcpyHostToDevice, m->s_copy_in));
         BB_CUDA(cudaEventRecord(m->ev_in[s], m->s_copy_in));
         BB_CUDA(cudaStreamWaitEvent(m->s_compute, m->ev_in[s], 0));
-        rc = bb_colminmax_launch(m->ctx, dst, rows, F, fmin, fmax, k == 0, m->s_compute);
+        rc = bb_colminmax_launch(m->ctx, dst, x_dtype, rows, F, fmin, fmax, k == 0, m->s_compute);
         if (rc != BB_OK) return rc;
         BB_CUDA(cudaEventRecord(m->ev_done[s], m->s_compute));
       }
-      range_kernel<<<(F + 127) / 128, 128, 0, m->s_compute>>>(fmin, fmax, frange, F);
-      BB_CUDA(cudaMemcpyAsync(features_host, fmin, 2 * F * sizeof(float), cudaMemcpyDeviceToHost, m->s_compute));
+      launch_range(fmin, fmax, frange, F, x_dtype, m->s_compute);
+      BB_CUDA(cudaMemcpyAsync(features_host, fmin, 2 * F * xs, cudaMemcpyDeviceToHost, m->s_compute));
       BB_CUDA(cudaStreamSynchronize(m->s_compute));
     }
   } else if (norm) {
-    BB_CUDA(cudaMemcpyAsync(fmin, features_host, 2 * F * sizeof(float), cudaMemcpyHostToDevice, m->s_compute));
+    BB_CUDA(cudaMemcpyAsync(fmin, features_host, 2 * F * xs, cudaMemcpyHostToDevice, m->s_compute));
   }
   struct EvGuard {  // the per-chunk upload events live for this call only
     std::vector<cudaEvent_t>& v;
     ~EvGuard() { for (cudaEvent_t e : v) if (e) cudaEventDestroy(e); }
   } ev_guard{ev_up};
 
-  std::vector<float> widen_tmp;
-  float* pinned_out[2] = {nullptr, nullptr};
-  if (z_dtype == BB_F64 && n_rows) {
-    if (pinned_init(m, 1, (size_t)chunk * Z * sizeof(float)) != BB_OK) return BB_ERR_NOMEM;
+  const bool widen = z_dtype == BB_F64 && dev_dtype != BB_F64;  // float32 on the device, float64 in the caller's buffer
+  // a float64 latent from the float64 chain lands in a pinned slot and is copied out on host threads when the caller's
+  // buffer is pageable (a device-to-pageable copy runs at a fraction of the PCIe rate)
+  const bool bounce = dev_dtype == BB_F64 && n_rows && !host_pinned(z_host);
+  void* pinned_out[2] = {nullptr, nullptr};
+  if ((widen || bounce) && n_rows) {
+    if (pinned_init(m, 1, (size_t)chunk * Z * dtype_size(dev_dtype)) != BB_OK) return BB_ERR_NOMEM;
     pinned_out[0] = m->pinned_f32[1][0]; pinned_out[1] = m->pinned_f32[1][1];
   }
-  auto finish_chunk = [&](int64_t k) -> int {  // host side of chunk k: wait for its D2H, widen if needed
+  auto finish_chunk = [&](int64_t k) -> int {  // host side of chunk k: wait for its D2H, widen / copy out if needed
     const int s = (int)(k & 1);
     BB_CUDA(cudaEventSynchronize(m->ev_out[s]));
-    if (z_dtype == BB_F64) {
-      const int64_t r0 = k * chunk, rows = std::min(chunk, n_rows - r0);
-      widen_f32_f64(pinned_out[s], (double*)z_host + (size_t)r0 * Z, (size_t)rows * Z);
-    }
+    const int64_t r0 = k * chunk, rows = std::min(chunk, n_rows - r0);
+    if (widen) widen_f32_f64((const float*)pinned_out[s], (double*)z_host + (size_t)r0 * Z, (size_t)rows * Z);
+    else if (bounce) copy_parallel((double*)z_host + (size_t)r0 * Z, pinned_out[s], (size_t)rows * Z * sizeof(double));
     return BB_OK;
   };
   rc = BB_OK;
   for (int64_t k = 0; k < n_chunks && rc == BB_OK; ++k) {
     const int64_t r0 = k * chunk, rows = std::min(chunk, n_rows - r0);
     const int s = (int)(k & 1);
-    const float* src;
+    const char* src;
     if (resident) {
-      src = resident + (size_t)r0 * F;
+      src = resident + (size_t)r0 * F * xs;
       if (!ev_up.empty()) BB_CUDA(cudaStreamWaitEvent(m->s_compute, ev_up[(size_t)k], 0));
     } else {
       if (k >= 2) BB_CUDA(cudaStreamWaitEvent(m->s_copy_in, m->ev_done[s], 0));  // slot's previous kernel finished
-      BB_CUDA(cudaMemcpyAsync(m->stage_dev[0][s], x_host + (size_t)r0 * F, (size_t)rows * F * sizeof(float), cudaMemcpyHostToDevice, m->s_copy_in));
+      BB_CUDA(cudaMemcpyAsync(m->stage_dev[0][s], xh + (size_t)r0 * F * xs, (size_t)rows * F * xs, cudaMemcpyHostToDevice, m->s_copy_in));
       BB_CUDA(cudaEventRecord(m->ev_in[s], m->s_copy_in));
       BB_CUDA(cudaStreamWaitEvent(m->s_compute, m->ev_in[s], 0));
-      src = (const float*)m->stage_dev[0][s];
+      src = (const char*)m->stage_dev[0][s];
     }
     if (k >= 2) {
       rc = finish_chunk(k - 2);  // frees output slot s on the host side (and its pinned buffer)
       if (rc != BB_OK) break;
       BB_CUDA(cudaStreamWaitEvent(m->s_compute, m->ev_out[s], 0));
     }
-    rc = run_chain(m, &m->enc, src, BB_F32, rows, norm ? fmin : nullptr, norm ? frange : nullptr, nullptr, nullptr,
+    rc = run_chain(m, &m->enc, src, x_dtype, rows, norm ? fmin : nullptr, norm ? frange : nullptr, nullptr, nullptr, x_dtype,
                    m->stage_dev[1][s], dev_dtype, precision, m->s_compute);
     if (rc != BB_OK) break;
     BB_CUDA(cudaEventRecord(m->ev_done[s], m->s_compute));
     BB_CUDA(cudaStreamWaitEvent(m->s_copy_out, m->ev_done[s], 0));
-    void* dst = (z_dtype == BB_F64) ? (void*)pinned_out[s] : (void*)((char*)z_host + (size_t)r0 * Z * dtype_size(z_dtype));
+    void* dst = (widen || bounce) ? pinned_out[s] : (void*)((char*)z_host + (size_t)r0 * Z * dtype_size(z_dtype));
     BB_CUDA(cudaMemcpyAsync(dst, m->stage_dev[1][s], (size_t)rows * Z * dtype_size(dev_dtype), cudaMemcpyDeviceToHost, m->s_copy_out));
     BB_CUDA(cudaEventRecord(m->ev_out[s], m->s_copy_out));
   }
@@ -773,49 +851,62 @@ int bb_compress_host(bb_model* m, const float* x_host, int64_t n_rows, float* fe
   if (rc == BB_OK && precision == BB_PREC_AUTO && chain_has_tc(&m->enc)) {
     int tripped = 0;  // fp16 range guard of the split path: redo on the fp32 kernel (features are already known)
     rc = bb_model_range_flag(m, 1, &tripped);
-    if (rc == BB_OK && tripped) return bb_compress_host(m, x_host, n_rows, features_host, 0, z_host, z_dtype, BB_PREC_FP32);
+    if (rc == BB_OK && tripped)
+      return compress_host(m, x_host, x_dtype, n_rows, features_host, 0, z_host, z_dtype, BB_PREC_FP32);
   }
   return rc;
 }
 
-int bb_decompress_host(bb_model* m, const void* z_host, int z_dtype, int64_t n_rows,
-                       const float* features_host, void* y_host, int y_dtype, int precision) {
+// The host-buffer decompress pipeline of bb_decompress_host (float32 features) and bb_decompress_host_f64 (feat_dtype
+// BB_F64: float64 features, latent and reconstruction, precision BB_PREC_FP64).
+int decompress_host(bb_model* m, const void* z_host, int z_dtype, int64_t n_rows, const void* features_host,
+                    int feat_dtype, void* y_host, int y_dtype, int precision) {
   if (!m || (!z_host && n_rows) || (!y_host && n_rows) || n_rows < 0) return BB_ERR_INVALID;
   if (z_dtype != BB_F32 && z_dtype != BB_F16 && z_dtype != BB_F64) return BB_ERR_INVALID;
   if (y_dtype != BB_F32 && y_dtype != BB_F64) return BB_ERR_INVALID;
+  if (feat_dtype == BB_F64 && precision != BB_PREC_FP64) return BB_ERR_INVALID;
   BB_CUDA(cudaSetDevice(m->ctx->device));
   const int F = m->dec.desc.out_dim, Z = m->dec.desc.in_dim;
-  const int dev_in = (z_dtype == BB_F16) ? BB_F16 : BB_F32;
+  const bool f64 = precision == BB_PREC_FP64;
+  // device dtypes: the float32 / fp16 kernels read a float64 latent narrowed on the host and write float32; the float64
+  // kernel reads and writes the caller's dtypes
+  const int dev_in = (z_dtype == BB_F64 && !f64) ? BB_F32 : z_dtype;
+  const int dev_out = f64 ? y_dtype : BB_F32;
+  const bool narrow = dev_in != z_dtype, widen = dev_out != y_dtype;
+  // float64 chunks of the float64 chain go through the pinned slots when the caller's buffer is pageable
+  const bool bounce_in = dev_in == BB_F64 && n_rows && !host_pinned(z_host);
+  const bool bounce_out = dev_out == BB_F64 && n_rows && !host_pinned(y_host);
   const int64_t chunk = pipe_chunk_rows(n_rows);
   const int64_t n_chunks = n_rows ? (n_rows + chunk - 1) / chunk : 0;
-  const size_t in_b = (size_t)chunk * Z * dtype_size(dev_in), out_b = (size_t)chunk * F * sizeof(float);
+  const size_t in_b = (size_t)chunk * Z * dtype_size(dev_in), out_b = (size_t)chunk * F * dtype_size(dev_out);
   int rc = pipe_init(m, in_b, out_b);
   if (rc != BB_OK) return rc;
-  float* fmin = m->feat_dev;
-  float* frange = m->feat_dev + F;
+  char* feat = nullptr;
+  rc = features_dev(m, feat_dtype, &feat);
+  if (rc != BB_OK) return rc;
+  char* fmin = feat;
+  char* frange = feat + F * dtype_size(feat_dtype);
   const bool norm = features_host != nullptr;
-  if (norm) BB_CUDA(cudaMemcpyAsync(fmin, features_host, 2 * F * sizeof(float), cudaMemcpyHostToDevice, m->s_compute));
+  if (norm) BB_CUDA(cudaMemcpyAsync(fmin, features_host, 2 * F * dtype_size(feat_dtype), cudaMemcpyHostToDevice, m->s_compute));
 
-  float* pin_in[2] = {nullptr, nullptr};
-  float* pin_out[2] = {nullptr, nullptr};
-  auto cleanup = [&]() {};  // the bounce buffers belong to the model
-  if (n_rows) {
-    if (z_dtype == BB_F64) {
-      if (pinned_init(m, 0, (size_t)chunk * Z * sizeof(float)) != BB_OK) return BB_ERR_NOMEM;
+  void* pin_in[2] = {nullptr, nullptr};
+  void* pin_out[2] = {nullptr, nullptr};
+  if (n_rows) {  // (the bounce buffers belong to the model)
+    if (narrow || bounce_in) {
+      if (pinned_init(m, 0, (size_t)chunk * Z * dtype_size(dev_in)) != BB_OK) return BB_ERR_NOMEM;
       pin_in[0] = m->pinned_f32[0][0]; pin_in[1] = m->pinned_f32[0][1];
     }
-    if (y_dtype == BB_F64) {
-      if (pinned_init(m, 1, (size_t)chunk * F * sizeof(float)) != BB_OK) return BB_ERR_NOMEM;
+    if (widen || bounce_out) {
+      if (pinned_init(m, 1, (size_t)chunk * F * dtype_size(dev_out)) != BB_OK) return BB_ERR_NOMEM;
       pin_out[0] = m->pinned_f32[1][0]; pin_out[1] = m->pinned_f32[1][1];
     }
   }
   auto finish_chunk = [&](int64_t k) -> int {
     const int s = (int)(k & 1);
     BB_CUDA(cudaEventSynchronize(m->ev_out[s]));
-    if (y_dtype == BB_F64) {
-      const int64_t r0 = k * chunk, rows = std::min(chunk, n_rows - r0);
-      widen_f32_f64(pin_out[s], (double*)y_host + (size_t)r0 * F, (size_t)rows * F);
-    }
+    const int64_t r0 = k * chunk, rows = std::min(chunk, n_rows - r0);
+    if (widen) widen_f32_f64((const float*)pin_out[s], (double*)y_host + (size_t)r0 * F, (size_t)rows * F);
+    else if (bounce_out) copy_parallel((double*)y_host + (size_t)r0 * F, pin_out[s], (size_t)rows * F * sizeof(double));
     return BB_OK;
   };
   rc = BB_OK;
@@ -827,8 +918,11 @@ int bb_decompress_host(bb_model* m, const void* z_host, int z_dtype, int64_t n_r
       BB_CUDA(cudaStreamWaitEvent(m->s_copy_in, m->ev_done[s], 0));
     }
     const void* src = (const char*)z_host + (size_t)r0 * Z * dtype_size(z_dtype);
-    if (z_dtype == BB_F64) {
-      narrow_f64_f32((const double*)src, pin_in[s], (size_t)rows * Z);
+    if (narrow) {
+      narrow_f64_f32((const double*)src, (float*)pin_in[s], (size_t)rows * Z);
+      src = pin_in[s];
+    } else if (bounce_in) {
+      copy_parallel(pin_in[s], src, (size_t)rows * Z * sizeof(double));
       src = pin_in[s];
     }
     BB_CUDA(cudaMemcpyAsync(m->stage_dev[0][s], src, (size_t)rows * Z * dtype_size(dev_in), cudaMemcpyHostToDevice, m->s_copy_in));
@@ -840,24 +934,48 @@ int bb_decompress_host(bb_model* m, const void* z_host, int z_dtype, int64_t n_r
       BB_CUDA(cudaStreamWaitEvent(m->s_compute, m->ev_out[s], 0));
     }
     rc = run_chain(m, &m->dec, m->stage_dev[0][s], dev_in, rows, nullptr, nullptr, norm ? fmin : nullptr,
-                   norm ? frange : nullptr, m->stage_dev[1][s], BB_F32, precision, m->s_compute);
+                   norm ? frange : nullptr, feat_dtype, m->stage_dev[1][s], dev_out, precision, m->s_compute);
     if (rc != BB_OK) break;
     BB_CUDA(cudaEventRecord(m->ev_done[s], m->s_compute));
     BB_CUDA(cudaStreamWaitEvent(m->s_copy_out, m->ev_done[s], 0));
-    void* dst = (y_dtype == BB_F64) ? (void*)pin_out[s] : (void*)((float*)y_host + (size_t)r0 * F);
-    BB_CUDA(cudaMemcpyAsync(dst, m->stage_dev[1][s], (size_t)rows * F * sizeof(float), cudaMemcpyDeviceToHost, m->s_copy_out));
+    void* dst = (widen || bounce_out) ? pin_out[s] : (void*)((char*)y_host + (size_t)r0 * F * dtype_size(y_dtype));
+    BB_CUDA(cudaMemcpyAsync(dst, m->stage_dev[1][s], (size_t)rows * F * dtype_size(dev_out), cudaMemcpyDeviceToHost, m->s_copy_out));
     BB_CUDA(cudaEventRecord(m->ev_out[s], m->s_copy_out));
   }
   for (int64_t k = std::max<int64_t>(0, n_chunks - 2); k < n_chunks && rc == BB_OK; ++k) rc = finish_chunk(k);
   cudaStreamSynchronize(m->s_compute);
   cudaStreamSynchronize(m->s_copy_out);
-  cleanup();
   if (rc == BB_OK && precision == BB_PREC_AUTO && chain_has_tc(&m->dec)) {
     int tripped = 0;
     rc = bb_model_range_flag(m, 1, &tripped);
-    if (rc == BB_OK && tripped) return bb_decompress_host(m, z_host, z_dtype, n_rows, features_host, y_host, y_dtype, BB_PREC_FP32);
+    if (rc == BB_OK && tripped)
+      return decompress_host(m, z_host, z_dtype, n_rows, features_host, feat_dtype, y_host, y_dtype, BB_PREC_FP32);
   }
   return rc;
+}
+
+}  // namespace
+
+extern "C" {
+
+int bb_compress_host(bb_model* m, const float* x_host, int64_t n_rows, float* features_host,
+                     int recompute_minmax, void* z_host, int z_dtype, int precision) {
+  return compress_host(m, x_host, BB_F32, n_rows, features_host, recompute_minmax, z_host, z_dtype, precision);
+}
+
+int bb_decompress_host(bb_model* m, const void* z_host, int z_dtype, int64_t n_rows,
+                       const float* features_host, void* y_host, int y_dtype, int precision) {
+  return decompress_host(m, z_host, z_dtype, n_rows, features_host, BB_F32, y_host, y_dtype, precision);
+}
+
+int bb_compress_host_f64(bb_model* m, const double* x_host, int64_t n_rows, double* features_host,
+                         int recompute_minmax, double* z_host) {
+  return compress_host(m, x_host, BB_F64, n_rows, features_host, recompute_minmax, z_host, BB_F64, BB_PREC_FP64);
+}
+
+int bb_decompress_host_f64(bb_model* m, const double* z_host, int64_t n_rows, const double* features_host,
+                           double* y_host) {
+  return decompress_host(m, z_host, BB_F64, n_rows, features_host, BB_F64, y_host, BB_F64, BB_PREC_FP64);
 }
 
 }  // extern "C"

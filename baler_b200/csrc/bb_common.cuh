@@ -42,6 +42,20 @@ struct ChainDesc {
   ChainLayer layer[BB_MAX_LAYERS];
 };
 
+// One layer / one direction of the float64 chain (bb_chain_f64.cu); filled lazily by bb_chain_f64_prepare.
+struct F64Layer {
+  int K, Kpad, N, Npad;  // in features (padded to whole weight chunks), out features (padded to the thread tile)
+  int act, tn;           // BB_ACT_*, columns per thread
+  int w_off, b_off;      // double offsets of Wt[Kpad][Npad] (k-major, zero padded) and bias[Npad] in the blob
+};
+struct F64Desc {
+  int n_layers, in_dim, out_dim;
+  int tr;              // rows per tile (64 or 32)
+  int max_npad;        // widest padded layer: row length of the weight ring
+  int buf_rows[2];     // rows ([feature] index) of the two ping-pong activation buffers
+  F64Layer layer[BB_MAX_LAYERS];
+};
+
 // Launch plan of the statically shaped tcgen05 kernel (bb_chain_tc4.cu); filled by bb_tc_prepare.
 struct Tc4Plan {
   bool ok = false;
@@ -80,6 +94,10 @@ struct Chain {
   size_t g5_w_off[BB_MAX_LAYERS] = {0}, g5_b_off[BB_MAX_LAYERS] = {0};
   float g5_unscale[BB_MAX_LAYERS] = {0};
   int lay_max_ld = 0;
+  // float64 path (bb_chain_f64.cu): packed on the first BB_PREC_FP64 call, released by bb_model_trim
+  mutable F64Desc f64 = {};
+  mutable double* f64_blob_dev = nullptr;
+  mutable size_t f64_smem = 0;
   std::vector<double> w_host[BB_MAX_LAYERS];  // kept for re-packing
   std::vector<double> b_host[BB_MAX_LAYERS];
 };
@@ -94,12 +112,13 @@ struct bb_model {
   size_t stage_bytes[2] = {0, 0};
   cudaEvent_t ev_in[2] = {nullptr, nullptr}, ev_done[2] = {nullptr, nullptr}, ev_out[2] = {nullptr, nullptr};
   float* feat_dev = nullptr;  // [min | range | max] x n_features
+  double* feat64_dev = nullptr;  // the same for float64 tables (bb_compress_host_f64 / bb_decompress_host_f64), lazily
   // kept between calls (a 9.6 GB cudaMalloc + cudaFree costs ~0.12 s, a 240 MB cudaMallocHost ~0.05 s): the table that
   // stays resident between the min/max pass and the encode pass of bb_compress_host, and the pinned float32 bounce
   // buffers of the float64 host paths; released by bb_model_destroy / bb_model_trim
   float* resident_dev = nullptr;
   size_t resident_bytes = 0;
-  float* pinned_f32[2][2] = {{nullptr, nullptr}, {nullptr, nullptr}};  // [in/out][slot]
+  float* pinned_f32[2][2] = {{nullptr, nullptr}, {nullptr, nullptr}};  // [in/out][slot] (float64 chunks of the fp64 path too)
   size_t pinned_bytes[2] = {0, 0};
 };
 
@@ -118,8 +137,15 @@ size_t bb_gemm_tc5_buf_bytes(const Chain* c, int64_t rows);
 int bb_gemm_tc5_chunk(bb_ctx* ctx, const Chain* c, const void* in, int in_dtype, int64_t rows, const float* pre_min,
                       const float* pre_range, void* buf0, void* buf1, int* flag_dev, int* out_buf, int* ld_out,
                       cudaStream_t stream);
-int bb_colminmax_launch(bb_ctx* ctx, const float* x, int64_t n_rows, int n_cols, float* min_dev,
-                        float* max_dev, int reset, cudaStream_t stream);
+// x / min / max of element type dtype (BB_F32 or BB_F64)
+int bb_colminmax_launch(bb_ctx* ctx, const void* x, int dtype, int64_t n_rows, int n_cols, void* min_dev,
+                        void* max_dev, int reset, cudaStream_t stream);
+int bb_chain_f64_prepare(bb_ctx* ctx, const Chain* c);
+void bb_chain_f64_release(const Chain* c);
+// features (pre_* on the way in, post_* on the way out) are of type feat_dtype (BB_F32 or BB_F64)
+int bb_chain_f64_launch(bb_ctx* ctx, const Chain* c, const void* in, int in_dtype, int64_t n_rows, const void* pre_min,
+                        const void* pre_range, const void* post_min, const void* post_range, int feat_dtype, void* out,
+                        int out_dtype, cudaStream_t stream);
 int bb_tc_prepare(bb_ctx* ctx, Chain* c);
 void bb_tc_release(Chain* c);
 int bb_tc_launch_dbg(bb_ctx* ctx, const Chain* c, const void* in, int in_dtype, int64_t n_rows, const float* pre_min,

@@ -6,10 +6,12 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import BB_ACT_LEAKY, BB_ACT_NONE, BB_ACT_RELU, BB_F16, BB_F32, BB_F64, PRECISIONS, check
+from ._lib import BB_ACT_LEAKY, BB_ACT_NONE, BB_ACT_RELU, BB_F16, BB_F32, BB_F64, BB_PREC_FP64, PRECISIONS, check
 
 _NP2BB = {np.dtype(np.float32): BB_F32, np.dtype(np.float16): BB_F16, np.dtype(np.float64): BB_F64}
-_T2BB = {torch.float32: BB_F32, torch.float16: BB_F16}
+_T2BB = {torch.float32: BB_F32, torch.float16: BB_F16, torch.float64: BB_F64}
+# shapes the float64 chain takes (precision "fp64"; include/baler_b200.h, BB_PREC_FP64)
+FP64_MAX_LAYERS, FP64_MAX_WIDTH = 8, 256
 _contexts = {}
 
 
@@ -82,14 +84,24 @@ def host_convert(a, dtype):
 
 
 def colminmax(x, ctx=None):
-    """per-column (min, max) of a row-major CUDA float32 table -> two float32 CUDA vectors"""
+    """per-column (min, max) of a row-major CUDA float32 or float64 table -> two CUDA vectors of the table's dtype"""
     ctx = ctx or get_context(x.device)
-    assert x.is_cuda and x.dtype == torch.float32 and x.dim() == 2 and x.is_contiguous()
-    mn = torch.empty(x.shape[1], dtype=torch.float32, device=x.device)
+    assert x.is_cuda and x.dtype in (torch.float32, torch.float64) and x.dim() == 2 and x.is_contiguous()
+    mn = torch.empty(x.shape[1], dtype=x.dtype, device=x.device)
     mx = torch.empty_like(mn)
-    check(_lib.lib().bb_colminmax_f32(ctx.handle, _ptr(x), x.shape[0], x.shape[1], _ptr(mn), _ptr(mx), _stream(ctx)),
-          "bb_colminmax_f32")
+    name = "bb_colminmax_f64" if x.dtype == torch.float64 else "bb_colminmax_f32"
+    check(getattr(_lib.lib(), name)(ctx.handle, _ptr(x), x.shape[0], x.shape[1], _ptr(mn), _ptr(mx), _stream(ctx)), name)
     return mn, mx
+
+
+def fp64_refusal(chains):
+    """None when the float64 kernel takes every chain in `chains` ({name: [width of each layer boundary]}), else the
+    message of the NotImplementedError precision "fp64" raises for it"""
+    for name, dims in chains.items():
+        if len(dims) - 1 > FP64_MAX_LAYERS or max(dims) > FP64_MAX_WIDTH:
+            return ("precision='fp64' takes dense chains of at most %d layers with every width <= %d; the %s is %s"
+                    % (FP64_MAX_LAYERS, FP64_MAX_WIDTH, name, "-".join(str(d) for d in dims)))
+    return None
 
 
 def normalize_table(x, mn, rg, inverse=False, out=None, ctx=None):
@@ -122,12 +134,13 @@ class DenseCodec:
     def __init__(self, enc_layers, dec_layers, device=None):
         self.ctx = get_context(device)
         self.handle = C.c_void_p()
-        keep = []
+        keep, widths = [], []
 
         def pack(layers):
             w = [np.ascontiguousarray(l[0], dtype=np.float64) for l in layers]
             b = [np.ascontiguousarray(l[1], dtype=np.float64) for l in layers]
-            dims = (C.c_int * (len(layers) + 1))(*([w[0].shape[1]] + [x.shape[0] for x in w]))
+            widths.append([w[0].shape[1]] + [x.shape[0] for x in w])
+            dims = (C.c_int * (len(layers) + 1))(*widths[-1])
             acts = (C.c_int * len(layers))(*[self._ACT[l[2]] for l in layers])
             keep.extend(w + b)
             return len(layers), dims, acts, _host_ptrs(w), _host_ptrs(b)
@@ -139,6 +152,23 @@ class DenseCodec:
                                                    C.byref(self.handle)), "bb_model_create_dense")
         self.n_features = _lib.lib().bb_model_n_features(self.handle)
         self.z_dim = _lib.lib().bb_model_z_dim(self.handle)
+        self.widths = {"encoder": widths[0], "decoder": widths[1]}
+
+    def require_fp64(self, precision="fp64"):
+        """True for precision "fp64" (raises NotImplementedError when the float64 kernel does not take this model's
+        chains), False for the other precisions"""
+        if _prec(precision) != _lib.BB_PREC_FP64:
+            return False
+        msg = fp64_refusal(self.widths)
+        if msg:
+            raise NotImplementedError(msg)
+        return True
+
+    def _fp64_input(self, precision):
+        """float64 inputs run the float64 chain: precision "auto" or "fp64" """
+        if _prec(precision) not in (_lib.BB_PREC_AUTO, _lib.BB_PREC_FP64):
+            raise ValueError("float64 tensors run on precision 'fp64' only")
+        self.require_fp64()
 
     def __del__(self):
         try:
@@ -174,8 +204,19 @@ class DenseCodec:
 
     # ---- device-resident tensors
     def encode(self, x, fmin=None, frange=None, out_dtype=torch.float32, precision="auto", out=None, check_range=True):
-        assert x.is_cuda and x.dtype == torch.float32 and x.is_contiguous() and x.shape[-1] == self.n_features
+        """z = encode((x - fmin) / frange).  A float64 `x` (with float64 fmin / frange) runs the float64 chain and gives a
+        float64 latent; precision "fp64" runs it on a float32 `x`, normalised in float32 first (out_dtype may be float64)."""
+        assert x.is_cuda and x.dtype in (torch.float32, torch.float64) and x.is_contiguous() and x.shape[-1] == self.n_features
         n = x.numel() // self.n_features
+        if x.dtype == torch.float64:
+            self._fp64_input(precision)
+            assert fmin is None or (fmin.dtype == frange.dtype == torch.float64)
+            z = out if out is not None else torch.empty((n, self.z_dim), dtype=torch.float64, device=x.device)
+            assert z.dtype == torch.float64
+            check(_lib.lib().bb_encode_f64(self.handle, _ptr(x), n, _ptr(fmin), _ptr(frange), _ptr(z), _stream(self.ctx)),
+                  "bb_encode_f64")
+            return z
+        self.require_fp64(precision)
         z = out if out is not None else torch.empty((n, self.z_dim), dtype=out_dtype, device=x.device)
         self._guarded(lambda p: check(_lib.lib().bb_encode_f32(
             self.handle, _ptr(x), n, _ptr(fmin), _ptr(frange), _ptr(z), _T2BB[z.dtype], p, _stream(self.ctx)),
@@ -183,8 +224,20 @@ class DenseCodec:
         return z
 
     def decode(self, z, fmin=None, frange=None, precision="auto", out=None, check_range=True):
+        """y = decode(z) * frange + fmin.  A float64 `z` runs the float64 chain and gives float64 rows (float32 features
+        are widened exactly); precision "fp64" runs it on a float32 / float16 `z` with float32 rows out."""
         assert z.is_cuda and z.dtype in _T2BB and z.is_contiguous() and z.shape[-1] == self.z_dim
         n = z.numel() // self.z_dim
+        if z.dtype == torch.float64:
+            self._fp64_input(precision)
+            if fmin is not None:
+                fmin, frange = fmin.to(torch.float64).contiguous(), frange.to(torch.float64).contiguous()
+            y = out if out is not None else torch.empty((n, self.n_features), dtype=torch.float64, device=z.device)
+            assert y.dtype == torch.float64
+            check(_lib.lib().bb_decode_f64(self.handle, _ptr(z), n, _ptr(fmin), _ptr(frange), _ptr(y), _stream(self.ctx)),
+                  "bb_decode_f64")
+            return y
+        self.require_fp64(precision)
         y = out if out is not None else torch.empty((n, self.n_features), dtype=torch.float32, device=z.device)
         self._guarded(lambda p: check(_lib.lib().bb_decode_f32(
             self.handle, _ptr(z), _T2BB[z.dtype], n, _ptr(fmin), _ptr(frange), _ptr(y), p, _stream(self.ctx)),
@@ -194,7 +247,11 @@ class DenseCodec:
     # ---- host buffers (numpy), chunked copy/compute pipeline inside the library
     def compress_host(self, x, features=None, recompute_minmax=False, z_dtype=np.float32, precision="auto", out=None):
         """x: (n, F) float32 ndarray.  features: None (no normalisation) or (2, F) float32 [min; range]
-        (overwritten when recompute_minmax).  Returns (z, features)."""
+        (overwritten when recompute_minmax).  Returns (z, features).
+        precision "fp64": the float64 chain; a float32 table is normalised in float32 as above, any other table in
+        float64 with (2, F) float64 features (bb_compress_host_f64, float64 latent)."""
+        if self.require_fp64(precision) and np.asarray(x).dtype != np.float32:
+            return self._compress_host_f64(x, features, recompute_minmax, z_dtype, out)
         x = host_convert(x, np.float32)  # (float64 tables: narrowed on the worker threads)
         n = x.shape[0]
         z = out if out is not None else np.empty((n, self.z_dim), dtype=z_dtype)
@@ -207,7 +264,32 @@ class DenseCodec:
                                           z.ctypes.data, _NP2BB[z.dtype], _prec(precision)), "bb_compress_host")
         return z, feats
 
+    def _compress_host_f64(self, x, features, recompute_minmax, z_dtype, out):
+        """float64 table: float64 features and latent (narrowed on the host when z_dtype asks for less)"""
+        x = host_convert(x, np.float64)
+        n = x.shape[0]
+        z = out if out is not None else np.empty((n, self.z_dim), dtype=np.float64)
+        assert z.dtype == np.float64 and z.flags.c_contiguous
+        feats = None
+        if features is not None or recompute_minmax:
+            feats = np.zeros((2, self.n_features), dtype=np.float64) if features is None else \
+                np.ascontiguousarray(features, dtype=np.float64).copy()
+        check(_lib.lib().bb_compress_host_f64(self.handle, x.ctypes.data, n, None if feats is None else feats.ctypes.data,
+                                              int(bool(recompute_minmax)), z.ctypes.data), "bb_compress_host_f64")
+        return (z if out is not None else host_convert(z, z_dtype)), feats
+
     def decompress_host(self, z, features=None, y_dtype=np.float64, precision="auto", out=None):
+        """z: (n, z_dim) ndarray, features None or (2, F) [min; range] of the table (float32).  Returns y of y_dtype.
+        precision "fp64": the float64 chain; float64 features (a float64 table's) run bb_decompress_host_f64."""
+        if (self.require_fp64(precision) and features is not None and np.asarray(features).dtype == np.float64):
+            z = host_convert(z, np.float64)
+            n = z.shape[0]
+            y = out if out is not None else np.empty((n, self.n_features), dtype=np.float64)
+            assert y.dtype == np.float64 and y.flags.c_contiguous
+            feats = np.ascontiguousarray(features, dtype=np.float64)
+            check(_lib.lib().bb_decompress_host_f64(self.handle, z.ctypes.data, n, feats.ctypes.data, y.ctypes.data),
+                  "bb_decompress_host_f64")
+            return y if out is not None else host_convert(y, y_dtype)
         z = np.ascontiguousarray(z)
         n = z.shape[0]
         y = out if out is not None else np.empty((n, self.n_features), dtype=y_dtype)

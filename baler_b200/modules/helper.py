@@ -11,7 +11,7 @@ import numpy as np
 import torch
 
 from .. import engine
-from . import data_processing, training
+from . import data_processing, models, training
 
 sys.path.append(os.getcwd())
 
@@ -20,8 +20,12 @@ class Config:
     """Namespace the per-project `set_config(c)` fills (reference helper.py:150-179: a dataclass used as a
     class-level namespace; attributes that are never set raise AttributeError when read).
     Extra, optional knobs of this implementation (absent = reference behaviour):
-      precision        "auto" | "fp32" | "split16" | "fast"   arithmetic of the fused encode/decode kernels
-      latent_dtype     "float64" (AE default, what the reference writes) | "float32" | "float16"
+      precision        "auto" | "fp32" | "split16" | "fast" | "fp64"   arithmetic of the fused encode/decode kernels;
+                       "fp64" computes in float64 like the reference's float64 models (its files to ~1e-15, integer
+                       columns equal): dense models of <= 256 columns (AE, AE_Dropout_BN, CFD_dense_AE), float64 files
+                       normalised in float64 on the device, float32 files in float32 as numpy does; not with
+                       save_error_bounded_deltas
+      latent_dtype     "float64" (AE default, what the reference writes; any model under "fp64") | "float32" | "float16"
       l1_in_training   bool: add reg_param * L1 chain to the training loss (dead code upstream, SURVEY F2)
     """
 
@@ -150,14 +154,36 @@ def get_device():
 def _latent_np_dtype(model, config):
     name = getattr(config, "latent_dtype", None)
     if name is None:
-        return np.float64 if model.dtype == torch.float64 else np.float32
+        return np.float64 if model.dtype == torch.float64 or _fp64(config) else np.float32
     return np.dtype(name).type
+
+
+def _fp64(config):
+    """config.precision == "fp64": the float64 chain; refuses what it does not do before anything is read or written"""
+    if engine.PRECISIONS.get(getattr(config, "precision", "auto")) != engine.BB_PREC_FP64:
+        return False
+    if getattr(config, "save_error_bounded_deltas", False):
+        raise NotImplementedError("precision='fp64' does not compute error-bounded deltas (save_error_bounded_deltas); "
+                                  "use another precision for them")
+    return True
+
+
+def _refuse_fp64_shape(model):
+    """NotImplementedError naming the chain when the float64 kernel does not take `model` (Conv_AE, widths > 256)"""
+    if isinstance(model, models.Conv_AE):
+        raise NotImplementedError("precision='fp64' takes dense chains only; Conv_AE unrolls to dense layers up to %d wide"
+                                  % model.q_z_mid_dim)
+    dims = [model.n_features, *model.hidden, model.z_dim]
+    msg = engine.fp64_refusal({"encoder": dims, "decoder": dims[::-1]})
+    if msg:
+        raise NotImplementedError(msg)
 
 
 def compress(model_path, config):
     """reference helper.py:473-616 -> (compressed ndarray, eb_batch, eb_deltas, eb_index).
     Normalisation uses THIS file's column min/max (helper.py:500-502), fused into the encode kernel."""
     from .. import sharded
+    fp64 = _fp64(config)
     rank, world = sharded.dist_env()  # under torchrun: this rank's GPU, before anything touches a device
     loaded = np.load(config.input_path)
     data_before = loaded["data"]
@@ -184,11 +210,16 @@ def compress(model_path, config):
     model = data_processing.load_model(data_processing.initialise_model(config.model_name), model_path,
                                        n_features=n_features, z_dim=config.latent_space_size)
     model.eval()
+    if fp64:
+        _refuse_fp64_shape(model)
     normalise = bool(config.apply_normalization) and not config.custom_norm
     if config.apply_normalization:
         print("Normalizing...")
     table = None
-    if normalise and data_before.dtype == np.float64 and data_before.size:
+    if fp64 and data_before.dtype != np.float32:
+        # the float64 chain normalises a float64 table in float64 on the device (bb_compress_host_f64)
+        table = engine.host_convert(data_before.reshape(data_before.shape[0], -1), np.float64)
+    elif normalise and data_before.dtype == np.float64 and data_before.size:
         # a float64 file whose offset dwarfs its spread is normalised here in float64, as the reference's numpy does
         # (data_processing.F32_OFFSET_LIMIT); the kernels then take the normalised float32 table as it is
         flat64 = data_before.reshape(data_before.shape[0], -1)
@@ -303,6 +334,7 @@ def decompress(model_path, input_path, input_path_deltas, input_batch_index, mod
     `renormalize_features` ([min; range], optional, not in the reference signature) fuses the
     un-normalisation of baler.py:410-424 into the decode kernel."""
     from .. import sharded
+    fp64 = _fp64(config)
     rank, world = sharded.dist_env()  # under torchrun: this rank's GPU, before anything touches a device
     loaded = np.load(input_path)
     data, names, normalization_features = loaded["data"], loaded["names"], loaded["normalization_features"]
@@ -314,6 +346,9 @@ def decompress(model_path, input_path, input_path_deltas, input_batch_index, mod
     model = data_processing.load_model(data_processing.initialise_model(config.model_name), model_path,
                                        n_features=number_of_columns, z_dim=latent_space_size)
     model.eval()
+    if fp64:
+        _refuse_fp64_shape(model)
+        data = engine.host_convert(data, np.float64)  # the latent goes to the float64 chain as float64
     if data.dtype not in (np.float16, np.float32, np.float64):
         data = data.astype(np.float32)
     out_dtype = np.float64 if model.dtype == torch.float64 else np.float32
@@ -325,7 +360,7 @@ def decompress(model_path, input_path, input_path_deltas, input_batch_index, mod
     else:
         codec = model.codec()
     host_renorm = None
-    if renormalize_features is not None and out_dtype == np.float64:
+    if renormalize_features is not None and out_dtype == np.float64 and not fp64:
         f64 = np.asarray(renormalize_features, dtype=np.float64).reshape(2, -1)
         if data_processing._ill_conditioned(f64[0], f64[0] + f64[1]):
             # float32 could not hold y * range + min (data_processing.F32_OFFSET_LIMIT): decode to normalised values and

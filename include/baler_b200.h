@@ -51,6 +51,10 @@ extern "C" {
 #define BB_PREC_FP32 1    /* fp32 FFMA on CUDA cores; reference tolerance 1e-5 met with margin */
 #define BB_PREC_SPLIT16 2 /* tcgen05 tensor cores, fp16 hi/lo 3-product split, fp32 accumulate in TMEM */
 #define BB_PREC_FAST16 3  /* tcgen05 single fp16 product: OUTSIDE the 1e-5 tolerance (~3e-4), opt-in */
+#define BB_PREC_FP64 4    /* float64 DFMA chain, the reference's own arithmetic (its AE models are float64, helper.py:565):
+                             matches the reference's files to ~1e-15, opt-in.  Dense chains of <= 8 layers whose widths
+                             are all <= 256 (AE, CFD_dense_AE and AE_Dropout_BN up to 256 columns); other shapes return
+                             BB_ERR_UNSUPPORTED.  The float64 weight image is packed on the first call. */
 
 typedef struct bb_ctx bb_ctx;         /* one per device */
 typedef struct bb_model bb_model;     /* packed encoder + decoder weights of one autoencoder */
@@ -111,6 +115,10 @@ int bb_model_range_flag(bb_model* m, int reset, int* out);
  */
 int bb_colminmax_f32(bb_ctx* ctx, const float* x_dev, int64_t n_rows, int n_cols,
                      float* min_dev, float* max_dev, bb_stream_t stream);
+/* The same for a float64 table: data_processing.find_minmax (data_processing.py:113-130) on the float64 arrays the
+ * reference loads, exact (-0 < +0, NaN propagates per column). */
+int bb_colminmax_f64(bb_ctx* ctx, const double* x_dev, int64_t n_rows, int n_cols,
+                     double* min_dev, double* max_dev, bb_stream_t stream);
 
 /*
  * Stand-alone column normalisation and its inverse on device tables (row-major n x c float32):
@@ -131,6 +139,9 @@ int bb_renormalize_f32(bb_ctx* ctx, const float* y_dev, int64_t n_rows, int n_co
  * reference's IEEE divide, inside the 1e-5 bar); the stand-alone bb_normalize_f32 above is the
  * bit-equal subtract + divide.  min_dev/range_dev may both be NULL (apply_normalization = False).
  * z_dtype: BB_F32 or BB_F16 (row-major n_rows x z_dim).
+ * precision BB_PREC_FP64: the table is normalised in float32 (bit-equal to numpy's float32 arithmetic, the
+ * reference converts to a float64 tensor after normalising, data_processing.py:133-153), widened and run through
+ * the float64 chain; z_dtype may then also be BB_F64.
  */
 int bb_encode_f32(bb_model* m, const float* x_dev, int64_t n_rows,
                   const float* min_dev, const float* range_dev,
@@ -144,6 +155,20 @@ int bb_encode_f32(bb_model* m, const float* x_dev, int64_t n_rows,
 int bb_decode_f32(bb_model* m, const void* z_dev, int z_dtype, int64_t n_rows,
                   const float* min_dev, const float* range_dev,
                   float* y_dev, int precision, bb_stream_t stream);
+/* (bb_decode_f32 with BB_PREC_FP64: z_dtype BB_F32 / BB_F16 / BB_F64, chain and un-normalisation in float64, float32 out.) */
+
+/*
+ * Float64 tables (BB_PREC_FP64 arithmetic throughout): helper.compress / helper.decompress on the float64 files the
+ * reference reads and writes (helper.py:473-616, 619-733).
+ *   bb_encode_f64: z = encode((x - min) / range), normalised in float64 (data_processing.py:133-153) and fused with the
+ *                  `model.encode` loop (helper.py:583-611).
+ *   bb_decode_f64: y = decode(z) * range + min in float64 (helper.py:701-723 fused with data_processing.py:188-203).
+ * min_dev / range_dev may both be NULL.  BB_ERR_UNSUPPORTED for shapes outside BB_PREC_FP64's.
+ */
+int bb_encode_f64(bb_model* m, const double* x_dev, int64_t n_rows, const double* min_dev,
+                  const double* range_dev, double* z_dev, bb_stream_t stream);
+int bb_decode_f64(bb_model* m, const double* z_dev, int64_t n_rows, const double* min_dev,
+                  const double* range_dev, double* y_dev, bb_stream_t stream);
 
 /*
  * The host-side steps of the two pipelines below, callable on their own (no device needed):
@@ -167,12 +192,21 @@ int bb_host_colminmax_f32(const float* x_host, int64_t n_rows, int n_cols, float
  *     features_host == NULL: no normalisation.
  *   z_dtype / y_dtype: BB_F32, BB_F64 (what the reference writes for AE, helper.py:565) or, for z,
  *     BB_F16.  Pinned (page-locked) host buffers make the copies asynchronous; pageable works too.
+ *   precision BB_PREC_FP64: the float64 chain (see bb_encode_f32 / bb_decode_f32); BB_F64 latents and reconstructions
+ *     then cross PCIe as float64, with no float32 step on the host.
  */
 int bb_compress_host(bb_model* m, const float* x_host, int64_t n_rows,
                      float* features_host, int recompute_minmax,
                      void* z_host, int z_dtype, int precision);
 int bb_decompress_host(bb_model* m, const void* z_host, int z_dtype, int64_t n_rows,
                        const float* features_host, void* y_host, int y_dtype, int precision);
+/* The same pipelines for float64 tables, in float64 throughout (BB_PREC_FP64): helper.compress / helper.decompress
+ * (helper.py:473-616, 619-733) on a float64 file.  features_host is 2 x n_features float64 [min; range] (computed from
+ * THIS table when recompute_minmax != 0, exact float64 column min / max; helper.py:500-502), or NULL. */
+int bb_compress_host_f64(bb_model* m, const double* x_host, int64_t n_rows, double* features_host,
+                         int recompute_minmax, double* z_host);
+int bb_decompress_host_f64(bb_model* m, const double* z_host, int64_t n_rows, const double* features_host,
+                           double* y_host);
 
 /* ------------------------------------------------------------------ training (dense AE) */
 
