@@ -48,6 +48,7 @@ _SIGNATURES = {
     "bb_colminmax_f32": (C.c_int, [_P, _P, C.c_int64, C.c_int, _P, _P, _P]),
     "bb_colminmax_f64": (C.c_int, [_P, _P, C.c_int64, C.c_int, _P, _P, _P]),
     "bb_normalize_f32": (C.c_int, [_P, _P, C.c_int64, C.c_int, _P, _P, _P, _P]),
+    "bb_normalize_f64": (C.c_int, [_P, _P, C.c_int64, C.c_int, _P, _P, _P, _P]),
     "bb_renormalize_f32": (C.c_int, [_P, _P, C.c_int64, C.c_int, _P, _P, _P, _P]),
     "bb_encode_f32": (C.c_int, [_P, _P, C.c_int64, _P, _P, _P, C.c_int, C.c_int, _P]),
     "bb_decode_f32": (C.c_int, [_P, _P, C.c_int, C.c_int64, _P, _P, _P, C.c_int, _P]),
@@ -73,10 +74,15 @@ _SIGNATURES = {
     "bb_trainer_param_count": (C.c_int, [_P]),
     "bb_trainer_params_dev": (_P, [_P]),
     "bb_trainer_grads_dev": (_P, [_P]),
+    "bb_trainer_params_dev_f64": (_P, [_P]),
+    "bb_trainer_grads_dev_f64": (_P, [_P]),
     "bb_trainer_get_params": (C.c_int, [_P, _P, _P]),
     "bb_trainer_step": (C.c_int, [_P, _P, C.c_int, C.POINTER(TrainHyper), C.c_int, _P, _P]),
     "bb_trainer_epoch": (C.c_int, [_P, _P, C.c_int64, C.c_int, C.POINTER(TrainHyper), C.POINTER(C.c_double), _P]),
     "bb_trainer_validate": (C.c_int, [_P, _P, C.c_int64, C.c_int, C.POINTER(C.c_double), _P]),
+    "bb_trainer_step_f64": (C.c_int, [_P, _P, C.c_int, C.POINTER(TrainHyper), C.c_int, _P, _P]),
+    "bb_trainer_epoch_f64": (C.c_int, [_P, _P, C.c_int64, C.c_int, C.POINTER(TrainHyper), C.POINTER(C.c_double), _P]),
+    "bb_trainer_validate_f64": (C.c_int, [_P, _P, C.c_int64, C.c_int, C.POINTER(C.c_double), _P]),
     "bb_trainer_activation_means": (C.c_int, [_P, _P]),
     "bb_mse_sum_f32": (C.c_int, [_P, _P, _P, C.c_int64, _P, _P]),
     "bb_error_bounded_deltas_f32": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int, _P, _P, C.c_double, C.c_int64, C.c_int64, _P, _P, _P, _P, _P]),

@@ -63,10 +63,12 @@ def _latent_size(config, shape, original_shape):
 def perform_training(output_path, config, verbose):
     """reference baler.py:84-207"""
     from . import sharded
+    helper.refuse_fp64_training(config)  # precision "fp64": what the float64 trainer does not take, before any work
     sharded.dist_env()  # under torchrun: bind this rank to ITS GPU before helper.process allocates anything on a device
     train_set, test_set, normalization_features, original_shape = helper.process(
         config.input_path, config.custom_norm, config.test_size, config.apply_normalization,
-        config.convert_to_blocks if hasattr(config, "convert_to_blocks") else None, verbose)
+        config.convert_to_blocks if hasattr(config, "convert_to_blocks") else None, verbose,
+        precision=getattr(config, "precision", None))
     n_features, number_of_columns = _latent_size(config, train_set.shape, original_shape)
     if verbose:
         print(f"Intitalizing Model with Latent Size - {config.latent_space_size} and Features - {n_features}")

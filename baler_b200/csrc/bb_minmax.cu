@@ -231,9 +231,29 @@ __global__ void __launch_bounds__(256) colscale_kernel(const float* __restrict__
     out[e] = INVERSE ? fmaf(v, __ldg(rg + col), __ldg(mn + col)) : __fdiv_rn(__fsub_rn(v, __ldg(mn + col)), __ldg(rg + col));
   }
 }
+
+// (x - min) / range in float64, one rounding per operation like numpy
+__global__ void __launch_bounds__(256) normalize_f64_kernel(const double* __restrict__ x, const int64_t n_elems, const int c,
+                                                            const double* __restrict__ mn, const double* __restrict__ rg,
+                                                            double* __restrict__ out) {
+  const int64_t G = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n_elems; e += G) {
+    const int col = (int)(e % c);
+    out[e] = __ddiv_rn(__dsub_rn(x[e], __ldg(mn + col)), __ldg(rg + col));
+  }
+}
 }  // namespace
 
 extern "C" {
+int bb_normalize_f64(bb_ctx* ctx, const double* x_dev, int64_t n_rows, int n_cols, const double* min_dev,
+                     const double* range_dev, double* out_dev, bb_stream_t stream) {
+  if (!ctx || n_cols <= 0 || n_rows < 0 || !min_dev || !range_dev || ((!x_dev || !out_dev) && n_rows)) return BB_ERR_INVALID;
+  if (n_rows == 0) return BB_OK;
+  const int64_t n = n_rows * n_cols;
+  const int grid = (int)((n + 255) / 256 < (int64_t)ctx->sm_count * 8 ? (n + 255) / 256 : ctx->sm_count * 8);
+  normalize_f64_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(x_dev, n, n_cols, min_dev, range_dev, out_dev);
+  return (int)cudaGetLastError();
+}
 int bb_normalize_f32(bb_ctx* ctx, const float* x_dev, int64_t n_rows, int n_cols, const float* min_dev,
                      const float* range_dev, float* out_dev, bb_stream_t stream) {
   if (!ctx || n_cols <= 0 || n_rows < 0 || !min_dev || !range_dev || ((!x_dev || !out_dev) && n_rows)) return BB_ERR_INVALID;

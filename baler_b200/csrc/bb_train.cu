@@ -25,6 +25,7 @@
 #include <curand_philox4x32_x.h>
 
 #include "bb_common.cuh"
+#include "bb_train_f64.cuh"
 #include "bb_train_tc.cuh"
 
 namespace {
@@ -722,6 +723,11 @@ struct bb_trainer {
   int precision = BB_PREC_AUTO;      // BB_PREC_FP32 forces the fp32 kernels
   bool wt_fresh = true, tc_fresh = true;
   bool last_tc = false;              // which path ran the most recent forward pass (activation extraction)
+  // float64 path (bb_train_f64.cu, BB_PREC_FP64): its own float64 master parameters, Adam state and scratch, made by
+  // bb_trainer_set_precision from the float64 weights bb_trainer_create received (kept here until then)
+  F64Trainer* f64 = nullptr;
+  std::vector<double> params_host;
+  bool started = false;              // a step or an epoch has run (the precision of a float64 run is fixed from then on)
 };
 
 namespace {
@@ -919,6 +925,14 @@ int create_common(bb_ctx* ctx, int n_features, int z_dim, const double* const* w
       hnbt[i] = bn_nbt ? bn_nbt[i] : 0;
     }
   }
+  if (kind == 0) {
+    t->params_host.assign(p, 0.0);
+    for (int l = 0; l < NL; ++l) {
+      const int K = dims[l], N = dims[l + 1];
+      for (int i = 0; i < N * K; ++i) t->params_host[d.w_off[l] + i] = weights_host[l][i];
+      for (int n = 0; n < N; ++n) t->params_host[d.b_off[l] + n] = biases_host[l][n];
+    }
+  }
   t->n_tiles = (int)tiles.size();
   const int max_splits = (max_batch + DW_T - 1) / DW_T;
   const int max_ctas = (max_batch + RT - 1) / RT;
@@ -993,12 +1007,36 @@ int bb_trainer_destroy(bb_trainer* t) {
   for (void* p : ptrs)
     if (p) cudaFree(p);
   bb_tc_train_destroy(t->tc);
+  bb_f64_train_destroy(t->f64);
   delete t;
   return BB_OK;
 }
 
 int bb_trainer_set_precision(bb_trainer* t, int precision) {
-  if (!t || precision < BB_PREC_AUTO || precision > BB_PREC_SPLIT16) return BB_ERR_INVALID;
+  if (!t) return BB_ERR_INVALID;
+  if (precision == BB_PREC_FP64) {
+    if (t->kind != 0) return BB_ERR_UNSUPPORTED;
+    if (t->started) return BB_ERR_INVALID;
+    if (!t->f64) {
+      F64TrainLayout fl;
+      const TrainDims& d = t->d;
+      memcpy(fl.dims, d.dims, sizeof(fl.dims));
+      memcpy(fl.act, d.act, sizeof(fl.act));
+      memcpy(fl.w_off, d.w_off, sizeof(fl.w_off));
+      memcpy(fl.b_off, d.b_off, sizeof(fl.b_off));
+      memcpy(fl.wt_off, d.wt_off, sizeof(fl.wt_off));
+      memcpy(fl.a_off, d.a_off, sizeof(fl.a_off));
+      memcpy(fl.z_off, d.z_off, sizeof(fl.z_off));
+      fl.a_stride = d.a_stride; fl.z_stride = d.z_stride; fl.n_params = d.n_params; fl.max_dim = d.max_dim;
+      BB_CUDA(cudaSetDevice(t->ctx->device));
+      const int rc = bb_f64_train_create(t->ctx, fl, t->params_host.data(), t->max_batch, &t->f64);
+      if (rc != BB_OK) return rc;
+    }
+    t->precision = BB_PREC_FP64;
+    return BB_OK;
+  }
+  if (precision < BB_PREC_AUTO || precision > BB_PREC_SPLIT16) return BB_ERR_INVALID;
+  if (t->precision == BB_PREC_FP64 && t->started) return BB_ERR_INVALID;
   if (precision == BB_PREC_SPLIT16 && !t->tc) return BB_ERR_UNSUPPORTED;
   t->precision = precision;
   return BB_OK;
@@ -1006,12 +1044,14 @@ int bb_trainer_set_precision(bb_trainer* t, int precision) {
 
 int bb_trainer_precision(const bb_trainer* t) {
   if (!t) return BB_ERR_INVALID;
+  if (t->precision == BB_PREC_FP64) return BB_PREC_FP64;
   return t->tc && t->precision != BB_PREC_FP32 ? BB_PREC_SPLIT16 : BB_PREC_FP32;
 }
 
 int bb_trainer_range_flag(bb_trainer* t, int reset, int* out) {
   if (!t || !out) return BB_ERR_INVALID;
   *out = 0;
+  if (t->precision == BB_PREC_FP64) return BB_OK;
   return t->tc ? bb_tc_train_range_flag(t->tc, reset, out) : BB_OK;
 }
 
@@ -1021,12 +1061,12 @@ int bb_trainer_debug_layer(bb_trainer* t, int which, int layer, int rows, float*
 }
 
 int bb_trainer_dp_export(bb_trainer* t, int world_size, unsigned char* handle_out_64) {
-  if (!t || !t->tc) return BB_ERR_UNSUPPORTED;
+  if (!t || !t->tc || t->precision == BB_PREC_FP64) return BB_ERR_UNSUPPORTED;
   return bb_tc_train_dp_export(t->tc, world_size, handle_out_64);
 }
 
 int bb_trainer_dp_connect(bb_trainer* t, int rank, int world_size, const unsigned char* handles) {
-  if (!t || !t->tc) return BB_ERR_UNSUPPORTED;
+  if (!t || !t->tc || t->precision == BB_PREC_FP64) return BB_ERR_UNSUPPORTED;
   return bb_tc_train_dp_connect(t->tc, rank, world_size, handles);
 }
 
@@ -1038,9 +1078,22 @@ int bb_trainer_profile(bb_trainer* t, int step, long long* out_128) {
 int bb_trainer_param_count(const bb_trainer* t) { return t ? t->d.n_params : 0; }
 float* bb_trainer_params_dev(bb_trainer* t) { return t ? t->params : nullptr; }
 float* bb_trainer_grads_dev(bb_trainer* t) { return t ? t->grads : nullptr; }
+double* bb_trainer_params_dev_f64(bb_trainer* t) { return t && t->precision == BB_PREC_FP64 ? bb_f64_train_params(t->f64) : nullptr; }
+double* bb_trainer_grads_dev_f64(bb_trainer* t) { return t && t->precision == BB_PREC_FP64 ? bb_f64_train_grads(t->f64) : nullptr; }
 
 int bb_trainer_get_params(bb_trainer* t, double* const* weights_host, double* const* biases_host) {
   if (!t || !weights_host || !biases_host) return BB_ERR_INVALID;
+  if (t->precision == BB_PREC_FP64) {  // the float64 master as it is
+    std::vector<double> hp(t->d.n_params);
+    const int rc = bb_f64_train_get_params(t->f64, hp.data());
+    if (rc != BB_OK) return rc;
+    for (int l = 0; l < NL; ++l) {
+      const int K = t->d.dims[l], N = t->d.dims[l + 1];
+      memcpy(weights_host[l], hp.data() + t->d.w_off[l], sizeof(double) * N * K);
+      memcpy(biases_host[l], hp.data() + t->d.b_off[l], sizeof(double) * N);
+    }
+    return BB_OK;
+  }
   std::vector<float> hp(t->d.n_params);
   BB_CUDA(cudaMemcpy(hp.data(), t->params, sizeof(float) * hp.size(), cudaMemcpyDeviceToHost));
   for (int l = 0; l < NL; ++l) {
@@ -1051,10 +1104,84 @@ int bb_trainer_get_params(bb_trainer* t, double* const* weights_host, double* co
   return BB_OK;
 }
 
+}  // extern "C"
+
+namespace {
+// BB_PREC_FP64: the float64 step of bb_train_f64.cu on a float32 table (widened exactly) or a float64 one
+int step_f64(bb_trainer* t, const void* x, int x_is_f64, int rows, const bb_train_hyper* h, int phase, double* loss_accum,
+             cudaStream_t s) {
+  if (!t || !h || !x || rows < 1 || rows > t->max_batch || phase < 0 || phase > 2) return BB_ERR_INVALID;
+  if (t->precision != BB_PREC_FP64) return BB_ERR_INVALID;
+  t->started = true;
+  const long long step = phase != 1 ? t->step + 1 : t->step;
+  const int rc = bb_f64_train_step(t->f64, x, x_is_f64, rows, h, phase, step, loss_accum, s);
+  if (rc == BB_OK) t->step = step;
+  return rc;
+}
+
+int epoch_f64(bb_trainer* t, const void* x, int x_is_f64, int64_t n_rows, int batch, const bb_train_hyper* h,
+              double* epoch_loss_host, cudaStream_t s) {
+  if (!t || !h || !x || n_rows < 1 || batch < 1 || batch > t->max_batch || !epoch_loss_host) return BB_ERR_INVALID;
+  if (t->precision != BB_PREC_FP64) return BB_ERR_INVALID;
+  if (h->world_size > 1) return BB_ERR_UNSUPPORTED;  // data parallel: phases 1 and 2 around the caller's all-reduce
+  BB_CUDA(cudaMemsetAsync(t->loss_accum, 0, sizeof(double), s));
+  const size_t row_bytes = (size_t)t->d.dims[0] * (x_is_f64 ? sizeof(double) : sizeof(float));
+  int64_t n_batches = 0;
+  for (int64_t r0 = 0; r0 < n_rows; r0 += batch, ++n_batches) {
+    const int rows = (int)(n_rows - r0 < batch ? n_rows - r0 : batch);
+    const int rc = step_f64(t, (const char*)x + (size_t)r0 * row_bytes, x_is_f64, rows, h, 0, t->loss_accum, s);
+    if (rc != BB_OK) return rc;
+  }
+  double total = 0.0;
+  BB_CUDA(cudaMemcpyAsync(&total, t->loss_accum, sizeof(double), cudaMemcpyDeviceToHost, s));
+  BB_CUDA(cudaStreamSynchronize(s));
+  *epoch_loss_host = total / (double)n_batches;
+  return BB_OK;
+}
+
+int validate_f64(bb_trainer* t, const void* x, int x_is_f64, int64_t n_rows, int batch, double* epoch_loss_host,
+                 cudaStream_t s) {
+  if (!t || !x || n_rows < 1 || batch < 1 || batch > t->max_batch || !epoch_loss_host) return BB_ERR_INVALID;
+  if (t->precision != BB_PREC_FP64) return BB_ERR_INVALID;
+  BB_CUDA(cudaMemsetAsync(t->loss_accum, 0, sizeof(double), s));
+  const size_t row_bytes = (size_t)t->d.dims[0] * (x_is_f64 ? sizeof(double) : sizeof(float));
+  int64_t n_batches = 0;
+  for (int64_t r0 = 0; r0 < n_rows; r0 += batch, ++n_batches) {
+    const int rows = (int)(n_rows - r0 < batch ? n_rows - r0 : batch);
+    const int rc = bb_f64_train_eval(t->f64, (const char*)x + (size_t)r0 * row_bytes, x_is_f64, rows, t->loss_accum, s);
+    if (rc != BB_OK) return rc;
+  }
+  double total = 0.0;
+  BB_CUDA(cudaMemcpyAsync(&total, t->loss_accum, sizeof(double), cudaMemcpyDeviceToHost, s));
+  BB_CUDA(cudaStreamSynchronize(s));
+  *epoch_loss_host = total / (double)n_batches;
+  return BB_OK;
+}
+}  // namespace
+
+extern "C" {
+
+int bb_trainer_step_f64(bb_trainer* t, const double* x_dev, int batch_rows, const bb_train_hyper* h, int phase,
+                        double* loss_accum_dev, bb_stream_t stream) {
+  return step_f64(t, x_dev, 1, batch_rows, h, phase, loss_accum_dev, (cudaStream_t)stream);
+}
+
+int bb_trainer_epoch_f64(bb_trainer* t, const double* x_dev, int64_t n_rows, int batch, const bb_train_hyper* h,
+                         double* epoch_loss_host, bb_stream_t stream) {
+  return epoch_f64(t, x_dev, 1, n_rows, batch, h, epoch_loss_host, (cudaStream_t)stream);
+}
+
+int bb_trainer_validate_f64(bb_trainer* t, const double* x_dev, int64_t n_rows, int batch, double* epoch_loss_host,
+                            bb_stream_t stream) {
+  return validate_f64(t, x_dev, 1, n_rows, batch, epoch_loss_host, (cudaStream_t)stream);
+}
+
 int bb_trainer_step(bb_trainer* t, const float* x_dev, int batch_rows, const bb_train_hyper* h, int phase,
                     double* loss_accum_dev, bb_stream_t stream) {
   if (!t || !h || !x_dev || batch_rows < 1 || batch_rows > t->max_batch || phase < 0 || phase > 2) return BB_ERR_INVALID;
   cudaStream_t s = (cudaStream_t)stream;
+  if (t->precision == BB_PREC_FP64) return step_f64(t, x_dev, 0, batch_rows, h, phase, loss_accum_dev, s);
+  t->started = true;
   int urc;
   if (use_tc(t, h, s, &urc)) {
     if (urc != BB_OK) return urc;
@@ -1102,6 +1229,8 @@ int bb_trainer_step(bb_trainer* t, const float* x_dev, int batch_rows, const bb_
 int bb_trainer_epoch(bb_trainer* t, const float* x_dev, int64_t n_rows, int batch, const bb_train_hyper* h,
                      double* epoch_loss_host, bb_stream_t stream) {
   if (!t || !h || !x_dev || n_rows < 1 || batch < 1 || !epoch_loss_host) return BB_ERR_INVALID;
+  if (t->precision == BB_PREC_FP64) return epoch_f64(t, x_dev, 0, n_rows, batch, h, epoch_loss_host, (cudaStream_t)stream);
+  t->started = true;
   if (h->world_size <= 1 && batch > t->max_batch) return BB_ERR_INVALID;
   const int dp_world = t->tc ? bb_tc_train_dp_world(t->tc) : 1;
   if (h->world_size > 1 && h->world_size != dp_world) return BB_ERR_INVALID;  // data parallel needs bb_trainer_dp_connect
@@ -1143,6 +1272,7 @@ int bb_trainer_validate(bb_trainer* t, const float* x_dev, int64_t n_rows, int b
                         bb_stream_t stream) {
   if (!t || !x_dev || n_rows < 1 || batch < 1 || batch > t->max_batch || !epoch_loss_host) return BB_ERR_INVALID;
   cudaStream_t s = (cudaStream_t)stream;
+  if (t->precision == BB_PREC_FP64) return validate_f64(t, x_dev, 0, n_rows, batch, epoch_loss_host, s);
   BB_CUDA(cudaMemsetAsync(t->loss_accum, 0, sizeof(double), s));
   int64_t n_batches = 0;
   int urc;
@@ -1182,6 +1312,7 @@ int bb_trainer_validate(bb_trainer* t, const float* x_dev, int64_t n_rows, int b
 
 int bb_trainer_activation_means(bb_trainer* t, double* out) {
   if (!t || !out) return BB_ERR_INVALID;
+  if (t->precision == BB_PREC_FP64) return bb_f64_train_activation_means(t->f64, out);
   if (t->last_tc) return bb_tc_train_activation_means(t->tc, t->last_rows, out);
   const int rows = t->last_rows, stride = t->d.a_stride;
   std::vector<float> h((size_t)rows * stride);

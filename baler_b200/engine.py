@@ -115,6 +115,18 @@ def normalize_table(x, mn, rg, inverse=False, out=None, ctx=None):
     return out
 
 
+def normalize_table_f64(x, mn, rg, out=None, ctx=None):
+    """(x - min) / range on a CUDA float64 table, one IEEE subtract and divide per element (bit-equal to numpy)"""
+    ctx = ctx or get_context(x.device)
+    assert x.is_cuda and x.dtype == torch.float64 and x.is_contiguous()
+    assert mn.dtype == rg.dtype == torch.float64 and mn.is_contiguous() and rg.is_contiguous()
+    out = torch.empty_like(x) if out is None else out
+    c = x.shape[-1]
+    check(_lib.lib().bb_normalize_f64(ctx.handle, _ptr(x), x.numel() // c, c, _ptr(mn), _ptr(rg), _ptr(out), _stream(ctx)),
+          "bb_normalize_f64")
+    return out
+
+
 def mse_sum(a, b, ctx=None):
     """sum((a - b)^2) of two CUDA float32 tensors -> python float (one device->host read)"""
     ctx = ctx or get_context(a.device)
@@ -335,7 +347,7 @@ class Trainer:
         except Exception:
             pass
 
-    def _flat(self, ptr, n=None):
+    def _flat(self, ptr, n=None, typestr="<f4"):
         # zero-copy torch view of library-owned device memory
         from torch.utils import dlpack  # noqa: F401  (documented route; below uses __cuda_array_interface__)
 
@@ -343,16 +355,30 @@ class Trainer:
             pass
 
         a = _Arr()
-        a.__cuda_array_interface__ = {"shape": (n or self.n_params,), "typestr": "<f4", "data": (int(ptr), False), "version": 2}
+        a.__cuda_array_interface__ = {"shape": (n or self.n_params,), "typestr": typestr, "data": (int(ptr), False), "version": 2}
         return torch.as_tensor(a, device=self.ctx.device)
 
     def set_precision(self, precision):
-        """"auto" / "split16": tensor-core step (AE family, MSE loss); "fp32": the fp32 FFMA kernels"""
+        """"auto" / "split16": tensor-core step (AE family, MSE loss); "fp32": the fp32 FFMA kernels; "fp64": the float64
+        kernels with float64 master parameters (AE / CFD_dense_AE, before the first step; params_view / grads_view are
+        float64 from then on, step / epoch / validate take float32 or float64 tables)"""
         check(_lib.lib().bb_trainer_set_precision(self.handle, _prec(precision)), "bb_trainer_set_precision")
 
     @property
     def precision(self):
-        return {_lib.BB_PREC_FP32: "fp32", _lib.BB_PREC_SPLIT16: "split16"}[_lib.lib().bb_trainer_precision(self.handle)]
+        return {_lib.BB_PREC_FP32: "fp32", _lib.BB_PREC_SPLIT16: "split16", _lib.BB_PREC_FP64: "fp64"}[
+            _lib.lib().bb_trainer_precision(self.handle)]
+
+    @property
+    def _fp64(self):
+        return _lib.lib().bb_trainer_precision(self.handle) == _lib.BB_PREC_FP64
+
+    def _x(self, x, name):
+        """(pointer, C entry point) of a float32 or float64 CUDA table"""
+        assert x.is_cuda and x.is_contiguous() and x.dtype in (torch.float32, torch.float64)
+        if x.dtype == torch.float64:
+            name += "_f64"  # BB_PREC_FP64 trainers only: the library refuses the others
+        return _ptr(x), getattr(_lib.lib(), name), name
 
     def range_flag(self, reset=True):
         """sticky flag of the split16 step: a batch loss was not finite (values beyond the fp16 range); synchronises"""
@@ -386,27 +412,31 @@ class Trainer:
         return out[:n * rows].reshape(n, rows)
 
     def params_view(self):
+        """flat parameters (float32; float64 under precision "fp64")"""
+        if self._fp64:
+            return self._flat(_lib.lib().bb_trainer_params_dev_f64(self.handle), typestr="<f8")
         return self._flat(_lib.lib().bb_trainer_params_dev(self.handle))
 
     def grads_view(self):
-        """n_params gradient entries followed by the batch loss (one flat buffer = one all-reduce)"""
+        """n_params gradient entries followed by the batch loss (one flat buffer = one all-reduce); float64 under "fp64" """
+        if self._fp64:
+            return self._flat(_lib.lib().bb_trainer_grads_dev_f64(self.handle), self.n_params + 1, "<f8")
         return self._flat(_lib.lib().bb_trainer_grads_dev(self.handle), self.n_params + 1)
 
     def step(self, x, hyper, phase=0):
-        assert x.is_cuda and x.dtype == torch.float32 and x.is_contiguous()
-        check(_lib.lib().bb_trainer_step(self.handle, _ptr(x), x.shape[0], C.byref(hyper), phase,
-                                         _ptr(self.loss_accum), _stream(self.ctx)), "bb_trainer_step")
+        ptr, fn, name = self._x(x, "bb_trainer_step")
+        check(fn(self.handle, ptr, x.shape[0], C.byref(hyper), phase, _ptr(self.loss_accum), _stream(self.ctx)), name)
 
     def epoch(self, x, batch, hyper):
         out = C.c_double()
-        check(_lib.lib().bb_trainer_epoch(self.handle, _ptr(x), x.shape[0], batch, C.byref(hyper), C.byref(out),
-                                          _stream(self.ctx)), "bb_trainer_epoch")
+        ptr, fn, name = self._x(x, "bb_trainer_epoch")
+        check(fn(self.handle, ptr, x.shape[0], batch, C.byref(hyper), C.byref(out), _stream(self.ctx)), name)
         return out.value
 
     def validate(self, x, batch):
         out = C.c_double()
-        check(_lib.lib().bb_trainer_validate(self.handle, _ptr(x), x.shape[0], batch, C.byref(out), _stream(self.ctx)),
-              "bb_trainer_validate")
+        ptr, fn, name = self._x(x, "bb_trainer_validate")
+        check(fn(self.handle, ptr, x.shape[0], batch, C.byref(out), _stream(self.ctx)), name)
         return out.value
 
     def set_dropout(self, seed=0, masks=None):

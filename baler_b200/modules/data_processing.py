@@ -118,6 +118,26 @@ def normalize(data, custom_norm):
     return out if arr.dtype == np.float32 else engine.host_convert(out, np.float64)
 
 
+def minmax_normalize_f64(data, normalise=True):
+    """precision "fp64" on a float64 table: ([min; max - min] exact in float64, the table normalised in float64 on the
+    device when `normalise`, else as it is) - what the reference's float64 numpy computes (data_processing.py:113-153),
+    bit for bit, with no float32 step and no host pass over the table"""
+    engine.require_cuda()
+    arr = np.asarray(data)
+    assert arr.dtype == np.float64
+    flat = np.ascontiguousarray(arr.reshape(arr.shape[0], -1) if arr.ndim > 1 else arr.reshape(-1, 1))
+    x = torch.from_numpy(flat).cuda()
+    mn, mx = engine.colminmax(x)
+    mn_h, mx_h = mn.cpu().numpy(), mx.cpu().numpy()
+    rg_h = mx_h - mn_h  # one float64 subtraction per column, as numpy
+    feats = np.array([mn_h, rg_h])
+    feats = feats.reshape((2,) + arr.shape[1:]) if arr.ndim > 1 else feats.reshape(2)
+    if not normalise:
+        return feats, arr
+    out = engine.normalize_table_f64(x, mn, torch.from_numpy(rg_h).cuda(), out=x)
+    return feats, out.cpu().numpy().reshape(arr.shape)
+
+
 def renormalize_std(input_data, true_min, feature_range):
     """reference data_processing.py:171-185 (one column)"""
     return renormalize_func(np.asarray(input_data).reshape(-1, 1), [true_min], [feature_range]).reshape(-1)

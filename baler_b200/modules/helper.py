@@ -24,7 +24,11 @@ class Config:
                        "fp64" computes in float64 like the reference's float64 models (its files to ~1e-15, integer
                        columns equal): dense models of <= 256 columns (AE, AE_Dropout_BN, CFD_dense_AE), float64 files
                        normalised in float64 on the device, float32 files in float32 as numpy does; not with
-                       save_error_bounded_deltas
+                       save_error_bounded_deltas.  "fp64" also governs --mode train: the float64 training step
+                       (float64 parameters, gradients and Adam state; the reference's training to ~1e-14) for AE and
+                       CFD_dense_AE of <= 100 columns with the MSE loss or l1_in_training, float64 files normalised in
+                       float64 on the device; AE_Dropout_BN, Conv_AE and loss_function_swae are refused.  The other
+                       values leave training on its default step (split16 tensor cores, fp32 for the L1 chain)
       latent_dtype     "float64" (AE default, what the reference writes; any model under "fp64") | "float32" | "float16"
       l1_in_training   bool: add reg_param * L1 chain to the training loss (dead code upstream, SURVEY F2)
     """
@@ -112,18 +116,27 @@ def renormalize(data, true_min_list, feature_range_list):
     return data_processing.renormalize_func(data, true_min_list, feature_range_list)
 
 
-def process(input_path, custom_norm, test_size, apply_normalization, convert_to_blocks, verbose):
-    """reference helper.py:277-319 -> (train_set, test_set, normalization_features, original_shape)"""
+def process(input_path, custom_norm, test_size, apply_normalization, convert_to_blocks, verbose, precision=None):
+    """reference helper.py:277-319 -> (train_set, test_set, normalization_features, original_shape).
+    `precision` (optional, not in the reference signature): "fp64" normalises a float64 file in float64 on the device,
+    bit-equal to the reference's numpy (float32 files stay float32-normalised, as upstream)."""
     data = np.load(input_path)["data"]
     if verbose:
         print("Original Dataset Shape - ", data.shape)
     original_shape = data.shape
     if convert_to_blocks:
         data = data_processing.convert_to_blocks_util(convert_to_blocks, data)
-    normalization_features = data_processing.find_minmax(data)
-    if apply_normalization:
-        print("Normalizing the data...")
-        data = normalize(data, custom_norm)
+    if training.is_fp64(precision):
+        engine.require_cuda()  # the float64 trainer, like every compute path, has no CPU fallback
+    if training.is_fp64(precision) and data.dtype == np.float64 and data.size:
+        if apply_normalization:
+            print("Normalizing the data...")
+        normalization_features, data = data_processing.minmax_normalize_f64(data, apply_normalization and not custom_norm)
+    else:
+        normalization_features = data_processing.find_minmax(data)
+        if apply_normalization:
+            print("Normalizing the data...")
+            data = normalize(data, custom_norm)
     if not test_size:
         train_set = test_set = data
     else:
@@ -131,6 +144,28 @@ def process(input_path, custom_norm, test_size, apply_normalization, convert_to_
 
         train_set, test_set = train_test_split(data, test_size=test_size, random_state=1)
     return train_set, test_set, normalization_features, original_shape
+
+
+def _npz_shape(path, key="data"):
+    """shape of array `key` of an .npz file from its header, without reading the array"""
+    import zipfile
+    with zipfile.ZipFile(path) as z, z.open(key + ".npy") as f:
+        version = np.lib.format.read_magic(f)
+        read = np.lib.format.read_array_header_1_0 if version == (1, 0) else np.lib.format.read_array_header_2_0
+        return read(f)[0]
+
+
+def refuse_fp64_training(config):
+    """--mode train with config.precision == "fp64": NotImplementedError naming what the float64 trainer does not take,
+    before any file is read or written (training.refuse_fp64_training).  True when "fp64" trains."""
+    if not training.is_fp64(getattr(config, "precision", None)):
+        return False
+    blocks = getattr(config, "convert_to_blocks", None)
+    shape = _npz_shape(config.input_path)
+    n_features = int(blocks[1]) * int(blocks[2]) if blocks else int(np.prod(shape[1:]))
+    training.refuse_fp64_training(config.model_name, n_features,
+                                  getattr(config, "custom_loss_function", None) == "loss_function_swae")
+    return True
 
 
 def train(model, number_of_columns, train_set, test_set, project_path, config):

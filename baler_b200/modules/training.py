@@ -12,6 +12,25 @@ from . import utils
 
 dist_env = sharded.dist_env
 FUSED_TRAINER_MAX_FEATURES = 100  # bb_trainer stages whole weight matrices in shared memory (widest: 200 x 100)
+FP64_TRAINING_MODELS = ("AE", "CFD_dense_AE")  # what precision "fp64" trains: the fused trainer's models without BatchNorm
+
+
+def is_fp64(precision):
+    return engine.PRECISIONS.get(precision or "auto") == engine.BB_PREC_FP64
+
+
+def refuse_fp64_training(model_name, n_features, swae=False):
+    """NotImplementedError naming what the float64 trainer (precision "fp64") does not take: models other than AE /
+    CFD_dense_AE (AE_Dropout_BN's BatchNorm, Conv_AE), loss_function_swae, rows wider than the fused trainer's"""
+    if model_name not in FP64_TRAINING_MODELS:
+        raise NotImplementedError("precision='fp64' trains %s only; %s is not trained in float64 (use another precision)"
+                                  % (" and ".join(FP64_TRAINING_MODELS), model_name))
+    if swae:
+        raise NotImplementedError("precision='fp64' trains with the MSE loss (and l1_in_training) only, not "
+                                  "custom_loss_function = 'loss_function_swae'")
+    if n_features > FUSED_TRAINER_MAX_FEATURES:
+        raise NotImplementedError("precision='fp64' trains models of at most %d columns (the fused trainer); %s has %d"
+                                  % (FUSED_TRAINER_MAX_FEATURES, model_name, n_features))
 
 
 def broadcast_initial_state(model):
@@ -42,9 +61,13 @@ class DeviceBatches:
 
 class DeviceAdam:
     """Stands in for torch.optim.Adam(model.parameters(), lr) (training.py:266): Adam state lives in
-    the bb_trainer; `lr` is what LRScheduler adjusts."""
+    the bb_trainer; `lr` is what LRScheduler adjusts.  precision "fp64": the float64 step of the fused trainer (AE /
+    CFD_dense_AE up to FUSED_TRAINER_MAX_FEATURES columns; refuse_fp64_training names what it does not take)."""
 
-    def __init__(self, model, lr, max_batch, l1=False, reg_param=0.0, dropout_seed=0, block_hw=None, swae=False):
+    def __init__(self, model, lr, max_batch, l1=False, reg_param=0.0, dropout_seed=0, block_hw=None, swae=False,
+                 precision=None):
+        if is_fp64(precision):
+            refuse_fp64_training(type(model).__name__, getattr(model, "n_features", 0), swae)
         self.rank, self.world = dist_env()
         broadcast_initial_state(model)
         self.model = model
@@ -64,6 +87,12 @@ class DeviceAdam:
             self.dp = sharded.DataParallelTrainer(self.trainer) if self.world > 1 else None
             return
         w, b = model.linear_tensors()
+        if is_fp64(precision):
+            # no layered fallback: the float64 step is the fused trainer's; data parallel all-reduces its float64 gradient
+            self.trainer = engine.Trainer(w, b, model.n_features, model.z_dim, max_batch)
+            self.trainer.set_precision("fp64")
+            self.dp = sharded.DataParallelTrainer(self.trainer, fused=False) if self.world > 1 else None
+            return
         if not swae and (self.has_bn or model.n_features <= FUSED_TRAINER_MAX_FEATURES):
             try:
                 self.trainer = engine.Trainer(w, b, model.n_features, model.z_dim, max_batch,
@@ -148,13 +177,16 @@ def validate(model, test_dl, model_children, reg_param, optimizer=None):
 
 
 def _to_device_table(data, config):
+    """the (normalised) table on the device: float32, or float64 as it is under precision "fp64" (the float64 step widens
+    a float32 table exactly, as the reference's torch.tensor(..., float64) does, training.py:230)"""
     arr = np.asarray(data)
+    dtype = np.float64 if is_fp64(getattr(config, "precision", None)) and arr.dtype == np.float64 else np.float32
     if config.data_dimension == 2:
         if config.model_type == "convolutional" and config.model_name != "Conv_AE":
             raise NotImplementedError("convolutional models other than Conv_AE: see DESIGN.md (out of scope)")
         # dense: (N, H * W) rows (training.py:195-204); Conv_AE: (N, 1, H, W) batches (:222-228), the same memory
         arr = arr.reshape(arr.shape[0], arr.shape[1] * arr.shape[2])
-    return torch.from_numpy(np.ascontiguousarray(arr, dtype=np.float32)).cuda()
+    return torch.from_numpy(np.ascontiguousarray(arr, dtype=dtype)).cuda()
 
 
 def train(model, variables, train_data, test_data, project_path, config):
@@ -178,7 +210,8 @@ def train(model, variables, train_data, test_data, project_path, config):
     optimizer = DeviceAdam(model, config.lr, max_batch=bs, l1=bool(getattr(config, "l1_in_training", False)),
                            reg_param=config.reg_param, dropout_seed=int(torch.initial_seed()) & 0x7FFFFFFFFFFFFFFF,
                            block_hw=tuple(np.asarray(train_data).shape[1:3]) if conv else None,
-                           swae=getattr(config, "custom_loss_function", None) == "loss_function_swae")
+                           swae=getattr(config, "custom_loss_function", None) == "loss_function_swae",
+                           precision=getattr(config, "precision", None))
     early_stopping = utils.EarlyStopping(config.early_stopping_patience, config.min_delta) if config.early_stopping else None
     lr_scheduler = utils.LRScheduler(optimizer, config.lr_scheduler_patience) if config.lr_scheduler else None
     train_loss, val_loss = [], []

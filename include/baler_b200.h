@@ -130,6 +130,11 @@ int bb_normalize_f32(bb_ctx* ctx, const float* x_dev, int64_t n_rows, int n_cols
                      const float* range_dev, float* out_dev, bb_stream_t stream);
 int bb_renormalize_f32(bb_ctx* ctx, const float* y_dev, int64_t n_rows, int n_cols, const float* min_dev,
                        const float* range_dev, float* out_dev, bb_stream_t stream);
+/* out = (x - min) / range on a row-major n x c float64 table: the reference's float64 numpy normalisation of a float64
+ * file (data_processing.py:133-153), one IEEE subtract and one IEEE divide per element, bit-equal to numpy (0 / 0 gives
+ * NaN as there).  `out_dev` may alias the input. */
+int bb_normalize_f64(bb_ctx* ctx, const double* x_dev, int64_t n_rows, int n_cols, const double* min_dev,
+                     const double* range_dev, double* out_dev, bb_stream_t stream);
 
 /*
  * z = encode((x - min) / range)  for n_rows rows of the row-major table x (n_rows x n_features).
@@ -262,6 +267,13 @@ int bb_trainer_destroy(bb_trainer* t);
  *                    kernel per epoch; the default (BB_PREC_AUTO) for `AE` / `CFD_dense_AE` / `AE_Dropout_BN` with the
  *                    MSE loss.
  *   BB_PREC_FP32     fp32 FFMA kernels; always used for the opt-in L1 chain.
+ *   BB_PREC_FP64     float64 DFMA kernels with float64 master parameters and Adam state: the reference's float64
+ *                    training to rounding (~1e-14), MSE and L1 chain.  Trainers of bb_trainer_create only
+ *                    (bb_trainer_create_dbn: BB_ERR_UNSUPPORTED), and only before the first step or epoch (later:
+ *                    BB_ERR_INVALID).  It uploads the float64 weights bb_trainer_create received, exactly.  The float32
+ *                    table entry points widen x exactly; the *_f64 ones below take float64 tables.  The in-kernel
+ *                    exchange (bb_trainer_dp_export / _connect) is not available: data parallel runs phase 1, an
+ *                    all-reduce of the float64 gradient (bb_trainer_grads_dev_f64) and phase 2.
  * bb_trainer_precision returns what the next MSE step will run on.  Values beyond +-65504 (un-normalised tables) leave
  * the fp16 range on the SPLIT16 path: the batch loss turns non-finite, a sticky flag is raised and
  * bb_trainer_range_flag reports it (synchronises the device); the caller restarts with BB_PREC_FP32.
@@ -284,7 +296,11 @@ int bb_trainer_profile(bb_trainer* t, int step, long long* out_host_128);
 int bb_trainer_param_count(const bb_trainer* t);
 float* bb_trainer_params_dev(bb_trainer* t);
 float* bb_trainer_grads_dev(bb_trainer* t);
-/* copy parameters back as the reference's float64 state_dict tensors */
+/* BB_PREC_FP64: the float64 master parameters and the float64 gradient (n_params entries, then the batch loss), same
+ * layout; NULL for the other precisions (the float32 views above keep their meaning and are not updated by fp64 steps) */
+double* bb_trainer_params_dev_f64(bb_trainer* t);
+double* bb_trainer_grads_dev_f64(bb_trainer* t);
+/* copy parameters back as the reference's float64 state_dict tensors (BB_PREC_FP64: the float64 master as it is) */
 int bb_trainer_get_params(bb_trainer* t, double* const* weights_host, double* const* biases_host);
 
 /*
@@ -325,6 +341,14 @@ int bb_trainer_epoch(bb_trainer* t, const float* x_dev, int64_t n_rows, int batc
  * (training.py:104-137) */
 int bb_trainer_validate(bb_trainer* t, const float* x_dev, int64_t n_rows, int batch,
                         double* epoch_loss_host, bb_stream_t stream);
+/* bb_trainer_step / _epoch / _validate on a float64 table (the reference's float64 training tensor, training.py:230):
+ * BB_PREC_FP64 trainers only (BB_ERR_INVALID otherwise) */
+int bb_trainer_step_f64(bb_trainer* t, const double* x_dev, int batch_rows, const bb_train_hyper* h,
+                        int phase, double* loss_accum_dev, bb_stream_t stream);
+int bb_trainer_epoch_f64(bb_trainer* t, const double* x_dev, int64_t n_rows, int batch,
+                         const bb_train_hyper* h, double* epoch_loss_host, bb_stream_t stream);
+int bb_trainer_validate_f64(bb_trainer* t, const double* x_dev, int64_t n_rows, int batch,
+                            double* epoch_loss_host, bb_stream_t stream);
 
 /*
  * Per-node mean activation of the six hidden layers (en1,en2,en3,de1,de2,de3) over the rows of the LAST
