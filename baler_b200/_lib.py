@@ -63,6 +63,9 @@ _SIGNATURES = {
     "bb_trainer_set_dropout": (C.c_int, [_P, C.c_uint64, _P]),
     "bb_trainer_get_bn": (C.c_int, [_P, _P, _P, _P, _P, _P]),
     "bb_trainer_bn_running_dev": (C.c_int, [_P, _PP, _PP, C.POINTER(C.c_int)]),
+    "bb_trainer_bn_running_dev_f64": (C.c_int, [_P, _PP, _PP, C.POINTER(C.c_int)]),
+    "bb_trainer_set_dropout_mt19937": (C.c_int, [_P, _P, C.c_int]),
+    "bb_trainer_get_dropout_mt19937": (C.c_int, [_P, _P, C.POINTER(C.c_int)]),
     "bb_trainer_destroy": (C.c_int, [_P]),
     "bb_trainer_set_precision": (C.c_int, [_P, C.c_int]),
     "bb_trainer_precision": (C.c_int, [_P]),

@@ -366,12 +366,7 @@ struct DbnArgs {
 
 __device__ __forceinline__ bool dropout_keep(const DbnArgs& a, const int l, const int grow, const int j, const int N) {
   if (a.mask[l] != nullptr) return a.mask[l][(size_t)grow * N + j] != 0;
-  // Philox4x32-10 keyed by (seed, step), counter (column / 4, row, layer): stateless, any launch geometry
-  const uint4 r = curand_Philox4x32_10(make_uint4((unsigned)(j >> 2), (unsigned)grow, (unsigned)l, (unsigned)a.step),
-                                       make_uint2((unsigned)a.seed, (unsigned)(a.seed >> 32) ^ (unsigned)(a.step >> 32)));
-  const unsigned v = (j & 3) == 0 ? r.x : (j & 3) == 1 ? r.y : (j & 3) == 2 ? r.z : r.w;
-  const float keep_p[4] = {0.5f, 0.6f, 0.7f, 0.8f};  // 1 - p of models.py:263-275
-  return v < (unsigned)(keep_p[l] * 4294967296.0);
+  return bb_philox_keep(a.seed, a.step, l, grow, j);
 }
 
 __global__ void __launch_bounds__(NT_FB)
@@ -727,6 +722,8 @@ struct bb_trainer {
   // bb_trainer_set_precision from the float64 weights bb_trainer_create received (kept here until then)
   F64Trainer* f64 = nullptr;
   std::vector<double> params_host;
+  std::vector<double> bn_stats_host;  // AE_Dropout_BN: float64 running_mean then running_var (bn_f_total each)
+  long long nbt_host[4] = {0, 0, 0, 0};
   bool started = false;              // a step or an epoch has run (the precision of a float64 run is fixed from then on)
 };
 
@@ -813,8 +810,31 @@ int bb_trainer_set_dropout(bb_trainer* t, unsigned long long seed, const unsigne
   if (!t || t->kind != 1) return BB_ERR_INVALID;
   t->seed = seed;
   for (int i = 0; i < 4; ++i) t->mask_dev[i] = masks_dev ? masks_dev[i] : nullptr;
+  if (t->f64) {
+    const int rc = bb_f64_train_set_dropout(t->f64, seed, masks_dev);
+    if (rc != BB_OK) return rc;
+  }
   if (t->tc) return bb_tc_train_set_dropout(t->tc, seed, masks_dev);
   return BB_OK;
+}
+
+int bb_trainer_set_dropout_mt19937(bb_trainer* t, const uint32_t* key_624, int pos) {
+  if (!t || t->kind != 1 || !key_624) return BB_ERR_INVALID;
+  if (t->precision != BB_PREC_FP64) return BB_ERR_UNSUPPORTED;
+  return bb_f64_train_set_mt19937(t->f64, key_624, pos);
+}
+
+int bb_trainer_get_dropout_mt19937(bb_trainer* t, uint32_t* key_out_624, int* pos_out) {
+  if (!t || t->kind != 1 || !key_out_624 || !pos_out) return BB_ERR_INVALID;
+  if (t->precision != BB_PREC_FP64) return BB_ERR_UNSUPPORTED;
+  return bb_f64_train_get_mt19937(t->f64, key_out_624, pos_out);
+}
+
+int bb_trainer_bn_running_dev_f64(bb_trainer* t, double** running_mean_dev, double** running_var_dev, int* n) {
+  if (!t || t->kind != 1 || !running_mean_dev || !running_var_dev || !n) return BB_ERR_INVALID;
+  if (t->precision != BB_PREC_FP64) return BB_ERR_UNSUPPORTED;
+  *n = t->d.bn_f_total;
+  return bb_f64_train_bn_running(t->f64, running_mean_dev, running_var_dev);
 }
 
 int bb_trainer_bn_running_dev(bb_trainer* t, float** running_mean_dev, float** running_var_dev, int* n) {
@@ -827,6 +847,20 @@ int bb_trainer_get_bn(bb_trainer* t, double* const* bn_weight_host, double* cons
                       double* const* bn_mean_host, double* const* bn_var_host, long long* bn_batches_tracked) {
   if (!t || t->kind != 1 || !bn_weight_host || !bn_bias_host || !bn_mean_host || !bn_var_host || !bn_batches_tracked)
     return BB_ERR_INVALID;
+  if (t->precision == BB_PREC_FP64) {  // the float64 master as it is
+    std::vector<double> hp(t->d.n_params), hm(t->d.bn_f_total), hv(t->d.bn_f_total);
+    int rc = bb_f64_train_get_params(t->f64, hp.data());
+    if (rc == BB_OK) rc = bb_f64_train_get_bn_stats(t->f64, hm.data(), hv.data(), bn_batches_tracked);
+    if (rc != BB_OK) return rc;
+    for (int i = 0; i < 4; ++i) {
+      const int n = t->d.dims[5 + i];
+      memcpy(bn_weight_host[i], hp.data() + t->d.bn_g_off[i], sizeof(double) * n);
+      memcpy(bn_bias_host[i], hp.data() + t->d.bn_b_off[i], sizeof(double) * n);
+      memcpy(bn_mean_host[i], hm.data() + t->d.bn_f_off[i], sizeof(double) * n);
+      memcpy(bn_var_host[i], hv.data() + t->d.bn_f_off[i], sizeof(double) * n);
+    }
+    return BB_OK;
+  }
   std::vector<float> hp(t->d.n_params), hm(t->d.bn_f_total), hv(t->d.bn_f_total);
   BB_CUDA(cudaMemcpy(hp.data(), t->params, sizeof(float) * hp.size(), cudaMemcpyDeviceToHost));
   BB_CUDA(cudaMemcpy(hm.data(), t->rm, sizeof(float) * hm.size(), cudaMemcpyDeviceToHost));
@@ -925,12 +959,23 @@ int create_common(bb_ctx* ctx, int n_features, int z_dim, const double* const* w
       hnbt[i] = bn_nbt ? bn_nbt[i] : 0;
     }
   }
-  if (kind == 0) {
-    t->params_host.assign(p, 0.0);
-    for (int l = 0; l < NL; ++l) {
-      const int K = dims[l], N = dims[l + 1];
-      for (int i = 0; i < N * K; ++i) t->params_host[d.w_off[l] + i] = weights_host[l][i];
-      for (int n = 0; n < N; ++n) t->params_host[d.b_off[l] + n] = biases_host[l][n];
+  // float64 copies of what create received, for bb_trainer_set_precision(BB_PREC_FP64)
+  t->params_host.assign(p, 0.0);
+  for (int l = 0; l < NL; ++l) {
+    const int K = dims[l], N = dims[l + 1];
+    for (int i = 0; i < N * K; ++i) t->params_host[d.w_off[l] + i] = weights_host[l][i];
+    for (int n = 0; n < N; ++n) t->params_host[d.b_off[l] + n] = biases_host[l][n];
+  }
+  if (kind == 1) {
+    t->bn_stats_host.assign(2 * (size_t)d.bn_f_total, 0.0);
+    for (int i = 0; i < 4; ++i) {
+      for (int j = 0; j < dims[5 + i]; ++j) {
+        t->params_host[d.bn_g_off[i] + j] = bn_gamma[i][j];
+        t->params_host[d.bn_b_off[i] + j] = bn_beta[i][j];
+        t->bn_stats_host[d.bn_f_off[i] + j] = bn_mean[i][j];
+        t->bn_stats_host[d.bn_f_total + d.bn_f_off[i] + j] = bn_var[i][j];
+      }
+      t->nbt_host[i] = hnbt[i];
     }
   }
   t->n_tiles = (int)tiles.size();
@@ -1015,7 +1060,6 @@ int bb_trainer_destroy(bb_trainer* t) {
 int bb_trainer_set_precision(bb_trainer* t, int precision) {
   if (!t) return BB_ERR_INVALID;
   if (precision == BB_PREC_FP64) {
-    if (t->kind != 0) return BB_ERR_UNSUPPORTED;
     if (t->started) return BB_ERR_INVALID;
     if (!t->f64) {
       F64TrainLayout fl;
@@ -1028,9 +1072,21 @@ int bb_trainer_set_precision(bb_trainer* t, int precision) {
       memcpy(fl.a_off, d.a_off, sizeof(fl.a_off));
       memcpy(fl.z_off, d.z_off, sizeof(fl.z_off));
       fl.a_stride = d.a_stride; fl.z_stride = d.z_stride; fl.n_params = d.n_params; fl.max_dim = d.max_dim;
+      fl.kind = t->kind;
+      memcpy(fl.bn_g_off, d.bn_g_off, sizeof(fl.bn_g_off));
+      memcpy(fl.bn_b_off, d.bn_b_off, sizeof(fl.bn_b_off));
+      memcpy(fl.bn_f_off, d.bn_f_off, sizeof(fl.bn_f_off));
+      fl.bn_f_total = d.bn_f_total;
+      if (t->kind == 1) fl.act[3] = BB_ACT_LEAKY;  // AE_Dropout_BN activates the latent too (models.py:273-275)
       BB_CUDA(cudaSetDevice(t->ctx->device));
-      const int rc = bb_f64_train_create(t->ctx, fl, t->params_host.data(), t->max_batch, &t->f64);
-      if (rc != BB_OK) return rc;
+      int rc = bb_f64_train_create(t->ctx, fl, t->params_host.data(), t->kind == 1 ? t->bn_stats_host.data() : nullptr,
+                                   t->nbt_host, t->max_batch, &t->f64);
+      if (rc == BB_OK && t->kind == 1) rc = bb_f64_train_set_dropout(t->f64, t->seed, t->mask_dev);
+      if (rc != BB_OK) {
+        bb_f64_train_destroy(t->f64);
+        t->f64 = nullptr;
+        return rc;
+      }
     }
     t->precision = BB_PREC_FP64;
     return BB_OK;

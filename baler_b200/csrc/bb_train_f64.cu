@@ -28,6 +28,8 @@
 #include <cstring>
 #include <new>
 
+#include <cooperative_groups.h>
+
 #include "bb_train_f64.cuh"
 
 namespace {
@@ -287,6 +289,282 @@ train_fwd_bwd_f64_kernel(const __grid_constant__ F64TrainLayout d, const double*
   }
 }
 
+// ------------------------------------------------------------------------------------------------ AE_Dropout_BN
+// reference baler/modules/models.py:256-313 in float64, in torch's arithmetic:
+//   encoder 4 x (Linear -> Dropout(p = .5,.4,.3,.2) -> LeakyReLU)   [activation also on the latent]
+//   decoder 3 x (Linear -> LeakyReLU -> BatchNorm1d) + Linear -> BatchNorm1d -> ReLU
+// Dropout multiplies by the noise torch builds, bernoulli / (1 - p): 0 or the rounded float64 1 / (1 - p), in the
+// forward and the backward pass.  BatchNorm in train mode normalises with the statistics of the whole batch (biased
+// variance, eps 1e-5) and updates the float64 running statistics as torch does (momentum 0.1, unbiased variance).
+// The batch is spread over CTAs of RT rows, so the kernel is launched cooperatively; the statistics are two passes
+// (the mean, then the sum of squared deviations: no E[x^2] - mean^2 cancellation), each a per-CTA partial sum combined
+// in CTA order after a grid-wide barrier, so a run is reproducible.  The backward pass needs one more barrier per
+// BatchNorm for the batch sums of dy and dy * xhat; gamma / beta gradients are those totals.
+struct F64DbnArgs {
+  const void* x;
+  int x_is_f64, batch_rows;
+  int mode;                      // 0: train forward + backward, 1: eval forward (no dropout, running statistics), loss only
+  double* act_g;
+  double* dz_g;
+  double* loss_part;
+  double* bn_part;               // [12 slots][gridDim.x][2 * max_dim] partial sums
+  double* rm;                    // running mean / var, bn_f_total each
+  double* rv;
+  long long* nbt;                // num_batches_tracked[4]
+  double* bn_grad;               // split 0 of the gradient partials (the BatchNorm gamma / beta gradients land there)
+  const unsigned char* mask[4];  // keep-masks [batch][N_l] (injected, or drawn from torch's stream) or nullptr (Philox)
+  unsigned long long seed, step;
+  double keep_scale[4];          // 1 / (1 - p) rounded, what noise.div_(1 - p) leaves in a kept element
+};
+
+__device__ __forceinline__ bool dbn_keep(const F64DbnArgs& a, int l, int grow, int j, int N) {
+  if (a.mask[l] != nullptr) return a.mask[l][(size_t)grow * N + j] != 0;
+  return bb_philox_keep(a.seed, a.step, l, grow, j);
+}
+
+// sum over the CTAs, in CTA order, of entry j of this barrier slot's partials
+__device__ __forceinline__ double cta_total(const double* slot, int n_cta, int stride, int j) {
+  double s = 0.0;
+  for (int c = 0; c < n_cta; ++c) s = __dadd_rn(s, __ldcg(slot + (size_t)c * stride + j));
+  return s;
+}
+
+__global__ void __launch_bounds__(NT_FB)
+train_dbn_f64_kernel(const __grid_constant__ F64TrainLayout d, const double* __restrict__ params,
+                     const double* __restrict__ wt, const __grid_constant__ F64DbnArgs a) {
+  namespace cg = cooperative_groups;
+  cg::grid_group grid = cg::this_grid();
+  extern __shared__ __align__(16) double smem[];
+  __shared__ double warp_loss[NT_FB / 32];
+  double* act_s = smem;                                            // a_stride * RT
+  double* dz_s0 = act_s + d.a_stride * RT;                         // max_dim * RT
+  double* dz_s1 = dz_s0 + d.max_dim * RT;
+  double* red_s = dz_s1 + d.max_dim * RT;                          // max(max_dim, NT_FB) * RT
+  double* xhat_s = red_s + (d.max_dim > NT_FB ? d.max_dim : NT_FB) * RT;  // bn_f_total * RT: normalised BN inputs
+  double* u_s = xhat_s + d.bn_f_total * RT;                        // bn_f_total * RT: BN inputs
+  double* inv_s = u_s + d.bn_f_total * RT;                         // bn_f_total (+1): 1 / sqrt(var + eps)
+  double* tot_s = inv_s + ((d.bn_f_total + 1) & ~1);               // 2 * max_dim: batch mean / batch sums
+  const bool train = a.mode == 0;
+  Stream s;
+  s.ring = tot_s + 2 * d.max_dim;
+  s.stage_elems = (KC * d.max_dim + 2 + 1) & ~1;
+  s.n = 0;
+  s.next_p = 0; s.next_i0 = 0;
+  s.per_chain = train ? 2 * NL - 1 : NL;
+  s.total = s.per_chain;
+  issue_next(d, params, wt, s, 0);
+
+  const int B = a.batch_rows;
+  const int n_cta = gridDim.x;
+  const int slot = 2 * d.max_dim;
+  const int row0 = blockIdx.x * RT;
+  const int rows = min(RT, B - row0);
+  const int F = d.dims[0];
+  for (int o = threadIdx.x; o < RT * F; o += NT_FB) {
+    const int r = o / F, j = o - r * F;
+    double v = 0.0;
+    if (r < rows) {
+      const size_t e = (size_t)(row0 + r) * F + j;
+      v = a.x_is_f64 ? __ldg(reinterpret_cast<const double*>(a.x) + e) : (double)__ldg(reinterpret_cast<const float*>(a.x) + e);
+      a.act_g[(size_t)(row0 + r) * d.a_stride + j] = v;
+    }
+    act_s[j * RT + r] = v;
+  }
+  __syncthreads();
+
+  // ---------------- forward: encoder
+  for (int l = 0; l < 4; ++l) {
+    int K, N;
+    const double* src = pass_src(d, params, wt, l, K, N);
+    const int KP = gemv_f64(d, params, wt, s, src, act_s + d.a_off[l] * RT, K, N, red_s);
+    const double* bias = params + d.b_off[l];
+    double* out_s = act_s + d.a_off[l + 1] * RT;
+    for (int o = threadIdx.x; o < RT * N; o += NT_FB) {
+      const int r = o / N, j = o - r * N;
+      double v = __dadd_rn(red_sum(red_s, KP, N, r, j), __ldg(bias + j));
+      if (train && r < rows) v = __dmul_rn(v, dbn_keep(a, l, row0 + r, j, N) ? a.keep_scale[l] : 0.0);
+      v = act_fwd(v, BB_ACT_LEAKY);
+      out_s[j * RT + r] = v;
+      if (r < rows) a.act_g[(size_t)(row0 + r) * d.a_stride + d.a_off[l + 1] + j] = v;
+    }
+    __syncthreads();
+  }
+  // ---------------- forward: decoder with BatchNorm
+  for (int i = 0; i < 4; ++i) {
+    const int l = 4 + i, fo = d.bn_f_off[i];
+    int K, N;
+    const double* src = pass_src(d, params, wt, l, K, N);
+    const int KP = gemv_f64(d, params, wt, s, src, act_s + d.a_off[l] * RT, K, N, red_s);
+    const double* bias = params + d.b_off[l];
+    for (int o = threadIdx.x; o < RT * N; o += NT_FB) {
+      const int r = o / N, j = o - r * N;
+      double v = __dadd_rn(red_sum(red_s, KP, N, r, j), __ldg(bias + j));
+      if (i < 3) v = act_fwd(v, BB_ACT_LEAKY);
+      u_s[(fo + j) * RT + r] = r < rows ? v : 0.0;
+    }
+    __syncthreads();
+    if (train) {
+      double* part = a.bn_part + ((size_t)(2 * i) * n_cta + blockIdx.x) * slot;
+      for (int j = threadIdx.x; j < N; j += NT_FB) {
+        double s1 = 0.0;
+        for (int r = 0; r < rows; ++r) s1 = __dadd_rn(s1, u_s[(fo + j) * RT + r]);
+        part[j] = s1;
+      }
+      __threadfence();
+      grid.sync();
+      const double* all = a.bn_part + (size_t)(2 * i) * n_cta * slot;
+      for (int j = threadIdx.x; j < N; j += NT_FB) tot_s[j] = __ddiv_rn(cta_total(all, n_cta, slot, j), (double)B);
+      __syncthreads();
+      part = a.bn_part + ((size_t)(2 * i + 1) * n_cta + blockIdx.x) * slot;
+      for (int j = threadIdx.x; j < N; j += NT_FB) {
+        double s2 = 0.0;
+        for (int r = 0; r < rows; ++r) {
+          const double dv = __dsub_rn(u_s[(fo + j) * RT + r], tot_s[j]);
+          s2 = __dadd_rn(s2, __dmul_rn(dv, dv));
+        }
+        part[j] = s2;
+      }
+      __threadfence();
+      grid.sync();
+      all = a.bn_part + (size_t)(2 * i + 1) * n_cta * slot;
+      for (int j = threadIdx.x; j < N; j += NT_FB) {
+        const double m2 = cta_total(all, n_cta, slot, j);
+        inv_s[fo + j] = __ddiv_rn(1.0, __dsqrt_rn(__dadd_rn(__ddiv_rn(m2, (double)B), 1e-5)));
+        if (blockIdx.x == 0) {  // running statistics: momentum * batch + (1 - momentum) * running, unbiased variance
+          const double unbiased = __ddiv_rn(m2, (double)(B > 1 ? B - 1 : 1));
+          a.rm[fo + j] = __dadd_rn(__dmul_rn(0.1, tot_s[j]), __dmul_rn(1.0 - 0.1, a.rm[fo + j]));
+          a.rv[fo + j] = __dadd_rn(__dmul_rn(0.1, unbiased), __dmul_rn(1.0 - 0.1, a.rv[fo + j]));
+          if (j == 0) a.nbt[i] += 1;
+        }
+      }
+    } else {
+      for (int j = threadIdx.x; j < N; j += NT_FB) {
+        tot_s[j] = a.rm[fo + j];
+        inv_s[fo + j] = __ddiv_rn(1.0, __dsqrt_rn(__dadd_rn(a.rv[fo + j], 1e-5)));
+      }
+    }
+    __syncthreads();
+    const double* gam = params + d.bn_g_off[i];
+    const double* bet = params + d.bn_b_off[i];
+    double* out_s = act_s + d.a_off[l + 1] * RT;
+    for (int o = threadIdx.x; o < RT * N; o += NT_FB) {
+      const int r = o / N, j = o - r * N;
+      const double xh = __dmul_rn(__dsub_rn(u_s[(fo + j) * RT + r], tot_s[j]), inv_s[fo + j]);
+      double h = __dadd_rn(__dmul_rn(xh, __ldg(gam + j)), __ldg(bet + j));
+      if (i == 3) h = act_fwd(h, BB_ACT_RELU);
+      xhat_s[(fo + j) * RT + r] = xh;
+      out_s[j * RT + r] = h;
+      if (r < rows && l + 1 < NL) a.act_g[(size_t)(row0 + r) * d.a_stride + d.a_off[l + 1] + j] = h;
+    }
+    __syncthreads();
+  }
+  // ---------------- loss and the seed gradient (through the final ReLU)
+  double loss_local = 0.0;
+  double* dz_cur = dz_s0;
+  double* dz_nxt = dz_s1;
+  {
+    const double* out_s = act_s + d.a_off[NL] * RT;
+    for (int o = threadIdx.x; o < RT * F; o += NT_FB) {
+      const int r = o / F, j = o - r * F;
+      double g = 0.0;
+      if (r < rows) {
+        const double rec = out_s[j * RT + r];
+        const double diff = __dsub_rn(rec, act_s[j * RT + r]);
+        loss_local = __dadd_rn(loss_local, __ddiv_rn(__dmul_rn(diff, diff), (double)F));
+        g = rec > 0.0 ? __ddiv_rn(__dmul_rn(2.0, diff), (double)F) : 0.0;
+      }
+      dz_cur[j * RT + r] = g;
+    }
+    __syncthreads();
+  }
+  if (train) {
+    // ---------------- backward: decoder (dz_cur = gradient w.r.t. the BatchNorm output)
+    for (int i = 3; i >= 0; --i) {
+      const int l = 4 + i, fo = d.bn_f_off[i];
+      const int N = d.dims[l + 1];
+      double* part = a.bn_part + ((size_t)(8 + 3 - i) * n_cta + blockIdx.x) * slot;
+      for (int j = threadIdx.x; j < N; j += NT_FB) {
+        double t1 = 0.0, t2 = 0.0;
+        for (int r = 0; r < rows; ++r) {
+          const double g = dz_cur[j * RT + r];
+          t1 = __dadd_rn(t1, g);
+          t2 = __dadd_rn(t2, __dmul_rn(g, xhat_s[(fo + j) * RT + r]));
+        }
+        part[j] = t1; part[N + j] = t2;
+      }
+      __threadfence();
+      grid.sync();
+      const double* all = a.bn_part + (size_t)(8 + 3 - i) * n_cta * slot;
+      for (int j = threadIdx.x; j < N; j += NT_FB) {
+        const double T1 = cta_total(all, n_cta, slot, j), T2 = cta_total(all, n_cta, slot, N + j);
+        tot_s[j] = __ddiv_rn(T1, (double)B);
+        tot_s[d.max_dim + j] = __ddiv_rn(T2, (double)B);
+        if (blockIdx.x == 0) { a.bn_grad[d.bn_b_off[i] + j] = T1; a.bn_grad[d.bn_g_off[i] + j] = T2; }
+      }
+      __syncthreads();
+      const double* gam = params + d.bn_g_off[i];
+      for (int o = threadIdx.x; o < RT * N; o += NT_FB) {
+        const int r = o / N, j = o - r * N;
+        // torch's batch-norm backward: dx = (dy - mean(dy) - xhat * mean(dy * xhat)) * invstd * gamma
+        double dx = __dsub_rn(__dsub_rn(dz_cur[j * RT + r], tot_s[j]), __dmul_rn(xhat_s[(fo + j) * RT + r], tot_s[d.max_dim + j]));
+        dx = __dmul_rn(__dmul_rn(dx, inv_s[fo + j]), __ldg(gam + j));
+        if (i < 3 && !(u_s[(fo + j) * RT + r] > 0.0)) dx = __dmul_rn(dx, 0.01);
+        if (r >= rows) dx = 0.0;
+        dz_nxt[j * RT + r] = dx;
+        if (r < rows) a.dz_g[(size_t)(row0 + r) * d.z_stride + d.z_off[l] + j] = dx;
+      }
+      __syncthreads();
+      {  // dX = dZ W_l: the gradient w.r.t. the output of the previous block
+        int Nn, K;
+        const double* src = pass_src(d, params, wt, 2 * NL - 1 - l, Nn, K);
+        const int KP = gemv_f64(d, params, wt, s, src, dz_nxt, Nn, K, red_s);
+        for (int o = threadIdx.x; o < RT * K; o += NT_FB) {
+          const int r = o / K, j = o - r * K;
+          dz_cur[j * RT + r] = red_sum(red_s, KP, K, r, j);
+        }
+        __syncthreads();
+      }
+    }
+    // ---------------- backward: encoder (dz_cur = gradient w.r.t. the output of encoder layer l)
+    for (int l = 3; l >= 0; --l) {
+      const int N = d.dims[l + 1];
+      const double* a_out = act_s + d.a_off[l + 1] * RT;
+      for (int o = threadIdx.x; o < RT * N; o += NT_FB) {
+        const int r = o / N, j = o - r * N;
+        double g = 0.0;
+        if (r < rows) {
+          g = dz_cur[j * RT + r];
+          if (!(a_out[j * RT + r] > 0.0)) g = __dmul_rn(g, 0.01);
+          g = __dmul_rn(g, dbn_keep(a, l, row0 + r, j, N) ? a.keep_scale[l] : 0.0);
+          a.dz_g[(size_t)(row0 + r) * d.z_stride + d.z_off[l] + j] = g;
+        }
+        dz_nxt[j * RT + r] = g;
+      }
+      __syncthreads();
+      if (l >= 1) {
+        int Nn, K;
+        const double* src = pass_src(d, params, wt, 2 * NL - 1 - l, Nn, K);
+        const int KP = gemv_f64(d, params, wt, s, src, dz_nxt, Nn, K, red_s);
+        for (int o = threadIdx.x; o < RT * K; o += NT_FB) {
+          const int r = o / K, j = o - r * K;
+          dz_cur[j * RT + r] = red_sum(red_s, KP, K, r, j);
+        }
+        __syncthreads();
+      }
+    }
+  }
+  cp_async_wait_all();
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) loss_local = __dadd_rn(loss_local, __shfl_xor_sync(0xffffffffu, loss_local, off));
+  if ((threadIdx.x & 31) == 0) warp_loss[threadIdx.x >> 5] = loss_local;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double v = 0.0;
+    for (int w = 0; w < NT_FB / 32; ++w) v = __dadd_rn(v, warp_loss[w]);
+    a.loss_part[blockIdx.x] = v;
+  }
+}
+
 // partial[split][w_off[l] + n * K + k] = sum_{r in split} dZ_l[r][n] * A_l[r][k]  (+ the second chain), b likewise
 __global__ void __launch_bounds__(NT)
 train_dw_f64_kernel(const __grid_constant__ F64TrainLayout d, const Tile* __restrict__ tiles, const double* __restrict__ act_g,
@@ -406,18 +684,41 @@ struct F64Trainer {
   double *act_g = nullptr, *dz_g = nullptr, *partial = nullptr, *loss_part = nullptr;
   int* wt_index = nullptr;
   Tile* tiles = nullptr;
+  // AE_Dropout_BN
+  double *bn_part = nullptr, *rm = nullptr, *rv = nullptr;
+  long long* nbt = nullptr;
+  size_t dbn_smem = 0;
+  int dbn_max_ctas = 0;
+  const unsigned char* mask_dev[4] = {nullptr, nullptr, nullptr, nullptr};
+  unsigned long long seed = 0;
+  // torch's stream: the twister state (624 words + position) and two mask slots [rows][sum N_l] filled on a side stream
+  bool mt_armed = false;
+  uint32_t* mt_state = nullptr;
+  unsigned char* mt_slot[2] = {nullptr, nullptr};
+  cudaStream_t mt_stream = nullptr;
+  cudaEvent_t mt_ready[2] = {nullptr, nullptr}, mt_free[2] = {nullptr, nullptr};
+  long long mt_draws = 0;
 };
 
 void bb_f64_train_destroy(F64Trainer* f) {
   if (!f) return;
-  void* ptrs[] = {f->params, f->wt, f->grads, f->m, f->v, f->act_g, f->dz_g, f->partial, f->loss_part, f->wt_index, f->tiles};
+  if (f->mt_stream) cudaStreamSynchronize(f->mt_stream);
+  void* ptrs[] = {f->params, f->wt, f->grads, f->m, f->v, f->act_g, f->dz_g, f->partial, f->loss_part, f->wt_index, f->tiles,
+                  f->bn_part, f->rm, f->rv, f->nbt, f->mt_state, f->mt_slot[0], f->mt_slot[1]};
   for (void* p : ptrs)
     if (p) cudaFree(p);
+  for (int i = 0; i < 2; ++i) {
+    if (f->mt_ready[i]) cudaEventDestroy(f->mt_ready[i]);
+    if (f->mt_free[i]) cudaEventDestroy(f->mt_free[i]);
+  }
+  if (f->mt_stream) cudaStreamDestroy(f->mt_stream);
   delete f;
 }
 
-int bb_f64_train_create(bb_ctx* ctx, const F64TrainLayout& d, const double* params_host, int max_batch, F64Trainer** out) {
+int bb_f64_train_create(bb_ctx* ctx, const F64TrainLayout& d, const double* params_host, const double* bn_stats_host,
+                        const long long* nbt_host, int max_batch, F64Trainer** out) {
   if (!ctx || !params_host || !out || max_batch < 1) return BB_ERR_INVALID;
+  if (d.kind == 1 && (!bn_stats_host || !nbt_host)) return BB_ERR_INVALID;
   if (d.max_dim > NT_FB) return BB_ERR_UNSUPPORTED;
   const size_t stage = (size_t)((KC * d.max_dim + 2 + 1) & ~1);
   const size_t smem = ((size_t)(d.a_stride + 2 * d.max_dim + (d.max_dim > NT_FB ? d.max_dim : NT_FB)) * RT + 2 * stage) * sizeof(double);
@@ -469,8 +770,27 @@ int bb_f64_train_create(bb_ctx* ctx, const F64TrainLayout& d, const double* para
   if (rc == BB_OK) rc = (int)cudaMemset(f->m, 0, sizeof(double) * p);
   if (rc == BB_OK) rc = (int)cudaMemset(f->v, 0, sizeof(double) * p);
   if (rc == BB_OK) rc = (int)cudaMemset(f->grads, 0, sizeof(double) * (p + 1));
+  // the BatchNorm entries of splits > 0 stay zero: the dW kernel writes Linear entries only
+  if (rc == BB_OK) rc = (int)cudaMemset(f->partial, 0, sizeof(double) * (size_t)max_splits * p);
   if (rc == BB_OK)
     rc = (int)cudaFuncSetAttribute(train_fwd_bwd_f64_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (rc == BB_OK && d.kind == 1) {
+    const int nb = d.bn_f_total;
+    alloc((void**)&f->bn_part, sizeof(double) * 12 * (size_t)max_ctas * 2 * d.max_dim);
+    alloc((void**)&f->rm, sizeof(double) * nb);
+    alloc((void**)&f->rv, sizeof(double) * nb);
+    alloc((void**)&f->nbt, sizeof(long long) * 4);
+    if (rc == BB_OK) rc = (int)cudaMemcpy(f->rm, bn_stats_host, sizeof(double) * nb, cudaMemcpyHostToDevice);
+    if (rc == BB_OK) rc = (int)cudaMemcpy(f->rv, bn_stats_host + nb, sizeof(double) * nb, cudaMemcpyHostToDevice);
+    if (rc == BB_OK) rc = (int)cudaMemcpy(f->nbt, nbt_host, sizeof(long long) * 4, cudaMemcpyHostToDevice);
+    f->dbn_smem = smem + ((size_t)2 * nb * RT + ((nb + 1) & ~1) + 2 * d.max_dim) * sizeof(double);
+    if (rc == BB_OK && f->dbn_smem > ctx->smem_optin) rc = BB_ERR_UNSUPPORTED;
+    if (rc == BB_OK)
+      rc = (int)cudaFuncSetAttribute(train_dbn_f64_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)f->dbn_smem);
+    int per_sm = 0;
+    if (rc == BB_OK) rc = (int)cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, train_dbn_f64_kernel, NT_FB, f->dbn_smem);
+    f->dbn_max_ctas = per_sm * ctx->sm_count;
+  }
   if (rc == BB_OK) rc = (int)cudaDeviceSynchronize();
   if (rc != BB_OK) { bb_f64_train_destroy(f); return rc; }
   *out = f;
@@ -486,6 +806,50 @@ int launch_fwd(F64Trainer* f, const void* x, int x_is_f64, int rows, int backwar
                          f->wt, x, x_is_f64, rows, f->act_g, f->dz_g, (size_t)f->max_batch * f->d.a_stride,
                          (size_t)f->max_batch * f->d.z_stride, backward, h ? h->l1 : 0, reg_inv_rows, f->loss_part);
 }
+
+// the keep-masks of this batch from torch's stream: drawn on the side stream into the slot the step before last read
+int draw_mt(F64Trainer* f, int rows, const unsigned char** masks, cudaStream_t s) {
+  const int k = (int)(f->mt_draws & 1);
+  int widths[4], tot = 0;
+  unsigned char* out[4];
+  for (int l = 0; l < 4; ++l) {
+    widths[l] = f->d.dims[l + 1];
+    out[l] = f->mt_slot[k] + (size_t)rows * tot;
+    masks[l] = out[l];
+    tot += widths[l];
+  }
+  const double keep[4] = {1.0 - 0.5, 1.0 - 0.4, 1.0 - 0.3, 1.0 - 0.2};  // models.py:263-275
+  BB_CUDA(cudaStreamWaitEvent(f->mt_stream, f->mt_free[k], 0));
+  int rc = bb_mt_dropout_launch(f->mt_state, rows, widths, keep, out, f->mt_stream);
+  if (rc != BB_OK) return rc;
+  BB_CUDA(cudaEventRecord(f->mt_ready[k], f->mt_stream));
+  BB_CUDA(cudaStreamWaitEvent(s, f->mt_ready[k], 0));
+  ++f->mt_draws;
+  return BB_OK;
+}
+
+int launch_dbn(F64Trainer* f, const void* x, int x_is_f64, int rows, int mode, long long step, cudaStream_t s) {
+  const int grid = (rows + RT - 1) / RT;
+  if (grid > f->dbn_max_ctas) return BB_ERR_UNSUPPORTED;  // cooperative launch: every CTA must be resident
+  f->last_rows = rows;
+  F64DbnArgs a;
+  a.x = x; a.x_is_f64 = x_is_f64; a.batch_rows = rows; a.mode = mode;
+  a.act_g = f->act_g; a.dz_g = f->dz_g; a.loss_part = f->loss_part; a.bn_part = f->bn_part;
+  a.rm = f->rm; a.rv = f->rv; a.nbt = f->nbt; a.bn_grad = f->partial;
+  for (int i = 0; i < 4; ++i) a.mask[i] = f->mask_dev[i];
+  a.seed = f->seed; a.step = (unsigned long long)step;
+  const double p[4] = {0.5, 0.4, 0.3, 0.2};
+  for (int i = 0; i < 4; ++i) a.keep_scale[i] = 1.0 / (1.0 - p[i]);
+  const bool mt = mode == 0 && f->mt_armed;
+  if (mt) {
+    const int rc = draw_mt(f, rows, a.mask, s);
+    if (rc != BB_OK) return rc;
+  }
+  void* args[] = {(void*)&f->d, (void*)&f->params, (void*)&f->wt, (void*)&a};
+  BB_CUDA(cudaLaunchCooperativeKernel((const void*)train_dbn_f64_kernel, dim3(grid), dim3(NT_FB), args, f->dbn_smem, s));
+  if (mt) BB_CUDA(cudaEventRecord(f->mt_free[(f->mt_draws - 1) & 1], s));
+  return BB_OK;
+}
 }  // namespace
 
 int bb_f64_train_step(F64Trainer* f, const void* x_dev, int x_is_f64, int rows, const bb_train_hyper* h, int phase,
@@ -494,7 +858,14 @@ int bb_f64_train_step(F64Trainer* f, const void* x_dev, int x_is_f64, int rows, 
   const int p = f->d.n_params;
   const int n_splits = (rows + DW_T - 1) / DW_T;
   if (phase != 2) {
-    int rc = launch_fwd(f, x_dev, x_is_f64, rows, 1, h, s);
+    int rc;
+    if (f->d.kind == 1) {
+      // AE_Dropout_BN: MSE only; the Philox counter takes the step the kernel's update will be (bb_train.cu's t->step)
+      if (h->l1) return BB_ERR_UNSUPPORTED;
+      rc = launch_dbn(f, x_dev, x_is_f64, rows, 0, phase == 0 ? step - 1 : step, s);
+    } else {
+      rc = launch_fwd(f, x_dev, x_is_f64, rows, 1, h, s);
+    }
     if (rc != BB_OK) return rc;
     BB_CUDA(pdl_launch(train_dw_f64_kernel, dim3(f->n_tiles, n_splits), dim3(NT), 0, s, f->d, f->tiles, f->act_g, f->dz_g,
                        (size_t)f->max_batch * f->d.a_stride, (size_t)f->max_batch * f->d.z_stride, h->l1 ? 2 : 1, rows,
@@ -517,7 +888,7 @@ int bb_f64_train_step(F64Trainer* f, const void* x_dev, int x_is_f64, int rows, 
 
 int bb_f64_train_eval(F64Trainer* f, const void* x_dev, int x_is_f64, int rows, double* loss_accum_dev, cudaStream_t s) {
   if (!f || !x_dev || rows < 1 || rows > f->max_batch) return BB_ERR_INVALID;
-  int rc = launch_fwd(f, x_dev, x_is_f64, rows, 0, nullptr, s);
+  int rc = f->d.kind == 1 ? launch_dbn(f, x_dev, x_is_f64, rows, 1, 0, s) : launch_fwd(f, x_dev, x_is_f64, rows, 0, nullptr, s);
   if (rc != BB_OK) return rc;
   const AdamArgs a = {};
   // mode 1 with zero parameters only folds the loss partials into the gradient's loss slot ...
@@ -558,3 +929,63 @@ int bb_f64_train_get_params(F64Trainer* f, double* params_host) {
 
 double* bb_f64_train_params(F64Trainer* f) { return f ? f->params : nullptr; }
 double* bb_f64_train_grads(F64Trainer* f) { return f ? f->grads : nullptr; }
+
+int bb_f64_train_set_dropout(F64Trainer* f, unsigned long long seed, const unsigned char* const* masks_dev) {
+  if (!f || f->d.kind != 1) return BB_ERR_INVALID;
+  f->seed = seed;
+  for (int i = 0; i < 4; ++i) f->mask_dev[i] = masks_dev ? masks_dev[i] : nullptr;
+  f->mt_armed = false;
+  return BB_OK;
+}
+
+int bb_f64_train_set_mt19937(F64Trainer* f, const uint32_t* key_624, int pos) {
+  if (!f || f->d.kind != 1 || !key_624 || pos < 0 || pos > 624) return BB_ERR_INVALID;
+  int rc = BB_OK;
+  if (!f->mt_stream) {
+    rc = (int)cudaStreamCreateWithFlags(&f->mt_stream, cudaStreamNonBlocking);
+    for (int i = 0; i < 2 && rc == BB_OK; ++i) {
+      rc = (int)cudaEventCreateWithFlags(&f->mt_ready[i], cudaEventDisableTiming);
+      if (rc == BB_OK) rc = (int)cudaEventCreateWithFlags(&f->mt_free[i], cudaEventDisableTiming);
+    }
+    size_t per_row = 0;
+    for (int l = 0; l < 4; ++l) per_row += f->d.dims[l + 1];
+    if (rc == BB_OK) rc = (int)cudaMalloc((void**)&f->mt_state, sizeof(uint32_t) * 625);
+    for (int i = 0; i < 2 && rc == BB_OK; ++i) rc = (int)cudaMalloc((void**)&f->mt_slot[i], per_row * f->max_batch);
+    if (rc != BB_OK) return rc;
+  }
+  uint32_t h[625];
+  memcpy(h, key_624, sizeof(uint32_t) * 624);
+  h[624] = (uint32_t)pos;
+  BB_CUDA(cudaMemcpyAsync(f->mt_state, h, sizeof(h), cudaMemcpyHostToDevice, f->mt_stream));
+  BB_CUDA(cudaStreamSynchronize(f->mt_stream));
+  for (int i = 0; i < 4; ++i) f->mask_dev[i] = nullptr;
+  f->mt_armed = true;
+  return BB_OK;
+}
+
+int bb_f64_train_get_mt19937(F64Trainer* f, uint32_t* key_624, int* pos) {
+  if (!f || !key_624 || !pos) return BB_ERR_INVALID;
+  if (!f->mt_armed) return BB_ERR_INVALID;
+  uint32_t h[625];
+  BB_CUDA(cudaMemcpyAsync(h, f->mt_state, sizeof(h), cudaMemcpyDeviceToHost, f->mt_stream));
+  BB_CUDA(cudaStreamSynchronize(f->mt_stream));
+  memcpy(key_624, h, sizeof(uint32_t) * 624);
+  *pos = (int)h[624];
+  return BB_OK;
+}
+
+int bb_f64_train_bn_running(F64Trainer* f, double** rm_dev, double** rv_dev) {
+  if (!f || f->d.kind != 1 || !rm_dev || !rv_dev) return BB_ERR_INVALID;
+  *rm_dev = f->rm; *rv_dev = f->rv;
+  return BB_OK;
+}
+
+int bb_f64_train_get_bn_stats(F64Trainer* f, double* rm_host, double* rv_host, long long* nbt_host) {
+  if (!f || f->d.kind != 1 || !rm_host || !rv_host || !nbt_host) return BB_ERR_INVALID;
+  BB_CUDA(cudaMemcpy(rm_host, f->rm, sizeof(double) * f->d.bn_f_total, cudaMemcpyDeviceToHost));
+  BB_CUDA(cudaMemcpy(rv_host, f->rv, sizeof(double) * f->d.bn_f_total, cudaMemcpyDeviceToHost));
+  BB_CUDA(cudaMemcpy(nbt_host, f->nbt, sizeof(long long) * 4, cudaMemcpyDeviceToHost));
+  return BB_OK;
+}
+
+int bb_f64_train_dbn_max_ctas(F64Trainer* f) { return f ? f->dbn_max_ctas : 0; }

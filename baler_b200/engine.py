@@ -312,6 +312,34 @@ class DenseCodec:
         return y
 
 
+# torch's CPU generator state (torch.Generator.get_state(), 5056 bytes): the MT19937 engine as
+# {uint64 seed, int32 left, int32 seeded, uint64 next, uint64 state[624]} followed by the cached normal samples.
+# The next word is state[next] unless left == 1, when the engine twists first: numpy's position 624 - (left - 1).
+_MT_LEFT, _MT_NEXT, _MT_KEY = 8, 16, 24
+_MT_STATE_BYTES = 5056
+
+
+def mt19937_from_torch_state(blob):
+    """(key uint32[624], position 0..624) of a torch CPU generator state"""
+    b = blob.numpy().tobytes()
+    if len(b) != _MT_STATE_BYTES:
+        raise ValueError("not a torch CPU generator state (%d bytes, expected %d)" % (len(b), _MT_STATE_BYTES))
+    left = int(np.frombuffer(b, np.int32, 1, _MT_LEFT)[0])
+    key = np.frombuffer(b, np.uint64, 624, _MT_KEY).astype(np.uint32)
+    return key, 624 - (left - 1)
+
+
+def mt19937_to_torch_state(blob, key, pos):
+    """`blob` with its MT19937 key and position replaced (everything else, e.g. the seed and the normal cache, kept)"""
+    b = bytearray(blob.numpy().tobytes())
+    if len(b) != _MT_STATE_BYTES or not 0 <= pos <= 624:
+        raise ValueError("bad torch CPU generator state or position")
+    b[_MT_LEFT:_MT_LEFT + 4] = np.int32(625 - pos).tobytes()
+    b[_MT_NEXT:_MT_NEXT + 8] = np.uint64(pos % 624).tobytes()
+    b[_MT_KEY:_MT_KEY + 8 * 624] = np.asarray(key, dtype=np.uint32).astype(np.uint64).tobytes()
+    return torch.frombuffer(b, dtype=torch.uint8).clone()
+
+
 class Trainer:
     """bb_trainer: parameters, Adam state and scratch of one dense-AE training run on one GPU."""
 
@@ -360,8 +388,9 @@ class Trainer:
 
     def set_precision(self, precision):
         """"auto" / "split16": tensor-core step (AE family, MSE loss); "fp32": the fp32 FFMA kernels; "fp64": the float64
-        kernels with float64 master parameters (AE / CFD_dense_AE, before the first step; params_view / grads_view are
-        float64 from then on, step / epoch / validate take float32 or float64 tables)"""
+        kernels with float64 master parameters (before the first step; params_view / grads_view / bn_running_views are
+        float64 from then on, step / epoch / validate take float32 or float64 tables).  AE_Dropout_BN under "fp64": batches
+        up to 4 rows x resident CTAs (592 on a B200), dropout from Philox, injected masks or set_dropout_torch"""
         check(_lib.lib().bb_trainer_set_precision(self.handle, _prec(precision)), "bb_trainer_set_precision")
 
     @property
@@ -450,8 +479,25 @@ class Trainer:
     def bn_running_views(self):
         """AE_Dropout_BN: zero-copy views (running_mean, running_var) of the concatenated BatchNorm buffers"""
         rm, rv, n = C.c_void_p(), C.c_void_p(), C.c_int()
-        check(_lib.lib().bb_trainer_bn_running_dev(self.handle, C.byref(rm), C.byref(rv), C.byref(n)), "bb_trainer_bn_running_dev")
-        return self._flat(rm.value, n.value), self._flat(rv.value, n.value)
+        name, typestr = ("bb_trainer_bn_running_dev_f64", "<f8") if self._fp64 else ("bb_trainer_bn_running_dev", "<f4")
+        check(getattr(_lib.lib(), name)(self.handle, C.byref(rm), C.byref(rv), C.byref(n)), name)
+        return self._flat(rm.value, n.value, typestr), self._flat(rv.value, n.value, typestr)
+
+    def set_dropout_torch(self, generator=None):
+        """AE_Dropout_BN under "fp64": the following steps draw their dropout masks on the device from `generator`'s
+        Mersenne Twister (torch's default CPU generator when None) exactly as the reference's bernoulli_ calls would;
+        write_back_dropout_torch() then leaves the generator where the reference's would be"""
+        self._torch_gen = torch.default_generator if generator is None else generator
+        key, pos = mt19937_from_torch_state(self._torch_gen.get_state())
+        check(_lib.lib().bb_trainer_set_dropout_mt19937(self.handle, key.ctypes.data, pos), "bb_trainer_set_dropout_mt19937")
+
+    def write_back_dropout_torch(self):
+        """set the generator of set_dropout_torch to the device's state after the last drawn word (synchronises)"""
+        key = np.empty(624, dtype=np.uint32)
+        pos = C.c_int()
+        check(_lib.lib().bb_trainer_get_dropout_mt19937(self.handle, key.ctypes.data, C.byref(pos)),
+              "bb_trainer_get_dropout_mt19937")
+        self._torch_gen.set_state(mt19937_to_torch_state(self._torch_gen.get_state(), key, pos.value))
 
     def get_bn(self):
         out = {k: [np.empty_like(a) for a in self._bn[k]] for k in ("weight", "bias", "running_mean", "running_var")}

@@ -27,8 +27,15 @@ class Config:
                        save_error_bounded_deltas.  "fp64" also governs --mode train: the float64 training step
                        (float64 parameters, gradients and Adam state; the reference's training to ~1e-14) for AE and
                        CFD_dense_AE of <= 100 columns with the MSE loss or l1_in_training, float64 files normalised in
-                       float64 on the device; AE_Dropout_BN, Conv_AE and loss_function_swae are refused.  The other
-                       values leave training on its default step (split16 tensor cores, fp32 for the L1 chain)
+                       float64 on the device; AE_Dropout_BN with dropout_stream = "torch" (below); Conv_AE and
+                       loss_function_swae are refused.  The other values leave training on its default step (split16
+                       tensor cores, fp32 for the L1 chain)
+      dropout_stream   "torch": AE_Dropout_BN under precision "fp64" draws its dropout masks on the device from torch's
+                       default CPU generator, exactly the masks the reference's run draws, and leaves the generator where
+                       the reference's would be: the float64 run then reproduces the reference's training.  One process,
+                       batch_size <= 4 rows x the GPU's SMs (592 on a B200).  Without it AE_Dropout_BN is not trained
+                       in float64 (a float64 run with other masks is no closer to the reference than split16); with any
+                       other precision the key is refused
       latent_dtype     "float64" (AE default, what the reference writes; any model under "fp64") | "float32" | "float16"
       l1_in_training   bool: add reg_param * L1 chain to the training loss (dead code upstream, SURVEY F2)
     """
@@ -158,13 +165,17 @@ def _npz_shape(path, key="data"):
 def refuse_fp64_training(config):
     """--mode train with config.precision == "fp64": NotImplementedError naming what the float64 trainer does not take,
     before any file is read or written (training.refuse_fp64_training).  True when "fp64" trains."""
+    stream = getattr(config, "dropout_stream", None)
     if not training.is_fp64(getattr(config, "precision", None)):
+        training.refuse_dropout_stream(config.model_name, getattr(config, "precision", None), stream)
         return False
     blocks = getattr(config, "convert_to_blocks", None)
     shape = _npz_shape(config.input_path)
     n_features = int(blocks[1]) * int(blocks[2]) if blocks else int(np.prod(shape[1:]))
     training.refuse_fp64_training(config.model_name, n_features,
-                                  getattr(config, "custom_loss_function", None) == "loss_function_swae")
+                                  getattr(config, "custom_loss_function", None) == "loss_function_swae",
+                                  dropout_stream=stream, batch_size=config.batch_size,
+                                  world=int(os.environ.get("WORLD_SIZE", "1")))
     return True
 
 

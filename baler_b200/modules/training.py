@@ -13,16 +13,54 @@ from . import utils
 dist_env = sharded.dist_env
 FUSED_TRAINER_MAX_FEATURES = 100  # bb_trainer stages whole weight matrices in shared memory (widest: 200 x 100)
 FP64_TRAINING_MODELS = ("AE", "CFD_dense_AE")  # what precision "fp64" trains: the fused trainer's models without BatchNorm
+DROPOUT_STREAMS = ("torch",)
+# AE_Dropout_BN's float64 step is one cooperative kernel of 4-row CTAs, one CTA per SM: every CTA of a batch must be
+# resident (148 SMs on a B200: 592 rows)
+FP64_DBN_ROWS_PER_CTA = 4
+B200_SM_COUNT = 148
 
 
 def is_fp64(precision):
     return engine.PRECISIONS.get(precision or "auto") == engine.BB_PREC_FP64
 
 
-def refuse_fp64_training(model_name, n_features, swae=False):
+def fp64_dbn_max_batch():
+    """largest AE_Dropout_BN batch of the float64 step: 4 rows x the SMs of the current GPU (a B200's without one)"""
+    sms = torch.cuda.get_device_properties(torch.cuda.current_device()).multi_processor_count \
+        if torch.cuda.is_available() else B200_SM_COUNT
+    return FP64_DBN_ROWS_PER_CTA * sms
+
+
+def refuse_dropout_stream(model_name, precision, dropout_stream):
+    """config.dropout_stream outside precision "fp64": ValueError for an unknown value, NotImplementedError for
+    AE_Dropout_BN (only the float64 step draws from torch's stream)"""
+    if dropout_stream is None:
+        return
+    if dropout_stream not in DROPOUT_STREAMS:
+        raise ValueError("dropout_stream must be one of %s, not %r" % (DROPOUT_STREAMS, dropout_stream))
+    if model_name == "AE_Dropout_BN" and not is_fp64(precision):
+        raise NotImplementedError("dropout_stream = %r is drawn by the float64 step of AE_Dropout_BN only; set "
+                                  "precision = 'fp64' (precision is %r)" % (dropout_stream, precision))
+
+
+def refuse_fp64_training(model_name, n_features, swae=False, dropout_stream=None, batch_size=None, world=1):
     """NotImplementedError naming what the float64 trainer (precision "fp64") does not take: models other than AE /
-    CFD_dense_AE (AE_Dropout_BN's BatchNorm, Conv_AE), loss_function_swae, rows wider than the fused trainer's"""
-    if model_name not in FP64_TRAINING_MODELS:
+    CFD_dense_AE and AE_Dropout_BN with dropout_stream = "torch" (Conv_AE), loss_function_swae, rows wider than the
+    fused trainer's; for AE_Dropout_BN also several processes and batches beyond the resident limit"""
+    refuse_dropout_stream(model_name, "fp64", dropout_stream)
+    if model_name == "AE_Dropout_BN":
+        if dropout_stream != "torch":
+            raise NotImplementedError(
+                "precision='fp64' trains AE_Dropout_BN only with dropout_stream = 'torch' (the reference's own dropout "
+                "masks, drawn on the device from torch's generator); with other masks a float64 run is no closer to "
+                "the reference than the default precision")
+        if world > 1:
+            raise NotImplementedError("precision='fp64' trains AE_Dropout_BN in one process (BatchNorm over the global "
+                                      "batch of %d ranks is not implemented for float64)" % world)
+        if batch_size is not None and batch_size > fp64_dbn_max_batch():
+            raise NotImplementedError("precision='fp64' trains AE_Dropout_BN with batch_size <= %d (every CTA of a "
+                                      "batch resident); batch_size is %d" % (fp64_dbn_max_batch(), batch_size))
+    elif model_name not in FP64_TRAINING_MODELS:
         raise NotImplementedError("precision='fp64' trains %s only; %s is not trained in float64 (use another precision)"
                                   % (" and ".join(FP64_TRAINING_MODELS), model_name))
     if swae:
@@ -48,6 +86,12 @@ def broadcast_initial_state(model):
     model.load_state_dict(sd)
 
 
+def consume_loader_seed(n_rows, batch_size):
+    """draw from torch's default generator what iter() of the reference's DataLoader(shuffle=False) over n_rows rows
+    draws (its base seed), by making that iterator over a placeholder of the same length"""
+    iter(torch.utils.data.DataLoader(range(n_rows), batch_size=batch_size, shuffle=False))
+
+
 class DeviceBatches:
     """Stands in for the reference's DataLoader(shuffle=False, drop_last=False) (training.py:253-263):
     the whole (normalised, float32) table resident in HBM plus the batch size."""
@@ -65,9 +109,15 @@ class DeviceAdam:
     CFD_dense_AE up to FUSED_TRAINER_MAX_FEATURES columns; refuse_fp64_training names what it does not take)."""
 
     def __init__(self, model, lr, max_batch, l1=False, reg_param=0.0, dropout_seed=0, block_hw=None, swae=False,
-                 precision=None):
+                 precision=None, dropout_stream=None):
+        """dropout_stream = "torch" (AE_Dropout_BN under precision "fp64"): every epoch draws its dropout masks on the
+        device from torch's default CPU generator, as the reference's fit does, and writes the state back"""
         if is_fp64(precision):
-            refuse_fp64_training(type(model).__name__, getattr(model, "n_features", 0), swae)
+            refuse_fp64_training(type(model).__name__, getattr(model, "n_features", 0), swae, dropout_stream, max_batch,
+                                 dist_env()[1])
+        else:
+            refuse_dropout_stream(type(model).__name__, precision, dropout_stream)
+        self.torch_stream = is_fp64(precision) and dropout_stream == "torch" and hasattr(model, "bn_tensors")
         self.rank, self.world = dist_env()
         broadcast_initial_state(model)
         self.model = model
@@ -89,7 +139,8 @@ class DeviceAdam:
         w, b = model.linear_tensors()
         if is_fp64(precision):
             # no layered fallback: the float64 step is the fused trainer's; data parallel all-reduces its float64 gradient
-            self.trainer = engine.Trainer(w, b, model.n_features, model.z_dim, max_batch)
+            self.trainer = engine.Trainer(w, b, model.n_features, model.z_dim, max_batch,
+                                          bn=model.bn_tensors() if self.has_bn else None)
             self.trainer.set_precision("fp64")
             self.dp = sharded.DataParallelTrainer(self.trainer, fused=False) if self.world > 1 else None
             return
@@ -117,6 +168,13 @@ class DeviceAdam:
     def epoch(self, data, batch_size):
         """one pass over `data` in the reference's batch order; data-parallel when launched with several ranks"""
         self.steps += (data.shape[0] + batch_size - 1) // batch_size
+        if self.torch_stream:
+            # the reference's fit iterates a fresh iter(train_dl) (one draw for its base seed), then draws every mask
+            consume_loader_seed(data.shape[0], batch_size)
+            self.trainer.set_dropout_torch()
+            loss = self.trainer.epoch(data, batch_size, self.hyper())
+            self.trainer.write_back_dropout_torch()
+            return loss
         if self.dp is None:
             return self.trainer.epoch(data, batch_size, self.hyper())
         return self.dp.epoch_table(data, batch_size, self.hyper(), self.rank, self.world)
@@ -171,6 +229,8 @@ def validate(model, test_dl, model_children, reg_param, optimizer=None):
     """reference training.py:104-137: eval-mode forward + sum-MSE / n_columns, mean over batches"""
     print("### Beginning Validating")
     model.eval()
+    if getattr(optimizer, "torch_stream", False):
+        consume_loader_seed(test_dl.data.shape[0], test_dl.batch_size)  # the reference's iter(test_dl)
     epoch_loss = optimizer.trainer.validate(test_dl.data, test_dl.batch_size)
     print(f"# Finished. Validation Loss: {epoch_loss:.6f}")
     return epoch_loss
@@ -211,7 +271,8 @@ def train(model, variables, train_data, test_data, project_path, config):
                            reg_param=config.reg_param, dropout_seed=int(torch.initial_seed()) & 0x7FFFFFFFFFFFFFFF,
                            block_hw=tuple(np.asarray(train_data).shape[1:3]) if conv else None,
                            swae=getattr(config, "custom_loss_function", None) == "loss_function_swae",
-                           precision=getattr(config, "precision", None))
+                           precision=getattr(config, "precision", None),
+                           dropout_stream=getattr(config, "dropout_stream", None))
     early_stopping = utils.EarlyStopping(config.early_stopping_patience, config.min_delta) if config.early_stopping else None
     lr_scheduler = utils.LRScheduler(optimizer, config.lr_scheduler_patience) if config.lr_scheduler else None
     train_loss, val_loss = [], []

@@ -251,12 +251,25 @@ int bb_trainer_create_dbn(bb_ctx* ctx, int n_features, int z_dim,
                           const double* const* bn_mean_host, const double* const* bn_var_host,
                           const long long* bn_batches_tracked, int max_batch, bb_trainer** out);
 /* dropout: in-kernel Philox4x32-10 keyed by (seed, step, layer, row, column); `masks_dev` (4 device pointers to
- * [batch x width] uint8 keep-masks, or NULL) injects torch-generated masks for parity tests */
+ * [batch x width] uint8 keep-masks, or NULL) injects torch-generated masks for parity tests.  Disarms the torch stream. */
 int bb_trainer_set_dropout(bb_trainer* t, unsigned long long seed, const unsigned char* const* masks_dev);
+/* dropout from torch's CPU generator (BB_PREC_FP64 only; other precisions: BB_ERR_UNSUPPORTED).  The reference draws
+ * every mask with bernoulli_(1 - p) on torch's default generator, an MT19937: per batch, layer 0..3, [rows x width]
+ * row-major, two words per element (first word high), keep = (random64 & (2^53 - 1)) * 2^-53 < 1 - p.
+ * set_dropout_mt19937 arms that stream for the following steps from the generator's state: its 624-word key and the
+ * position 0..624 of the next word (numpy's count; 624 - (left - 1) of torch.Generator.get_state()).  Each training
+ * step then draws its batch's masks on the device, on a side stream one step ahead, without a host synchronisation.
+ * get_dropout_mt19937 returns the state after the last drawn word (synchronises the side stream); writing it back into
+ * the generator leaves it where the reference's would be.  BB_ERR_INVALID before the stream is armed. */
+int bb_trainer_set_dropout_mt19937(bb_trainer* t, const uint32_t* key_624, int pos);
+int bb_trainer_get_dropout_mt19937(bb_trainer* t, uint32_t* key_out_624, int* pos_out);
 /* device views of the concatenated BatchNorm running statistics (4 layers, 50 + 100 + 200 + n_features values each).
  * Data parallel inside the library keeps them identical on every rank; host-loop data parallel (per-rank statistics)
  * averages them over ranks (torch DDP broadcasts rank 0's buffers instead; models.py:275-296) */
 int bb_trainer_bn_running_dev(bb_trainer* t, float** running_mean_dev, float** running_var_dev, int* n);
+/* BB_PREC_FP64: the float64 running statistics the float64 step updates (BB_ERR_UNSUPPORTED for other precisions) */
+int bb_trainer_bn_running_dev_f64(bb_trainer* t, double** running_mean_dev, double** running_var_dev, int* n);
+/* gamma / beta, running statistics and num_batches_tracked as float64 (BB_PREC_FP64: the float64 master as it is) */
 int bb_trainer_get_bn(bb_trainer* t, double* const* bn_weight_host, double* const* bn_bias_host,
                       double* const* bn_mean_host, double* const* bn_var_host, long long* bn_batches_tracked);
 int bb_trainer_destroy(bb_trainer* t);
@@ -268,12 +281,16 @@ int bb_trainer_destroy(bb_trainer* t);
  *                    MSE loss.
  *   BB_PREC_FP32     fp32 FFMA kernels; always used for the opt-in L1 chain.
  *   BB_PREC_FP64     float64 DFMA kernels with float64 master parameters and Adam state: the reference's float64
- *                    training to rounding (~1e-14), MSE and L1 chain.  Trainers of bb_trainer_create only
- *                    (bb_trainer_create_dbn: BB_ERR_UNSUPPORTED), and only before the first step or epoch (later:
- *                    BB_ERR_INVALID).  It uploads the float64 weights bb_trainer_create received, exactly.  The float32
- *                    table entry points widen x exactly; the *_f64 ones below take float64 tables.  The in-kernel
+ *                    training to rounding (~1e-14), MSE and L1 chain.  Only before the first step or epoch (later:
+ *                    BB_ERR_INVALID).  It uploads the float64 weights (and for bb_trainer_create_dbn the BatchNorm
+ *                    gamma / beta, running statistics and num_batches_tracked) that create received, exactly.  The
+ *                    float32 table entry points widen x exactly; the *_f64 ones below take float64 tables.  The in-kernel
  *                    exchange (bb_trainer_dp_export / _connect) is not available: data parallel runs phase 1, an
  *                    all-reduce of the float64 gradient (bb_trainer_grads_dev_f64) and phase 2.
+ *                    AE_Dropout_BN: one cooperative kernel with whole-batch float64 BatchNorm statistics, MSE loss only,
+ *                    batches up to 4 rows x resident CTAs (592 on B200; beyond: BB_ERR_UNSUPPORTED), one GPU's
+ *                    statistics; dropout from Philox (the same masks as BB_PREC_FP32), injected masks or torch's
+ *                    stream (bb_trainer_set_dropout_mt19937).
  * bb_trainer_precision returns what the next MSE step will run on.  Values beyond +-65504 (un-normalised tables) leave
  * the fp16 range on the SPLIT16 path: the batch loss turns non-finite, a sticky flag is raised and
  * bb_trainer_range_flag reports it (synchronises the device); the caller restarts with BB_PREC_FP32.
