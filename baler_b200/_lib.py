@@ -102,6 +102,10 @@ _SIGNATURES = {
     "bb_ltrainer_step_swae": (C.c_int, [_P, _P, C.c_int, C.POINTER(TrainHyper), C.c_int, _P, _P, C.c_int, C.c_int, C.c_float, _P, _P]),
     "bb_ltrainer_epoch": (C.c_int, [_P, _P, C.c_int64, C.c_int, C.POINTER(TrainHyper), C.POINTER(C.c_double), _P]),
     "bb_ltrainer_validate": (C.c_int, [_P, _P, C.c_int64, C.c_int, C.POINTER(C.c_double), _P]),
+    "bb_ltrainer_create_dbn": (C.c_int, [_P, C.c_int, C.c_int, _P, _P, _P, _P, _P, _P, _P, C.c_int, _PP]),
+    "bb_ltrainer_set_dropout": (C.c_int, [_P, C.c_uint64, _P]),
+    "bb_ltrainer_bn_batches_tracked": (C.c_int, [_P, _P]),
+    "bb_ltrainer_activation_means": (C.c_int, [_P, _P]),
 }
 
 _handle = None

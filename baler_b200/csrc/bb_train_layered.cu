@@ -21,11 +21,19 @@
 // running statistics), one block per channel:
 //     forward   xhat = (z - mean) * rstd,  y = gamma * xhat + beta
 //     backward  dgamma = sum(dy * xhat),  dbeta = sum(dy),  dz = gamma * rstd * (dy - dbeta / M - xhat * dgamma / M)
+//
+// `AE_Dropout_BN` (models.py:256-313) trains through the same chain (bb_ltrainer_create_dbn) at any batch size; the fused
+// dbn steps need every CTA of a batch resident.  Its two extra layer kinds:
+//     dropout   encoder: Linear -> Dropout(p) -> LeakyReLU; keep-bits from bb_philox_keep(seed, step, layer, row, column)
+//               (the stream of the fused fp32 / tensor-core dbn steps) or injected masks, kept values x fp32(1 / (1 - p))
+//     BN after  decoder layers 0-2: Linear -> LeakyReLU -> BatchNorm1d (the last one keeps Linear -> BatchNorm1d -> ReLU);
+//               the pre-BatchNorm activation is kept for LeakyReLU' in the backward pass
 #include <cmath>
 #include <cstdlib>
 #include <vector>
 
 #include "bb_common.cuh"
+#include "bb_train_f64.cuh"  // bb_philox_keep
 
 namespace {
 
@@ -190,11 +198,12 @@ constexpr float LBN_EPS = 1e-5f, LBN_MOMENTUM = 0.1f;
 
 // BatchNorm over channel c = blockIdx.x of Z[rows][N] (channel c = columns c*S .. c*S + S - 1), then the activation, in
 // place.  training: batch statistics (saved for the backward pass in mean_rstd, running statistics updated);
-// otherwise the running statistics.  xhat (nullable) receives the normalised values.
+// otherwise the running statistics.  xhat (nullable) receives the normalised values, pre (nullable) the input values.
 __global__ void __launch_bounds__(256) bn_fwd_kernel(float* __restrict__ Z, float* __restrict__ xhat, const int rows, const int N,
                                                      const int S, const int C, const float* __restrict__ gamma,
                                                      const float* __restrict__ beta, float* __restrict__ running,
-                                                     float* __restrict__ mean_rstd, const int training, const int act) {
+                                                     float* __restrict__ mean_rstd, const int training, const int act,
+                                                     float* __restrict__ pre) {
   __shared__ float red[256];
   const int c = blockIdx.x, M = rows * S;
   float mean, rstd;
@@ -222,7 +231,8 @@ __global__ void __launch_bounds__(256) bn_fwd_kernel(float* __restrict__ Z, floa
   const float g = gamma[c], b = beta[c];
   for (int e = threadIdx.x; e < M; e += 256) {
     const int64_t i = (int64_t)(e / S) * N + c * S + e % S;
-    const float xh = (Z[i] - mean) * rstd;
+    const float z = Z[i], xh = (z - mean) * rstd;
+    if (pre) pre[i] = z;
     if (xhat) xhat[i] = xh;
     Z[i] = act_fwd(g * xh + b, act);
   }
@@ -248,6 +258,61 @@ __global__ void __launch_bounds__(256) bn_bwd_kernel(float* __restrict__ dY, con
   for (int e = threadIdx.x; e < M; e += 256) {
     const int64_t i = (int64_t)(e / S) * N + c * S + e % S;
     dY[i] = k * (dY[i] - m1 - xhat[i] * m2);
+  }
+}
+
+// AE_Dropout_BN encoder: Z[rows][N] = act(keep ? Z * scale : 0) in place (dropout before the activation, models.py:263-275)
+__device__ __forceinline__ bool ldrop_keep(const unsigned char* mask, const unsigned long long seed, const unsigned long long step,
+                                           const int l, const int r, const int j, const int N) {
+  return mask ? mask[(int64_t)r * N + j] != 0 : bb_philox_keep(seed, step, l, r, j);
+}
+
+__global__ void __launch_bounds__(256) dropout_fwd_kernel(float* __restrict__ Z, const int rows, const int N, const int l,
+                                                          const unsigned long long seed, const unsigned long long step,
+                                                          const unsigned char* __restrict__ mask, const float scale, const int act) {
+  const int64_t total = (int64_t)rows * N;
+  for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
+    const int r = (int)(e / N), j = (int)(e - (int64_t)r * N);
+    Z[e] = act_fwd(ldrop_keep(mask, seed, step, l, r, j, N) ? Z[e] * scale : 0.f, act);
+  }
+}
+
+// its backward in place: dA (w.r.t. the layer output A) -> dZ = keep ? dA * act'(A) * scale : 0
+__global__ void __launch_bounds__(256) dropout_bwd_kernel(float* __restrict__ dA, const float* __restrict__ A_out, const int rows,
+                                                          const int N, const int l, const unsigned long long seed,
+                                                          const unsigned long long step, const unsigned char* __restrict__ mask,
+                                                          const float scale, const int act) {
+  const int64_t total = (int64_t)rows * N;
+  for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
+    const int r = (int)(e / N), j = (int)(e - (int64_t)r * N);
+    float g = dA[e];
+    if (act == BB_ACT_LEAKY) g *= A_out[e] > 0.f ? 1.f : BB_LEAKY;
+    else if (act == BB_ACT_RELU) g *= A_out[e] > 0.f ? 1.f : 0.f;
+    dA[e] = ldrop_keep(mask, seed, step, l, r, j, N) ? g * scale : 0.f;
+  }
+}
+
+// activation extraction: out[i][j] = mean over `rows` rows of column j of src[i] ([rows][n[i]]), NaN for j >= n[i]; a block
+// takes 32 columns of one matrix, 8 row groups add their rows in ascending order in double, combined in group order
+struct ColMeanSrc {
+  const float* a[6];
+  int n[6];
+};
+
+__global__ void __launch_bounds__(256) col_means_kernel(const __grid_constant__ ColMeanSrc src, const int rows, const int width,
+                                                        double* __restrict__ out) {
+  __shared__ double red[8][33];
+  const int i = blockIdx.y, c = threadIdx.x & 31, rg = threadIdx.x >> 5, j = blockIdx.x * 32 + c, n = src.n[i];
+  double s = 0.0;
+  if (j < n)
+    for (int r = rg; r < rows; r += 8) s += (double)src.a[i][(int64_t)r * n + j];
+  red[rg][c] = s;
+  __syncthreads();
+  if (rg == 0 && j < width) {
+    double v = 0.0;
+#pragma unroll
+    for (int q = 0; q < 8; ++q) v += red[q][c];
+    out[i * width + j] = j < n && rows > 0 ? v / rows : (double)NAN;
   }
 }
 
@@ -384,6 +449,11 @@ struct LLayer {
   float* dense = nullptr;                    // owns Wd | bd | gWd | gbd when tied
   int32_t *map = nullptr, *csr_ptr = nullptr, *csr_idx = nullptr;
   float *xhat = nullptr, *mean_rstd = nullptr, *running = nullptr;  // BatchNorm: saved xhat, batch (mean, rstd), running (mean | var)
+  long long nbt = 0;                         // BatchNorm: num_batches_tracked (training forward passes)
+  bool bn_post = false;                      // BatchNorm after the activation (AE_Dropout_BN decoder layers 0-2) ...
+  float* pre = nullptr;                      // ... and the activation it normalised, kept for act' in the backward pass
+  int drop = -1;                             // dropout before the activation: Philox layer / mask slot (-1: none)
+  float drop_scale = 1.f;                    // fp32(1 / (1 - p))
 };
 
 struct bb_ltrainer {
@@ -401,6 +471,11 @@ struct bb_ltrainer {
   long long step = 0;
   float* splitk = nullptr;                // split-K partials: SPLIT_MAX x the largest GEMM output
   size_t splitk_floats = 0;
+  int last_rows = 0;                      // rows of the most recent forward pass (activation extraction)
+  // AE_Dropout_BN (bb_ltrainer_create_dbn): dropout from Philox (seed, step = Adam updates before this one) or injected masks
+  bool dbn = false;
+  unsigned long long seed = 0;
+  const unsigned char* mask_dev[4] = {nullptr, nullptr, nullptr, nullptr};
 };
 
 namespace {
@@ -465,16 +540,25 @@ struct SwaeArgs {
 
 int lforward_backward(bb_ltrainer* t, const float* x, int rows, bool backward, cudaStream_t s, const SwaeArgs* sw = nullptr) {
   const int L = t->n_layers;
+  const int ew_blocks = t->ctx->sm_count * 2;  // elementwise kernels
+  t->last_rows = rows;
   BB_CUDA(cudaMemcpyAsync(t->act + t->a_off[0], x, sizeof(float) * (size_t)rows * t->lay[0].K, cudaMemcpyDeviceToDevice, s));
   for (int l = 0; l < L; ++l) {
-    const LLayer& y = t->lay[l];
+    LLayer& y = t->lay[l];
+    const bool drop = backward && y.drop >= 0;  // eval mode: dropout is the identity
+    float* A = t->act + t->a_off[l + 1];
     // A_{l+1}[rows x N] = act(A_l[rows x K] . W_l[N x K]^T + b_l)
-    lgemm(t, s, t->act + t->a_off[l], y.K, 1, y.Wd, 1, y.K, t->act + t->a_off[l + 1], y.N, rows, y.N, y.K, y.bd,
-          y.bn_c ? BB_ACT_NONE : y.act);
-    if (y.bn_c)
-      bn_fwd_kernel<<<y.bn_c, 256, 0, s>>>(t->act + t->a_off[l + 1], backward ? y.xhat : nullptr, rows, y.N, y.N / y.bn_c, y.bn_c,
-                                           t->params + y.g_off, t->params + y.g_off + y.bn_c, y.running, y.mean_rstd,
-                                           backward ? 1 : 0, y.act);
+    lgemm(t, s, t->act + t->a_off[l], y.K, 1, y.Wd, 1, y.K, A, y.N, rows, y.N, y.K, y.bd,
+          (y.bn_c && !y.bn_post) || drop ? BB_ACT_NONE : y.act);
+    if (drop)
+      dropout_fwd_kernel<<<ew_blocks, 256, 0, s>>>(A, rows, y.N, y.drop, t->seed, (unsigned long long)t->step, t->mask_dev[y.drop],
+                                                   y.drop_scale, y.act);
+    if (y.bn_c) {
+      bn_fwd_kernel<<<y.bn_c, 256, 0, s>>>(A, backward ? y.xhat : nullptr, rows, y.N, y.N / y.bn_c, y.bn_c, t->params + y.g_off,
+                                           t->params + y.g_off + y.bn_c, y.running, y.mean_rstd, backward ? 1 : 0,
+                                           y.bn_post ? BB_ACT_NONE : y.act, backward && y.bn_post ? y.pre : nullptr);
+      if (backward) y.nbt += 1;
+    }
   }
   const int C = t->lay[L - 1].N;
   float* dA = t->dz[0];
@@ -502,10 +586,19 @@ int lforward_backward(bb_ltrainer* t, const float* x, int rows, bool backward, c
     float* dZ = t->dz[cur];
     if (sw && l == sw->latent_layer)  // the encoder sees the decoder's gradient plus the sliced-Wasserstein one
       add_inplace_kernel<<<t->ctx->sm_count, 256, 0, s>>>(dZ, t->sw_dz, (int64_t)rows * N);
-    act_bwd_kernel<<<t->ctx->sm_count * 2, 256, 0, s>>>(dZ, t->act + t->a_off[l + 1], (int64_t)rows * N, y.act);
-    if (y.bn_c)
-      bn_bwd_kernel<<<y.bn_c, 256, 0, s>>>(dZ, y.xhat, rows, N, N / y.bn_c, y.bn_c, t->params + y.g_off, y.mean_rstd,
-                                           t->grads + y.g_off, t->grads + y.g_off + y.bn_c);
+    if (y.drop >= 0) {
+      dropout_bwd_kernel<<<ew_blocks, 256, 0, s>>>(dZ, t->act + t->a_off[l + 1], rows, N, y.drop, t->seed, (unsigned long long)t->step,
+                                                   t->mask_dev[y.drop], y.drop_scale, y.act);
+    } else if (y.bn_post) {  // Linear -> act -> BatchNorm: through the BatchNorm first, then act' of its input
+      bn_bwd_kernel<<<y.bn_c, 256, 0, s>>>(dZ, y.xhat, rows, N, 1, y.bn_c, t->params + y.g_off, y.mean_rstd, t->grads + y.g_off,
+                                           t->grads + y.g_off + y.bn_c);
+      act_bwd_kernel<<<ew_blocks, 256, 0, s>>>(dZ, y.pre, (int64_t)rows * N, y.act);
+    } else {
+      act_bwd_kernel<<<ew_blocks, 256, 0, s>>>(dZ, t->act + t->a_off[l + 1], (int64_t)rows * N, y.act);
+      if (y.bn_c)
+        bn_bwd_kernel<<<y.bn_c, 256, 0, s>>>(dZ, y.xhat, rows, N, N / y.bn_c, y.bn_c, t->params + y.g_off, y.mean_rstd,
+                                             t->grads + y.g_off, t->grads + y.g_off + y.bn_c);
+    }
     // dW_l[N x K] = dZ^T[N x rows] . A_l[rows x K]
     lgemm(t, s, dZ, 1, N, t->act + t->a_off[l], K, 1, y.gWd, K, N, K, rows, nullptr, BB_ACT_NONE);
     colsum_kernel<<<(N + 31) / 32, 256, 0, s>>>(dZ, rows, N, y.gbd);
@@ -647,6 +740,88 @@ int bb_ltrainer_create(bb_ctx* ctx, int n_layers, const int* dims, const int* ac
                                max_batch, out);
 }
 
+int bb_ltrainer_create_dbn(bb_ctx* ctx, int n_features, int z_dim, const double* const* weights_host,
+                           const double* const* biases_host, const double* const* bn_weight_host,
+                           const double* const* bn_bias_host, const double* const* bn_mean_host,
+                           const double* const* bn_var_host, const long long* bn_batches_tracked, int max_batch,
+                           bb_ltrainer** out) {
+  if (!bn_weight_host || !bn_bias_host || !bn_mean_host || !bn_var_host || n_features < 1 || z_dim < 1) return BB_ERR_INVALID;
+  // models.py:256-313: encoder 4 x (Linear -> Dropout -> LeakyReLU), decoder 3 x (Linear -> LeakyReLU -> BatchNorm1d),
+  // then Linear -> BatchNorm1d -> ReLU
+  const int dims[9] = {n_features, 200, 100, 50, z_dim, 50, 100, 200, n_features};
+  const int acts[8] = {BB_ACT_LEAKY, BB_ACT_LEAKY, BB_ACT_LEAKY, BB_ACT_LEAKY, BB_ACT_LEAKY, BB_ACT_LEAKY, BB_ACT_LEAKY, BB_ACT_RELU};
+  const float drop_scale[4] = {1.f / 0.5f, 1.f / 0.6f, 1.f / 0.7f, 1.f / 0.8f};  // the fused dbn steps' keep_scale
+  int bn_c[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+  std::vector<double> bn[4];
+  const double* bn_ptr[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+  for (int i = 0; i < 4; ++i) {
+    const int n = dims[5 + i];
+    if (!bn_weight_host[i] || !bn_bias_host[i] || !bn_mean_host[i] || !bn_var_host[i]) return BB_ERR_INVALID;
+    bn[i].resize(4 * (size_t)n);
+    for (int j = 0; j < n; ++j) {
+      bn[i][j] = bn_weight_host[i][j];
+      bn[i][n + j] = bn_bias_host[i][j];
+      bn[i][2 * n + j] = bn_mean_host[i][j];
+      bn[i][3 * n + j] = bn_var_host[i][j];
+    }
+    bn_c[4 + i] = n;
+    bn_ptr[4 + i] = bn[i].data();
+  }
+  bb_ltrainer* t = nullptr;
+  int rc = bb_ltrainer_create_ex(ctx, 8, dims, acts, nullptr, nullptr, nullptr, bn_c, weights_host, biases_host, bn_ptr, 0,
+                                 max_batch, &t);
+  if (rc != BB_OK) return rc;
+  t->dbn = true;
+  for (int l = 0; l < 4; ++l) {
+    t->lay[l].drop = l;
+    t->lay[l].drop_scale = drop_scale[l];
+  }
+  for (int i = 0; i < 4 && rc == BB_OK; ++i) {
+    LLayer& y = t->lay[4 + i];
+    y.nbt = bn_batches_tracked ? bn_batches_tracked[i] : 0;
+    y.bn_post = i < 3;
+    if (y.bn_post) rc = (int)cudaMalloc(&y.pre, sizeof(float) * (size_t)max_batch * y.N);
+  }
+  if (rc != BB_OK) { bb_ltrainer_destroy(t); return rc; }
+  *out = t;
+  return BB_OK;
+}
+
+int bb_ltrainer_set_dropout(bb_ltrainer* t, unsigned long long seed, const unsigned char* const* masks_dev) {
+  if (!t || !t->dbn) return BB_ERR_INVALID;
+  t->seed = seed;
+  for (int i = 0; i < 4; ++i) t->mask_dev[i] = masks_dev ? masks_dev[i] : nullptr;
+  return BB_OK;
+}
+
+int bb_ltrainer_bn_batches_tracked(bb_ltrainer* t, long long* out) {
+  if (!t || !out) return BB_ERR_INVALID;
+  for (int l = 0; l < t->n_layers; ++l) out[l] = t->lay[l].bn_c ? t->lay[l].nbt : 0;
+  return BB_OK;
+}
+
+int bb_ltrainer_activation_means(bb_ltrainer* t, double* out_host_6x200) {
+  if (!t || !out_host_6x200) return BB_ERR_INVALID;
+  // the 8-Linear autoencoders (AE family): A_l = output of layer l - 1 for l = 1, 2, 3, 5, 6, 7, as bb_trainer_activation_means
+  const int layers[6] = {1, 2, 3, 5, 6, 7}, width = 200;
+  if (t->n_layers != 8) return BB_ERR_UNSUPPORTED;
+  ColMeanSrc src;
+  for (int i = 0; i < 6; ++i) {
+    src.a[i] = t->act + t->a_off[layers[i]];
+    src.n[i] = t->lay[layers[i] - 1].N;
+    if (src.n[i] > width) return BB_ERR_UNSUPPORTED;
+  }
+  BB_CUDA(cudaSetDevice(t->ctx->device));
+  double* dev = nullptr;
+  BB_CUDA(cudaDeviceSynchronize());  // the last forward pass ran on the caller's stream
+  BB_CUDA(cudaMalloc(&dev, sizeof(double) * 6 * width));
+  col_means_kernel<<<dim3(width / 32 + 1, 6), 256>>>(src, t->last_rows, width, dev);
+  int rc = (int)cudaGetLastError();
+  if (rc == BB_OK) rc = (int)cudaMemcpy(out_host_6x200, dev, sizeof(double) * 6 * width, cudaMemcpyDeviceToHost);
+  cudaFree(dev);
+  return rc;
+}
+
 int bb_ltrainer_destroy(bb_ltrainer* t) {
   if (!t) return BB_OK;
   void* ptrs[] = {t->params, t->grads, t->m, t->v, t->act, t->dz[0], t->dz[1], t->loss_part, t->loss_accum, t->running_all,
@@ -655,7 +830,7 @@ int bb_ltrainer_destroy(bb_ltrainer* t) {
     if (p) cudaFree(p);
   for (int l = 0; l < t->n_layers; ++l) {
     LLayer& y = t->lay[l];
-    void* lp[] = {y.dense, y.map, y.csr_ptr, y.csr_idx, y.xhat, y.mean_rstd};
+    void* lp[] = {y.dense, y.map, y.csr_ptr, y.csr_idx, y.xhat, y.mean_rstd, y.pre};
     for (void* p : lp)
       if (p) cudaFree(p);
   }

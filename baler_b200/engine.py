@@ -542,9 +542,11 @@ def error_bounded_deltas(x, y, mn, rg, bound_percent, row0=0):
 
 class LayeredTrainer:
     """bb_ltrainer: the layer-by-layer trainer for dense autoencoders too wide for the fused training kernels
-    (CFD_dense_AE on 2500-feature snapshots).  Same surface as Trainer for what training.train uses."""
+    (CFD_dense_AE on 2500-feature snapshots), and for AE_Dropout_BN batches beyond the fused step's (LayeredTrainer.dbn).
+    Same surface as Trainer for what training.train uses."""
 
     _ACT = {"none": 0, "leaky": 1, "relu": 2}
+    dbn_kind = False
 
     def __init__(self, weights, biases, acts, max_batch, device=None, dims=None, w_maps=None, bn=None, loss_columns=0):
         """plain Linears: weights[l] is the (out, in) matrix.  Conv_AE (weight sharing, BatchNorm2d; see
@@ -580,6 +582,38 @@ class LayeredTrainer:
                                                    C.byref(self.handle)), "bb_ltrainer_create_ex")
         self.n_params = _lib.lib().bb_ltrainer_param_count(self.handle)
         self.loss_accum = torch.zeros(1, dtype=torch.float64, device=self.ctx.device)
+
+    @classmethod
+    def dbn(cls, weights, biases, n_features, z_dim, max_batch, bn, device=None):
+        """AE_Dropout_BN (bb_ltrainer_create_dbn): the arguments of Trainer(..., bn=bn) - the 8 Linears (out, in), and bn
+        = {weight, bias, running_mean, running_var: 4 arrays each, num_batches_tracked: 4 ints}.  No batch limit beyond
+        memory.  get_bn() then returns that dict."""
+        self = cls.__new__(cls)
+        self.ctx = get_context(device)
+        self.handle = C.c_void_p()
+        self.dbn_kind = True
+        self._w = [np.ascontiguousarray(w, dtype=np.float64) for w in weights]
+        self._b = [np.ascontiguousarray(b, dtype=np.float64) for b in biases]
+        self._bn = {k: [np.ascontiguousarray(a, dtype=np.float64) for a in bn[k]]
+                    for k in ("weight", "bias", "running_mean", "running_var")}
+        self.dims = [n_features, 200, 100, 50, z_dim, 50, 100, 200, n_features]
+        nbt = (C.c_longlong * 4)(*[int(v) for v in bn.get("num_batches_tracked", [0] * 4)])
+        with torch.cuda.device(self.ctx.device):
+            check(_lib.lib().bb_ltrainer_create_dbn(self.ctx.handle, n_features, z_dim, _host_ptrs(self._w), _host_ptrs(self._b),
+                                                    _host_ptrs(self._bn["weight"]), _host_ptrs(self._bn["bias"]),
+                                                    _host_ptrs(self._bn["running_mean"]), _host_ptrs(self._bn["running_var"]),
+                                                    nbt, max_batch, C.byref(self.handle)), "bb_ltrainer_create_dbn")
+        self.n_params = _lib.lib().bb_ltrainer_param_count(self.handle)
+        self.loss_accum = torch.zeros(1, dtype=torch.float64, device=self.ctx.device)
+        return self
+
+    def set_dropout(self, seed=0, masks=None):
+        """AE_Dropout_BN: Philox seed (the fused trainer's stream), or 4 CUDA uint8 keep-masks [batch, width]"""
+        self._masks = None if masks is None else [m.contiguous() for m in masks]
+        ptrs = None
+        if self._masks is not None:
+            ptrs = (C.c_void_p * 4)(*[m.data_ptr() for m in self._masks])
+        check(_lib.lib().bb_ltrainer_set_dropout(self.handle, int(seed), ptrs), "bb_ltrainer_set_dropout")
 
     def __del__(self):
         try:
@@ -631,14 +665,25 @@ class LayeredTrainer:
         return w, b
 
     def get_bn(self):
-        """per layer None or (4, channels): gamma / beta / running_mean / running_var"""
-        out = [None if b is None else np.empty_like(b) for b in self._bn]
+        """per layer None or (4, channels): gamma / beta / running_mean / running_var.  AE_Dropout_BN (dbn): Trainer.get_bn's
+        dict, num_batches_tracked included"""
+        if not self.dbn_kind:
+            out = [None if b is None else np.empty_like(b) for b in self._bn]
+        else:
+            out = [None] * 4 + [np.empty((4, n)) for n in self.dims[5:]]
         ptrs = (C.c_void_p * len(out))()
         for l, a in enumerate(out):
             if a is not None:
                 ptrs[l] = a.ctypes.data
         check(_lib.lib().bb_ltrainer_get_bn(self.handle, ptrs), "bb_ltrainer_get_bn")
-        return out
+        if not self.dbn_kind:
+            return out
+        nbt = (C.c_longlong * 8)()
+        check(_lib.lib().bb_ltrainer_bn_batches_tracked(self.handle, nbt), "bb_ltrainer_bn_batches_tracked")
+        keys = ("weight", "bias", "running_mean", "running_var")
+        res = {k: [out[4 + i][j].copy() for i in range(4)] for j, k in enumerate(keys)}
+        res["num_batches_tracked"] = [int(v) for v in nbt[4:]]
+        return res
 
     def bn_running_views(self):
         """zero-copy view of the running statistics of all BatchNorm layers (one tensor; DataParallelTrainer averages it)"""
@@ -647,7 +692,14 @@ class LayeredTrainer:
         return (self._flat(ptr, n.value),)
 
     def activation_means(self):
-        raise NotImplementedError("activation extraction is implemented for the fused trainer (n_features <= 31)")
+        """bb_ltrainer_activation_means: the (6, 200) NaN-padded matrix of Trainer.activation_means, from the last forward
+        pass; the 8-Linear autoencoders only"""
+        if len(self.dims) != 9:
+            raise NotImplementedError("activation extraction is implemented for the dense autoencoders (8 Linears), not "
+                                      "for a %d-layer chain" % (len(self.dims) - 1))
+        out = np.empty((6, 200), dtype=np.float64)
+        check(_lib.lib().bb_ltrainer_activation_means(self.handle, out.ctypes.data), "bb_ltrainer_activation_means")
+        return out
 
 
 def make_hyper(lr=1e-3, reg_param=0.0, l1=False, world_size=1, beta1=0.9, beta2=0.999, eps=1e-8):

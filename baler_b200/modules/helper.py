@@ -164,10 +164,12 @@ def _npz_shape(path, key="data"):
 
 def refuse_fp64_training(config):
     """--mode train with config.precision == "fp64": NotImplementedError naming what the float64 trainer does not take,
-    before any file is read or written (training.refuse_fp64_training).  True when "fp64" trains."""
+    before any file is read or written (training.refuse_fp64_training).  True when "fp64" trains.  Other precisions:
+    the dropout_stream key and AE_Dropout_BN's per-rank batch under torchrun (training.refuse_dbn_rank_share)."""
     stream = getattr(config, "dropout_stream", None)
     if not training.is_fp64(getattr(config, "precision", None)):
         training.refuse_dropout_stream(config.model_name, getattr(config, "precision", None), stream)
+        training.refuse_dbn_rank_share(config.model_name, config.batch_size, int(os.environ.get("WORLD_SIZE", "1")))
         return False
     blocks = getattr(config, "convert_to_blocks", None)
     shape = _npz_shape(config.input_path)

@@ -18,17 +18,43 @@ DROPOUT_STREAMS = ("torch",)
 # resident (148 SMs on a B200: 592 rows)
 FP64_DBN_ROWS_PER_CTA = 4
 B200_SM_COUNT = 148
+# AE_Dropout_BN's fused step (tensor cores) keeps every 16-row tile of a batch resident, one CTA per SM (2368 rows on a
+# B200); larger batches train on the layer-by-layer trainer
+DBN_FUSED_ROWS_PER_CTA = 16
 
 
 def is_fp64(precision):
     return engine.PRECISIONS.get(precision or "auto") == engine.BB_PREC_FP64
 
 
+def _sm_count():
+    """SMs of the current GPU (a B200's without one)"""
+    return torch.cuda.get_device_properties(torch.cuda.current_device()).multi_processor_count \
+        if torch.cuda.is_available() else B200_SM_COUNT
+
+
 def fp64_dbn_max_batch():
     """largest AE_Dropout_BN batch of the float64 step: 4 rows x the SMs of the current GPU (a B200's without one)"""
-    sms = torch.cuda.get_device_properties(torch.cuda.current_device()).multi_processor_count \
-        if torch.cuda.is_available() else B200_SM_COUNT
-    return FP64_DBN_ROWS_PER_CTA * sms
+    return FP64_DBN_ROWS_PER_CTA * _sm_count()
+
+
+def dbn_fused_max_batch():
+    """largest AE_Dropout_BN batch of the fused step: 16 rows x the SMs of the current GPU (a B200's without one); larger
+    batches of one process train on the layer-by-layer trainer"""
+    return DBN_FUSED_ROWS_PER_CTA * _sm_count()
+
+
+def refuse_dbn_rank_share(model_name, batch_size, world):
+    """NotImplementedError for AE_Dropout_BN under torchrun when a rank's share of the global batch exceeds the fused step's
+    batch: the layer-by-layer trainer normalises over one process's batch only"""
+    if model_name != "AE_Dropout_BN" or world <= 1 or batch_size is None:
+        return
+    share = (batch_size + world - 1) // world
+    if share > dbn_fused_max_batch():
+        raise NotImplementedError("AE_Dropout_BN with %d ranks trains per-rank shares of at most %d rows (the fused step); "
+                                  "batch_size %d gives %d per rank.  BatchNorm over the global batch of larger shares is "
+                                  "not implemented: lower batch_size or train in one process"
+                                  % (world, dbn_fused_max_batch(), batch_size, share))
 
 
 def refuse_dropout_stream(model_name, precision, dropout_stream):
@@ -111,12 +137,14 @@ class DeviceAdam:
     def __init__(self, model, lr, max_batch, l1=False, reg_param=0.0, dropout_seed=0, block_hw=None, swae=False,
                  precision=None, dropout_stream=None):
         """dropout_stream = "torch" (AE_Dropout_BN under precision "fp64"): every epoch draws its dropout masks on the
-        device from torch's default CPU generator, as the reference's fit does, and writes the state back"""
+        device from torch's default CPU generator, as the reference's fit does, and writes the state back.
+        AE_Dropout_BN batches beyond dbn_fused_max_batch() train on the layer-by-layer trainer (one process)."""
         if is_fp64(precision):
             refuse_fp64_training(type(model).__name__, getattr(model, "n_features", 0), swae, dropout_stream, max_batch,
                                  dist_env()[1])
         else:
             refuse_dropout_stream(type(model).__name__, precision, dropout_stream)
+            refuse_dbn_rank_share(type(model).__name__, max_batch, int(os.environ.get("WORLD_SIZE", "1")))
         self.torch_stream = is_fp64(precision) and dropout_stream == "torch" and hasattr(model, "bn_tensors")
         self.rank, self.world = dist_env()
         broadcast_initial_state(model)
@@ -144,7 +172,10 @@ class DeviceAdam:
             self.trainer.set_precision("fp64")
             self.dp = sharded.DataParallelTrainer(self.trainer, fused=False) if self.world > 1 else None
             return
-        if not swae and (self.has_bn or model.n_features <= FUSED_TRAINER_MAX_FEATURES):
+        if self.has_bn and self.world == 1 and max_batch > dbn_fused_max_batch():
+            # batches the fused AE_Dropout_BN step cannot hold resident: the layer-by-layer trainer, same dropout stream
+            self.trainer = engine.LayeredTrainer.dbn(w, b, model.n_features, model.z_dim, max_batch, model.bn_tensors())
+        elif not swae and (self.has_bn or model.n_features <= FUSED_TRAINER_MAX_FEATURES):
             try:
                 self.trainer = engine.Trainer(w, b, model.n_features, model.z_dim, max_batch,
                                               bn=model.bn_tensors() if self.has_bn else None)

@@ -427,6 +427,31 @@ int bb_ltrainer_epoch(bb_ltrainer* t, const float* x_dev, int64_t n_rows, int ba
                       double* epoch_loss_host, bb_stream_t stream);
 int bb_ltrainer_validate(bb_ltrainer* t, const float* x_dev, int64_t n_rows, int batch, double* epoch_loss_host,
                          bb_stream_t stream);
+/*
+ * AE_Dropout_BN (models.py:256-313) on the layer-by-layer trainer, at any batch size that fits in memory (the fused
+ * bb_trainer_create_dbn step needs every tile of a batch resident: 16 rows x SMs on the tensor-core step).  Same
+ * arguments as bb_trainer_create_dbn.  The chain: encoder 4 x (Linear -> Dropout p = .5/.4/.3/.2 -> LeakyReLU), the latent
+ * included; decoder 3 x (Linear -> LeakyReLU -> BatchNorm1d), then Linear -> BatchNorm1d -> ReLU.  Training steps draw
+ * their keep-masks as the fused dbn steps do (bb_trainer_set_dropout: Philox keyed by the seed and the number of earlier
+ * Adam updates, or injected masks) and use batch statistics (biased variance, eps 1e-5, running statistics with momentum
+ * 0.1 and the unbiased variance); bb_ltrainer_validate uses no dropout and the running statistics.  MSE only
+ * (h->l1: BB_ERR_UNSUPPORTED), one process (bb_ltrainer_epoch).  The flat parameters hold, layer after layer,
+ * weights | biases | gamma | beta; bb_ltrainer_get_params / bb_ltrainer_get_bn (layers 4-7) read them back.
+ */
+int bb_ltrainer_create_dbn(bb_ctx* ctx, int n_features, int z_dim, const double* const* weights_host,
+                           const double* const* biases_host, const double* const* bn_weight_host,
+                           const double* const* bn_bias_host, const double* const* bn_mean_host,
+                           const double* const* bn_var_host, const long long* bn_batches_tracked, int max_batch,
+                           bb_ltrainer** out);
+/* AE_Dropout_BN trainers: dropout source of the following steps, as bb_trainer_set_dropout (seed, or 4 device uint8
+ * keep-masks [batch][width_l], kept while they are in use; NULL: Philox) */
+int bb_ltrainer_set_dropout(bb_ltrainer* t, unsigned long long seed, const unsigned char* const* masks_dev);
+/* num_batches_tracked of every layer (n_layers entries; 0 for layers without BatchNorm) */
+int bb_ltrainer_bn_batches_tracked(bb_ltrainer* t, long long* out_n_layers);
+/* bb_trainer_activation_means of the 8-Linear autoencoders (AE, CFD_dense_AE, AE_Dropout_BN): column means of the outputs
+ * of layers 0, 1, 2, 4, 5, 6 over the rows of the last forward pass (training step or validate), NaN beyond a layer's
+ * width; synchronises the device.  Other chains or layers wider than 200: BB_ERR_UNSUPPORTED. */
+int bb_ltrainer_activation_means(bb_ltrainer* t, double* out_host_6x200);
 
 /*
  * Error-bounded deltas: helper.save_error_bounded_requirement (helper.py:442-470) for n_rows rows at once.  `x_dev` raw
