@@ -86,6 +86,12 @@ _SIGNATURES = {
     "bb_trainer_step_f64": (C.c_int, [_P, _P, C.c_int, C.POINTER(TrainHyper), C.c_int, _P, _P]),
     "bb_trainer_epoch_f64": (C.c_int, [_P, _P, C.c_int64, C.c_int, C.POINTER(TrainHyper), C.POINTER(C.c_double), _P]),
     "bb_trainer_validate_f64": (C.c_int, [_P, _P, C.c_int64, C.c_int, C.POINTER(C.c_double), _P]),
+    "bb_trainer_epoch_host": (C.c_int, [_P, _P, C.c_int, C.c_int64, C.c_int, C.POINTER(TrainHyper), C.c_int64,
+                                        C.POINTER(C.c_double), _P]),
+    "bb_trainer_validate_host": (C.c_int, [_P, _P, C.c_int, C.c_int64, C.c_int, C.c_int64, C.POINTER(C.c_double), _P]),
+    "bb_ltrainer_epoch_host": (C.c_int, [_P, _P, C.c_int, C.c_int64, C.c_int, C.POINTER(TrainHyper), C.c_int64,
+                                         C.POINTER(C.c_double), _P]),
+    "bb_ltrainer_validate_host": (C.c_int, [_P, _P, C.c_int, C.c_int64, C.c_int, C.c_int64, C.POINTER(C.c_double), _P]),
     "bb_trainer_activation_means": (C.c_int, [_P, _P]),
     "bb_mse_sum_f32": (C.c_int, [_P, _P, _P, C.c_int64, _P, _P]),
     "bb_error_bounded_deltas_f32": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int, _P, _P, C.c_double, C.c_int64, C.c_int64, _P, _P, _P, _P, _P]),

@@ -979,3 +979,122 @@ int bb_decompress_host_f64(bb_model* m, const double* z_host, int64_t n_rows, co
 }
 
 }  // extern "C"
+
+// ------------------------------------------------------------------ host tables streamed through a device window
+
+struct HostWindow {
+  cudaStream_t copy = nullptr;
+  cudaEvent_t landed[2] = {nullptr, nullptr};    // slot's upload complete (copy stream)
+  cudaEvent_t consumed[2] = {nullptr, nullptr};  // slot's kernels complete (caller's stream)
+  cudaEvent_t staged[2] = {nullptr, nullptr};    // pinned buffer's upload complete (copy stream)
+  void* dev[2] = {nullptr, nullptr};
+  size_t dev_bytes = 0;
+  void* pin[2] = {nullptr, nullptr};
+  size_t pin_bytes = 0;
+};
+
+namespace {
+// pinned staging of a pageable table: 2 x 64 MiB, whatever the window (the window's size is bounded by device memory, the
+// staging by what page-locking a shared host can spare)
+constexpr size_t WINDOW_STAGE_BYTES = (size_t)64 << 20;
+
+int window_create(HostWindow* w) {
+  BB_CUDA(cudaStreamCreateWithFlags(&w->copy, cudaStreamNonBlocking));
+  for (int i = 0; i < 2; ++i) {
+    BB_CUDA(cudaEventCreateWithFlags(&w->landed[i], cudaEventDisableTiming));
+    BB_CUDA(cudaEventCreateWithFlags(&w->consumed[i], cudaEventDisableTiming));
+    BB_CUDA(cudaEventCreateWithFlags(&w->staged[i], cudaEventDisableTiming));
+  }
+  return BB_OK;
+}
+
+// upload `bytes` of the host table at src into dst on the copy stream (after whatever the copy stream already waits for)
+int window_upload(HostWindow* w, void* dst, const char* src, size_t bytes, bool pinned, unsigned* stage_k) {
+  if (pinned) {
+    BB_CUDA(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, w->copy));
+    return BB_OK;
+  }
+  for (size_t off = 0; off < bytes; off += w->pin_bytes) {
+    const size_t n = std::min(w->pin_bytes, bytes - off);
+    const int p = (int)((*stage_k)++ & 1u);
+    BB_CUDA(cudaEventSynchronize(w->staged[p]));  // the buffer's previous upload has left it (never recorded: returns)
+    copy_parallel(w->pin[p], src + off, n);
+    BB_CUDA(cudaMemcpyAsync((char*)dst + off, w->pin[p], n, cudaMemcpyHostToDevice, w->copy));
+    BB_CUDA(cudaEventRecord(w->staged[p], w->copy));
+  }
+  return BB_OK;
+}
+}  // namespace
+
+void bb_host_window_free(HostWindow* w) {
+  if (!w) return;
+  if (w->copy) cudaStreamSynchronize(w->copy);
+  for (int i = 0; i < 2; ++i) {
+    if (w->dev[i]) cudaFree(w->dev[i]);
+    if (w->pin[i]) cudaFreeHost(w->pin[i]);
+    if (w->landed[i]) cudaEventDestroy(w->landed[i]);
+    if (w->consumed[i]) cudaEventDestroy(w->consumed[i]);
+    if (w->staged[i]) cudaEventDestroy(w->staged[i]);
+  }
+  if (w->copy) cudaStreamDestroy(w->copy);
+  delete w;
+}
+
+int bb_host_window_run(HostWindow** win, const void* x_host, size_t row_bytes, int64_t n_rows, int64_t window_rows,
+                       cudaStream_t s, const std::function<int(const void*, int64_t)>& body) {
+  if (!win || !x_host || row_bytes == 0 || n_rows < 1 || window_rows < 1) return BB_ERR_INVALID;
+  if (!*win) {
+    HostWindow* w = new (std::nothrow) HostWindow();
+    if (!w) return BB_ERR_NOMEM;
+    const int rc = window_create(w);
+    if (rc != BB_OK) {
+      bb_host_window_free(w);
+      return rc;
+    }
+    *win = w;
+  }
+  HostWindow* w = *win;
+  const int64_t rows_per = std::min(window_rows, n_rows);
+  const size_t slot_bytes = (size_t)rows_per * row_bytes;
+  if (w->dev_bytes < slot_bytes) {
+    BB_CUDA(cudaStreamSynchronize(w->copy));
+    for (int i = 0; i < 2; ++i) {
+      if (w->dev[i]) cudaFree(w->dev[i]);  // (waits for the kernels still reading it)
+      w->dev[i] = nullptr;
+    }
+    w->dev_bytes = 0;
+    for (int i = 0; i < 2; ++i)
+      if (cudaMalloc(&w->dev[i], slot_bytes) != cudaSuccess) { cudaGetLastError(); return BB_ERR_NOMEM; }
+    w->dev_bytes = slot_bytes;
+  }
+  const bool pinned = host_pinned(x_host);
+  const size_t stage = std::min(WINDOW_STAGE_BYTES, slot_bytes);
+  if (!pinned && w->pin_bytes < stage) {
+    BB_CUDA(cudaStreamSynchronize(w->copy));
+    for (int i = 0; i < 2; ++i) {
+      if (w->pin[i]) cudaFreeHost(w->pin[i]);
+      w->pin[i] = nullptr;
+    }
+    w->pin_bytes = 0;
+    for (int i = 0; i < 2; ++i)
+      if (cudaMallocHost(&w->pin[i], stage) != cudaSuccess) { cudaGetLastError(); return BB_ERR_NOMEM; }
+    w->pin_bytes = stage;
+  }
+  // the slots' previous users (an earlier call on another stream) are done before this call writes them
+  for (int i = 0; i < 2; ++i) BB_CUDA(cudaEventRecord(w->consumed[i], s));
+  const char* x = (const char*)x_host;
+  unsigned stage_k = 0;
+  int rc = BB_OK;
+  for (int64_t k = 0, r0 = 0; r0 < n_rows && rc == BB_OK; ++k, r0 += rows_per) {
+    const int slot = (int)(k & 1);
+    const int64_t rows = std::min(rows_per, n_rows - r0);
+    rc = (int)cudaStreamWaitEvent(w->copy, w->consumed[slot], 0);  // the kernels of window k - 2 are done with the slot
+    if (rc == BB_OK) rc = window_upload(w, w->dev[slot], x + (size_t)r0 * row_bytes, (size_t)rows * row_bytes, pinned, &stage_k);
+    if (rc == BB_OK) rc = (int)cudaEventRecord(w->landed[slot], w->copy);
+    if (rc == BB_OK) rc = (int)cudaStreamWaitEvent(s, w->landed[slot], 0);
+    if (rc == BB_OK) rc = body(w->dev[slot], rows);
+    if (rc == BB_OK) rc = (int)cudaEventRecord(w->consumed[slot], s);
+  }
+  const cudaError_t sync = cudaStreamSynchronize(w->copy);  // (the staging buffers are free again when this returns)
+  return rc != BB_OK ? rc : (int)sync;
+}

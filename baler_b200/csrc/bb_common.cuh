@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <cuda_fp16.h>
 #include <stdint.h>
+#include <functional>
 #include <vector>
 
 #include "../../include/baler_b200.h"
@@ -158,3 +159,14 @@ int bb_tc_launch(bb_ctx* ctx, const Chain* c, const void* in, int in_dtype, int6
                  const float* pre_min, const float* pre_range, const float* post_min,
                  const float* post_range, void* out, int out_dtype, int fast, int* flag_dev,
                  cudaStream_t stream);
+
+// --- host tables streamed through the device (bb_api.cu): the training entry points *_epoch_host / *_validate_host
+// Two device slots of window_rows rows, filled on an internal copy stream while `body` runs on `s` on the other one; events
+// order the reuse of each slot.  A pageable table goes through two pinned staging buffers (copied on the worker pool), a
+// pinned one is copied directly.  `body(x_dev, rows)` enqueues the work of one window on `s`; windows are cut every
+// window_rows rows, so a caller that passes a multiple of its batch sees whole batches.  The slots and streams are kept in
+// *win between calls (created on first use, released by bb_host_window_free).
+struct HostWindow;
+int bb_host_window_run(HostWindow** win, const void* x_host, size_t row_bytes, int64_t n_rows, int64_t window_rows,
+                       cudaStream_t s, const std::function<int(const void*, int64_t)>& body);
+void bb_host_window_free(HostWindow* win);

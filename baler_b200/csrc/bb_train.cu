@@ -725,6 +725,7 @@ struct bb_trainer {
   std::vector<double> bn_stats_host;  // AE_Dropout_BN: float64 running_mean then running_var (bn_f_total each)
   long long nbt_host[4] = {0, 0, 0, 0};
   bool started = false;              // a step or an epoch has run (the precision of a float64 run is fixed from then on)
+  HostWindow* win = nullptr;         // device window of bb_trainer_epoch_host / _validate_host (kept between calls)
 };
 
 namespace {
@@ -1053,6 +1054,7 @@ int bb_trainer_destroy(bb_trainer* t) {
     if (p) cudaFree(p);
   bb_tc_train_destroy(t->tc);
   bb_f64_train_destroy(t->f64);
+  bb_host_window_free(t->win);
   delete t;
   return BB_OK;
 }
@@ -1175,43 +1177,137 @@ int step_f64(bb_trainer* t, const void* x, int x_is_f64, int rows, const bb_trai
   return rc;
 }
 
-int epoch_f64(bb_trainer* t, const void* x, int x_is_f64, int64_t n_rows, int batch, const bb_train_hyper* h,
-              double* epoch_loss_host, cudaStream_t s) {
-  if (!t || !h || !x || n_rows < 1 || batch < 1 || batch > t->max_batch || !epoch_loss_host) return BB_ERR_INVALID;
-  if (t->precision != BB_PREC_FP64) return BB_ERR_INVALID;
-  if (h->world_size > 1) return BB_ERR_UNSUPPORTED;  // data parallel: phases 1 and 2 around the caller's all-reduce
-  BB_CUDA(cudaMemsetAsync(t->loss_accum, 0, sizeof(double), s));
-  const size_t row_bytes = (size_t)t->d.dims[0] * (x_is_f64 ? sizeof(double) : sizeof(float));
-  int64_t n_batches = 0;
-  for (int64_t r0 = 0; r0 < n_rows; r0 += batch, ++n_batches) {
-    const int rows = (int)(n_rows - r0 < batch ? n_rows - r0 : batch);
-    const int rc = step_f64(t, (const char*)x + (size_t)r0 * row_bytes, x_is_f64, rows, h, 0, t->loss_accum, s);
-    if (rc != BB_OK) return rc;
+// Arguments of an epoch on a table of float32 (x_is_f64 = 0) or float64 rows that the entry points refuse, else BB_OK
+int check_epoch(bb_trainer* t, int x_is_f64, int batch, const bb_train_hyper* h) {
+  if (x_is_f64 && t->precision != BB_PREC_FP64) return BB_ERR_INVALID;
+  if (t->precision == BB_PREC_FP64) {
+    if (batch > t->max_batch) return BB_ERR_INVALID;
+    return h->world_size > 1 ? BB_ERR_UNSUPPORTED : BB_OK;  // data parallel: phases 1 and 2 around the caller's all-reduce
   }
-  double total = 0.0;
-  BB_CUDA(cudaMemcpyAsync(&total, t->loss_accum, sizeof(double), cudaMemcpyDeviceToHost, s));
-  BB_CUDA(cudaStreamSynchronize(s));
-  *epoch_loss_host = total / (double)n_batches;
+  t->started = true;
+  if (h->world_size <= 1 && batch > t->max_batch) return BB_ERR_INVALID;
+  const int dp_world = t->tc ? bb_tc_train_dp_world(t->tc) : 1;
+  if (h->world_size > 1 && h->world_size != dp_world) return BB_ERR_INVALID;  // data parallel needs bb_trainer_dp_connect
+  if (h->world_size > 1 && (batch + dp_world - 1) / dp_world > t->max_batch) return BB_ERR_INVALID;
   return BB_OK;
 }
 
-int validate_f64(bb_trainer* t, const void* x, int x_is_f64, int64_t n_rows, int batch, double* epoch_loss_host,
-                 cudaStream_t s) {
-  if (!t || !x || n_rows < 1 || batch < 1 || batch > t->max_batch || !epoch_loss_host) return BB_ERR_INVALID;
-  if (t->precision != BB_PREC_FP64) return BB_ERR_INVALID;
-  BB_CUDA(cudaMemsetAsync(t->loss_accum, 0, sizeof(double), s));
+// The training steps of the batches of rows [0, n_rows) of x in order (the last one may be ragged), their losses added to
+// t->loss_accum.  The body of an epoch over a device table, and of every window of a streamed host table: windows hold
+// whole batches and the step counter runs on, so both run the same steps.
+int train_rows(bb_trainer* t, const void* x, int x_is_f64, int64_t n_rows, int batch, const bb_train_hyper* h, cudaStream_t s) {
   const size_t row_bytes = (size_t)t->d.dims[0] * (x_is_f64 ? sizeof(double) : sizeof(float));
-  int64_t n_batches = 0;
-  for (int64_t r0 = 0; r0 < n_rows; r0 += batch, ++n_batches) {
+  if (t->precision == BB_PREC_FP64) {
+    for (int64_t r0 = 0; r0 < n_rows; r0 += batch) {
+      const int rows = (int)(n_rows - r0 < batch ? n_rows - r0 : batch);
+      const int rc = step_f64(t, (const char*)x + (size_t)r0 * row_bytes, x_is_f64, rows, h, 0, t->loss_accum, s);
+      if (rc != BB_OK) return rc;
+    }
+    return BB_OK;
+  }
+  int urc;
+  if (use_tc(t, h, s, &urc)) {
+    // the whole epoch (window) is one persistent kernel: no launch and no host round trip between steps
+    if (urc != BB_OK) return urc;
+    const TcHyper th = tc_hyper(h);
+    const int64_t n_batches = (n_rows + batch - 1) / batch;
+    t->wt_fresh = false;
+    t->last_tc = true;
+    t->last_rows = (int)(n_rows - (n_batches - 1) * batch);
+    bb_tc_train_set_mode(t->tc, 1, (unsigned long long)t->step);
+    const int rc = bb_tc_train_run(t->tc, (const float*)x, n_rows, batch, TC_P1 | TC_DW | TC_ADAM, &th, t->step + 1,
+                                   t->loss_accum, h->world_size > 1 ? 1 : 0, s);
+    if (rc != BB_OK) return rc;
+    t->step += n_batches;
+    return BB_OK;
+  }
+  if (urc != BB_OK) return urc;
+  if (h->world_size > 1) return BB_ERR_UNSUPPORTED;  // the fused exchange lives in the tensor-core kernel
+  for (int64_t r0 = 0; r0 < n_rows; r0 += batch) {
     const int rows = (int)(n_rows - r0 < batch ? n_rows - r0 : batch);
-    const int rc = bb_f64_train_eval(t->f64, (const char*)x + (size_t)r0 * row_bytes, x_is_f64, rows, t->loss_accum, s);
+    const int rc = bb_trainer_step(t, (const float*)x + (size_t)r0 * t->d.dims[0], rows, h, 0, t->loss_accum, s);
     if (rc != BB_OK) return rc;
   }
+  return BB_OK;
+}
+
+// The eval-mode forward passes of the batches of rows [0, n_rows) of x, their losses added to t->loss_accum (validate;
+// windows as in train_rows)
+int eval_rows(bb_trainer* t, const void* x, int x_is_f64, int64_t n_rows, int batch, cudaStream_t s) {
+  if (t->precision == BB_PREC_FP64) {
+    const size_t row_bytes = (size_t)t->d.dims[0] * (x_is_f64 ? sizeof(double) : sizeof(float));
+    for (int64_t r0 = 0; r0 < n_rows; r0 += batch) {
+      const int rows = (int)(n_rows - r0 < batch ? n_rows - r0 : batch);
+      const int rc = bb_f64_train_eval(t->f64, (const char*)x + (size_t)r0 * row_bytes, x_is_f64, rows, t->loss_accum, s);
+      if (rc != BB_OK) return rc;
+    }
+    return BB_OK;
+  }
+  const float* xf = (const float*)x;
+  int urc;
+  const bool tc = use_tc(t, nullptr, s, &urc);
+  if (urc != BB_OK) return urc;
+  if (tc) {
+    TcHyper th;
+    memset(&th, 0, sizeof(th));
+    th.b1d = th.b2d = 0.5;
+    const int64_t n_batches = (n_rows + batch - 1) / batch;
+    t->last_tc = true;
+    t->last_rows = (int)(n_rows - (n_batches - 1) * batch);
+    bb_tc_train_set_mode(t->tc, 0, 0ull);
+    return bb_tc_train_run(t->tc, xf, n_rows, batch, TC_FWD_ONLY, &th, 1, t->loss_accum, 0, s);
+  }
+  for (int64_t r0 = 0; r0 < n_rows; r0 += batch) {
+    const int rows = (int)(n_rows - r0 < batch ? n_rows - r0 : batch);
+    t->last_tc = false;
+    int rc = t->kind == 1 ? launch_dbn(t, xf + (size_t)r0 * t->d.dims[0], rows, 1, s)
+                          : launch_fwd_bwd(t, xf + (size_t)r0 * t->d.dims[0], rows, 0, nullptr, s);
+    if (rc != BB_OK) return rc;
+    // mode 1 with zero splits: only folds the loss partials into the gradient's loss slot ...
+    train_adam_kernel<<<1, NT, 0, s>>>(0, 1, t->partial, 0, t->grads + t->d.n_params, nullptr, nullptr, nullptr, nullptr,
+                                       nullptr, 0.f, 0.f, 0.f, 0.f, 0.f, t->loss_part, (rows + RT - 1) / RT, nullptr);
+    // ... and mode 2 with zero parameters adds that slot to the accumulator
+    train_adam_kernel<<<1, NT, 0, s>>>(0, 2, nullptr, 0, t->grads + t->d.n_params, nullptr, nullptr, nullptr, nullptr,
+                                       nullptr, 0.f, 0.f, 0.f, 0.f, 0.f, nullptr, 0, t->loss_accum);
+    BB_CUDA(cudaGetLastError());
+  }
+  return BB_OK;
+}
+
+// epoch loss = the summed batch losses over the number of batches (training.py:99); synchronises s
+int finish_epoch(bb_trainer* t, int64_t n_rows, int batch, double* epoch_loss_host, cudaStream_t s) {
   double total = 0.0;
   BB_CUDA(cudaMemcpyAsync(&total, t->loss_accum, sizeof(double), cudaMemcpyDeviceToHost, s));
   BB_CUDA(cudaStreamSynchronize(s));
-  *epoch_loss_host = total / (double)n_batches;
+  *epoch_loss_host = total / (double)((n_rows + batch - 1) / batch);
   return BB_OK;
+}
+
+int epoch_dev(bb_trainer* t, const void* x, int x_is_f64, int64_t n_rows, int batch, const bb_train_hyper* h,
+              double* epoch_loss_host, cudaStream_t s) {
+  if (!t || !h || !x || n_rows < 1 || batch < 1 || !epoch_loss_host) return BB_ERR_INVALID;
+  int rc = check_epoch(t, x_is_f64, batch, h);
+  if (rc != BB_OK) return rc;
+  BB_CUDA(cudaMemsetAsync(t->loss_accum, 0, sizeof(double), s));
+  rc = train_rows(t, x, x_is_f64, n_rows, batch, h, s);
+  return rc != BB_OK ? rc : finish_epoch(t, n_rows, batch, epoch_loss_host, s);
+}
+
+int validate_dev(bb_trainer* t, const void* x, int x_is_f64, int64_t n_rows, int batch, double* epoch_loss_host,
+                 cudaStream_t s) {
+  if (!t || !x || n_rows < 1 || batch < 1 || batch > t->max_batch || !epoch_loss_host) return BB_ERR_INVALID;
+  if (x_is_f64 && t->precision != BB_PREC_FP64) return BB_ERR_INVALID;
+  BB_CUDA(cudaMemsetAsync(t->loss_accum, 0, sizeof(double), s));
+  const int rc = eval_rows(t, x, x_is_f64, n_rows, batch, s);
+  return rc != BB_OK ? rc : finish_epoch(t, n_rows, batch, epoch_loss_host, s);
+}
+
+// bytes per row of a host table of x_dtype for this trainer (0: a dtype it does not take); checks the window
+size_t host_row_bytes(bb_trainer* t, const void* x_host, int x_dtype, int64_t n_rows, int batch, int64_t window_rows) {
+  if (!x_host || n_rows < 1 || batch < 1 || window_rows < batch || window_rows % batch) return 0;
+  if (x_dtype == BB_F32) return (size_t)t->d.dims[0] * sizeof(float);
+  if (x_dtype == BB_F64 && t->precision == BB_PREC_FP64) return (size_t)t->d.dims[0] * sizeof(double);
+  return 0;
 }
 }  // namespace
 
@@ -1224,12 +1320,12 @@ int bb_trainer_step_f64(bb_trainer* t, const double* x_dev, int batch_rows, cons
 
 int bb_trainer_epoch_f64(bb_trainer* t, const double* x_dev, int64_t n_rows, int batch, const bb_train_hyper* h,
                          double* epoch_loss_host, bb_stream_t stream) {
-  return epoch_f64(t, x_dev, 1, n_rows, batch, h, epoch_loss_host, (cudaStream_t)stream);
+  return epoch_dev(t, x_dev, 1, n_rows, batch, h, epoch_loss_host, (cudaStream_t)stream);
 }
 
 int bb_trainer_validate_f64(bb_trainer* t, const double* x_dev, int64_t n_rows, int batch, double* epoch_loss_host,
                             bb_stream_t stream) {
-  return validate_f64(t, x_dev, 1, n_rows, batch, epoch_loss_host, (cudaStream_t)stream);
+  return validate_dev(t, x_dev, 1, n_rows, batch, epoch_loss_host, (cudaStream_t)stream);
 }
 
 int bb_trainer_step(bb_trainer* t, const float* x_dev, int batch_rows, const bb_train_hyper* h, int phase,
@@ -1284,86 +1380,44 @@ int bb_trainer_step(bb_trainer* t, const float* x_dev, int batch_rows, const bb_
 
 int bb_trainer_epoch(bb_trainer* t, const float* x_dev, int64_t n_rows, int batch, const bb_train_hyper* h,
                      double* epoch_loss_host, bb_stream_t stream) {
-  if (!t || !h || !x_dev || n_rows < 1 || batch < 1 || !epoch_loss_host) return BB_ERR_INVALID;
-  if (t->precision == BB_PREC_FP64) return epoch_f64(t, x_dev, 0, n_rows, batch, h, epoch_loss_host, (cudaStream_t)stream);
-  t->started = true;
-  if (h->world_size <= 1 && batch > t->max_batch) return BB_ERR_INVALID;
-  const int dp_world = t->tc ? bb_tc_train_dp_world(t->tc) : 1;
-  if (h->world_size > 1 && h->world_size != dp_world) return BB_ERR_INVALID;  // data parallel needs bb_trainer_dp_connect
-  cudaStream_t s = (cudaStream_t)stream;
-  BB_CUDA(cudaMemsetAsync(t->loss_accum, 0, sizeof(double), s));
-  int64_t n_batches = 0;
-  int urc;
-  if (h->world_size > 1 && (batch + dp_world - 1) / dp_world > t->max_batch) return BB_ERR_INVALID;
-  if (use_tc(t, h, s, &urc)) {
-    // the whole epoch is one persistent kernel: no launch and no host round trip between steps
-    if (urc != BB_OK) return urc;
-    const TcHyper th = tc_hyper(h);
-    n_batches = (n_rows + batch - 1) / batch;
-    t->wt_fresh = false;
-    t->last_tc = true;
-    t->last_rows = (int)(n_rows - (n_batches - 1) * batch);
-    bb_tc_train_set_mode(t->tc, 1, (unsigned long long)t->step);
-    const int rc = bb_tc_train_run(t->tc, x_dev, n_rows, batch, TC_P1 | TC_DW | TC_ADAM, &th, t->step + 1, t->loss_accum,
-                                   h->world_size > 1 ? 1 : 0, s);
-    if (rc != BB_OK) return rc;
-    t->step += n_batches;
-  } else {
-    if (urc != BB_OK) return urc;
-    if (h->world_size > 1) return BB_ERR_UNSUPPORTED;  // the fused exchange lives in the tensor-core kernel
-    for (int64_t r0 = 0; r0 < n_rows; r0 += batch, ++n_batches) {
-      const int rows = (int)(n_rows - r0 < batch ? n_rows - r0 : batch);
-      const int rc = bb_trainer_step(t, x_dev + (size_t)r0 * t->d.dims[0], rows, h, 0, t->loss_accum, s);
-      if (rc != BB_OK) return rc;
-    }
-  }
-  double total = 0.0;
-  BB_CUDA(cudaMemcpyAsync(&total, t->loss_accum, sizeof(double), cudaMemcpyDeviceToHost, s));
-  BB_CUDA(cudaStreamSynchronize(s));
-  *epoch_loss_host = total / (double)n_batches;
-  return BB_OK;
+  return epoch_dev(t, x_dev, 0, n_rows, batch, h, epoch_loss_host, (cudaStream_t)stream);
 }
 
 int bb_trainer_validate(bb_trainer* t, const float* x_dev, int64_t n_rows, int batch, double* epoch_loss_host,
                         bb_stream_t stream) {
-  if (!t || !x_dev || n_rows < 1 || batch < 1 || batch > t->max_batch || !epoch_loss_host) return BB_ERR_INVALID;
+  return validate_dev(t, x_dev, 0, n_rows, batch, epoch_loss_host, (cudaStream_t)stream);
+}
+
+int bb_trainer_epoch_host(bb_trainer* t, const void* x_host, int x_dtype, int64_t n_rows, int batch, const bb_train_hyper* h,
+                          int64_t window_rows, double* epoch_loss_host, bb_stream_t stream) {
+  if (!t || !h || !epoch_loss_host) return BB_ERR_INVALID;
+  const size_t row_bytes = host_row_bytes(t, x_host, x_dtype, n_rows, batch, window_rows);
+  if (!row_bytes) return BB_ERR_INVALID;
+  const int x_is_f64 = x_dtype == BB_F64;
+  int rc = check_epoch(t, x_is_f64, batch, h);
+  if (rc != BB_OK) return rc;
   cudaStream_t s = (cudaStream_t)stream;
-  if (t->precision == BB_PREC_FP64) return validate_f64(t, x_dev, 0, n_rows, batch, epoch_loss_host, s);
+  BB_CUDA(cudaSetDevice(t->ctx->device));
   BB_CUDA(cudaMemsetAsync(t->loss_accum, 0, sizeof(double), s));
-  int64_t n_batches = 0;
-  int urc;
-  const bool tc = use_tc(t, nullptr, s, &urc);
-  if (urc != BB_OK) return urc;
-  if (tc) {
-    TcHyper th;
-    memset(&th, 0, sizeof(th));
-    th.b1d = th.b2d = 0.5;
-    n_batches = (n_rows + batch - 1) / batch;
-    t->last_tc = true;
-    t->last_rows = (int)(n_rows - (n_batches - 1) * batch);
-    bb_tc_train_set_mode(t->tc, 0, 0ull);
-    const int rc = bb_tc_train_run(t->tc, x_dev, n_rows, batch, TC_FWD_ONLY, &th, 1, t->loss_accum, 0, s);
-    if (rc != BB_OK) return rc;
-  }
-  for (int64_t r0 = 0; !tc && r0 < n_rows; r0 += batch, ++n_batches) {
-    const int rows = (int)(n_rows - r0 < batch ? n_rows - r0 : batch);
-    t->last_tc = false;
-    int rc = t->kind == 1 ? launch_dbn(t, x_dev + (size_t)r0 * t->d.dims[0], rows, 1, s)
-                          : launch_fwd_bwd(t, x_dev + (size_t)r0 * t->d.dims[0], rows, 0, nullptr, s);
-    if (rc != BB_OK) return rc;
-    // mode 1 with zero splits: only folds the loss partials into the gradient's loss slot ...
-    train_adam_kernel<<<1, NT, 0, s>>>(0, 1, t->partial, 0, t->grads + t->d.n_params, nullptr, nullptr, nullptr, nullptr,
-                                       nullptr, 0.f, 0.f, 0.f, 0.f, 0.f, t->loss_part, (rows + RT - 1) / RT, nullptr);
-    // ... and mode 2 with zero parameters adds that slot to the accumulator
-    train_adam_kernel<<<1, NT, 0, s>>>(0, 2, nullptr, 0, t->grads + t->d.n_params, nullptr, nullptr, nullptr, nullptr,
-                                       nullptr, 0.f, 0.f, 0.f, 0.f, 0.f, nullptr, 0, t->loss_accum);
-    BB_CUDA(cudaGetLastError());
-  }
-  double total = 0.0;
-  BB_CUDA(cudaMemcpyAsync(&total, t->loss_accum, sizeof(double), cudaMemcpyDeviceToHost, s));
-  BB_CUDA(cudaStreamSynchronize(s));
-  *epoch_loss_host = total / (double)n_batches;
-  return BB_OK;
+  rc = bb_host_window_run(&t->win, x_host, row_bytes, n_rows, window_rows, s, [&](const void* x, int64_t rows) {
+    return train_rows(t, x, x_is_f64, rows, batch, h, s);
+  });
+  return rc != BB_OK ? rc : finish_epoch(t, n_rows, batch, epoch_loss_host, s);
+}
+
+int bb_trainer_validate_host(bb_trainer* t, const void* x_host, int x_dtype, int64_t n_rows, int batch, int64_t window_rows,
+                             double* epoch_loss_host, bb_stream_t stream) {
+  if (!t || !epoch_loss_host || batch > t->max_batch) return BB_ERR_INVALID;
+  const size_t row_bytes = host_row_bytes(t, x_host, x_dtype, n_rows, batch, window_rows);
+  if (!row_bytes) return BB_ERR_INVALID;
+  const int x_is_f64 = x_dtype == BB_F64;
+  cudaStream_t s = (cudaStream_t)stream;
+  BB_CUDA(cudaSetDevice(t->ctx->device));
+  BB_CUDA(cudaMemsetAsync(t->loss_accum, 0, sizeof(double), s));
+  const int rc = bb_host_window_run(&t->win, x_host, row_bytes, n_rows, window_rows, s, [&](const void* x, int64_t rows) {
+    return eval_rows(t, x, x_is_f64, rows, batch, s);
+  });
+  return rc != BB_OK ? rc : finish_epoch(t, n_rows, batch, epoch_loss_host, s);
 }
 
 int bb_trainer_activation_means(bb_trainer* t, double* out) {

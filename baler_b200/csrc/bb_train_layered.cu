@@ -476,6 +476,7 @@ struct bb_ltrainer {
   bool dbn = false;
   unsigned long long seed = 0;
   const unsigned char* mask_dev[4] = {nullptr, nullptr, nullptr, nullptr};
+  HostWindow* win = nullptr;              // device window of bb_ltrainer_epoch_host / _validate_host (kept between calls)
 };
 
 namespace {
@@ -834,6 +835,7 @@ int bb_ltrainer_destroy(bb_ltrainer* t) {
     for (void* p : lp)
       if (p) cudaFree(p);
   }
+  bb_host_window_free(t->win);
   delete t;
   return BB_OK;
 }
@@ -928,34 +930,25 @@ int bb_ltrainer_step_swae(bb_ltrainer* t, const float* x_dev, int batch_rows, co
   return lstep(t, x_dev, batch_rows, h, phase, loss_accum_dev, stream, &sw);
 }
 
-int bb_ltrainer_epoch(bb_ltrainer* t, const float* x_dev, int64_t n_rows, int batch, const bb_train_hyper* h,
-                      double* epoch_loss_host, bb_stream_t stream) {
-  if (!t || !h || !x_dev || n_rows < 1 || batch < 1 || batch > t->max_batch || !epoch_loss_host) return BB_ERR_INVALID;
-  if (h->world_size > 1) return BB_ERR_INVALID;
-  cudaStream_t s = (cudaStream_t)stream;
-  BB_CUDA(cudaMemsetAsync(t->loss_accum, 0, sizeof(double), s));
-  int64_t n_batches = 0;
-  for (int64_t r0 = 0; r0 < n_rows; r0 += batch, ++n_batches) {
+}  // extern "C"
+
+namespace {
+// the training steps of the batches of rows [0, n_rows) of x in order, their losses added to t->loss_accum: the body of an
+// epoch over a device table and of every window of a streamed host table (windows hold whole batches)
+int ltrain_rows(bb_ltrainer* t, const float* x, int64_t n_rows, int batch, const bb_train_hyper* h, cudaStream_t s) {
+  for (int64_t r0 = 0; r0 < n_rows; r0 += batch) {
     const int rows = (int)(n_rows - r0 < batch ? n_rows - r0 : batch);
-    const int rc = bb_ltrainer_step(t, x_dev + (size_t)r0 * t->lay[0].K, rows, h, 0, t->loss_accum, s);
+    const int rc = bb_ltrainer_step(t, x + (size_t)r0 * t->lay[0].K, rows, h, 0, t->loss_accum, s);
     if (rc != BB_OK) return rc;
   }
-  double total = 0.0;
-  BB_CUDA(cudaMemcpyAsync(&total, t->loss_accum, sizeof(double), cudaMemcpyDeviceToHost, s));
-  BB_CUDA(cudaStreamSynchronize(s));
-  *epoch_loss_host = total / (double)n_batches;
   return BB_OK;
 }
 
-int bb_ltrainer_validate(bb_ltrainer* t, const float* x_dev, int64_t n_rows, int batch, double* epoch_loss_host,
-                         bb_stream_t stream) {
-  if (!t || !x_dev || n_rows < 1 || batch < 1 || batch > t->max_batch || !epoch_loss_host) return BB_ERR_INVALID;
-  cudaStream_t s = (cudaStream_t)stream;
-  BB_CUDA(cudaMemsetAsync(t->loss_accum, 0, sizeof(double), s));
-  int64_t n_batches = 0;
-  for (int64_t r0 = 0; r0 < n_rows; r0 += batch, ++n_batches) {
+// the eval-mode forward passes of the same batches, their losses added to t->loss_accum
+int leval_rows(bb_ltrainer* t, const float* x, int64_t n_rows, int batch, cudaStream_t s) {
+  for (int64_t r0 = 0; r0 < n_rows; r0 += batch) {
     const int rows = (int)(n_rows - r0 < batch ? n_rows - r0 : batch);
-    int rc = lforward_backward(t, x_dev + (size_t)r0 * t->lay[0].K, rows, false, s);
+    int rc = lforward_backward(t, x + (size_t)r0 * t->lay[0].K, rows, false, s);
     if (rc != BB_OK) return rc;
     // mode 1 folds the loss partials into grads[n_params]; mode 2 with zero parameters adds that slot to the accumulator
     ladam_kernel<<<1, 256, 0, s>>>(t->n_params, 1, t->grads, nullptr, nullptr, nullptr, 0.f, 0.f, 0.f, 0.f, 0.f, t->loss_part,
@@ -964,11 +957,72 @@ int bb_ltrainer_validate(bb_ltrainer* t, const float* x_dev, int64_t n_rows, int
                                    t->loss_accum);
     BB_CUDA(cudaGetLastError());
   }
+  return BB_OK;
+}
+
+// epoch loss = the summed batch losses over the number of batches (training.py:99); synchronises s
+int lfinish(bb_ltrainer* t, int64_t n_rows, int batch, double* epoch_loss_host, cudaStream_t s) {
   double total = 0.0;
   BB_CUDA(cudaMemcpyAsync(&total, t->loss_accum, sizeof(double), cudaMemcpyDeviceToHost, s));
   BB_CUDA(cudaStreamSynchronize(s));
-  *epoch_loss_host = total / (double)n_batches;
+  *epoch_loss_host = total / (double)((n_rows + batch - 1) / batch);
   return BB_OK;
+}
+
+// a host table this trainer streams: float32 rows, a window of whole batches
+bool lhost_ok(bb_ltrainer* t, const void* x_host, int x_dtype, int64_t n_rows, int batch, int64_t window_rows,
+              const double* epoch_loss_host) {
+  return t && x_host && x_dtype == BB_F32 && n_rows >= 1 && batch >= 1 && batch <= t->max_batch && window_rows >= batch &&
+         window_rows % batch == 0 && epoch_loss_host;
+}
+}  // namespace
+
+extern "C" {
+
+int bb_ltrainer_epoch(bb_ltrainer* t, const float* x_dev, int64_t n_rows, int batch, const bb_train_hyper* h,
+                      double* epoch_loss_host, bb_stream_t stream) {
+  if (!t || !h || !x_dev || n_rows < 1 || batch < 1 || batch > t->max_batch || !epoch_loss_host) return BB_ERR_INVALID;
+  if (h->world_size > 1) return BB_ERR_INVALID;
+  cudaStream_t s = (cudaStream_t)stream;
+  BB_CUDA(cudaMemsetAsync(t->loss_accum, 0, sizeof(double), s));
+  const int rc = ltrain_rows(t, x_dev, n_rows, batch, h, s);
+  return rc != BB_OK ? rc : lfinish(t, n_rows, batch, epoch_loss_host, s);
+}
+
+int bb_ltrainer_validate(bb_ltrainer* t, const float* x_dev, int64_t n_rows, int batch, double* epoch_loss_host,
+                         bb_stream_t stream) {
+  if (!t || !x_dev || n_rows < 1 || batch < 1 || batch > t->max_batch || !epoch_loss_host) return BB_ERR_INVALID;
+  cudaStream_t s = (cudaStream_t)stream;
+  BB_CUDA(cudaMemsetAsync(t->loss_accum, 0, sizeof(double), s));
+  const int rc = leval_rows(t, x_dev, n_rows, batch, s);
+  return rc != BB_OK ? rc : lfinish(t, n_rows, batch, epoch_loss_host, s);
+}
+
+int bb_ltrainer_epoch_host(bb_ltrainer* t, const void* x_host, int x_dtype, int64_t n_rows, int batch,
+                           const bb_train_hyper* h, int64_t window_rows, double* epoch_loss_host, bb_stream_t stream) {
+  if (!h || !lhost_ok(t, x_host, x_dtype, n_rows, batch, window_rows, epoch_loss_host)) return BB_ERR_INVALID;
+  if (h->world_size > 1) return BB_ERR_INVALID;
+  cudaStream_t s = (cudaStream_t)stream;
+  BB_CUDA(cudaSetDevice(t->ctx->device));
+  BB_CUDA(cudaMemsetAsync(t->loss_accum, 0, sizeof(double), s));
+  const size_t row_bytes = (size_t)t->lay[0].K * sizeof(float);
+  const int rc = bb_host_window_run(&t->win, x_host, row_bytes, n_rows, window_rows, s, [&](const void* x, int64_t rows) {
+    return ltrain_rows(t, (const float*)x, rows, batch, h, s);
+  });
+  return rc != BB_OK ? rc : lfinish(t, n_rows, batch, epoch_loss_host, s);
+}
+
+int bb_ltrainer_validate_host(bb_ltrainer* t, const void* x_host, int x_dtype, int64_t n_rows, int batch,
+                              int64_t window_rows, double* epoch_loss_host, bb_stream_t stream) {
+  if (!lhost_ok(t, x_host, x_dtype, n_rows, batch, window_rows, epoch_loss_host)) return BB_ERR_INVALID;
+  cudaStream_t s = (cudaStream_t)stream;
+  BB_CUDA(cudaSetDevice(t->ctx->device));
+  BB_CUDA(cudaMemsetAsync(t->loss_accum, 0, sizeof(double), s));
+  const size_t row_bytes = (size_t)t->lay[0].K * sizeof(float);
+  const int rc = bb_host_window_run(&t->win, x_host, row_bytes, n_rows, window_rows, s, [&](const void* x, int64_t rows) {
+    return leval_rows(t, (const float*)x, rows, batch, s);
+  });
+  return rc != BB_OK ? rc : lfinish(t, n_rows, batch, epoch_loss_host, s);
 }
 
 }  // extern "C"

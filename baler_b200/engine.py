@@ -94,6 +94,16 @@ def colminmax(x, ctx=None):
     return mn, mx
 
 
+def _host_table(x, window_rows, batch):
+    """(pointer, BB dtype) of a C-contiguous 2-D float32 / float64 numpy table streamed through device windows of
+    `window_rows` rows (bb_*_epoch_host: a positive multiple of the batch)"""
+    if not (isinstance(x, np.ndarray) and x.ndim == 2 and x.flags.c_contiguous and x.dtype in (np.float32, np.float64)):
+        raise ValueError("a host table is a C-contiguous 2-D float32 / float64 numpy array")
+    if window_rows is None or window_rows < batch or window_rows % batch:
+        raise ValueError("window_rows must be a positive multiple of the batch (%d), not %r" % (batch, window_rows))
+    return x.ctypes.data, _NP2BB[x.dtype]
+
+
 def fp64_refusal(chains):
     """None when the float64 kernel takes every chain in `chains` ({name: [width of each layer boundary]}), else the
     message of the NotImplementedError precision "fp64" raises for it"""
@@ -456,14 +466,27 @@ class Trainer:
         ptr, fn, name = self._x(x, "bb_trainer_step")
         check(fn(self.handle, ptr, x.shape[0], C.byref(hyper), phase, _ptr(self.loss_accum), _stream(self.ctx)), name)
 
-    def epoch(self, x, batch, hyper):
+    def epoch(self, x, batch, hyper, window_rows=None):
+        """one epoch over a CUDA table, or over a C-contiguous numpy table streamed through two device windows of
+        `window_rows` rows (a multiple of `batch`; bb_trainer_epoch_host): the same steps, bit for bit"""
         out = C.c_double()
+        if isinstance(x, np.ndarray):
+            ptr, dt = _host_table(x, window_rows, batch)
+            check(_lib.lib().bb_trainer_epoch_host(self.handle, ptr, dt, x.shape[0], batch, C.byref(hyper), int(window_rows),
+                                                   C.byref(out), _stream(self.ctx)), "bb_trainer_epoch_host")
+            return out.value
         ptr, fn, name = self._x(x, "bb_trainer_epoch")
         check(fn(self.handle, ptr, x.shape[0], batch, C.byref(hyper), C.byref(out), _stream(self.ctx)), name)
         return out.value
 
-    def validate(self, x, batch):
+    def validate(self, x, batch, window_rows=None):
+        """validate over a CUDA table, or a numpy table streamed as in epoch()"""
         out = C.c_double()
+        if isinstance(x, np.ndarray):
+            ptr, dt = _host_table(x, window_rows, batch)
+            check(_lib.lib().bb_trainer_validate_host(self.handle, ptr, dt, x.shape[0], batch, int(window_rows), C.byref(out),
+                                                      _stream(self.ctx)), "bb_trainer_validate_host")
+            return out.value
         ptr, fn, name = self._x(x, "bb_trainer_validate")
         check(fn(self.handle, ptr, x.shape[0], batch, C.byref(out), _stream(self.ctx)), name)
         return out.value
@@ -646,14 +669,25 @@ class LayeredTrainer:
                                                proj.shape[0], latent_layer, float(reg_weight), _ptr(self.loss_accum),
                                                _stream(self.ctx)), "bb_ltrainer_step_swae")
 
-    def epoch(self, x, batch, hyper):
+    def epoch(self, x, batch, hyper, window_rows=None):
+        """Trainer.epoch: a CUDA table, or a float32 numpy table streamed in windows (bb_ltrainer_epoch_host)"""
         out = C.c_double()
+        if isinstance(x, np.ndarray):
+            ptr, dt = _host_table(x, window_rows, batch)
+            check(_lib.lib().bb_ltrainer_epoch_host(self.handle, ptr, dt, x.shape[0], batch, C.byref(hyper), int(window_rows),
+                                                    C.byref(out), _stream(self.ctx)), "bb_ltrainer_epoch_host")
+            return out.value
         check(_lib.lib().bb_ltrainer_epoch(self.handle, _ptr(x), x.shape[0], batch, C.byref(hyper), C.byref(out),
                                            _stream(self.ctx)), "bb_ltrainer_epoch")
         return out.value
 
-    def validate(self, x, batch):
+    def validate(self, x, batch, window_rows=None):
         out = C.c_double()
+        if isinstance(x, np.ndarray):
+            ptr, dt = _host_table(x, window_rows, batch)
+            check(_lib.lib().bb_ltrainer_validate_host(self.handle, ptr, dt, x.shape[0], batch, int(window_rows),
+                                                       C.byref(out), _stream(self.ctx)), "bb_ltrainer_validate_host")
+            return out.value
         check(_lib.lib().bb_ltrainer_validate(self.handle, _ptr(x), x.shape[0], batch, C.byref(out), _stream(self.ctx)),
               "bb_ltrainer_validate")
         return out.value

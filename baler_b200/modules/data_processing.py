@@ -76,14 +76,46 @@ def normalize_float64_host(flat, mn, rg, out_dtype=np.float64):
         return ((np.asarray(flat, dtype=np.float64) - mn) / rg).astype(out_dtype, copy=False)
 
 
+# Device buffer of the row-chunked preprocessing passes: find_minmax / normalize / minmax_normalize_f64 / renormalize_func
+# upload the table in chunks of at most this many bytes, so a table larger than device memory is preprocessed too
+PREPROCESS_CHUNK_BYTES = 1 << 28
+
+
+def _row_chunks(flat):
+    """(r0, rows) of the row chunks of a C-contiguous 2-D host table (one empty chunk for an empty table)"""
+    rows = max(1, PREPROCESS_CHUNK_BYTES // max(1, flat.shape[1] * flat.itemsize))
+    return [(r0, flat[r0:r0 + rows]) for r0 in range(0, len(flat), rows)] or [(0, flat)]
+
+
 def _minmax_dev(flat):
-    x = torch.from_numpy(flat).cuda()
-    mn, mx = engine.colminmax(x)
-    return x, mn, mx
+    """(device table or None, column min, column max) of a C-contiguous host table.  Per-chunk min / max, combined by the
+    same kernel over the stacked chunk results (min of mins, max of maxes: exact, -0 < +0 and NaN kept as in one pass).
+    A table of one chunk stays on the device for the caller's second pass."""
+    chunks = _row_chunks(flat)
+    mins, maxs, x = [], [], None
+    for _, c in chunks:
+        x = torch.from_numpy(c).cuda()
+        mn, mx = engine.colminmax(x)
+        mins.append(mn)
+        maxs.append(mx)
+    if len(chunks) == 1:
+        return x, mins[0], maxs[0]
+    return None, engine.colminmax(torch.stack(mins))[0], engine.colminmax(torch.stack(maxs))[1]
+
+
+def _map_chunks(flat, x, fn, out_dtype):
+    """host array of fn(device chunk) over the row chunks of `flat` (x: the device copy of a one-chunk table, or None)"""
+    if x is not None:
+        return fn(x).cpu().numpy()
+    out = np.empty(flat.shape, dtype=out_dtype)
+    for r0, c in _row_chunks(flat):
+        out[r0:r0 + len(c)] = fn(torch.from_numpy(c).cuda()).cpu().numpy()
+    return out
 
 
 def find_minmax(data):
-    """[min; max - min] per column (reference data_processing.py:113-130), computed on the GPU.
+    """[min; max - min] per column (reference data_processing.py:113-130), computed on the GPU in row chunks of at most
+    PREPROCESS_CHUNK_BYTES.
     float32 arithmetic: exact for float32 / small-integer tables (what the CMS path feeds); float64 tables whose offset
     dwarfs their spread get exact float64 statistics from the host (float64_stats)."""
     arr = np.asarray(data)
@@ -113,29 +145,29 @@ def normalize(data, custom_norm):
             return normalize_float64_host(flat64, st[0], st[1]).reshape(arr.shape)
     arr, flat = _table(data)
     x, mn, mx = _minmax_dev(flat)
-    out = engine.normalize_table(x, mn, mx - mn).cpu().numpy()  # max - min: one float32 subtraction per column
-    out = out.reshape(arr.shape)
+    rg = mx - mn  # one float32 subtraction per column
+    out = _map_chunks(flat, x, lambda c: engine.normalize_table(c, mn, rg, out=c), np.float32).reshape(arr.shape)
     return out if arr.dtype == np.float32 else engine.host_convert(out, np.float64)
 
 
 def minmax_normalize_f64(data, normalise=True):
     """precision "fp64" on a float64 table: ([min; max - min] exact in float64, the table normalised in float64 on the
     device when `normalise`, else as it is) - what the reference's float64 numpy computes (data_processing.py:113-153),
-    bit for bit, with no float32 step and no host pass over the table"""
+    bit for bit, with no float32 step and no host pass over the table; row chunks as find_minmax"""
     engine.require_cuda()
     arr = np.asarray(data)
     assert arr.dtype == np.float64
     flat = np.ascontiguousarray(arr.reshape(arr.shape[0], -1) if arr.ndim > 1 else arr.reshape(-1, 1))
-    x = torch.from_numpy(flat).cuda()
-    mn, mx = engine.colminmax(x)
+    x, mn, mx = _minmax_dev(flat)
     mn_h, mx_h = mn.cpu().numpy(), mx.cpu().numpy()
     rg_h = mx_h - mn_h  # one float64 subtraction per column, as numpy
     feats = np.array([mn_h, rg_h])
     feats = feats.reshape((2,) + arr.shape[1:]) if arr.ndim > 1 else feats.reshape(2)
     if not normalise:
         return feats, arr
-    out = engine.normalize_table_f64(x, mn, torch.from_numpy(rg_h).cuda(), out=x)
-    return feats, out.cpu().numpy().reshape(arr.shape)
+    rg = torch.from_numpy(rg_h).cuda()
+    out = _map_chunks(flat, x, lambda c: engine.normalize_table_f64(c, mn, rg, out=c), np.float64)
+    return feats, out.reshape(arr.shape)
 
 
 def renormalize_std(input_data, true_min, feature_range):
@@ -152,8 +184,7 @@ def renormalize_func(norm_data, min_list, range_list):
         flat64 = (arr.reshape(arr.shape[0], -1) if arr.ndim > 1 else arr.reshape(-1, 1)).astype(np.float64)
         return (flat64 * rg64 + mn64).reshape(arr.shape)
     arr, flat = _table(norm_data)
-    x = torch.from_numpy(flat).cuda()
     mn = torch.as_tensor(np.asarray(min_list, dtype=np.float32).reshape(-1)).cuda()
     rg = torch.as_tensor(np.asarray(range_list, dtype=np.float32).reshape(-1)).cuda()
-    out = engine.normalize_table(x, mn, rg, inverse=True).cpu().numpy()
+    out = _map_chunks(flat, None, lambda c: engine.normalize_table(c, mn, rg, inverse=True, out=c), np.float32)
     return engine.host_convert(out, np.float64).reshape(arr.shape)

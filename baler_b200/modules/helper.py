@@ -38,6 +38,9 @@ class Config:
                        other precision the key is refused
       latent_dtype     "float64" (AE default, what the reference writes; any model under "fp64") | "float32" | "float16"
       l1_in_training   bool: add reg_param * L1 chain to the training loss (dead code upstream, SURVEY F2)
+    No key is needed for tables larger than device memory: --mode train normalises the table in row chunks, keeps it
+    resident when it fits the device memory the trainer leaves (training.device_table_budget), and otherwise streams
+    every epoch and validation from host memory through two device windows of whole batches, with the same results.
     """
 
     model_type = str  # reference helper.py:163: defaults to the *type* `str`

@@ -118,12 +118,37 @@ def consume_loader_seed(n_rows, batch_size):
     iter(torch.utils.data.DataLoader(range(n_rows), batch_size=batch_size, shuffle=False))
 
 
-class DeviceBatches:
-    """Stands in for the reference's DataLoader(shuffle=False, drop_last=False) (training.py:253-263):
-    the whole (normalised, float32) table resident in HBM plus the batch size."""
+# Device memory kept free of training tables (torch's allocator, the library's per-call scratch, other work on the GPU)
+DEVICE_TABLE_RESERVE = 1 << 30
+# Largest device window of a streamed table, per slot.  The upload of the first window is not overlapped with training, so
+# windows are kept well below what the budget would allow: 256 MiB is ~10 ms of PCIe and millions of rows per window.
+STREAM_WINDOW_MAX_BYTES = 1 << 28
 
-    def __init__(self, data, batch_size):
-        self.data, self.batch_size = data, int(batch_size)
+
+def device_table_budget():
+    """bytes of device memory the training tables may take: what cudaMemGetInfo reports free (once the trainer and its
+    scratch exist) less DEVICE_TABLE_RESERVE"""
+    free, _ = torch.cuda.mem_get_info()
+    return max(0, free - DEVICE_TABLE_RESERVE)
+
+
+def stream_window_rows(row_bytes, batch_size, budget):
+    """rows of each of the two device windows a streamed table of `row_bytes` rows gets from `budget` bytes: the largest
+    multiple of the batch that fits twice, up to STREAM_WINDOW_MAX_BYTES per window.  MemoryError below one batch."""
+    rows = min(budget // 2, STREAM_WINDOW_MAX_BYTES) // row_bytes // batch_size * batch_size
+    if rows < batch_size:
+        raise MemoryError("device memory left for the training table (%d bytes) does not hold two batches of %d rows of %d "
+                          "bytes" % (budget, batch_size, row_bytes))
+    return int(rows)
+
+
+class DeviceBatches:
+    """Stands in for the reference's DataLoader(shuffle=False, drop_last=False) (training.py:253-263): the (normalised)
+    table plus the batch size.  The table is a CUDA tensor resident in HBM (window_rows None), or a C-contiguous numpy
+    array in host memory that every pass streams through two device windows of window_rows rows."""
+
+    def __init__(self, data, batch_size, window_rows=None):
+        self.data, self.batch_size, self.window_rows = data, int(batch_size), window_rows
 
     def __len__(self):
         return (self.data.shape[0] + self.batch_size - 1) // self.batch_size
@@ -196,19 +221,20 @@ class DeviceAdam:
         return engine.make_hyper(lr=self.lr, reg_param=self.reg_param, l1=self.l1,
                                  world_size=self.world if world_size is None else world_size)
 
-    def epoch(self, data, batch_size):
-        """one pass over `data` in the reference's batch order; data-parallel when launched with several ranks"""
+    def epoch(self, data, batch_size, window_rows=None):
+        """one pass over `data` in the reference's batch order; data-parallel when launched with several ranks.  A numpy
+        `data` streams from host memory in windows of `window_rows` rows (DeviceBatches)"""
         self.steps += (data.shape[0] + batch_size - 1) // batch_size
         if self.torch_stream:
             # the reference's fit iterates a fresh iter(train_dl) (one draw for its base seed), then draws every mask
             consume_loader_seed(data.shape[0], batch_size)
             self.trainer.set_dropout_torch()
-            loss = self.trainer.epoch(data, batch_size, self.hyper())
+            loss = self.trainer.epoch(data, batch_size, self.hyper(), window_rows)
             self.trainer.write_back_dropout_torch()
             return loss
         if self.dp is None:
-            return self.trainer.epoch(data, batch_size, self.hyper())
-        return self.dp.epoch_table(data, batch_size, self.hyper(), self.rank, self.world)
+            return self.trainer.epoch(data, batch_size, self.hyper(), window_rows)
+        return self.dp.epoch_table(data, batch_size, self.hyper(), self.rank, self.world, window_rows)
 
     SWAE_PROJECTIONS, SWAE_REG_WEIGHT = 2000, 100.0  # defaults of utils.loss_function_swae (utils.py:27-36)
 
@@ -222,6 +248,8 @@ class DeviceAdam:
         n_batches = 0
         for r0 in range(0, data.shape[0], batch_size):
             xb = data[r0:r0 + batch_size]
+            if isinstance(xb, np.ndarray):  # a table in host memory: one batch on the device at a time
+                xb = torch.from_numpy(np.ascontiguousarray(xb)).to(tr.loss_accum.device)
             prior = torch.randn((xb.shape[0], latent_dim), dtype=torch.float32)
             proj = torch.randn(self.SWAE_PROJECTIONS, latent_dim)
             proj = proj / proj.norm(dim=1).view(-1, 1)
@@ -251,7 +279,7 @@ def fit(config, model, train_dl, model_children, regular_param, optimizer, laten
     if hasattr(config, "custom_loss_function") and config.custom_loss_function == "loss_function_swae":
         epoch_loss = optimizer.epoch_swae(train_dl.data, train_dl.batch_size, latent_dim)
     else:
-        epoch_loss = optimizer.epoch(train_dl.data, train_dl.batch_size)
+        epoch_loss = optimizer.epoch(train_dl.data, train_dl.batch_size, train_dl.window_rows)
     print(f"# Finished. Training Loss: {epoch_loss:.6f}")
     return epoch_loss, epoch_loss, 0, model
 
@@ -262,22 +290,44 @@ def validate(model, test_dl, model_children, reg_param, optimizer=None):
     model.eval()
     if getattr(optimizer, "torch_stream", False):
         consume_loader_seed(test_dl.data.shape[0], test_dl.batch_size)  # the reference's iter(test_dl)
-    epoch_loss = optimizer.trainer.validate(test_dl.data, test_dl.batch_size)
+    epoch_loss = optimizer.trainer.validate(test_dl.data, test_dl.batch_size, test_dl.window_rows)
     print(f"# Finished. Validation Loss: {epoch_loss:.6f}")
     return epoch_loss
 
 
-def _to_device_table(data, config):
-    """the (normalised) table on the device: float32, or float64 as it is under precision "fp64" (the float64 step widens
-    a float32 table exactly, as the reference's torch.tensor(..., float64) does, training.py:230)"""
+def _refuse_table_model(config):
+    if config.data_dimension == 2 and config.model_type == "convolutional" and config.model_name != "Conv_AE":
+        raise NotImplementedError("convolutional models other than Conv_AE: see DESIGN.md (out of scope)")
+
+
+def _training_table(data, config):
+    """the (normalised) table as the trainers read it, in host memory: C-contiguous rows of float32, or float64 as it is
+    under precision "fp64" (the float64 step widens a float32 table exactly, as the reference's torch.tensor(...,
+    float64) does, training.py:230)"""
     arr = np.asarray(data)
     dtype = np.float64 if is_fp64(getattr(config, "precision", None)) and arr.dtype == np.float64 else np.float32
     if config.data_dimension == 2:
-        if config.model_type == "convolutional" and config.model_name != "Conv_AE":
-            raise NotImplementedError("convolutional models other than Conv_AE: see DESIGN.md (out of scope)")
+        _refuse_table_model(config)
         # dense: (N, H * W) rows (training.py:195-204); Conv_AE: (N, 1, H, W) batches (:222-228), the same memory
         arr = arr.reshape(arr.shape[0], arr.shape[1] * arr.shape[2])
-    return torch.from_numpy(np.ascontiguousarray(arr, dtype=dtype)).cuda()
+    return np.ascontiguousarray(arr, dtype=dtype)
+
+
+def _to_device_table(data, config):
+    """the (normalised) table resident on the device (_training_table's rows)"""
+    return torch.from_numpy(_training_table(data, config)).cuda()
+
+
+def _place_table(data, config, batch_size, budget, window_rows=None):
+    """(table, window_rows, device bytes it holds): the table resident on the device when it fits `budget` bytes, else
+    the host table streamed in windows - `window_rows` when given (the windows another streamed table already holds),
+    else the largest the budget allows (stream_window_rows).  Both run the same steps and give the same bits."""
+    arr = _training_table(data, config)
+    if arr.nbytes <= budget:
+        return _to_device_table(data, config), None, arr.nbytes
+    row_bytes = max(1, arr.strides[0])
+    window_rows = window_rows or stream_window_rows(row_bytes, batch_size, budget)
+    return arr, window_rows, 2 * window_rows * row_bytes
 
 
 def train(model, variables, train_data, test_data, project_path, config):
@@ -293,9 +343,7 @@ def train(model, variables, train_data, test_data, project_path, config):
         torch.manual_seed(0)
         np.random.seed(0)
     bs = config.batch_size
-    train_ds = _to_device_table(train_data, config)
-    valid_ds = train_ds if test_data is train_data else _to_device_table(test_data, config)
-    train_dl, valid_dl = DeviceBatches(train_ds, bs), DeviceBatches(valid_ds, bs)
+    _refuse_table_model(config)  # before the trainer is built
     model_children = list(model.children())
     conv = config.data_dimension == 2 and config.model_type == "convolutional"
     optimizer = DeviceAdam(model, config.lr, max_batch=bs, l1=bool(getattr(config, "l1_in_training", False)),
@@ -304,6 +352,14 @@ def train(model, variables, train_data, test_data, project_path, config):
                            swae=getattr(config, "custom_loss_function", None) == "loss_function_swae",
                            precision=getattr(config, "precision", None),
                            dropout_stream=getattr(config, "dropout_stream", None))
+    # tables that fit the device memory the trainer left are resident; larger ones stream from host memory
+    budget = device_table_budget()
+    train_ds, train_win, used = _place_table(train_data, config, bs, budget)
+    if test_data is train_data:
+        valid_ds, valid_win = train_ds, train_win
+    else:
+        valid_ds, valid_win, _ = _place_table(test_data, config, bs, budget - used, train_win)
+    train_dl, valid_dl = DeviceBatches(train_ds, bs, train_win), DeviceBatches(valid_ds, bs, valid_win)
     early_stopping = utils.EarlyStopping(config.early_stopping_patience, config.min_delta) if config.early_stopping else None
     lr_scheduler = utils.LRScheduler(optimizer, config.lr_scheduler_patience) if config.lr_scheduler else None
     train_loss, val_loss = [], []

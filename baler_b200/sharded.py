@@ -8,6 +8,7 @@ contiguous sub-batches; the flat gradient (+ batch loss in its last slot) is all
 not mean - because the reference loss is a sum over rows (utils.py:195-199), then every rank applies
 the identical Adam step.
 """
+import numpy as np
 import torch
 import torch.distributed as dist
 
@@ -108,23 +109,31 @@ class DataParallelTrainer:
     def _dummy(self, x_local):
         return torch.zeros((1, x_local.shape[1]), dtype=x_local.dtype, device=x_local.device)
 
-    def epoch_table(self, data, batch_size, hyper, rank, world):
-        """one pass over the full (replicated) table in global batches of `batch_size`; returns the epoch loss"""
+    def epoch_table(self, data, batch_size, hyper, rank, world, window_rows=None):
+        """one pass over the full (replicated) table in global batches of `batch_size`; returns the epoch loss.  `data` is
+        a CUDA table, or a numpy table in host memory (streamed in windows of `window_rows` rows by the fused step, one
+        slice at a time otherwise)"""
         if self.fused:
             # the library returns this rank's share of every batch loss; one reduction per epoch completes the sum
-            loss = torch.tensor([self.trainer.epoch(data, batch_size, hyper)], dtype=torch.float64, device=data.device)
+            loss = torch.tensor([self.trainer.epoch(data, batch_size, hyper, window_rows)], dtype=torch.float64,
+                                device=self.grads.device)
             dist.all_reduce(loss, op=dist.ReduceOp.SUM, group=self.group)
             return loss.item()
         slices = dp_batch_slices(data.shape[0], batch_size, rank, world)
-        return self.epoch([data[lo:hi] for lo, hi in slices], hyper)
+        return self.epoch((data[lo:hi] for lo, hi in slices), hyper)
 
     def epoch(self, x_local_batches, hyper):
-        """x_local_batches: list of this rank's slices, one per global batch; returns the epoch loss"""
+        """x_local_batches: this rank's slices, one per global batch (CUDA tensors, or numpy arrays uploaded one at a
+        time); returns the epoch loss"""
         self.trainer.loss_accum.zero_()
+        n = 0
         for xb in x_local_batches:
+            if not isinstance(xb, torch.Tensor):
+                xb = torch.from_numpy(np.ascontiguousarray(xb)).to(self.grads.device)
             self.step(xb, hyper)
+            n += 1
         self.sync_running_stats()
-        return self.trainer.loss_accum.item() / max(len(x_local_batches), 1)
+        return self.trainer.loss_accum.item() / max(n, 1)
 
 
 def global_minmax(shard, group=None):

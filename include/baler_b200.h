@@ -366,6 +366,24 @@ int bb_trainer_epoch_f64(bb_trainer* t, const double* x_dev, int64_t n_rows, int
                          const bb_train_hyper* h, double* epoch_loss_host, bb_stream_t stream);
 int bb_trainer_validate_f64(bb_trainer* t, const double* x_dev, int64_t n_rows, int batch,
                             double* epoch_loss_host, bb_stream_t stream);
+/*
+ * bb_trainer_epoch / _validate (and their _f64 forms) on a HOST table, for tables larger than device memory: the reference
+ * trains on the CPU (training.py:253-263), so it takes whatever fits in host memory.  x_host is row-major n_rows x
+ * n_features of x_dtype: BB_F32, or BB_F64 for BB_PREC_FP64 trainers (others: BB_ERR_INVALID).  The library keeps two
+ * device slots of `window_rows` rows (a positive multiple of `batch`, else BB_ERR_INVALID; allocated on first use, kept
+ * until bb_trainer_destroy).  An internal copy stream fills one slot while the epoch's kernels run on `stream` over the
+ * other; events order the reuse of each slot.  A pageable table is staged through two 64 MiB pinned buffers on the
+ * library's worker threads (the table itself is never pinned); a pinned one is copied directly.
+ * Windows are cut at batch boundaries and the step counter runs on across them (Philox dropout keys, Adam's bias
+ * correction, data-parallel packet tags), the torch-stream masks are drawn per batch in order, batch losses go into the
+ * same device accumulator in batch order, and BatchNorm statistics advance per batch: the results are bit-identical to
+ * the resident calls on the same table, for every trainer and precision (h->world_size > 1 included: every rank passes the
+ * full table and the global batch).  Returns after synchronising `stream`.
+ */
+int bb_trainer_epoch_host(bb_trainer* t, const void* x_host, int x_dtype, int64_t n_rows, int batch, const bb_train_hyper* h,
+                          int64_t window_rows, double* epoch_loss_host, bb_stream_t stream);
+int bb_trainer_validate_host(bb_trainer* t, const void* x_host, int x_dtype, int64_t n_rows, int batch, int64_t window_rows,
+                             double* epoch_loss_host, bb_stream_t stream);
 
 /*
  * Per-node mean activation of the six hidden layers (en1,en2,en3,de1,de2,de3) over the rows of the LAST
@@ -427,6 +445,11 @@ int bb_ltrainer_epoch(bb_ltrainer* t, const float* x_dev, int64_t n_rows, int ba
                       double* epoch_loss_host, bb_stream_t stream);
 int bb_ltrainer_validate(bb_ltrainer* t, const float* x_dev, int64_t n_rows, int batch, double* epoch_loss_host,
                          bb_stream_t stream);
+/* bb_ltrainer_epoch / _validate on a host table, streamed as bb_trainer_epoch_host does (x_dtype BB_F32 only) */
+int bb_ltrainer_epoch_host(bb_ltrainer* t, const void* x_host, int x_dtype, int64_t n_rows, int batch,
+                           const bb_train_hyper* h, int64_t window_rows, double* epoch_loss_host, bb_stream_t stream);
+int bb_ltrainer_validate_host(bb_ltrainer* t, const void* x_host, int x_dtype, int64_t n_rows, int batch,
+                              int64_t window_rows, double* epoch_loss_host, bb_stream_t stream);
 /*
  * AE_Dropout_BN (models.py:256-313) on the layer-by-layer trainer, at any batch size that fits in memory (the fused
  * bb_trainer_create_dbn step needs every tile of a batch resident: 16 rows x SMs on the tensor-core step).  Same
