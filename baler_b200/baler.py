@@ -2,6 +2,7 @@
 
 Keeps the reference's CLI, per-project config files and output layout (reference baler/baler.py:36-456):
   output/compressed_output/model.pt, compressed.npz {data, names, normalization_features}
+    (latent_dtype "q8" adds latent_min, latent_step, latent_block_rows: baler_b200/latent_q8.py)
   output/decompressed_output/decompressed.npz {data, names}
   output/training/normalization_features.npy, loss_data.npy, activations.npy, model_{epoch}.pt
 """
@@ -11,6 +12,7 @@ from math import ceil
 
 import numpy as np
 
+from . import latent_q8
 from .modules import helper
 
 __all__ = ("perform_compression", "perform_decompression", "perform_training", "print_info")
@@ -101,7 +103,9 @@ def perform_compression(output_path, config, verbose):
         return  # sharded launch (torchrun): rank 0 holds the gathered latent and writes the file
     names = np.load(config.input_path)["names"]
     save = np.savez_compressed if config.extra_compression else np.savez
-    save(os.path.join(output_path, "compressed_output", "compressed.npz"), data=compressed, names=names,
+    # latent_dtype "q8": uint8 codes in `data` plus their per-block parameters (latent_q8.npz_arrays)
+    latent = latent_q8.npz_arrays(compressed) if isinstance(compressed, latent_q8.Q8Latent) else {"data": compressed}
+    save(os.path.join(output_path, "compressed_output", "compressed.npz"), **latent, names=names,
          normalization_features=normalization_features)
     if getattr(config, "save_error_bounded_deltas", False):
         # reference baler.py:316-338: two gzip'd np.save files of object arrays (per batch: the deltas; the batch indices

@@ -28,8 +28,13 @@ def dist_env():
     return 0, 1
 
 
-def row_range(n_rows, rank, world):
-    """contiguous shard [lo, hi) of n_rows rows for `rank` (first n_rows % world ranks get one extra row)"""
+def row_range(n_rows, rank, world, align=1):
+    """contiguous shard [lo, hi) of n_rows rows for `rank` (first n_rows % world ranks get one extra row).  With `align` > 1
+    the shards are cut from whole groups of `align` rows (the 128-row blocks of a q8 latent) the same way, so every shard
+    starts on a group boundary; only the last group may be short."""
+    if align > 1:
+        lo, hi = row_range((n_rows + align - 1) // align, rank, world)
+        return min(n_rows, lo * align), min(n_rows, hi * align)
     base, extra = divmod(n_rows, world)
     lo = rank * base + min(rank, extra)
     return lo, lo + base + (1 if rank < extra else 0)
@@ -153,10 +158,10 @@ def global_minmax(shard, group=None):
     return np.stack([mn, mx - mn])
 
 
-def gather_rows_to_rank0(shard, n_rows, group=None, chunk_rows=1 << 22):
-    """contiguous row shards (numpy [rows_r, C], rank order = row order) -> the full [n_rows, C] array on rank 0, None on
-    the other ranks.  Point to point in chunks through a device staging buffer, so no rank ever holds more than its own
-    shard plus one chunk on the GPU."""
+def gather_rows_to_rank0(shard, n_rows, group=None, chunk_rows=1 << 22, align=1):
+    """contiguous row shards (numpy [rows_r, C], rank order = row order, cut by row_range(n_rows, rank, world, align)) ->
+    the full [n_rows, C] array on rank 0, None on the other ranks.  Point to point in chunks through a device staging
+    buffer, so no rank ever holds more than its own shard plus one chunk on the GPU."""
     import numpy as np
     rank, world = (dist.get_rank(group), dist.get_world_size(group)) if dist.is_initialized() else (0, 1)
     if world == 1:
@@ -167,7 +172,7 @@ def gather_rows_to_rank0(shard, n_rows, group=None, chunk_rows=1 << 22):
         out = np.empty((n_rows, c), dtype=shard.dtype)
         out[:len(shard)] = shard
         for src in range(1, world):
-            lo, hi = row_range(n_rows, src, world)
+            lo, hi = row_range(n_rows, src, world, align)
             for r0 in range(lo, hi, chunk_rows):
                 r1 = min(hi, r0 + chunk_rows)
                 buf = torch.empty((r1 - r0, c), dtype=torch.from_numpy(shard[:0]).dtype, device=dev)

@@ -213,6 +213,33 @@ int bb_compress_host_f64(bb_model* m, const double* x_host, int64_t n_rows, doub
 int bb_decompress_host_f64(bb_model* m, const double* z_host, int64_t n_rows, const double* features_host,
                            double* y_host);
 
+/* ------------------------------------------------------------------ 8-bit latent (latent_dtype "q8") */
+/*
+ * The latent [n_rows, z_dim] as uint8 codes plus a float32 pair (lo, step) per latent column and block of
+ * BB_Q8_BLOCK_ROWS consecutive rows, counted from row 0 of the arrays passed (the last block may be short):
+ *   lo / hi   min / max of the block column's finite values (-0 < +0; 0 when it has none)
+ *   step      float32((float64(hi) - float64(lo)) / 254)
+ *   code      255 for a non-finite value (it decodes to NaN); 0 when step == 0;
+ *             else clamp(rint((float64(v) - lo) * (1.0 / float64(step))), 0, 254), each float64 operation IEEE
+ *   decoded   float32(float64(lo) + float64(code) * float64(step)): |decoded - v| <= step / 2 plus float32 rounding
+ * lo_dev / step_dev hold ceil(n_rows / BB_Q8_BLOCK_ROWS) x z_dim floats.  The reference has no counterpart: it writes the
+ * latent as float64 (helper.py:565).
+ */
+#define BB_Q8_BLOCK_ROWS 128
+int bb_latent_quantize_q8(bb_ctx* ctx, const float* z_dev, int64_t n_rows, int z_dim, uint8_t* codes_dev, float* lo_dev,
+                          float* step_dev, bb_stream_t stream);
+int bb_latent_dequantize_q8(bb_ctx* ctx, const uint8_t* codes_dev, const float* lo_dev, const float* step_dev,
+                            int64_t n_rows, int z_dim, float* z_dev, bb_stream_t stream);
+/* bb_compress_host / bb_decompress_host with the 8-bit latent: encode a chunk -> quantise on the device -> copy codes and
+ * parameters out (and back: copy in -> dequantise -> decode with the fused un-normalisation).  Same chunking, streams and
+ * features as the float pipelines; chunks start on block boundaries, so the result does not depend on the chunking.
+ * codes_host is n_rows x z_dim bytes, lo_host / step_host ceil(n_rows / 128) x z_dim floats.  y_dtype BB_F32 or BB_F64.
+ * BB_PREC_FP64 returns BB_ERR_UNSUPPORTED: an 8-bit latent discards far more than float64 arithmetic gains. */
+int bb_compress_host_q8(bb_model* m, const float* x_host, int64_t n_rows, float* features_host, int recompute_minmax,
+                        uint8_t* codes_host, float* lo_host, float* step_host, int precision);
+int bb_decompress_host_q8(bb_model* m, const uint8_t* codes_host, const float* lo_host, const float* step_host, int64_t n_rows,
+                          const float* features_host, void* y_host, int y_dtype, int precision);
+
 /* ------------------------------------------------------------------ training (dense AE) */
 
 typedef struct bb_train_hyper {
