@@ -635,6 +635,16 @@ int bb_debug_tc_chain(bb_model* m, int decode, const void* in_dev, int64_t n_row
                           m->flag_dev, dbg_step, dbg_out_dev, force_groups, (cudaStream_t)stream);
 }
 
+// Test hook (not part of the public header): the kernel (a BbRoute) and tile rows of the last launch of one direction
+// (0 encoder, 1 decoder), so that tests can show which kernel a shape, precision, dtype and alignment were dispatched to.
+int bb_debug_last_route(bb_model* m, int direction, int* kernel, int* tile_rows) {
+  if (!m || direction < 0 || direction > 1 || !kernel || !tile_rows) return BB_ERR_INVALID;
+  const Chain* c = direction == 0 ? &m->enc : &m->dec;
+  *kernel = c->last_route;
+  *tile_rows = c->last_tile_rows;
+  return BB_OK;
+}
+
 int bb_model_range_flag(bb_model* m, int reset, int* out) {
   if (!m || !out) return BB_ERR_INVALID;
   BB_CUDA(cudaMemcpy(out, m->flag_dev, sizeof(int), cudaMemcpyDeviceToHost));

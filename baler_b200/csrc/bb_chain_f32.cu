@@ -207,7 +207,8 @@ int bb_chain_f32_prepare(bb_ctx* ctx, Chain* c) {
   c->f32_tr = chosen;
   c->smem_bytes = f32_smem_bytes(d, chosen);
 
-  std::vector<float> blob((size_t)d.blob_floats, 0.f);
+  // whole float4s: the kernel copies the blob to shared memory with (blob_floats + 3) / 4 float4 loads (zero tail)
+  std::vector<float> blob(((size_t)d.blob_floats + 3) & ~(size_t)3, 0.f);
   for (int l = 0; l < d.n_layers; ++l) {
     const ChainLayer& L = d.layer[l];
     const std::vector<double>& w = c->w_host[l];
@@ -235,6 +236,8 @@ int bb_chain_f32_launch(bb_ctx* ctx, const Chain* c, const void* in, int in_dtyp
   const int tr = c->f32_tr;
   const int64_t n_tiles = (n_rows + tr - 1) / tr;
   const int grid = (int)(n_tiles < ctx->sm_count ? n_tiles : ctx->sm_count);
+  c->last_route = BB_ROUTE_F32;
+  c->last_tile_rows = tr;
   switch (tr) {
     case 80:
       chain_f32_kernel<80><<<grid, NT, c->smem_bytes, stream>>>(c->desc, c->blob_dev, in, in_dtype, n_rows, pre_min, pre_range, post_min, post_range, out, out_dtype);

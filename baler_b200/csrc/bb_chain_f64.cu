@@ -315,6 +315,8 @@ int bb_chain_f64_launch(bb_ctx* ctx, const Chain* c, const void* in, int in_dtyp
   const int tr = c->f64.tr;
   const int64_t n_tiles = (n_rows + tr - 1) / tr;
   const int grid = (int)(n_tiles < ctx->sm_count ? n_tiles : ctx->sm_count);
+  c->last_route = BB_ROUTE_F64;
+  c->last_tile_rows = tr;
   if (tr == 64)
     chain_f64_kernel<64><<<grid, NT, c->f64_smem, stream>>>(c->f64, c->f64_blob_dev, in, in_dtype, n_rows, pre_min, pre_range,
                                                             post_min, post_range, feat_dtype, out, out_dtype);

@@ -391,6 +391,8 @@ int bb_chain_layered_launch(bb_ctx* ctx, const Chain* c, const void* in, int in_
     BB_CUDA(cudaMalloc(&c->lay_scratch, need));
     c->lay_scratch_bytes = need;
   }
+  c->last_route = tc5 ? BB_ROUTE_LAYERED_TC5 : tensor_cores ? BB_ROUTE_LAYERED_MMA : BB_ROUTE_LAYERED_F32;
+  c->last_tile_rows = (int)chunk;
   if (tc5) {
     const size_t in_esz5 = in_dtype == BB_F16 ? 2 : 4, out_esz5 = out_dtype == BB_F16 ? 2 : 4;
     char* b0 = reinterpret_cast<char*>(c->lay_scratch);

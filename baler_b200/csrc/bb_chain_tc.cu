@@ -766,6 +766,10 @@ int bb_tc_launch_dbg(bb_ctx* ctx, const Chain* c, const void* in, int in_dtype, 
     // the statically shaped kernel: exact and fast arithmetic, float32 or (on the latent side) float16 rows
     const int rc = bb_tc4_launch(ctx, c, in, in_dtype, n_rows, pre_min, pre_range, post_min, post_range, out, out_dtype, fast,
                                  flag_dev, dbg_step == -2 ? reinterpret_cast<uint32_t*>(dbg_out) : nullptr, stream);
+    if (rc == BB_OK) {
+      c->last_route = BB_ROUTE_TC4;
+      c->last_tile_rows = 2 * TILE;  // two pipelines per CTA (NPIPE of bb_chain_tc4.cu)
+    }
     if (rc != BB_ERR_UNSUPPORTED) return rc;
   }
   const TcHost* h = reinterpret_cast<const TcHost*>(c->tc_host);
@@ -774,6 +778,8 @@ int bb_tc_launch_dbg(bb_ctx* ctx, const Chain* c, const void* in, int in_dtype, 
   const int64_t want = (n_tiles + groups - 1) / groups;
   const int grid = (int)(want < ctx->sm_count ? want : ctx->sm_count);
   const int aligned = (reinterpret_cast<uintptr_t>(in) & 15u) == 0;
+  c->last_route = BB_ROUTE_TC;
+  c->last_tile_rows = groups * TILE;
   if (groups == 2)
     chain_tc_kernel<2><<<grid, 2 * (GROUP_T + 32), h->smem_bytes, stream>>>(h->prog, (const uint8_t*)c->tc_blob_dev, in, in_dtype, aligned,
                                                                      n_rows, pre_min, pre_range, post_min, post_range, out,

@@ -64,6 +64,18 @@ struct Tc4Plan {
   float c1[4] = {0, 0, 0, 0}, c2[4] = {0, 0, 0, 0};  // y = c1 * acc + c2 * |acc| per layer
 };
 
+// Kernel that ran a direction's last launch (Chain::last_route; read back by the test hook bb_debug_last_route).
+enum BbRoute {
+  BB_ROUTE_NONE = 0,
+  BB_ROUTE_F32 = 1,          // chain_f32_kernel (bb_chain_f32.cu)
+  BB_ROUTE_TC4 = 2,          // chain_tc4_kernel (bb_chain_tc4.cu)
+  BB_ROUTE_TC = 3,           // chain_tc_kernel, table-driven (bb_chain_tc.cu)
+  BB_ROUTE_LAYERED_F32 = 4,  // dense_layer_kernel per layer (bb_chain_layered.cu)
+  BB_ROUTE_LAYERED_MMA = 5,  // dense_layer_tc_kernel per layer, mma.sync (bb_chain_layered.cu)
+  BB_ROUTE_LAYERED_TC5 = 6,  // gemm_tc5_kernel per layer, tcgen05 (bb_gemm_tc5.cu)
+  BB_ROUTE_F64 = 7,          // chain_f64_kernel (bb_chain_f64.cu)
+};
+
 // Host + device state of one direction (encoder or decoder).
 struct Chain {
   ChainDesc desc;
@@ -101,6 +113,10 @@ struct Chain {
   mutable size_t f64_smem = 0;
   std::vector<double> w_host[BB_MAX_LAYERS];  // kept for re-packing
   std::vector<double> b_host[BB_MAX_LAYERS];
+  // what the last launch of this direction ran, set by the host-side launchers: a BbRoute and the rows of its tile (fused
+  // fp32 / fp64 chains), rows per chunk (layered GEMMs) or rows in flight per CTA (tcgen05 kernels: 128 per pipeline)
+  mutable int last_route = BB_ROUTE_NONE;
+  mutable int last_tile_rows = 0;
 };
 
 struct bb_model {

@@ -107,11 +107,12 @@ def test_layered_path_ragged_rows_and_chunks(golden, chunk, monkeypatch):
 
 
 @pytest.mark.parametrize("rows", [1, 127, 129, 5000, 20000])
-@pytest.mark.parametrize("mode", ["tcgen05", "mma"])
+@pytest.mark.parametrize("mode", ["tcgen05", "mma", "fp32"])
 def test_layered_gemm_odd_shapes_vs_float64(rows, mode, monkeypatch):
-    """the per-layer tensor-core GEMMs (tcgen05 gemm_tc5_kernel; mma.sync dense_layer_tc_kernel) on a chain with widths that
-    are multiples of nothing, a long contraction (3001: partial accumulators) and ragged row counts (20000: enough row
-    tiles for the resident-A mode of the 70 -> 1111 layer), against float64 numpy"""
+    """the per-layer GEMMs (tcgen05 gemm_tc5_kernel; mma.sync dense_layer_tc_kernel; fp32 dense_layer_kernel, what
+    precision "fp32" runs) on a chain with widths that are multiples of nothing, a long contraction (3001: partial
+    accumulators) and ragged row counts (20000: enough row tiles for the resident-A mode of the 70 -> 1111 layer), against
+    float64 numpy"""
     from baler_b200 import engine
     if mode == "mma":
         monkeypatch.setenv("BALER_B200_LAYERED_MMA", "1")
@@ -135,10 +136,11 @@ def test_layered_gemm_odd_shapes_vs_float64(rows, mode, monkeypatch):
             v = np.where(v > 0, v, 0.01 * v) if a == "leaky" else np.maximum(v, 0) if a == "relu" else v
         return v
 
-    z = codec.encode(torch.from_numpy(x).cuda())
+    precision = "fp32" if mode == "fp32" else "auto"
+    z = codec.encode(torch.from_numpy(x).cuda(), precision=precision)
     zr = ref(x, enc)
     assert rel_max(z.cpu().numpy(), zr) <= 1e-5 and rel_l2(z.cpu().numpy(), zr) <= 1e-5
-    y = codec.decode(z)
+    y = codec.decode(z, precision=precision)
     yr = ref(z.cpu().numpy(), dec)
     assert rel_max(y.cpu().numpy(), yr) <= 1e-5 and rel_l2(y.cpu().numpy(), yr) <= 1e-5
 

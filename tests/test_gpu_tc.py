@@ -130,7 +130,9 @@ def test_range_guard(ae):
 def test_tc_shape_family_vs_oracle(n_features, z_dim):
     """every instantiation of the statically shaped tcgen05 kernel (padded first K 16 / 32, padded last N 16 / 32, both
     directions): random reference-initialised AE(n_features, z_dim), fused normalisation / un-normalisation, ragged row
-    counts (single rows, tile tails whose byte count is not a multiple of 16, fewer tiles than SMs, many tiles)"""
+    counts (single rows, tile tails whose byte count is not a multiple of 16, fewer tiles than SMs, many tiles).  The same
+    shapes on the fused fp32 chain (precision "fp32") and in single-product mode ("fast": the table-driven kernel except
+    on the two CMS instantiations; documented as outside the 1e-5 bar)"""
     torch.manual_seed(100 * n_features + z_dim)
     m = models.AE(n_features, z_dim).eval()
     sd = {k: v.numpy().astype(np.float64) for k, v in m.state_dict().items()}
@@ -146,8 +148,9 @@ def test_tc_shape_family_vs_oracle(n_features, z_dim):
         yr = orc.ae_decode(sd, zr) * rg.astype(np.float64) + mn.astype(np.float64)
         x_dev = torch.from_numpy(raw).cuda()
         mn_d, rg_d = torch.from_numpy(mn).cuda(), torch.from_numpy(rg).cuda()
-        z = codec.encode(x_dev, mn_d, rg_d, precision="split16")
-        assert rel_max(z.cpu().numpy(), zr) <= 1e-5 and rel_l2(z.cpu().numpy(), zr) <= 1e-5, (n, rel_max(z.cpu().numpy(), zr))
-        y = codec.decode(torch.from_numpy(zr.astype(np.float32)).cuda(), mn_d, rg_d, precision="split16")
-        assert rel_max(y.cpu().numpy(), yr) <= 1e-5 and rel_l2(y.cpu().numpy(), yr) <= 1e-5, (n, rel_max(y.cpu().numpy(), yr))
+        for precision, tol in (("split16", 1e-5), ("fp32", 1e-5), ("fast", 1e-2)):
+            z = codec.encode(x_dev, mn_d, rg_d, precision=precision)
+            assert rel_max(z.cpu().numpy(), zr) <= tol and rel_l2(z.cpu().numpy(), zr) <= tol, (n, precision, rel_max(z.cpu().numpy(), zr))
+            y = codec.decode(torch.from_numpy(zr.astype(np.float32)).cuda(), mn_d, rg_d, precision=precision)
+            assert rel_max(y.cpu().numpy(), yr) <= tol and rel_l2(y.cpu().numpy(), yr) <= tol, (n, precision, rel_max(y.cpu().numpy(), yr))
     assert not codec.range_flag()
