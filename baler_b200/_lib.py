@@ -62,6 +62,10 @@ _SIGNATURES = {
     "bb_latent_dequantize_q8": (C.c_int, [_P, _P, _P, _P, C.c_int64, C.c_int, _P, _P]),
     "bb_compress_host_q8": (C.c_int, [_P, _P, C.c_int64, _P, C.c_int, _P, _P, _P, C.c_int]),
     "bb_decompress_host_q8": (C.c_int, [_P, _P, _P, _P, C.c_int64, _P, _P, C.c_int, C.c_int]),
+    "bb_latent_quantize_packed": (C.c_int, [_P, _P, C.c_int64, C.c_int, C.c_int, _P, _P, _P, _P]),
+    "bb_latent_dequantize_packed": (C.c_int, [_P, C.c_int, _P, _P, _P, C.c_int64, C.c_int, _P, _P]),
+    "bb_compress_host_packed": (C.c_int, [_P, _P, C.c_int64, _P, C.c_int, C.c_int, _P, _P, _P, C.c_int]),
+    "bb_decompress_host_packed": (C.c_int, [_P, C.c_int, _P, _P, _P, C.c_int64, _P, _P, C.c_int, C.c_int]),
     "bb_trainer_create": (C.c_int, [_P, C.c_int, C.c_int, _P, _P, C.c_int, _PP]),
     "bb_trainer_create_dbn": (C.c_int, [_P, C.c_int, C.c_int, _P, _P, _P, _P, _P, _P, _P, C.c_int, _PP]),
     "bb_trainer_set_dropout": (C.c_int, [_P, C.c_uint64, _P]),

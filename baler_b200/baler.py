@@ -2,7 +2,8 @@
 
 Keeps the reference's CLI, per-project config files and output layout (reference baler/baler.py:36-456):
   output/compressed_output/model.pt, compressed.npz {data, names, normalization_features}
-    (latent_dtype "q8" adds latent_min, latent_step, latent_block_rows: baler_b200/latent_q8.py)
+    (latent_dtype "q2" ... "q8" adds latent_min, latent_step, latent_block_rows and, below 8 bits, latent_bits:
+    baler_b200/latent_q8.py)
   output/decompressed_output/decompressed.npz {data, names}
   output/training/normalization_features.npy, loss_data.npy, activations.npy, model_{epoch}.pt
 """
@@ -103,8 +104,8 @@ def perform_compression(output_path, config, verbose):
         return  # sharded launch (torchrun): rank 0 holds the gathered latent and writes the file
     names = np.load(config.input_path)["names"]
     save = np.savez_compressed if config.extra_compression else np.savez
-    # latent_dtype "q8": uint8 codes in `data` plus their per-block parameters (latent_q8.npz_arrays)
-    latent = latent_q8.npz_arrays(compressed) if isinstance(compressed, latent_q8.Q8Latent) else {"data": compressed}
+    # latent_dtype "q2" ... "q8": packed codes in `data` plus their per-block parameters (latent_q8.npz_arrays)
+    latent = latent_q8.npz_arrays(compressed) if isinstance(compressed, latent_q8.PackedLatent) else {"data": compressed}
     save(os.path.join(output_path, "compressed_output", "compressed.npz"), **latent, names=names,
          normalization_features=normalization_features)
     if getattr(config, "save_error_bounded_deltas", False):

@@ -721,37 +721,40 @@ int bb_host_colminmax_f32(const float* x_host, int64_t n_rows, int n_cols, float
 
 namespace {
 
-// The 8-bit latent of bb_compress_host_q8 / bb_decompress_host_q8 in host memory: codes [n_rows, Z], lo / step
-// [ceil(n_rows / 128), Z]
-struct Q8Host {
+// The quantised latent of bb_compress_host_packed / bb_decompress_host_packed in host memory: codes [n_rows, row_bytes]
+// (row_bytes = ceil(Z * bits / 8)), lo / step [ceil(n_rows / 128), Z]
+struct QHost {
+  int bits;
   uint8_t* codes;
   float* lo;
   float* step;
+  size_t row_bytes(int Z) const { return ((size_t)Z * bits + 7) / 8; }
 };
 
-// A chunk's 8-bit latent in a device staging slot, behind its float32 latent: [float32 latent | codes | lo | step], each
-// part 256-byte aligned.  Chunks start on block boundaries (pipe_chunk_rows gives whole 128-row tiles), so a chunk's blocks
-// are the file's.
-struct Q8Slot {
+// A chunk's quantised latent in a device staging slot, behind its float32 latent: [float32 latent | codes | lo | step],
+// each part 256-byte aligned.  Chunks start on block boundaries (pipe_chunk_rows gives whole 128-row tiles), so a chunk's
+// blocks are the file's.
+struct QSlot {
   size_t codes_off, lo_off, step_off, bytes;
-  Q8Slot(int64_t rows, int Z) {
+  QSlot(int64_t rows, int Z, size_t row_bytes) {
     auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
     const size_t nb = (size_t)((rows + BB_Q8_BLOCK_ROWS - 1) / BB_Q8_BLOCK_ROWS);
     codes_off = up((size_t)rows * Z * sizeof(float));
-    lo_off = codes_off + up((size_t)rows * Z);
+    lo_off = codes_off + up((size_t)rows * row_bytes);
     step_off = lo_off + up(nb * Z * sizeof(float));
     bytes = step_off + up(nb * Z * sizeof(float));
   }
 };
 
 // The host-buffer compress pipeline of bb_compress_host (x_dtype BB_F32: float32 table and features),
-// bb_compress_host_f64 (x_dtype BB_F64: float64 table and features, precision BB_PREC_FP64) and bb_compress_host_q8 (q8:
-// the float32 latent of each chunk is quantised on the device and its codes and parameters are copied out instead).
+// bb_compress_host_f64 (x_dtype BB_F64: float64 table and features, precision BB_PREC_FP64) and bb_compress_host_packed
+// (q: the float32 latent of each chunk is quantised on the device and its codes and parameters are copied out instead).
 int compress_host(bb_model* m, const void* x_host, int x_dtype, int64_t n_rows, void* features_host,
-                  int recompute_minmax, void* z_host, int z_dtype, int precision, const Q8Host* q8 = nullptr) {
-  if (!m || (!x_host && n_rows) || (!z_host && !q8 && n_rows) || n_rows < 0) return BB_ERR_INVALID;
-  if (q8 && n_rows && (!q8->codes || !q8->lo || !q8->step)) return BB_ERR_INVALID;
-  if (q8 && (precision == BB_PREC_FP64 || x_dtype != BB_F32)) return BB_ERR_UNSUPPORTED;
+                  int recompute_minmax, void* z_host, int z_dtype, int precision, const QHost* q = nullptr) {
+  if (!m || (!x_host && n_rows) || (!z_host && !q && n_rows) || n_rows < 0) return BB_ERR_INVALID;
+  if (q && (q->bits < BB_LATENT_MIN_BITS || q->bits > BB_LATENT_MAX_BITS)) return BB_ERR_INVALID;
+  if (q && n_rows && (!q->codes || !q->lo || !q->step)) return BB_ERR_INVALID;
+  if (q && (precision == BB_PREC_FP64 || x_dtype != BB_F32)) return BB_ERR_UNSUPPORTED;
   if (z_dtype != BB_F32 && z_dtype != BB_F16 && z_dtype != BB_F64) return BB_ERR_INVALID;
   if (recompute_minmax && !features_host) return BB_ERR_INVALID;
   if (x_dtype == BB_F64 && precision != BB_PREC_FP64) return BB_ERR_INVALID;
@@ -760,11 +763,11 @@ int compress_host(bb_model* m, const void* x_host, int x_dtype, int64_t n_rows, 
   const size_t xs = dtype_size(x_dtype);  // bytes per element of the table and of its features
   // device output dtype: the float32 / fp16 kernels write float32 for a float64 latent (widened on the host below); the
   // float64 kernel writes whatever is asked
-  const int dev_dtype = q8 ? BB_F32 : (z_dtype == BB_F64 && precision != BB_PREC_FP64) ? BB_F32 : z_dtype;
+  const int dev_dtype = q ? BB_F32 : (z_dtype == BB_F64 && precision != BB_PREC_FP64) ? BB_F32 : z_dtype;
   const int64_t chunk = pipe_chunk_rows(n_rows);
   const int64_t n_chunks = n_rows ? (n_rows + chunk - 1) / chunk : 0;
-  const Q8Slot q8s(chunk, Z);
-  const size_t in_b = (size_t)chunk * F * xs, out_b = q8 ? q8s.bytes : (size_t)chunk * Z * dtype_size(dev_dtype);
+  const QSlot qs(chunk, Z, q ? q->row_bytes(Z) : 0);
+  const size_t in_b = (size_t)chunk * F * xs, out_b = q ? qs.bytes : (size_t)chunk * Z * dtype_size(dev_dtype);
   int rc = pipe_init(m, in_b, out_b);
   if (rc != BB_OK) return rc;
   char* feat = nullptr;
@@ -836,7 +839,7 @@ int compress_host(bb_model* m, const void* x_host, int x_dtype, int64_t n_rows, 
     ~EvGuard() { for (cudaEvent_t e : v) if (e) cudaEventDestroy(e); }
   } ev_guard{ev_up};
 
-  const bool widen = !q8 && z_dtype == BB_F64 && dev_dtype != BB_F64;  // float32 on the device, float64 in the caller's buffer
+  const bool widen = !q && z_dtype == BB_F64 && dev_dtype != BB_F64;  // float32 on the device, float64 in the caller's buffer
   // a float64 latent from the float64 chain lands in a pinned slot and is copied out on host threads when the caller's
   // buffer is pageable (a device-to-pageable copy runs at a fraction of the PCIe rate)
   const bool bounce = dev_dtype == BB_F64 && n_rows && !host_pinned(z_host);
@@ -877,18 +880,18 @@ int compress_host(bb_model* m, const void* x_host, int x_dtype, int64_t n_rows, 
                    m->stage_dev[1][s], dev_dtype, precision, m->s_compute);
     if (rc != BB_OK) break;
     char* out = (char*)m->stage_dev[1][s];
-    if (q8) {
-      rc = bb_latent_q8_quantize_launch(m->ctx, (const float*)out, rows, Z, (uint8_t*)(out + q8s.codes_off),
-                                        (float*)(out + q8s.lo_off), (float*)(out + q8s.step_off), m->s_compute);
+    if (q) {
+      rc = bb_latent_quantize_launch(m->ctx, (const float*)out, rows, Z, q->bits, (uint8_t*)(out + qs.codes_off),
+                                     (float*)(out + qs.lo_off), (float*)(out + qs.step_off), m->s_compute);
       if (rc != BB_OK) break;
     }
     BB_CUDA(cudaEventRecord(m->ev_done[s], m->s_compute));
     BB_CUDA(cudaStreamWaitEvent(m->s_copy_out, m->ev_done[s], 0));
-    if (q8) {
+    if (q) {
       const int64_t b0 = r0 / BB_Q8_BLOCK_ROWS, nb = (rows + BB_Q8_BLOCK_ROWS - 1) / BB_Q8_BLOCK_ROWS;
-      BB_CUDA(cudaMemcpyAsync(q8->codes + (size_t)r0 * Z, out + q8s.codes_off, (size_t)rows * Z, cudaMemcpyDeviceToHost, m->s_copy_out));
-      BB_CUDA(cudaMemcpyAsync(q8->lo + (size_t)b0 * Z, out + q8s.lo_off, (size_t)nb * Z * sizeof(float), cudaMemcpyDeviceToHost, m->s_copy_out));
-      BB_CUDA(cudaMemcpyAsync(q8->step + (size_t)b0 * Z, out + q8s.step_off, (size_t)nb * Z * sizeof(float), cudaMemcpyDeviceToHost, m->s_copy_out));
+      BB_CUDA(cudaMemcpyAsync(q->codes + (size_t)r0 * q->row_bytes(Z), out + qs.codes_off, (size_t)rows * q->row_bytes(Z), cudaMemcpyDeviceToHost, m->s_copy_out));
+      BB_CUDA(cudaMemcpyAsync(q->lo + (size_t)b0 * Z, out + qs.lo_off, (size_t)nb * Z * sizeof(float), cudaMemcpyDeviceToHost, m->s_copy_out));
+      BB_CUDA(cudaMemcpyAsync(q->step + (size_t)b0 * Z, out + qs.step_off, (size_t)nb * Z * sizeof(float), cudaMemcpyDeviceToHost, m->s_copy_out));
     } else {
       void* dst = (widen || bounce) ? pinned_out[s] : (void*)((char*)z_host + (size_t)r0 * Z * dtype_size(z_dtype));
       BB_CUDA(cudaMemcpyAsync(dst, out, (size_t)rows * Z * dtype_size(dev_dtype), cudaMemcpyDeviceToHost, m->s_copy_out));
@@ -902,20 +905,21 @@ int compress_host(bb_model* m, const void* x_host, int x_dtype, int64_t n_rows, 
     int tripped = 0;  // fp16 range guard of the split path: redo on the fp32 kernel (features are already known)
     rc = bb_model_range_flag(m, 1, &tripped);
     if (rc == BB_OK && tripped)
-      return compress_host(m, x_host, x_dtype, n_rows, features_host, 0, z_host, z_dtype, BB_PREC_FP32, q8);
+      return compress_host(m, x_host, x_dtype, n_rows, features_host, 0, z_host, z_dtype, BB_PREC_FP32, q);
   }
   return rc;
 }
 
 // The host-buffer decompress pipeline of bb_decompress_host (float32 features), bb_decompress_host_f64 (feat_dtype
-// BB_F64: float64 features, latent and reconstruction, precision BB_PREC_FP64) and bb_decompress_host_q8 (q8: codes and
-// parameters are copied in and dequantised to a float32 latent on the device; z_host and z_dtype are unused).
+// BB_F64: float64 features, latent and reconstruction, precision BB_PREC_FP64) and bb_decompress_host_packed (q: codes
+// and parameters are copied in and dequantised to a float32 latent on the device; z_host and z_dtype are unused).
 int decompress_host(bb_model* m, const void* z_host, int z_dtype, int64_t n_rows, const void* features_host,
-                    int feat_dtype, void* y_host, int y_dtype, int precision, const Q8Host* q8 = nullptr) {
-  if (!m || (!z_host && !q8 && n_rows) || (!y_host && n_rows) || n_rows < 0) return BB_ERR_INVALID;
-  if (q8 && n_rows && (!q8->codes || !q8->lo || !q8->step)) return BB_ERR_INVALID;
-  if (q8 && (precision == BB_PREC_FP64 || feat_dtype != BB_F32)) return BB_ERR_UNSUPPORTED;
-  if (q8) z_dtype = BB_F32;  // (the device latent)
+                    int feat_dtype, void* y_host, int y_dtype, int precision, const QHost* q = nullptr) {
+  if (!m || (!z_host && !q && n_rows) || (!y_host && n_rows) || n_rows < 0) return BB_ERR_INVALID;
+  if (q && (q->bits < BB_LATENT_MIN_BITS || q->bits > BB_LATENT_MAX_BITS)) return BB_ERR_INVALID;
+  if (q && n_rows && (!q->codes || !q->lo || !q->step)) return BB_ERR_INVALID;
+  if (q && (precision == BB_PREC_FP64 || feat_dtype != BB_F32)) return BB_ERR_UNSUPPORTED;
+  if (q) z_dtype = BB_F32;  // (the device latent)
   if (z_dtype != BB_F32 && z_dtype != BB_F16 && z_dtype != BB_F64) return BB_ERR_INVALID;
   if (y_dtype != BB_F32 && y_dtype != BB_F64) return BB_ERR_INVALID;
   if (feat_dtype == BB_F64 && precision != BB_PREC_FP64) return BB_ERR_INVALID;
@@ -932,8 +936,8 @@ int decompress_host(bb_model* m, const void* z_host, int z_dtype, int64_t n_rows
   const bool bounce_out = dev_out == BB_F64 && n_rows && !host_pinned(y_host);
   const int64_t chunk = pipe_chunk_rows(n_rows);
   const int64_t n_chunks = n_rows ? (n_rows + chunk - 1) / chunk : 0;
-  const Q8Slot q8s(chunk, Z);
-  const size_t in_b = q8 ? q8s.bytes : (size_t)chunk * Z * dtype_size(dev_in), out_b = (size_t)chunk * F * dtype_size(dev_out);
+  const QSlot qs(chunk, Z, q ? q->row_bytes(Z) : 0);
+  const size_t in_b = q ? qs.bytes : (size_t)chunk * Z * dtype_size(dev_in), out_b = (size_t)chunk * F * dtype_size(dev_out);
   int rc = pipe_init(m, in_b, out_b);
   if (rc != BB_OK) return rc;
   char* feat = nullptr;
@@ -973,11 +977,11 @@ int decompress_host(bb_model* m, const void* z_host, int z_dtype, int64_t n_rows
       BB_CUDA(cudaStreamWaitEvent(m->s_copy_in, m->ev_done[s], 0));
     }
     char* in = (char*)m->stage_dev[0][s];
-    if (q8) {
+    if (q) {
       const int64_t b0 = r0 / BB_Q8_BLOCK_ROWS, nb = (rows + BB_Q8_BLOCK_ROWS - 1) / BB_Q8_BLOCK_ROWS;
-      BB_CUDA(cudaMemcpyAsync(in + q8s.codes_off, q8->codes + (size_t)r0 * Z, (size_t)rows * Z, cudaMemcpyHostToDevice, m->s_copy_in));
-      BB_CUDA(cudaMemcpyAsync(in + q8s.lo_off, q8->lo + (size_t)b0 * Z, (size_t)nb * Z * sizeof(float), cudaMemcpyHostToDevice, m->s_copy_in));
-      BB_CUDA(cudaMemcpyAsync(in + q8s.step_off, q8->step + (size_t)b0 * Z, (size_t)nb * Z * sizeof(float), cudaMemcpyHostToDevice, m->s_copy_in));
+      BB_CUDA(cudaMemcpyAsync(in + qs.codes_off, q->codes + (size_t)r0 * q->row_bytes(Z), (size_t)rows * q->row_bytes(Z), cudaMemcpyHostToDevice, m->s_copy_in));
+      BB_CUDA(cudaMemcpyAsync(in + qs.lo_off, q->lo + (size_t)b0 * Z, (size_t)nb * Z * sizeof(float), cudaMemcpyHostToDevice, m->s_copy_in));
+      BB_CUDA(cudaMemcpyAsync(in + qs.step_off, q->step + (size_t)b0 * Z, (size_t)nb * Z * sizeof(float), cudaMemcpyHostToDevice, m->s_copy_in));
     } else {
       const void* src = (const char*)z_host + (size_t)r0 * Z * dtype_size(z_dtype);
       if (narrow) {
@@ -996,9 +1000,9 @@ int decompress_host(bb_model* m, const void* z_host, int z_dtype, int64_t n_rows
       if (rc != BB_OK) break;
       BB_CUDA(cudaStreamWaitEvent(m->s_compute, m->ev_out[s], 0));
     }
-    if (q8) {
-      rc = bb_latent_q8_dequantize_launch(m->ctx, (const uint8_t*)(in + q8s.codes_off), (const float*)(in + q8s.lo_off),
-                                          (const float*)(in + q8s.step_off), rows, Z, (float*)in, m->s_compute);
+    if (q) {
+      rc = bb_latent_dequantize_launch(m->ctx, q->bits, (const uint8_t*)(in + qs.codes_off), (const float*)(in + qs.lo_off),
+                                       (const float*)(in + qs.step_off), rows, Z, (float*)in, m->s_compute);
       if (rc != BB_OK) break;
     }
     rc = run_chain(m, &m->dec, m->stage_dev[0][s], dev_in, rows, nullptr, nullptr, norm ? fmin : nullptr,
@@ -1017,7 +1021,7 @@ int decompress_host(bb_model* m, const void* z_host, int z_dtype, int64_t n_rows
     int tripped = 0;
     rc = bb_model_range_flag(m, 1, &tripped);
     if (rc == BB_OK && tripped)
-      return decompress_host(m, z_host, z_dtype, n_rows, features_host, feat_dtype, y_host, y_dtype, BB_PREC_FP32, q8);
+      return decompress_host(m, z_host, z_dtype, n_rows, features_host, feat_dtype, y_host, y_dtype, BB_PREC_FP32, q);
   }
   return rc;
 }
@@ -1046,16 +1050,27 @@ int bb_decompress_host_f64(bb_model* m, const double* z_host, int64_t n_rows, co
   return decompress_host(m, z_host, BB_F64, n_rows, features_host, BB_F64, y_host, BB_F64, BB_PREC_FP64);
 }
 
+int bb_compress_host_packed(bb_model* m, const float* x_host, int64_t n_rows, float* features_host, int recompute_minmax,
+                            int bits, uint8_t* codes_host, float* lo_host, float* step_host, int precision) {
+  const QHost q{bits, codes_host, lo_host, step_host};
+  return compress_host(m, x_host, BB_F32, n_rows, features_host, recompute_minmax, nullptr, BB_F32, precision, &q);
+}
+
+int bb_decompress_host_packed(bb_model* m, int bits, const uint8_t* codes_host, const float* lo_host, const float* step_host,
+                              int64_t n_rows, const float* features_host, void* y_host, int y_dtype, int precision) {
+  const QHost q{bits, const_cast<uint8_t*>(codes_host), const_cast<float*>(lo_host), const_cast<float*>(step_host)};
+  return decompress_host(m, nullptr, BB_F32, n_rows, features_host, BB_F32, y_host, y_dtype, precision, &q);
+}
+
 int bb_compress_host_q8(bb_model* m, const float* x_host, int64_t n_rows, float* features_host, int recompute_minmax,
                         uint8_t* codes_host, float* lo_host, float* step_host, int precision) {
-  const Q8Host q8{codes_host, lo_host, step_host};
-  return compress_host(m, x_host, BB_F32, n_rows, features_host, recompute_minmax, nullptr, BB_F32, precision, &q8);
+  return bb_compress_host_packed(m, x_host, n_rows, features_host, recompute_minmax, 8, codes_host, lo_host, step_host,
+                                 precision);
 }
 
 int bb_decompress_host_q8(bb_model* m, const uint8_t* codes_host, const float* lo_host, const float* step_host, int64_t n_rows,
                           const float* features_host, void* y_host, int y_dtype, int precision) {
-  const Q8Host q8{const_cast<uint8_t*>(codes_host), const_cast<float*>(lo_host), const_cast<float*>(step_host)};
-  return decompress_host(m, nullptr, BB_F32, n_rows, features_host, BB_F32, y_host, y_dtype, precision, &q8);
+  return bb_decompress_host_packed(m, 8, codes_host, lo_host, step_host, n_rows, features_host, y_host, y_dtype, precision);
 }
 
 }  // extern "C"

@@ -163,11 +163,12 @@ void bb_chain_f64_release(const Chain* c);
 int bb_chain_f64_launch(bb_ctx* ctx, const Chain* c, const void* in, int in_dtype, int64_t n_rows, const void* pre_min,
                         const void* pre_range, const void* post_min, const void* post_range, int feat_dtype, void* out,
                         int out_dtype, cudaStream_t stream);
-// 8-bit latent (bb_latent_q8.cu): blocks of BB_Q8_BLOCK_ROWS rows start at row 0 of the arrays passed
-int bb_latent_q8_quantize_launch(bb_ctx* ctx, const float* z, int64_t n_rows, int Z, uint8_t* codes, float* lo, float* step,
-                                 cudaStream_t stream);
-int bb_latent_q8_dequantize_launch(bb_ctx* ctx, const uint8_t* codes, const float* lo, const float* step, int64_t n_rows,
-                                   int Z, float* z, cudaStream_t stream);
+// quantised latent of `bits` (2..8) bits per code (bb_latent_q8.cu): blocks of BB_Q8_BLOCK_ROWS rows start at row 0 of the
+// arrays passed; codes are n_rows x ceil(Z * bits / 8) bytes
+int bb_latent_quantize_launch(bb_ctx* ctx, const float* z, int64_t n_rows, int Z, int bits, uint8_t* codes, float* lo,
+                              float* step, cudaStream_t stream);
+int bb_latent_dequantize_launch(bb_ctx* ctx, int bits, const uint8_t* codes, const float* lo, const float* step,
+                                int64_t n_rows, int Z, float* z, cudaStream_t stream);
 int bb_tc_prepare(bb_ctx* ctx, Chain* c);
 void bb_tc_release(Chain* c);
 int bb_tc_launch_dbg(bb_ctx* ctx, const Chain* c, const void* in, int in_dtype, int64_t n_rows, const float* pre_min,

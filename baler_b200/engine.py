@@ -321,64 +321,86 @@ class DenseCodec:
                                             _NP2BB[y.dtype], _prec(precision)), "bb_decompress_host")
         return y
 
-    # ---- 8-bit latent (latent_q8: uint8 codes, float32 lo / step per 128-row block and column)
-    def quantize_q8(self, z):
-        """Q8Latent of CUDA tensors for a CUDA float32 latent [n, z_dim]; blocks start at its row 0"""
+    # ---- quantised latent (latent_q8: b-bit codes in packed rows, float32 lo / step per 128-row block and column); the
+    # *_q8 methods are the b = 8 calls, with Q8Latent in place of PackedLatent
+    def quantize_packed(self, z, bits):
+        """PackedLatent of CUDA tensors for a CUDA float32 latent [n, z_dim]; blocks start at its row 0"""
         assert z.is_cuda and z.dtype == torch.float32 and z.is_contiguous() and z.shape[-1] == self.z_dim
         n = z.numel() // self.z_dim
         nb = latent_q8.n_blocks(n)
-        q = latent_q8.Q8Latent(torch.empty((n, self.z_dim), dtype=torch.uint8, device=z.device),
-                               torch.empty((nb, self.z_dim), dtype=torch.float32, device=z.device),
-                               torch.empty((nb, self.z_dim), dtype=torch.float32, device=z.device))
-        check(_lib.lib().bb_latent_quantize_q8(self.ctx.handle, _ptr(z), n, self.z_dim, _ptr(q.codes), _ptr(q.lo), _ptr(q.step),
-                                               _stream(self.ctx)), "bb_latent_quantize_q8")
+        q = latent_q8.PackedLatent(torch.empty((n, latent_q8.row_bytes(self.z_dim, bits)), dtype=torch.uint8, device=z.device),
+                                   torch.empty((nb, self.z_dim), dtype=torch.float32, device=z.device),
+                                   torch.empty((nb, self.z_dim), dtype=torch.float32, device=z.device), int(bits))
+        check(_lib.lib().bb_latent_quantize_packed(self.ctx.handle, _ptr(z), n, self.z_dim, q.bits, _ptr(q.codes), _ptr(q.lo),
+                                                   _ptr(q.step), _stream(self.ctx)), "bb_latent_quantize_packed")
         return q
 
-    def dequantize_q8(self, q):
-        """the CUDA float32 latent [n, z_dim] of a Q8Latent of CUDA tensors"""
-        codes, lo, step = (t.contiguous() for t in q)
-        assert codes.is_cuda and codes.dtype == torch.uint8 and codes.shape[-1] == self.z_dim
-        n = codes.numel() // self.z_dim
+    def dequantize_packed(self, q):
+        """the CUDA float32 latent [n, z_dim] of a PackedLatent of CUDA tensors"""
+        codes, lo, step = (t.contiguous() for t in q[:3])
+        n = codes.shape[0]
+        assert codes.is_cuda and codes.dtype == torch.uint8 and codes.shape == (n, latent_q8.row_bytes(self.z_dim, q.bits))
         assert lo.dtype == step.dtype == torch.float32 and lo.shape == step.shape == (latent_q8.n_blocks(n), self.z_dim)
         z = torch.empty((n, self.z_dim), dtype=torch.float32, device=codes.device)
-        check(_lib.lib().bb_latent_dequantize_q8(self.ctx.handle, _ptr(codes), _ptr(lo), _ptr(step), n, self.z_dim, _ptr(z),
-                                                 _stream(self.ctx)), "bb_latent_dequantize_q8")
+        check(_lib.lib().bb_latent_dequantize_packed(self.ctx.handle, q.bits, _ptr(codes), _ptr(lo), _ptr(step), n, self.z_dim,
+                                                     _ptr(z), _stream(self.ctx)), "bb_latent_dequantize_packed")
         return z
 
-    def compress_host_q8(self, x, features=None, recompute_minmax=False, precision="auto", out=None):
-        """compress_host with the 8-bit latent (bb_compress_host_q8): returns (Q8Latent of numpy arrays, features).
-        `out`: a Q8Latent of host buffers to fill (latent_q8.empty).  precision "fp64" is refused."""
+    def compress_host_packed(self, x, bits, features=None, recompute_minmax=False, precision="auto", out=None):
+        """compress_host with the `bits`-bit latent (bb_compress_host_packed): returns (PackedLatent of numpy arrays,
+        features).  `out`: a PackedLatent of host buffers to fill (latent_q8.empty_packed).  precision "fp64" is refused."""
         if _prec(precision) == BB_PREC_FP64:
-            raise NotImplementedError("precision='fp64' does not write an 8-bit latent (latent_dtype='q8'): the 8-bit "
-                                      "codes discard far more than float64 arithmetic gains")
+            raise NotImplementedError("precision='fp64' does not write a quantised latent (latent_dtype='q%d'): the %d-bit "
+                                      "codes discard far more than float64 arithmetic gains" % (bits, bits))
         x = host_convert(x, np.float32)
         n = x.shape[0]
-        q = out if out is not None else latent_q8.empty(n, self.z_dim)
+        q = out if out is not None else latent_q8.empty_packed(n, self.z_dim, bits)
         feats = None
         if features is not None or recompute_minmax:
             feats = np.zeros((2, self.n_features), dtype=np.float32) if features is None else \
                 np.ascontiguousarray(features, dtype=np.float32).copy()
-        check(_lib.lib().bb_compress_host_q8(self.handle, x.ctypes.data, n, None if feats is None else feats.ctypes.data,
-                                             int(bool(recompute_minmax)), q.codes.ctypes.data, q.lo.ctypes.data,
-                                             q.step.ctypes.data, _prec(precision)), "bb_compress_host_q8")
+        check(_lib.lib().bb_compress_host_packed(self.handle, x.ctypes.data, n, None if feats is None else feats.ctypes.data,
+                                                 int(bool(recompute_minmax)), int(bits), q.codes.ctypes.data, q.lo.ctypes.data,
+                                                 q.step.ctypes.data, _prec(precision)), "bb_compress_host_packed")
         return q, feats
+
+    def decompress_host_packed(self, q, features=None, y_dtype=np.float64, precision="auto", out=None):
+        """decompress_host of a PackedLatent of numpy arrays (bb_decompress_host_packed): dequantised and decoded on the
+        device"""
+        if _prec(precision) == BB_PREC_FP64:
+            raise NotImplementedError("precision='fp64' does not read a quantised latent (latent_dtype='q%d')" % q.bits)
+        codes, lo, step = (np.ascontiguousarray(a) for a in q[:3])
+        n, width = codes.shape[0], latent_q8.row_bytes(self.z_dim, q.bits)
+        if codes.dtype != np.uint8 or codes.shape[1:] != (width,) or lo.dtype != np.float32 or step.dtype != np.float32 \
+                or lo.shape != (latent_q8.n_blocks(n), self.z_dim) or step.shape != lo.shape:
+            raise ValueError("a q%d latent of %d rows is uint8 codes (%d, %d) and float32 lo / step (%d, %d)"
+                             % (q.bits, n, n, width, latent_q8.n_blocks(n), self.z_dim))
+        y = out if out is not None else np.empty((n, self.n_features), dtype=y_dtype)
+        feats = None if features is None else np.ascontiguousarray(features, dtype=np.float32)
+        check(_lib.lib().bb_decompress_host_packed(self.handle, int(q.bits), codes.ctypes.data, lo.ctypes.data,
+                                                   step.ctypes.data, n, None if feats is None else feats.ctypes.data,
+                                                   y.ctypes.data, _NP2BB[y.dtype], _prec(precision)),
+              "bb_decompress_host_packed")
+        return y
+
+    def quantize_q8(self, z):
+        """Q8Latent of CUDA tensors for a CUDA float32 latent [n, z_dim]; blocks start at its row 0"""
+        return latent_q8.Q8Latent(*self.quantize_packed(z, 8)[:3])
+
+    def dequantize_q8(self, q):
+        """the CUDA float32 latent [n, z_dim] of a Q8Latent of CUDA tensors"""
+        return self.dequantize_packed(latent_q8.PackedLatent(*q, 8))
+
+    def compress_host_q8(self, x, features=None, recompute_minmax=False, precision="auto", out=None):
+        """compress_host with the 8-bit latent (bb_compress_host_q8): returns (Q8Latent of numpy arrays, features).
+        `out`: a Q8Latent of host buffers to fill (latent_q8.empty).  precision "fp64" is refused."""
+        q, feats = self.compress_host_packed(x, 8, features, recompute_minmax, precision,
+                                             None if out is None else latent_q8.PackedLatent(*out, 8))
+        return latent_q8.Q8Latent(*q[:3]), feats
 
     def decompress_host_q8(self, q, features=None, y_dtype=np.float64, precision="auto", out=None):
         """decompress_host of a Q8Latent of numpy arrays (bb_decompress_host_q8): dequantised and decoded on the device"""
-        if _prec(precision) == BB_PREC_FP64:
-            raise NotImplementedError("precision='fp64' does not read an 8-bit latent (latent_dtype='q8')")
-        codes, lo, step = (np.ascontiguousarray(a) for a in q)
-        n = codes.shape[0]
-        if codes.dtype != np.uint8 or codes.shape[1:] != (self.z_dim,) or lo.dtype != np.float32 or step.dtype != np.float32 \
-                or lo.shape != (latent_q8.n_blocks(n), self.z_dim) or step.shape != lo.shape:
-            raise ValueError("a q8 latent of %d rows is uint8 codes (%d, %d) and float32 lo / step (%d, %d)"
-                             % (n, n, self.z_dim, latent_q8.n_blocks(n), self.z_dim))
-        y = out if out is not None else np.empty((n, self.n_features), dtype=y_dtype)
-        feats = None if features is None else np.ascontiguousarray(features, dtype=np.float32)
-        check(_lib.lib().bb_decompress_host_q8(self.handle, codes.ctypes.data, lo.ctypes.data, step.ctypes.data, n,
-                                               None if feats is None else feats.ctypes.data, y.ctypes.data, _NP2BB[y.dtype],
-                                               _prec(precision)), "bb_decompress_host_q8")
-        return y
+        return self.decompress_host_packed(latent_q8.PackedLatent(*q, 8), features, y_dtype, precision, out)
 
 
 # torch's CPU generator state (torch.Generator.get_state(), 5056 bytes): the MT19937 engine as

@@ -39,8 +39,11 @@ class Config:
       latent_dtype     "float64" (AE default, what the reference writes; any model under "fp64") | "float32" | "float16"
                        | "q8": uint8 codes with a float32 (min, step) per latent column and 128-row block (latent_q8),
                        z + 8 z / 128 bytes per row (15.9 for z = 15, against 120 as float64 and 30 as float16); every
-                       latent value within half its block's step.  decompress recognises such a file by itself.  Not
-                       with precision "fp64"
+                       latent value within half its block's step
+                       | "q2" ... "q7": the same with b-bit codes, 2^b - 2 steps per block column, packed row by row:
+                       ceil(z b / 8) + 8 z / 128 bytes per row (8.94 for z = 15 at "q4"), the step / 2 error growing by
+                       about 2x per bit removed.  decompress recognises a quantised file by itself.  Not with precision
+                       "fp64"; another "q..." value is refused
       l1_in_training   bool: add reg_param * L1 chain to the training loss (dead code upstream, SURVEY F2)
     No key is needed for tables larger than device memory: --mode train normalises the table in row chunks, keeps it
     resident when it fits the device memory the trainer leaves (training.device_table_budget), and otherwise streams
@@ -207,22 +210,24 @@ def get_device():
 
 
 def _latent_np_dtype(model, config):
-    """numpy type of the latent compress writes, or latent_q8.NAME for the 8-bit latent"""
+    """numpy type of the latent compress writes, or the latent_dtype name ("q2" ... "q8") of a quantised latent"""
     name = getattr(config, "latent_dtype", None)
     if name is None:
         return np.float64 if model.dtype == torch.float64 or _fp64(config) else np.float32
-    if name == latent_q8.NAME:
-        return latent_q8.NAME
+    if latent_q8.bits_of(name) is not None:
+        return name
     return np.dtype(name).type
 
 
 def _fp64(config):
     """config.precision == "fp64": the float64 chain; refuses what it does not do before anything is read or written"""
+    bits = latent_q8.bits_of(getattr(config, "latent_dtype", None))  # (ValueError for an unknown "q..." value)
     if engine.PRECISIONS.get(getattr(config, "precision", "auto")) != engine.BB_PREC_FP64:
         return False
-    if getattr(config, "latent_dtype", None) == latent_q8.NAME:
-        raise NotImplementedError("precision='fp64' does not write or read an 8-bit latent (latent_dtype='q8'): the 8-bit "
-                                  "codes discard far more than float64 arithmetic gains; use another precision or latent_dtype")
+    if bits is not None:
+        raise NotImplementedError("precision='fp64' does not write or read a quantised latent (latent_dtype='q%d'): the "
+                                  "%d-bit codes discard far more than float64 arithmetic gains; use another precision or "
+                                  "latent_dtype" % (bits, bits))
     if getattr(config, "save_error_bounded_deltas", False):
         raise NotImplementedError("precision='fp64' does not compute error-bounded deltas (save_error_bounded_deltas); "
                                   "use another precision for them")
@@ -300,8 +305,9 @@ def compress(model_path, config):
     codec = model.codec(data_before.shape[1], data_before.shape[2]) if conv else model.codec()
     if getattr(config, "save_error_bounded_deltas", False):
         return _compress_with_deltas(codec, model, table, normalise, config, rank, world)
-    if _latent_np_dtype(model, config) == latent_q8.NAME:
-        return _compress_q8(codec, table, normalise, config, rank, world), [], [], []
+    bits = latent_q8.bits_of(getattr(config, "latent_dtype", None))
+    if bits is not None:
+        return _compress_packed(codec, table, normalise, config, rank, world, bits), [], [], []
     if world == 1:
         compressed, _ = codec.compress_host(table, recompute_minmax=normalise,
                                             z_dtype=_latent_np_dtype(model, config),
@@ -320,31 +326,31 @@ def compress(model_path, config):
     return sharded.gather_rows_to_rank0(z, len(table)), [], [], []
 
 
-def _compress_q8(codec, table, normalise, config, rank, world):
-    """latent_dtype "q8": the 8-bit latent (latent_q8.Q8Latent of numpy arrays).  Under torchrun the shards start on the
-    128-row blocks of the file, so each rank's blocks are the file's and rank 0's gathered result is the one-process
-    file byte for byte; the other ranks return None."""
+def _compress_packed(codec, table, normalise, config, rank, world, bits):
+    """latent_dtype "q2" ... "q8": the quantised latent (latent_q8.PackedLatent of numpy arrays).  Under torchrun the shards
+    start on the 128-row blocks of the file, so each rank's blocks are the file's and rank 0's gathered result is the
+    one-process file byte for byte; the other ranks return None."""
     from .. import sharded
     precision = getattr(config, "precision", "auto")
     if world == 1:
-        return codec.compress_host_q8(table, recompute_minmax=normalise, precision=precision)[0]
+        return codec.compress_host_packed(table, bits, recompute_minmax=normalise, precision=precision)[0]
     n = len(table)
     lo, hi = sharded.row_range(n, rank, world, latent_q8.BLOCK_ROWS)
     shard = table[lo:hi]
     feats = sharded.global_minmax(shard) if normalise else None
-    q = (codec.compress_host_q8(shard, features=feats, precision=precision)[0] if len(shard)
-         else latent_q8.empty(0, codec.z_dim))
-    return _gather_q8(q, n)
+    q = (codec.compress_host_packed(shard, bits, features=feats, precision=precision)[0] if len(shard)
+         else latent_q8.empty_packed(0, codec.z_dim, bits))
+    return _gather_packed(q, n)
 
 
-def _gather_q8(q, n_rows):
-    """this rank's block-aligned share of a q8 latent -> the whole Q8Latent on rank 0 (codes by rows, parameters by
-    blocks: the block ranges of aligned row shards are row_range of the block count), None on the other ranks"""
+def _gather_packed(q, n_rows):
+    """this rank's block-aligned share of a quantised latent -> the whole PackedLatent on rank 0 (codes by rows,
+    parameters by blocks: the block ranges of aligned row shards are row_range of the block count), None on the others"""
     from .. import sharded
     codes = sharded.gather_rows_to_rank0(q.codes, n_rows, align=latent_q8.BLOCK_ROWS)
     mins = sharded.gather_rows_to_rank0(q.lo, latent_q8.n_blocks(n_rows))
     steps = sharded.gather_rows_to_rank0(q.step, latent_q8.n_blocks(n_rows))
-    return None if codes is None else latent_q8.Q8Latent(codes, mins, steps)
+    return None if codes is None else latent_q8.PackedLatent(codes, mins, steps, q.bits)
 
 
 def _compress_with_deltas(codec, model, table, normalise, config, rank=0, world=1):
@@ -355,15 +361,16 @@ def _compress_with_deltas(codec, model, table, normalise, config, rank=0, world=
     config.batch_size rows on the host, in the reference's (batch index, deltas, (row-in-batch, column)) lists.
     Launched under torchrun every rank scans its contiguous row range (hits carry GLOBAL row numbers), rank 0 collects the
     latent rows and the hit lists and regroups them; the other ranks return (None, [], [], []).
-    latent_dtype "q8": each chunk's latent is quantised, and the deltas correct decode(dequantise(quantise(encode(x)))),
-    the rows decompress reproduces; shards and chunks start on 128-row blocks."""
+    latent_dtype "q2" ... "q8": each chunk's latent is quantised, and the deltas correct
+    decode(dequantise(quantise(encode(x)))), the rows decompress reproduces; shards and chunks start on 128-row blocks."""
     from .. import engine, sharded
     n, bs = len(table), int(config.batch_size)
     z_dtype = _latent_np_dtype(model, config)
-    q8 = z_dtype == latent_q8.NAME
-    lo, hi = sharded.row_range(n, rank, world, latent_q8.BLOCK_ROWS if q8 else 1)
+    bits = latent_q8.bits_of(z_dtype)
+    lo, hi = sharded.row_range(n, rank, world, latent_q8.BLOCK_ROWS if bits else 1)
     shard = table[lo:hi]
-    compressed = latent_q8.empty(hi - lo, codec.z_dim) if q8 else np.empty((hi - lo, codec.z_dim), dtype=z_dtype)
+    compressed = (latent_q8.empty_packed(hi - lo, codec.z_dim, bits) if bits
+                  else np.empty((hi - lo, codec.z_dim), dtype=z_dtype))
     mn = rg = None
     if normalise and n:
         # this file's own [min; range] (helper.py:500-502), over all ranks' rows
@@ -374,13 +381,13 @@ def _compress_with_deltas(codec, model, table, normalise, config, rank=0, world=
     for r0 in range(0, hi - lo, chunk):
         x = torch.from_numpy(shard[r0:r0 + chunk]).cuda()
         z = codec.encode(x, mn, rg, precision=getattr(config, "precision", "auto"))
-        if q8:  # (chunk is a multiple of the block)
-            qz = codec.quantize_q8(z)
+        if bits:  # (chunk is a multiple of the block)
+            qz = codec.quantize_packed(z, bits)
             b0 = r0 // latent_q8.BLOCK_ROWS
             compressed.codes[r0:r0 + chunk] = qz.codes.cpu().numpy()
             compressed.lo[b0:b0 + len(qz.lo)] = qz.lo.cpu().numpy()
             compressed.step[b0:b0 + len(qz.step)] = qz.step.cpu().numpy()
-            z = codec.dequantize_q8(qz)
+            z = codec.dequantize_packed(qz)
         else:
             compressed[r0:r0 + chunk] = z.cpu().numpy().astype(z_dtype, copy=False)
         y = codec.decode(z, precision=getattr(config, "precision", "auto"))  # still normalised, as upstream compares it
@@ -390,7 +397,7 @@ def _compress_with_deltas(codec, model, table, normalise, config, rank=0, world=
     cols = np.concatenate(cols) if cols else np.empty(0, np.int64)
     deltas = np.concatenate(deltas) if deltas else np.empty(0, np.float16)
     if world > 1:
-        compressed = _gather_q8(compressed, n) if q8 else sharded.gather_rows_to_rank0(compressed, n)
+        compressed = _gather_packed(compressed, n) if bits else sharded.gather_rows_to_rank0(compressed, n)
         hits = sharded.gather_objects_to_rank0((rows, cols, deltas))
         if rank != 0:
             return None, [], [], []
@@ -438,12 +445,12 @@ def decompress(model_path, input_path, input_path_deltas, input_batch_index, mod
     fp64 = _fp64(config)
     rank, world = sharded.dist_env()  # under torchrun: this rank's GPU, before anything touches a device
     loaded = np.load(input_path)
-    q8 = latent_q8.from_npz(loaded) if latent_q8.in_file(loaded) else None  # (checks the arrays before any work)
-    if q8 is not None and fp64:
-        raise NotImplementedError("%s holds an 8-bit latent (latent_dtype='q8'), which precision='fp64' does not read"
-                                  % input_path)
+    quant = latent_q8.read(loaded) if latent_q8.in_file(loaded) else None  # (checks the arrays before any work)
+    if quant is not None and fp64:
+        raise NotImplementedError("%s holds a %d-bit latent (latent_dtype='q%d'), which precision='fp64' does not read"
+                                  % (input_path, quant.bits, quant.bits))
     data, names, normalization_features = loaded["data"], loaded["names"], loaded["normalization_features"]
-    latent_space_size = data.shape[1]
+    latent_space_size = data.shape[1] if quant is None else quant.lo.shape[1]  # (packed rows are narrower than the latent)
     model_dict = torch.load(str(model_path), map_location="cpu")
     # the reference reads len() of the last state-dict entry, which crashes on AE_Dropout_BN's
     # num_batches_tracked scalar (SURVEY F7a); take the last tensor that has a length instead
@@ -454,7 +461,7 @@ def decompress(model_path, input_path, input_path_deltas, input_batch_index, mod
     if fp64:
         _refuse_fp64_shape(model)
         data = engine.host_convert(data, np.float64)  # the latent goes to the float64 chain as float64
-    if q8 is None and data.dtype not in (np.float16, np.float32, np.float64):
+    if quant is None and data.dtype not in (np.float16, np.float32, np.float64):
         data = data.astype(np.float32)
     out_dtype = np.float64 if model.dtype == torch.float64 else np.float32
     conv = config.data_dimension == 2 and config.model_type == "convolutional"
@@ -474,15 +481,15 @@ def decompress(model_path, input_path, input_path_deltas, input_batch_index, mod
     precision = getattr(config, "precision", "auto")
 
     def run(lo, hi):  # rows [lo, hi) of the file
-        if q8 is not None:
-            return codec.decompress_host_q8(latent_q8.rows(q8, lo, hi), features=renormalize_features, y_dtype=out_dtype,
-                                            precision=precision)
+        if quant is not None:
+            return codec.decompress_host_packed(latent_q8.rows(quant, lo, hi), features=renormalize_features,
+                                                y_dtype=out_dtype, precision=precision)
         return codec.decompress_host(np.ascontiguousarray(data[lo:hi]), features=renormalize_features, y_dtype=out_dtype,
                                      precision=precision)
     if world == 1:
         decompressed = run(0, len(data))
     else:  # under torchrun: every rank decodes its contiguous row range, rank 0 collects (the others return None data)
-        align = latent_q8.BLOCK_ROWS if q8 is not None else 1  # (a q8 latent is cut on its blocks)
+        align = latent_q8.BLOCK_ROWS if quant is not None else 1  # (a quantised latent is cut on its blocks)
         lo, hi = sharded.row_range(len(data), rank, world, align)
         part = run(lo, hi) if hi > lo else np.empty((0, codec.n_features), dtype=out_dtype)
         decompressed = sharded.gather_rows_to_rank0(part, len(data), align=align)

@@ -240,6 +240,29 @@ int bb_compress_host_q8(bb_model* m, const float* x_host, int64_t n_rows, float*
 int bb_decompress_host_q8(bb_model* m, const uint8_t* codes_host, const float* lo_host, const float* step_host, int64_t n_rows,
                           const float* features_host, void* y_host, int y_dtype, int precision);
 
+/* ------------------------------------------------------------------ b-bit latent (latent_dtype "q2" ... "q8") */
+/*
+ * The 8-bit latent above at `bits` bits per code, BB_LATENT_MIN_BITS <= bits <= BB_LATENT_MAX_BITS.  With L = 2^bits - 2:
+ *   step      float32((float64(hi) - float64(lo)) / L)
+ *   code      2^bits - 1 for a non-finite value; 0 when step == 0; else clamp(rint(...), 0, L) as above
+ * Row r of the codes is row_bytes = ceil(z_dim * bits / 8) bytes: column j's code is bits [j * bits, (j + 1) * bits) of the
+ * row, bit k being bit k % 8 of byte k / 8; the unused high bits of the last byte are 0.  codes are n_rows x row_bytes bytes,
+ * lo / step ceil(n_rows / BB_Q8_BLOCK_ROWS) x z_dim floats.  bits = 8 is the 8-bit latent, byte for byte: the four _q8
+ * entry points are these with bits = 8.  bits outside the range returns BB_ERR_INVALID; BB_PREC_FP64 BB_ERR_UNSUPPORTED.
+ * The quantise kernel stages a block's codes in shared memory: 128 x (row_bytes + z_dim) bytes (128 x z_dim for bits = 8)
+ * must fit a block's shared memory (z_dim up to about 1,700 at 8 bits on a B200), else BB_ERR_UNSUPPORTED.
+ */
+#define BB_LATENT_MIN_BITS 2
+#define BB_LATENT_MAX_BITS 8
+int bb_latent_quantize_packed(bb_ctx* ctx, const float* z_dev, int64_t n_rows, int z_dim, int bits, uint8_t* codes_dev,
+                              float* lo_dev, float* step_dev, bb_stream_t stream);
+int bb_latent_dequantize_packed(bb_ctx* ctx, int bits, const uint8_t* codes_dev, const float* lo_dev, const float* step_dev,
+                                int64_t n_rows, int z_dim, float* z_dev, bb_stream_t stream);
+int bb_compress_host_packed(bb_model* m, const float* x_host, int64_t n_rows, float* features_host, int recompute_minmax,
+                            int bits, uint8_t* codes_host, float* lo_host, float* step_host, int precision);
+int bb_decompress_host_packed(bb_model* m, int bits, const uint8_t* codes_host, const float* lo_host, const float* step_host,
+                              int64_t n_rows, const float* features_host, void* y_host, int y_dtype, int precision);
+
 /* ------------------------------------------------------------------ training (dense AE) */
 
 typedef struct bb_train_hyper {
