@@ -199,11 +199,13 @@ constexpr float LBN_EPS = 1e-5f, LBN_MOMENTUM = 0.1f;
 // BatchNorm over channel c = blockIdx.x of Z[rows][N] (channel c = columns c*S .. c*S + S - 1), then the activation, in
 // place.  training: batch statistics (saved for the backward pass in mean_rstd, running statistics updated);
 // otherwise the running statistics.  xhat (nullable) receives the normalised values, pre (nullable) the input values.
+// `updates`: running-statistics updates from this batch (2 for the encoder under loss_function_swae, which upstream
+// encodes a second time with the same batch statistics).
 __global__ void __launch_bounds__(256) bn_fwd_kernel(float* __restrict__ Z, float* __restrict__ xhat, const int rows, const int N,
                                                      const int S, const int C, const float* __restrict__ gamma,
                                                      const float* __restrict__ beta, float* __restrict__ running,
                                                      float* __restrict__ mean_rstd, const int training, const int act,
-                                                     float* __restrict__ pre) {
+                                                     float* __restrict__ pre, const int updates) {
   __shared__ float red[256];
   const int c = blockIdx.x, M = rows * S;
   float mean, rstd;
@@ -219,8 +221,10 @@ __global__ void __launch_bounds__(256) bn_fwd_kernel(float* __restrict__ Z, floa
     const float var = block_sum_256(s, red) / M;
     rstd = 1.f / sqrtf(var + LBN_EPS);
     if (threadIdx.x == 0) {
-      running[c] = (1.f - LBN_MOMENTUM) * running[c] + LBN_MOMENTUM * mean;
-      running[C + c] = (1.f - LBN_MOMENTUM) * running[C + c] + LBN_MOMENTUM * (M > 1 ? var * M / (M - 1) : var);
+      for (int u = 0; u < updates; ++u) {
+        running[c] = (1.f - LBN_MOMENTUM) * running[c] + LBN_MOMENTUM * mean;
+        running[C + c] = (1.f - LBN_MOMENTUM) * running[C + c] + LBN_MOMENTUM * (M > 1 ? var * M / (M - 1) : var);
+      }
       mean_rstd[c] = mean;
       mean_rstd[C + c] = rstd;
     }
@@ -393,6 +397,117 @@ __global__ void __launch_bounds__(256) swd_sort_kernel(float* __restrict__ lat, 
   if (threadIdx.x == 0) part[s] = acc;
 }
 
+// Batches above SWD_MAX_ROWS: the projections are kept transposed (latT / priT [S][rows], one contiguous segment per
+// projection) and one block sorts each segment in global memory with a stable LSD radix sort: SWR_PASSES passes of
+// SWR_BITS bits over order-preserving keys, -0 folded onto +0, so that equal values are ties kept in row order as
+// np.argsort(kind="stable") keeps them.  Each pass scatters the segment in chunks of 256 keys, in order: a key's slot is
+// its digit's running offset + the count of that digit in the chunk's earlier warps + its rank among its warp's equal
+// digits.  The loss partial and the scatter of the gradient are those of swd_sort_kernel.
+constexpr int SWR_BITS = 8, SWR_BINS = 1 << SWR_BITS, SWR_PASSES = 32 / SWR_BITS, SWR_WARPS = 256 / 32;
+static_assert(SWR_BINS == 256, "one digit per thread");
+
+__device__ __forceinline__ uint32_t swr_key(float f) {
+  uint32_t b = __float_as_uint(f);
+  if ((b << 1) == 0u) b = 0u;  // -0 -> +0
+  return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
+}
+
+__device__ __forceinline__ float swr_value(const uint32_t k) {
+  return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k);
+}
+
+struct SwrShared {
+  int hist[SWR_PASSES][SWR_BINS];
+  int wc[2][SWR_WARPS][SWR_BINS];  // per-warp digit counts, then their slots; two chunks in flight
+};
+
+// the digit histograms of all passes, from the float segment src[n]
+__device__ void swr_histogram(SwrShared& sh, const float* src, const int n) {
+  for (int i = threadIdx.x; i < SWR_PASSES * SWR_BINS; i += 256) (&sh.hist[0][0])[i] = 0;
+  __syncthreads();
+  for (int i = threadIdx.x; i < n; i += 256) {
+    const uint32_t k = swr_key(src[i]);
+#pragma unroll
+    for (int p = 0; p < SWR_PASSES; ++p) atomicAdd(&sh.hist[p][(k >> (p * SWR_BITS)) & (SWR_BINS - 1)], 1);
+  }
+  __syncthreads();
+}
+
+// one stable pass: keys of src (pass 0: the float segment fsrc, row i's index i) -> kdst / idst (idst nullable)
+__device__ void swr_pass(SwrShared& sh, const float* fsrc, const uint32_t* ksrc, const int* isrc, uint32_t* kdst, int* idst,
+                         const int n, const int pass) {
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, shift = pass * SWR_BITS;
+  int next = 0;  // thread t: first free slot of digit t
+  for (int d = 0; d < tid; ++d) next += sh.hist[pass][d];
+  for (int c0 = 0, buf = 0; c0 < n; c0 += 256, buf ^= 1) {
+    const int i = c0 + tid;
+    uint32_t k = 0;
+    int ix = i, d = -1 - lane;  // lanes past the end: a digit of their own
+    if (i < n) {
+      k = fsrc ? swr_key(fsrc[i]) : ksrc[i];
+      if (isrc) ix = isrc[i];
+      d = (int)((k >> shift) & (SWR_BINS - 1));
+    }
+    const unsigned peers = __match_any_sync(0xffffffffu, d);
+    const int rank = __popc(peers & ((1u << lane) - 1u));
+    if (d >= 0 && rank == 0) sh.wc[buf][warp][d] = __popc(peers);
+    __syncthreads();
+    int run = next;
+#pragma unroll
+    for (int w = 0; w < SWR_WARPS; ++w) {
+      const int cnt = sh.wc[buf][w][tid];
+      sh.wc[buf][w][tid] = run;
+      sh.wc[buf ^ 1][w][tid] = 0;  // the other buffer's last readers finished before the barrier above
+      run += cnt;
+    }
+    next = run;
+    __syncthreads();
+    if (d >= 0) {
+      const int pos = sh.wc[buf][warp][d] + rank;
+      kdst[pos] = k;
+      if (idst) idst[pos] = ix;
+    }
+  }
+  __syncthreads();  // the pass's writes are visible to the next pass's readers of the block ...
+#pragma unroll
+  for (int w = 0; w < SWR_WARPS; ++w) sh.wc[0][w][tid] = sh.wc[1][w][tid] = 0;  // ... which start from zero counts
+  __syncthreads();
+}
+
+// block s: sorts priT's segment (its keys end in priT) and latT's with its row indices (ending in kb / ib), then
+// part[s] and the gradient d latT[s][perm_i] = 2 w_i coef, written over latT
+__global__ void __launch_bounds__(256) swd_radix_kernel(float* __restrict__ latT, float* __restrict__ priT, const int rows,
+                                                        uint32_t* __restrict__ ka, uint32_t* __restrict__ kb,
+                                                        int* __restrict__ ia, int* __restrict__ ib, const float coef,
+                                                        float* __restrict__ part) {
+  static_assert(SWR_PASSES == 4, "the ping-pong below ends in kb / ib and priT");
+  __shared__ SwrShared sh;
+  __shared__ float red[256];
+  const size_t off = (size_t)blockIdx.x * rows;
+  float *lat = latT + off, *pri = priT + off;
+  uint32_t *a = ka + off, *b = kb + off, *pk = reinterpret_cast<uint32_t*>(pri);
+  int *xa = ia + off, *xb = ib + off;
+  for (int i = threadIdx.x; i < 2 * SWR_WARPS * SWR_BINS; i += 256) (&sh.wc[0][0][0])[i] = 0;  // (every pass leaves it so)
+  swr_histogram(sh, pri, rows);
+  swr_pass(sh, pri, nullptr, nullptr, a, nullptr, rows, 0);
+  swr_pass(sh, nullptr, a, nullptr, b, nullptr, rows, 1);
+  swr_pass(sh, nullptr, b, nullptr, a, nullptr, rows, 2);
+  swr_pass(sh, nullptr, a, nullptr, pk, nullptr, rows, 3);
+  swr_histogram(sh, lat, rows);
+  swr_pass(sh, lat, nullptr, nullptr, a, xa, rows, 0);
+  swr_pass(sh, nullptr, a, xa, b, xb, rows, 1);
+  swr_pass(sh, nullptr, b, xb, a, xa, rows, 2);
+  swr_pass(sh, nullptr, a, xa, b, xb, rows, 3);
+  float acc = 0.f;
+  for (int i = threadIdx.x; i < rows; i += 256) {
+    const float w = swr_value(b[i]) - swr_value(pk[i]);
+    acc += w * w;
+    lat[xb[i]] = 2.f * w * coef;
+  }
+  acc = block_sum_256(acc, red);
+  if (threadIdx.x == 0) part[blockIdx.x] = acc;
+}
+
 // loss_part[0] += coef * sum_s part[s] (fixed order);  dst[e] += src[e]
 __global__ void __launch_bounds__(256) swd_fold_kernel(const float* __restrict__ part, const int S, const float coef,
                                                        float* __restrict__ loss_part) {
@@ -466,6 +581,9 @@ struct bb_ltrainer {
   // loss_function_swae: projections of the latent batch / of the prior draws [max_batch][S], latent gradient, partials
   float *sw_lat = nullptr, *sw_pri = nullptr, *sw_dz = nullptr, *sw_part = nullptr;
   int sw_S = 0;
+  // batches above SWD_MAX_ROWS (max_batch > SWD_MAX_ROWS only): ping-pong keys and row indices of swd_radix_kernel
+  uint32_t* sw_key[2] = {nullptr, nullptr};
+  int* sw_idx[2] = {nullptr, nullptr};
   float* loss_part = nullptr;
   double* loss_accum = nullptr;
   long long step = 0;
@@ -555,10 +673,13 @@ int lforward_backward(bb_ltrainer* t, const float* x, int rows, bool backward, c
       dropout_fwd_kernel<<<ew_blocks, 256, 0, s>>>(A, rows, y.N, y.drop, t->seed, (unsigned long long)t->step, t->mask_dev[y.drop],
                                                    y.drop_scale, y.act);
     if (y.bn_c) {
+      // loss_function_swae: upstream's second model.encode(inputs) sees the same batch and weights, so the encoder's
+      // BatchNorm layers compute the same statistics again and update their running statistics a second time
+      const int updates = sw && l <= sw->latent_layer ? 2 : 1;
       bn_fwd_kernel<<<y.bn_c, 256, 0, s>>>(A, backward ? y.xhat : nullptr, rows, y.N, y.N / y.bn_c, y.bn_c, t->params + y.g_off,
                                            t->params + y.g_off + y.bn_c, y.running, y.mean_rstd, backward ? 1 : 0,
-                                           y.bn_post ? BB_ACT_NONE : y.act, backward && y.bn_post ? y.pre : nullptr);
-      if (backward) y.nbt += 1;
+                                           y.bn_post ? BB_ACT_NONE : y.act, backward && y.bn_post ? y.pre : nullptr, updates);
+      if (backward) y.nbt += updates;
     }
   }
   const int C = t->lay[L - 1].N;
@@ -569,15 +690,28 @@ int lforward_backward(bb_ltrainer* t, const float* x, int rows, bool backward, c
     // utils.compute_swd (utils.py:56-76): reg_weight / (B (B - 1)) * mean_{s, i} (sort(z P)_{s,i} - sort(prior P)_{s,i})^2
     const int D = t->lay[sw->latent_layer].N, S = sw->S;
     const float* Z = t->act + t->a_off[sw->latent_layer + 1];
-    lgemm(t, s, Z, D, 1, sw->proj, 1, D, t->sw_lat, S, rows, S, D, nullptr, BB_ACT_NONE);
-    lgemm(t, s, sw->prior, D, 1, sw->proj, 1, D, t->sw_pri, S, rows, S, D, nullptr, BB_ACT_NONE);
-    int n_pow2 = 1;
-    while (n_pow2 < rows) n_pow2 <<= 1;
-    const float coef = sw->reg_weight / ((float)rows * (float)(rows - 1)) / ((float)S * (float)rows);
-    swd_sort_kernel<<<S, 256, sizeof(float) * 3 * n_pow2, s>>>(t->sw_lat, t->sw_pri, rows, S, n_pow2, coef, t->sw_part);
-    swd_fold_kernel<<<1, 256, 0, s>>>(t->sw_part, S, coef, t->loss_part);
-    // d latent = d(z P) . P^T... as [rows][S] . [S][D]
-    if (backward) lgemm(t, s, t->sw_lat, S, 1, sw->proj, D, 1, t->sw_dz, D, rows, D, S, nullptr, BB_ACT_NONE);
+    if (rows <= SWD_MAX_ROWS) {
+      lgemm(t, s, Z, D, 1, sw->proj, 1, D, t->sw_lat, S, rows, S, D, nullptr, BB_ACT_NONE);
+      lgemm(t, s, sw->prior, D, 1, sw->proj, 1, D, t->sw_pri, S, rows, S, D, nullptr, BB_ACT_NONE);
+      int n_pow2 = 1;
+      while (n_pow2 < rows) n_pow2 <<= 1;
+      const float coef = sw->reg_weight / ((float)rows * (float)(rows - 1)) / ((float)S * (float)rows);
+      swd_sort_kernel<<<S, 256, sizeof(float) * 3 * n_pow2, s>>>(t->sw_lat, t->sw_pri, rows, S, n_pow2, coef, t->sw_part);
+      swd_fold_kernel<<<1, 256, 0, s>>>(t->sw_part, S, coef, t->loss_part);
+      // d latent = d(z P) . P^T... as [rows][S] . [S][D]
+      if (backward) lgemm(t, s, t->sw_lat, S, 1, sw->proj, D, 1, t->sw_dz, D, rows, D, S, nullptr, BB_ACT_NONE);
+    } else {
+      // transposed projections [S][rows] (the same products, k ascending), sorted segment by segment in global memory;
+      // the weight in float64, rounded once: B (B - 1) is not exact in float32 above 4096 rows
+      lgemm(t, s, sw->proj, D, 1, Z, 1, D, t->sw_lat, rows, S, rows, D, nullptr, BB_ACT_NONE);
+      lgemm(t, s, sw->proj, D, 1, sw->prior, 1, D, t->sw_pri, rows, S, rows, D, nullptr, BB_ACT_NONE);
+      const float coef = (float)((double)sw->reg_weight / ((double)rows * (double)(rows - 1)) / ((double)S * (double)rows));
+      swd_radix_kernel<<<S, 256, 0, s>>>(t->sw_lat, t->sw_pri, rows, t->sw_key[0], t->sw_key[1], t->sw_idx[0], t->sw_idx[1], coef,
+                                         t->sw_part);
+      swd_fold_kernel<<<1, 256, 0, s>>>(t->sw_part, S, coef, t->loss_part);
+      // d latent [rows][D] = (d latT)^T . P
+      if (backward) lgemm(t, s, t->sw_lat, 1, rows, sw->proj, D, 1, t->sw_dz, D, rows, D, S, nullptr, BB_ACT_NONE);
+    }
   }
   if (!backward) return (int)cudaGetLastError();
   int cur = 0;
@@ -826,7 +960,7 @@ int bb_ltrainer_activation_means(bb_ltrainer* t, double* out_host_6x200) {
 int bb_ltrainer_destroy(bb_ltrainer* t) {
   if (!t) return BB_OK;
   void* ptrs[] = {t->params, t->grads, t->m, t->v, t->act, t->dz[0], t->dz[1], t->loss_part, t->loss_accum, t->running_all,
-                  t->sw_lat, t->sw_pri, t->sw_dz, t->sw_part, t->splitk};
+                  t->sw_lat, t->sw_pri, t->sw_dz, t->sw_part, t->sw_key[0], t->sw_key[1], t->sw_idx[0], t->sw_idx[1], t->splitk};
   for (void* p : ptrs)
     if (p) cudaFree(p);
   for (int l = 0; l < t->n_layers; ++l) {
@@ -909,21 +1043,28 @@ int bb_ltrainer_step_swae(bb_ltrainer* t, const float* x_dev, int batch_rows, co
                           double* loss_accum_dev, bb_stream_t stream) {
   if (!t || !prior_dev || !proj_dev || n_projections < 1 || latent_layer < 0 || latent_layer >= t->n_layers - 1)
     return BB_ERR_INVALID;
-  if (batch_rows < 2 || batch_rows > SWD_MAX_ROWS) return BB_ERR_UNSUPPORTED;  // B (B - 1) in the weight; shared-memory sort
+  if (batch_rows < 2) return BB_ERR_UNSUPPORTED;  // B (B - 1) in the weight
   for (int l = 0; l < t->n_layers; ++l)
-    if (t->lay[l].bn_c) return BB_ERR_UNSUPPORTED;  // upstream runs the encoder twice per step: BatchNorm statistics move twice
+    if (t->lay[l].drop >= 0) return BB_ERR_UNSUPPORTED;  // upstream's second encode would draw other dropout masks
   if (t->sw_S != n_projections) {
     BB_CUDA(cudaSetDevice(t->ctx->device));
     BB_CUDA(cudaStreamSynchronize((cudaStream_t)stream));
-    void* old[] = {t->sw_lat, t->sw_pri, t->sw_dz, t->sw_part};
+    void* old[] = {t->sw_lat, t->sw_pri, t->sw_dz, t->sw_part, t->sw_key[0], t->sw_key[1], t->sw_idx[0], t->sw_idx[1]};
     for (void* p : old)
       if (p) cudaFree(p);
     t->sw_lat = t->sw_pri = t->sw_dz = t->sw_part = nullptr;
+    t->sw_key[0] = t->sw_key[1] = nullptr;
+    t->sw_idx[0] = t->sw_idx[1] = nullptr;
     t->sw_S = 0;
-    BB_CUDA(cudaMalloc(&t->sw_lat, sizeof(float) * (size_t)t->max_batch * n_projections));
-    BB_CUDA(cudaMalloc(&t->sw_pri, sizeof(float) * (size_t)t->max_batch * n_projections));
+    const size_t n = (size_t)t->max_batch * n_projections;
+    BB_CUDA(cudaMalloc(&t->sw_lat, sizeof(float) * n));
+    BB_CUDA(cudaMalloc(&t->sw_pri, sizeof(float) * n));
     BB_CUDA(cudaMalloc(&t->sw_dz, sizeof(float) * (size_t)t->max_batch * t->max_dim));
     BB_CUDA(cudaMalloc(&t->sw_part, sizeof(float) * n_projections));
+    for (int i = 0; i < 2 && t->max_batch > SWD_MAX_ROWS; ++i) {
+      BB_CUDA(cudaMalloc(&t->sw_key[i], sizeof(uint32_t) * n));
+      BB_CUDA(cudaMalloc(&t->sw_idx[i], sizeof(int) * n));
+    }
     t->sw_S = n_projections;
   }
   SwaeArgs sw{prior_dev, proj_dev, n_projections, latent_layer, reg_weight};

@@ -793,12 +793,16 @@ class LayeredTrainer:
         check(_lib.lib().bb_ltrainer_get_bn(self.handle, ptrs), "bb_ltrainer_get_bn")
         if not self.dbn_kind:
             return out
-        nbt = (C.c_longlong * 8)()
-        check(_lib.lib().bb_ltrainer_bn_batches_tracked(self.handle, nbt), "bb_ltrainer_bn_batches_tracked")
         keys = ("weight", "bias", "running_mean", "running_var")
         res = {k: [out[4 + i][j].copy() for i in range(4)] for j, k in enumerate(keys)}
-        res["num_batches_tracked"] = [int(v) for v in nbt[4:]]
+        res["num_batches_tracked"] = [int(v) for v in self.bn_batches_tracked()[4:]]
         return res
+
+    def bn_batches_tracked(self):
+        """int64 array, one entry per layer: the batches its BatchNorm counted (num_batches_tracked; 0 without one)"""
+        nbt = (C.c_longlong * (len(self.dims) - 1))()
+        check(_lib.lib().bb_ltrainer_bn_batches_tracked(self.handle, nbt), "bb_ltrainer_bn_batches_tracked")
+        return np.array(nbt[:], dtype=np.int64)
 
     def bn_running_views(self):
         """zero-copy view of the running statistics of all BatchNorm layers (one tensor; DataParallelTrainer averages it)"""

@@ -45,6 +45,10 @@ class Config:
                        about 2x per bit removed.  decompress recognises a quantised file by itself.  Not with precision
                        "fp64"; another "q..." value is refused
       l1_in_training   bool: add reg_param * L1 chain to the training loss (dead code upstream, SURVEY F2)
+    custom_loss_function = "loss_function_swae" (a reference key) trains AE, CFD_dense_AE and Conv_AE at any batch
+    size that fits device memory, in one process; Conv_AE's encoder BatchNorm2d counts two batches per step, as
+    upstream's second model.encode(inputs) leaves it.  AE_Dropout_BN (the second encode draws other dropout masks),
+    torchrun and precision "fp64" are refused.
     No key is needed for tables larger than device memory: --mode train normalises the table in row chunks, keeps it
     resident when it fits the device memory the trainer leaves (training.device_table_budget), and otherwise streams
     every epoch and validation from host memory through two device windows of whole batches, with the same results.

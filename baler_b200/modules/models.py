@@ -130,6 +130,7 @@ class AE(_DenseBase):
     none on latent / output)."""
 
     names = ("en1", "en2", "en3", "en4", "de1", "de2", "de3", "de4")
+    latent_layer = 3  # the latent is the output of en4 (what loss_function_swae's model.encode returns)
 
     def _build(self):
         dims = (self.n_features,) + self.hidden + (self.z_dim,) + self.hidden[::-1] + (self.n_features,)
@@ -393,6 +394,7 @@ class Conv_AE:
              ("q_z_lin.0", "lin", 0, None), ("q_z_lin.2", "lin", 0, None), ("p_x_lin.0", "lin", 0, None),
              ("p_x_lin.2", "lin", 0, None), ("p_x_conv.0", "convT", 0, "p_x_conv.1"), ("p_x_conv.3", "convT", 1, "p_x_conv.4"),
              ("p_x_conv.6", "convT", 1, None)]
+    latent_layer = [c[0] for c in _CONV].index("q_z_lin.2")  # training_spec layer whose output model.encode returns
 
     def training_spec(self, h=5, w=5):
         """dict(dims, acts, weights, biases, w_maps, bn) for engine.LayeredTrainer.  w_maps[l][i] is the flat index of the
@@ -432,16 +434,17 @@ class Conv_AE:
         return dict(dims=dims, acts=acts, weights=weights, biases=biases, w_maps=maps, bn=bn)
 
     def load_trained(self, weights, biases, bn, steps):
-        """write the trainer's parameters (training_spec order) back into the state_dict; `steps` training forward passes
-        were made (num_batches_tracked)"""
-        for (name, kind, pad, bn_name), wt, bs, b4 in zip(self._CONV, weights, biases, bn):
+        """write the trainer's parameters (training_spec order) back into the state_dict; `steps` batches were counted
+        (num_batches_tracked): one count for every BatchNorm, or one per training_spec layer"""
+        steps = np.broadcast_to(np.asarray(steps, dtype=np.int64), (len(self._CONV),))
+        for (name, kind, pad, bn_name), wt, bs, b4, n in zip(self._CONV, weights, biases, bn, steps):
             dt = self._sd[name + ".weight"].dtype
             self._sd[name + ".weight"] = torch.from_numpy(np.asarray(wt)).reshape(self._sd[name + ".weight"].shape).to(dt)
             self._sd[name + ".bias"] = torch.from_numpy(np.asarray(bs)).reshape(-1).to(dt)
             if bn_name is not None:
                 for k, row in zip(("weight", "bias", "running_mean", "running_var"), b4):
                     self._sd[bn_name + "." + k] = torch.from_numpy(np.asarray(row)).to(dt)
-                self._sd[bn_name + ".num_batches_tracked"] = self._sd[bn_name + ".num_batches_tracked"] + int(steps)
+                self._sd[bn_name + ".num_batches_tracked"] = self._sd[bn_name + ".num_batches_tracked"] + int(n)
         self._codec = None
 
     def codec(self, h=5, w=5):

@@ -178,15 +178,17 @@ class DeviceAdam:
         self.conv = hasattr(model, "training_spec")
         self.trainer, self.steps = None, 0
         self.lr, self.l1, self.reg_param, self.swae = lr, l1, reg_param, swae
-        if swae and (self.conv or self.has_bn or self.world > 1):
-            # upstream encodes twice per step with this loss (training.py:66-72): BatchNorm / dropout state would move twice
-            raise NotImplementedError("loss_function_swae: dense models without BatchNorm / dropout, one process")
+        if swae and (self.has_bn or self.world > 1):
+            # upstream encodes twice per step with this loss (training.py:66-72): the second encode of AE_Dropout_BN draws
+            # other dropout masks.  Conv_AE's BatchNorm2d sees the same batch twice, which its trainer reproduces.
+            raise NotImplementedError("loss_function_swae: models without dropout (AE, CFD_dense_AE, Conv_AE), one process")
         if self.conv:
             # Conv_AE: (transposed) convolutions as weight-sharing dense layers, BatchNorm2d on batch statistics; the loss
             # divisor is true_data.shape[1] = 1 channel (utils.py:197)
             sp = model.training_spec(*block_hw)
             self.trainer = engine.LayeredTrainer(sp["weights"], sp["biases"], sp["acts"], max_batch, dims=sp["dims"],
                                                  w_maps=sp["w_maps"], bn=sp["bn"], loss_columns=1)
+            self.nbt_synced = np.zeros(len(sp["dims"]) - 1, dtype=np.int64)  # batches counted into the model so far
             self.dp = sharded.DataParallelTrainer(self.trainer) if self.world > 1 else None
             return
         w, b = model.linear_tensors()
@@ -242,7 +244,8 @@ class DeviceAdam:
         """one pass with config.custom_loss_function = "loss_function_swae" (training.py:70-78).  The two random inputs of
         utils.compute_swd are drawn here from torch's global CPU generator in the reference's order - randn_like(z), then
         randn(num_projections, latent_dim) normalised per row (utils.py:57-90) - in float32 (upstream cannot run this loss on
-        the float64 AE: its float32 projections meet a double latent), and handed to the device step."""
+        the float64 AE: its float32 projections meet a double latent), and handed to the device step.  The latent is the
+        output of the model's layer `latent_layer` (q_z_lin.2 for Conv_AE, whose rows are _training_table's (N, H W))."""
         tr = self.trainer
         tr.loss_accum.zero_()
         n_batches = 0
@@ -253,15 +256,19 @@ class DeviceAdam:
             prior = torch.randn((xb.shape[0], latent_dim), dtype=torch.float32)
             proj = torch.randn(self.SWAE_PROJECTIONS, latent_dim)
             proj = proj / proj.norm(dim=1).view(-1, 1)
-            tr.step_swae(xb, self.hyper(), prior.cuda(), proj.cuda(), latent_layer=3, reg_weight=self.SWAE_REG_WEIGHT)
+            tr.step_swae(xb, self.hyper(), prior.cuda(), proj.cuda(), latent_layer=self.model.latent_layer,
+                         reg_weight=self.SWAE_REG_WEIGHT)
             n_batches += 1
         self.steps += n_batches
         return tr.loss_accum.item() / n_batches
 
     def sync_model(self):
         if self.conv:
+            # num_batches_tracked per BatchNorm layer: the encoder's counts 2 per loss_function_swae step
             w, b = self.trainer.get_params()
-            self.model.load_trained(w, b, self.trainer.get_bn(), self.steps)
+            nbt = self.trainer.bn_batches_tracked()
+            self.model.load_trained(w, b, self.trainer.get_bn(), nbt - self.nbt_synced)
+            self.nbt_synced = nbt
             self.steps = 0
             return
         w, b = self.trainer.get_params()

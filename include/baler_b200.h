@@ -485,8 +485,13 @@ int bb_ltrainer_step(bb_ltrainer* t, const float* x_dev, int batch_rows, const b
  * inputs of utils.compute_swd are the caller's: `prior_dev` [batch_rows][z_dim] (torch.randn_like(z)) and `proj_dev`
  * [n_projections][z_dim] unit rows (utils.get_random_projections), so a caller that draws them from torch's generator
  * in the reference's order reproduces the reference's stream.  Upstream encodes twice per step (model(inputs), then
- * model.encode(inputs)): identical values for a model without dropout / BatchNorm, which is what is accepted here
- * (BatchNorm layers: BB_ERR_UNSUPPORTED).  2 <= batch_rows <= 2048.  phase as in bb_ltrainer_step.
+ * model.encode(inputs)) with the same batch and weights: the same values and batch statistics, and the gradient of
+ * the two backward passes is this step's single one.  BatchNorm layers at or before `latent_layer` update their running
+ * statistics twice per step and count 2 batches (bb_ltrainer_bn_batches_tracked), later ones once.  Layers with dropout
+ * (the second encode would draw other masks): BB_ERR_UNSUPPORTED.  2 <= batch_rows <= max_batch: up to 2048 rows each
+ * projection is sorted in shared memory, above that by a stable radix sort in global memory (ties in row order), whose
+ * scratch (4 x max_batch x n_projections x 4 bytes) is allocated by the first step of a trainer with max_batch > 2048.
+ * phase as in bb_ltrainer_step.
  */
 int bb_ltrainer_step_swae(bb_ltrainer* t, const float* x_dev, int batch_rows, const bb_train_hyper* h, int phase,
                           const float* prior_dev, const float* proj_dev, int n_projections, int latent_layer, float reg_weight,
