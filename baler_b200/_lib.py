@@ -12,6 +12,7 @@ LIB_PATH = os.path.join(HERE, "libbaler_b200.so")
 BB_F32, BB_F16, BB_F64 = 0, 1, 2
 BB_ACT_NONE, BB_ACT_LEAKY, BB_ACT_RELU = 0, 1, 2
 BB_PREC_AUTO, BB_PREC_FP32, BB_PREC_SPLIT16, BB_PREC_FAST16, BB_PREC_FP64 = 0, 1, 2, 3, 4
+BB_ERROR_STATS_FIELDS = 24  # 8-byte words per column of a bb_error_stats record
 PRECISIONS = {"auto": BB_PREC_AUTO, "exact": BB_PREC_AUTO, "fp32": BB_PREC_FP32,
               "split16": BB_PREC_SPLIT16, "fast": BB_PREC_FAST16, "fast16": BB_PREC_FAST16, "fp64": BB_PREC_FP64}
 
@@ -102,6 +103,7 @@ _SIGNATURES = {
     "bb_ltrainer_validate_host": (C.c_int, [_P, _P, C.c_int, C.c_int64, C.c_int, C.c_int64, C.POINTER(C.c_double), _P]),
     "bb_trainer_activation_means": (C.c_int, [_P, _P]),
     "bb_mse_sum_f32": (C.c_int, [_P, _P, _P, C.c_int64, _P, _P]),
+    "bb_error_stats": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_int64, C.c_int, C.c_int64, _P, _P, _P, _P, _P, _P]),
     "bb_error_bounded_deltas_f32": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int, _P, _P, C.c_double, C.c_int64, C.c_int64, _P, _P, _P, _P, _P]),
     "bb_ltrainer_create": (C.c_int, [_P, C.c_int, _P, _P, _P, _P, C.c_int, _PP]),
     "bb_ltrainer_create_ex": (C.c_int, [_P, C.c_int, _P, _P, _P, _P, _P, _P, _P, _P, _P, C.c_int, C.c_int, _PP]),

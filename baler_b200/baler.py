@@ -13,7 +13,7 @@ from math import ceil
 
 import numpy as np
 
-from . import latent_q8
+from . import error_report, latent_q8
 from .modules import helper
 
 __all__ = ("perform_compression", "perform_decompression", "perform_training", "print_info")
@@ -92,17 +92,24 @@ def perform_training(output_path, config, verbose):
 
 def perform_compression(output_path, config, verbose):
     """reference baler.py:239-338"""
+    report = error_report.enabled(config)  # (ValueError for a non-bool value, before any file is read)
     print("Compressing...")
     start = time.time()
     normalization_features = []
     if config.apply_normalization:
         normalization_features = np.load(os.path.join(output_path, "training", "normalization_features.npy"))
-    compressed, error_bound_batch, error_bound_deltas, error_bound_index = helper.compress(
-        model_path=os.path.join(output_path, "compressed_output", "model.pt"), config=config)
+    extra = {}
+    if report:  # the features decompress un-normalises with (perform_decompression)
+        extra["renormalize_features"] = (np.asarray(normalization_features).reshape(2, -1) if config.apply_normalization
+                                         else None)
+    compressed, error_bound_batch, error_bound_deltas, error_bound_index, *record = helper.compress(
+        model_path=os.path.join(output_path, "compressed_output", "model.pt"), config=config, **extra)
     print("Compression took:", f"{(time.time() - start) / 60:.3} minutes")
     if compressed is None:
         return  # sharded launch (torchrun): rank 0 holds the gathered latent and writes the file
     names = np.load(config.input_path)["names"]
+    if report:
+        _write_error_report(output_path, config, record[0], names, normalization_features)
     save = np.savez_compressed if config.extra_compression else np.savez
     # latent_dtype "q2" ... "q8": packed codes in `data` plus their per-block parameters (latent_q8.npz_arrays)
     latent = latent_q8.npz_arrays(compressed) if isinstance(compressed, latent_q8.PackedLatent) else {"data": compressed}
@@ -125,6 +132,17 @@ def perform_compression(output_path, config, verbose):
                           ("compressed_batch_index_metadata.npz.gz", index)):
             with gzip.GzipFile(os.path.join(output_path, "compressed_output", name), "w") as f:
                 np.save(file=f, arr=arr, allow_pickle=True)
+
+
+def _write_error_report(output_path, config, record, names, normalization_features):
+    """output/compressed_output/error_report.npz (error_report.finalize) and its summary on stdout"""
+    if config.data_dimension != 1:  # block / snapshot positions
+        names = np.arange(record.n_cols)
+    features = np.asarray(normalization_features).reshape(2, -1) if config.apply_normalization else None
+    report = error_report.finalize(record, names, error_report.scale_range(features, record.n_cols), record.rows,
+                                   record.latent_dtype, record.precision)
+    np.savez(os.path.join(output_path, "compressed_output", "error_report.npz"), **report)
+    print(error_report.summary(report))
 
 
 def perform_decompression(output_path, config, verbose):

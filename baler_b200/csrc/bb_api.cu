@@ -56,6 +56,7 @@ int bb_ctx_create(int device, bb_ctx** out) {
 int bb_ctx_destroy(bb_ctx* ctx) {
   if (!ctx) return BB_OK;
   if (ctx->minmax_scratch) cudaFree(ctx->minmax_scratch);
+  if (ctx->err_scratch) cudaFree(ctx->err_scratch);
   delete ctx;
   return BB_OK;
 }

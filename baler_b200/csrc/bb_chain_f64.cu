@@ -283,7 +283,11 @@ int bb_chain_f64_prepare(bb_ctx* ctx, const Chain* c) {
   }
   double* dev = nullptr;
   BB_CUDA(cudaMalloc(&dev, blob.size() * sizeof(double)));
-  const cudaError_t e = cudaMemcpy(dev, blob.data(), blob.size() * sizeof(double), cudaMemcpyHostToDevice);
+  cudaError_t e = cudaMemcpy(dev, blob.data(), blob.size() * sizeof(double), cudaMemcpyHostToDevice);
+  // A copy from pageable memory may return before its DMA has landed, and the chain runs on the caller's stream or on the
+  // host pipelines' non-blocking streams, which are not ordered after that copy: without this wait the first chunks of
+  // bb_decompress_host_f64 were seen decoding with a partly uploaded weight image (rows off by up to ~30, run to run)
+  if (e == cudaSuccess) e = cudaDeviceSynchronize();
   if (e != cudaSuccess) {
     cudaFree(dev);
     return (int)e;

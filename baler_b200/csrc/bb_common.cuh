@@ -24,6 +24,8 @@ struct bb_ctx {
   float* minmax_scratch = nullptr;  // [2][blocks][cols] partials of the column min/max pass
   size_t minmax_scratch_bytes = 0;
   unsigned int* minmax_counter = nullptr;
+  void* err_scratch = nullptr;  // per-CTA partial records of bb_error_stats, grown to the widest call
+  size_t err_scratch_bytes = 0;
 };
 
 // One dense layer of a fused chain as the fp32 kernel sees it.

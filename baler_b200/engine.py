@@ -644,6 +644,25 @@ def error_bounded_deltas(x, y, mn, rg, bound_percent, row0=0):
     return r[order], cc[order], d[order]
 
 
+def error_stats(x, y, row0=0, post_min=None, post_range=None, scale_range=None, int_mask=None):
+    """bb_error_stats: the error_report.Record of rows y (what decompress writes) against the raw rows x, both CUDA float32 /
+    float64 [n, C].  post_min / post_range (CUDA float64 [C]): y * range + min first, in float64; scale_range (CUDA float64
+    [C]): the histogram's range; int_mask (CUDA uint8 [C]): columns truncated toward zero.  Global rows start at row0.
+    One device->host read of C x 192 bytes."""
+    from . import error_report
+    ctx = get_context(x.device)
+    assert x.is_cuda and y.is_cuda and x.dim() == 2 and x.shape == y.shape and x.is_contiguous() and y.is_contiguous()
+    assert x.dtype in (torch.float32, torch.float64) and y.dtype in (torch.float32, torch.float64)
+    for t, dt in ((post_min, torch.float64), (post_range, torch.float64), (scale_range, torch.float64), (int_mask, torch.uint8)):
+        assert t is None or (t.is_cuda and t.dtype == dt and t.is_contiguous() and t.numel() == x.shape[1])
+    n, c = x.shape
+    record = torch.empty(error_report.N_FIELDS * c, dtype=torch.int64, device=x.device)
+    check(_lib.lib().bb_error_stats(ctx.handle, _ptr(x), _T2BB[x.dtype], _ptr(y), _T2BB[y.dtype], n, c, int(row0),
+                                    _ptr(post_min), _ptr(post_range), _ptr(scale_range), _ptr(int_mask), _ptr(record),
+                                    _stream(ctx)), "bb_error_stats")
+    return error_report.Record.from_words(record.cpu().numpy(), c)
+
+
 class LayeredTrainer:
     """bb_ltrainer: the layer-by-layer trainer for dense autoencoders too wide for the fused training kernels
     (CFD_dense_AE on 2500-feature snapshots), and for AE_Dropout_BN batches beyond the fused step's (LayeredTrainer.dbn).

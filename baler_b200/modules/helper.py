@@ -45,6 +45,11 @@ class Config:
                        about 2x per bit removed.  decompress recognises a quantised file by itself.  Not with precision
                        "fp64"; another "q..." value is refused
       l1_in_training   bool: add reg_param * L1 chain to the training loss (dead code upstream, SURVEY F2)
+      error_report     bool: --mode compress also writes output/compressed_output/error_report.npz and prints a summary: the
+                       per-column error of the rows --mode decompress will write for this config (before error-bounded
+                       deltas) against the input rows, measured on the GPU chunk by chunk (baler_b200/error_report.py).
+                       Any precision and latent_dtype, with or without deltas, one process or torchrun.  Another value
+                       than True / False is refused before any file is read
     custom_loss_function = "loss_function_swae" (a reference key) trains AE, CFD_dense_AE and Conv_AE at any batch
     size that fits device memory, in one process; Conv_AE's encoder BatchNorm2d counts two batches per step, as
     upstream's second model.encode(inputs) leaves it.  AE_Dropout_BN (the second encode draws other dropout masks),
@@ -249,10 +254,17 @@ def _refuse_fp64_shape(model):
         raise NotImplementedError(msg)
 
 
-def compress(model_path, config):
+def compress(model_path, config, renormalize_features=None):
     """reference helper.py:473-616 -> (compressed ndarray, eb_batch, eb_deltas, eb_index).
-    Normalisation uses THIS file's column min/max (helper.py:500-502), fused into the encode kernel."""
-    from .. import sharded
+    Normalisation uses THIS file's column min/max (helper.py:500-502), fused into the encode kernel.
+    config.error_report = True (not in the reference): a fifth element, the error_report.Record of the rows decompress will
+    write (None on the ranks other than 0 under torchrun); `renormalize_features` ([min; range], optional, not in the
+    reference signature) are the training features decompress un-normalises with, needed when apply_normalization is set."""
+    from .. import error_report, sharded
+    report = error_report.enabled(config)  # (ValueError for a non-bool value, before any file is read)
+    if report and config.apply_normalization and renormalize_features is None:
+        raise ValueError("error_report with apply_normalization needs the training features decompress un-normalises with "
+                         "(renormalize_features)")
     fp64 = _fp64(config)
     rank, world = sharded.dist_env()  # under torchrun: this rank's GPU, before anything touches a device
     loaded = np.load(config.input_path)
@@ -307,6 +319,14 @@ def compress(model_path, config):
     if table is None:
         table = engine.host_convert(data_before.reshape(data_before.shape[0], -1), np.float32)
     codec = model.codec(data_before.shape[1], data_before.shape[2]) if conv else model.codec()
+    if report:
+        row_shape = (n_features,) if config.data_dimension == 1 else (
+            (1, original_shape[1], original_shape[2]) if conv else original_shape[1:])
+        if getattr(config, "convert_to_blocks", None) and error_report.int_columns(config, original_shape[1:]) is not None:
+            raise NotImplementedError("error_report does not follow integer type_list columns through convert_to_blocks")
+        spec = _ReportSpec(model, config, fp64, data_before.reshape(data_before.shape[0], -1), table, renormalize_features,
+                           error_report.int_columns(config, row_shape))
+        return _compress_with_deltas(codec, model, table, normalise, config, rank, world, spec)
     if getattr(config, "save_error_bounded_deltas", False):
         return _compress_with_deltas(codec, model, table, normalise, config, rank, world)
     bits = latent_q8.bits_of(getattr(config, "latent_dtype", None))
@@ -357,7 +377,68 @@ def _gather_packed(q, n_rows):
     return None if codes is None else latent_q8.PackedLatent(codes, mins, steps, q.bits)
 
 
-def _compress_with_deltas(codec, model, table, normalise, config, rank=0, world=1):
+class _ReportSpec:
+    """what error_report needs to reproduce decompress in compress's chunk loop (helper.decompress, baler.py:410-435): the
+    raw rows, the training features (fused into the decode kernel, or applied in float64 afterwards for a table beyond
+    data_processing.F32_OFFSET_LIMIT), the integer columns and the latent as it is stored"""
+
+    def __init__(self, model, config, fp64, raw, table, features, int_mask):
+        from .. import error_report
+        self.fp64 = fp64
+        self.precision = getattr(config, "precision", "auto")
+        self.z_dtype = _latent_np_dtype(model, config)
+        self.latent_name = self.z_dtype if isinstance(self.z_dtype, str) else np.dtype(self.z_dtype).name
+        n_cols = table.shape[1]
+        feats = None if features is None or not config.apply_normalization else np.asarray(features).reshape(2, -1)
+        self.scale = error_report.scale_range(feats, n_cols)
+        # the raw rows when the kernels read other ones: a float64 file narrowed to float32, or normalised on the host
+        self.raw = raw if raw.dtype == np.float64 and table.dtype != np.float64 else None
+        self.fused = self.post = None
+        if feats is not None:
+            if fp64:  # the float64 chain applies the features in their own dtype (widened exactly)
+                self.fused = feats
+            elif model.dtype == torch.float64 and data_processing._ill_conditioned(
+                    feats[0].astype(np.float64), feats[0].astype(np.float64) + feats[1].astype(np.float64)):
+                self.post = feats.astype(np.float64)  # decode to normalised rows, y * range + min in float64 on the host
+            else:
+                self.fused = feats.astype(np.float32)
+        dev = lambda a, dt: None if a is None else torch.from_numpy(np.ascontiguousarray(a, dtype=dt)).cuda()  # noqa: E731
+        self.fused_dev = None if self.fused is None else (dev(self.fused[0], self.fused.dtype), dev(self.fused[1], self.fused.dtype))
+        self.post_dev = (None, None) if self.post is None else (dev(self.post[0], np.float64), dev(self.post[1], np.float64))
+        self.scale_dev = dev(self.scale, np.float64)
+        self.mask_dev = dev(int_mask, np.uint8)
+
+    def record(self, codec, x, z, stored, lo, hi):
+        """the Record of rows [lo, hi): x their device rows as the kernels read them, z the device latent, `stored` the
+        latent as written (numpy rows, or None for a quantised latent, whose dequantised z is what decompress decodes)"""
+        from .. import engine
+        if stored is not None and stored.dtype != np.float64 and self.fp64:
+            z = torch.from_numpy(engine.host_convert(stored, np.float64)).cuda()  # decompress widens a narrower file
+        elif stored is not None and stored.dtype == np.float16:
+            z = torch.from_numpy(np.ascontiguousarray(stored)).cuda()  # the float16 rounding decompress decodes
+        fmin, frange = self.fused_dev if self.fused_dev is not None else (None, None)
+        y = codec.decode(z, fmin, frange, precision=self.precision)
+        if self.raw is not None:
+            x = torch.from_numpy(np.ascontiguousarray(self.raw[lo:hi])).cuda()
+        return engine.error_stats(x, y, row0=lo, post_min=self.post_dev[0], post_range=self.post_dev[1],
+                                  scale_range=self.scale_dev, int_mask=self.mask_dev)
+
+
+def _chunk_features(table, normalise, rank, world, shard):
+    """[min; range] device tensors the chunk loop normalises with (helper.py:500-502: this file's own), or (None, None)"""
+    from .. import sharded
+    if not (normalise and len(table)):
+        return None, None
+    if world > 1:
+        feats = sharded.global_minmax(shard)
+    elif table.dtype == np.float64:  # the float64 chain's exact float64 statistics (bb_compress_host_f64)
+        feats = data_processing.minmax_normalize_f64(table, normalise=False)[0]
+    else:
+        feats = data_processing.find_minmax(table)
+    return (torch.from_numpy(np.ascontiguousarray(feats[0])).cuda(), torch.from_numpy(np.ascontiguousarray(feats[1])).cuda())
+
+
+def _compress_with_deltas(codec, model, table, normalise, config, rank=0, world=1, report=None):
     """reference helper.py:583-611 with config.save_error_bounded_deltas: every batch is encoded, decoded again and
     compared with its (normalised) input; elements whose relative error exceeds config.error_bounded_requirement percent
     get a float16 delta (helper.save_error_bounded_requirement, helper.py:442-470).  Here the table goes through the GPU in
@@ -366,25 +447,30 @@ def _compress_with_deltas(codec, model, table, normalise, config, rank=0, world=
     Launched under torchrun every rank scans its contiguous row range (hits carry GLOBAL row numbers), rank 0 collects the
     latent rows and the hit lists and regroups them; the other ranks return (None, [], [], []).
     latent_dtype "q2" ... "q8": each chunk's latent is quantised, and the deltas correct
-    decode(dequantise(quantise(encode(x)))), the rows decompress reproduces; shards and chunks start on 128-row blocks."""
-    from .. import engine, sharded
+    decode(dequantise(quantise(encode(x)))), the rows decompress reproduces; shards and chunks start on 128-row blocks.
+    `report` (a _ReportSpec; config.error_report): every chunk is also decoded as decompress will decode it and measured by
+    bb_error_stats; a fifth element, the merged error_report.Record, is returned (None on ranks other than 0).  Without
+    save_error_bounded_deltas the loop then only writes the latent."""
+    from .. import engine, error_report, sharded
     n, bs = len(table), int(config.batch_size)
+    deltas_on = bool(getattr(config, "save_error_bounded_deltas", False))
+    precision = getattr(config, "precision", "auto")
     z_dtype = _latent_np_dtype(model, config)
     bits = latent_q8.bits_of(z_dtype)
     lo, hi = sharded.row_range(n, rank, world, latent_q8.BLOCK_ROWS if bits else 1)
     shard = table[lo:hi]
     compressed = (latent_q8.empty_packed(hi - lo, codec.z_dim, bits) if bits
                   else np.empty((hi - lo, codec.z_dim), dtype=z_dtype))
-    mn = rg = None
-    if normalise and n:
-        # this file's own [min; range] (helper.py:500-502), over all ranks' rows
-        feats = data_processing.find_minmax(table) if world == 1 else sharded.global_minmax(shard)
-        mn, rg = torch.from_numpy(np.ascontiguousarray(feats[0])).cuda(), torch.from_numpy(np.ascontiguousarray(feats[1])).cuda()
-    rows, cols, deltas = [], [], []
+    # this file's own [min; range] (helper.py:500-502), over all ranks' rows
+    mn, rg = _chunk_features(table, normalise, rank, world, shard)
+    # the float64 chain (precision "fp64") writes a float64 latent; the other kernels a float32 one
+    z_out = torch.float64 if report is not None and report.fp64 else torch.float32
+    rows, cols, deltas, records = [], [], [], []
     chunk = 1 << 20
     for r0 in range(0, hi - lo, chunk):
         x = torch.from_numpy(shard[r0:r0 + chunk]).cuda()
-        z = codec.encode(x, mn, rg, precision=getattr(config, "precision", "auto"))
+        z = codec.encode(x, mn, rg, out_dtype=z_out, precision=precision)
+        stored = None
         if bits:  # (chunk is a multiple of the block)
             qz = codec.quantize_packed(z, bits)
             b0 = r0 // latent_q8.BLOCK_ROWS
@@ -393,19 +479,37 @@ def _compress_with_deltas(codec, model, table, normalise, config, rank=0, world=
             compressed.step[b0:b0 + len(qz.step)] = qz.step.cpu().numpy()
             z = codec.dequantize_packed(qz)
         else:
-            compressed[r0:r0 + chunk] = z.cpu().numpy().astype(z_dtype, copy=False)
-        y = codec.decode(z, precision=getattr(config, "precision", "auto"))  # still normalised, as upstream compares it
-        r, c, d = engine.error_bounded_deltas(x, y, mn, rg, config.error_bounded_requirement, row0=lo + r0)
-        rows.append(r); cols.append(c); deltas.append(d)
+            stored = compressed[r0:r0 + chunk]
+            stored[...] = z.cpu().numpy().astype(z_dtype, copy=False)
+        if deltas_on:
+            y = codec.decode(z, precision=precision)  # still normalised, as upstream compares it
+            r, c, d = engine.error_bounded_deltas(x, y, mn, rg, config.error_bounded_requirement, row0=lo + r0)
+            rows.append(r); cols.append(c); deltas.append(d)
+        if report is not None:
+            records.append(report.record(codec, x, z, stored, lo + r0, lo + r0 + len(x)))
+    record = None
+    if report is not None:
+        record = error_report.merge(records) if records else error_report.Record.empty(table.shape[1])
+        record.rows, record.latent_dtype, record.precision = n, report.latent_name, report.precision
+    if not deltas_on:
+        if world > 1:
+            compressed = _gather_packed(compressed, n) if bits else sharded.gather_rows_to_rank0(compressed, n)
+            parts = sharded.gather_objects_to_rank0(record) if report is not None else None
+            if rank != 0:
+                return (None, [], [], []) + ((None,) if report is not None else ())
+            record = error_report.merge(parts) if report is not None else None  # rank order = row order
+        return (compressed, [], [], []) + ((record,) if report is not None else ())
     rows = np.concatenate(rows) if rows else np.empty(0, np.int64)
     cols = np.concatenate(cols) if cols else np.empty(0, np.int64)
     deltas = np.concatenate(deltas) if deltas else np.empty(0, np.float16)
     if world > 1:
         compressed = _gather_packed(compressed, n) if bits else sharded.gather_rows_to_rank0(compressed, n)
-        hits = sharded.gather_objects_to_rank0((rows, cols, deltas))
+        hits = sharded.gather_objects_to_rank0((rows, cols, deltas, record))
         if rank != 0:
-            return None, [], [], []
+            return (None, [], [], []) + ((None,) if report is not None else ())
         rows, cols, deltas = (np.concatenate([h[i] for h in hits]) for i in range(3))  # rank order = row order
+        if report is not None:
+            record = error_report.merge([h[3] for h in hits])
     print("Total Deltas Found - ", len(rows))
     # upstream appends an entry for EVERY batch (its `len(index) > 0` test is on a 2-tuple); batches without a hit get
     # empty lists here (upstream would reuse the previous batch's deltas or crash on the first one)
@@ -417,7 +521,7 @@ def _compress_with_deltas(codec, model, table, normalise, config, rank=0, world=
         eb_batch.append(b)
         eb_deltas.append(list(deltas[lo:hi]))
         eb_index.append((rows[lo:hi] - b * bs, cols[lo:hi]))
-    return compressed, eb_batch, eb_deltas, eb_index
+    return (compressed, eb_batch, eb_deltas, eb_index) + ((record,) if report is not None else ())
 
 
 def _apply_deltas(decompressed, input_path_deltas, input_batch_index, batch_size, col_scale):

@@ -543,6 +543,27 @@ int bb_error_bounded_deltas_f32(bb_ctx* ctx, const float* x_dev, const float* y_
                                 int64_t capacity, unsigned long long* count_dev, long long* rows_out_dev,
                                 int* cols_out_dev, void* deltas_f16_out_dev, bb_stream_t stream);
 
+/*
+ * Reconstruction error of n_rows rows (error_report = True; baler_b200/error_report.py defines the record, DESIGN §4.13).
+ * x_dev: the raw rows, y_dev: what decompress writes for them, both row-major n_rows x n_cols of x_dtype / y_dtype (BB_F32 or
+ * BB_F64).  post_min_dev / post_range_dev (float64, n_cols, both or neither): y is first replaced by y * range + min, two IEEE
+ * float64 operations.  int_mask_dev (uint8, n_cols, or NULL): y is truncated toward zero in the columns marked non-zero.
+ * scale_range_dev (float64, n_cols, or NULL = 1): the range the histogram measures |e| against (1 where it is not a
+ * positive finite number).  Over the rows where x and y are both finite, e = y - x in float64.
+ * Every pointer must be aligned to its element type (else BB_ERR_INVALID).  record_dev receives BB_ERROR_STATS_FIELDS x n_cols 8-byte words, field-major (word f * n_cols + j):
+ *   int64   0 count  1 nonfinite_x  2 nonfinite_y  3 response_count  4 int_mismatch  5 err_max_row (global row: row0 + r;
+ *           -1 when count is 0)  6..16 hist: |e| <= 1e-9 r, (1e-9 r, 1e-8 r], ..., (0.1 r, r], > r with r = edge * range
+ *   float64 17 x_min  18 x_max (over finite x; +inf / -inf when there is none)  19 sum e  20 sum e^2  21 err_max_abs (0 when
+ *           count is 0)  22 sum r  23 sum r^2, r = 100 * e / x over x != 0
+ * No floating-point atomics: a re-run gives the same bits.  The call only enqueues kernels on `stream`; the first call on a
+ * context (and a later one that needs more) allocates its scratch of at most 4 x SMs x 256 x 192 bytes beyond n_cols x 192
+ * (cudaMalloc).  One call at a time per context.
+ */
+#define BB_ERROR_STATS_FIELDS 24
+int bb_error_stats(bb_ctx* ctx, const void* x_dev, int x_dtype, const void* y_dev, int y_dtype, int64_t n_rows, int n_cols,
+                   int64_t row0, const double* post_min_dev, const double* post_range_dev, const double* scale_range_dev,
+                   const uint8_t* int_mask_dev, void* record_dev, bb_stream_t stream);
+
 /* sum((a - b)^2) over n float32 elements, ADDED to *out_dev (double): nn.MSELoss(reduction="sum") of
  * utils.mse_sum_loss_l1 (utils.py:195-196) on loose tensors. */
 int bb_mse_sum_f32(bb_ctx* ctx, const float* a_dev, const float* b_dev, int64_t n, double* out_dev, bb_stream_t stream);
